@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]                # our arm (N>1: launched by torchrun)
     python bench.py --impl reference [--steps K] [--warmup W]          # the reference's own code on the host CPU
+    python bench.py --dump-outputs DIR                                 # also write the last timed step's results as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic Coursera-shaped videos:
 forward -> loss.backward() -> gradient all-reduce(SUM) -> clip_grad_norm_(2.0) -> Adadelta(lr 0.5).step()
@@ -47,6 +48,7 @@ CFG5 = dict(batch=16, lt=4096, la=4096, li=2048, m=4096, steps=16)
 DROP = 0.2                                                           # train.py:209
 METRIC, UNIT = "mmbidaf_train_videos_per_s", "videos/s"
 N_ROTATE = 4
+DUMP_LIMIT = 64 << 20                                                # bytes --dump-outputs may write
 
 
 def measured_peaks():
@@ -123,6 +125,22 @@ def workload_config(n_gpus: int, **over):
            "l2": "inputs+activations per step exceed L2 (126 MB); BiDAF microbench rotates 4 input sets (4 x 144 MB)"}
     cfg.update(over)
     return cfg
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Write every tensor of ``arrays`` as ``directory/<name>.npy`` in float32 (float64 stays float64).  The inputs of a run are
+    seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the limit of {DUMP_LIMIT}")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -480,12 +498,19 @@ def run_gpu_arm(args):
     def run_resident():
         b = residents[turn["k"] % N_ROTATE]
         turn["k"] += 1
-        return trainer.step_graphed(b) if graphed else trainer.step(b)
+        turn["loss"] = trainer.step_graphed(b) if graphed else trainer.step(b)
 
     for _ in range(N_ROTATE):
         run_resident()
     with ClockSampler(local) as clocks:
         seconds = timed(run_resident, args.steps)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step holds after the last timed step (the sections below keep training the same model)
+        arrays = {"loss": turn["loss"], "grad_norm": trainer.last_grad_norm}
+        for name, p in trainer.model.named_parameters():
+            arrays["param." + name] = p
+            arrays["grad." + name] = p.grad
+        dump_outputs(args.dump_outputs, arrays)
     launches = launches_per_step * args.steps
     videos = CFG3["batch"] * world * args.steps
 
@@ -688,7 +713,11 @@ def main():
     ap.add_argument("--precision", default="fast", choices=["fast", "fp32"],
                     help="fast: bf16 tensor-core BiDAF + TF32 GEMMs (rel<=2e-2); fp32: rel<=1e-5 tier")
     ap.add_argument("--sections", default="step,e2e,cfg4,bidaf,cfg5,fp32,eager", help="profiling aid: which GPU sections to run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss, gradient norm, parameters and gradients as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -15,6 +15,7 @@ import torch
 import torch.nn as nn
 
 from . import functional as Fn
+from . import ops
 from .layers import BiDAFAttention, Embedding, ImageEmbedding, MultimodalAttentionDecoder, RNNEncoder
 
 __all__ = ["MMBiDAF"]
@@ -184,58 +185,60 @@ class MMBiDAF(nn.Module):
                 if not capturing and isinstance(t, torch.Tensor):
                     t.record_stream(stream)
 
-            for st in self._streams:
-                st.wait_stream(main)
-            # The audio chain (embedding -> 1024-step recurrence) is the critical path of the forward pass and the other two encoders
-            # have ~250 us of slack: they start when the audio EMBEDDING is done, so that its five small GEMMs / point-wise kernels do not
-            # share the chip with theirs (tools/step_timeline.py: 178 us from the start of the step to the start of the audio recurrence
-            # with all three chains launched together).
-            with torch.cuda.stream(s_audio):
-                audio_emb = self.a_emb(embedded_audio)
-                audio_emb_done = torch.cuda.Event()
-                audio_emb_done.record(s_audio)
-                branch["audio"] = self.audio_enc(audio_emb, original_audio_lengths)[0]
-            with torch.cuda.stream(s_text):
-                if self.stagger_encoders:
-                    s_text.wait_event(audio_emb_done)
-                branch["text"] = text_branch()[1]
-                text_done = torch.cuda.Event()
-                text_done.record(s_text)
-            with torch.cuda.stream(s_image):
-                if self.stagger_encoders:
-                    s_image.wait_event(audio_emb_done)
-                branch["image"] = image_branch()[1]
-            make_masks()                          # on the main stream, beside the encoders: needs only the lengths
-            # ... and so do the keep-masks of the two BiDAF blocks (shapes only): two mask draws less between the audio recurrence and
-            # the fused kernel, on the critical path
-            d2 = 2 * self.text_enc.rnn.hidden_size
-            dev = embedded_text.device
-            self.bidaf_att_audio.predraw_dropout((B, Lt, d2), (B, embedded_audio.size(1), d2), dev)
-            self.bidaf_att_image.predraw_dropout((B, Lt, d2), (B, transformed_images.size(1), d2), dev)
-            for att, st in ((self.bidaf_att_audio, s_audio), (self.bidaf_att_image, s_image)):
-                for t in (getattr(att, "_predrawn", None) or ()):
-                    keep(t, st)
-            masks_done = torch.cuda.Event()
-            masks_done.record(main)
-            with torch.cuda.stream(s_image):
-                s_image.wait_event(text_done)
-                s_image.wait_event(masks_done)
-                mod_text_image, text_img_hidden = image_aware()
-            with torch.cuda.stream(s_audio):
-                s_audio.wait_event(text_done)
-                s_audio.wait_event(masks_done)
-                mod_text_audio, text_audio_hidden = audio_aware()
-            decoder_start()                       # on the main stream, beside the recurrences
-            for st in self._streams:
-                main.wait_stream(st)
-            keep(branch["text"], s_audio)
-            keep(branch["text"], s_image)
-            for m in masks.values():
-                keep(m, s_audio)
-                keep(m, s_image)
-            for t in (mod_text_audio, text_audio_hidden, mod_text_image, text_img_hidden, branch["text"], branch["audio"], branch["image"],
-                      *side.values()):
-                keep(t, main)
+            # every dropout key of the forward pass is drawn on the main stream, in issue order (ops.keys_drawn_on)
+            with ops.keys_drawn_on(main):
+                for st in self._streams:
+                    st.wait_stream(main)
+                # The audio chain (embedding -> 1024-step recurrence) is the critical path of the forward pass and the other two encoders
+                # have ~250 us of slack: they start when the audio EMBEDDING is done, so that its five small GEMMs / point-wise kernels do not
+                # share the chip with theirs (tools/step_timeline.py: 178 us from the start of the step to the start of the audio recurrence
+                # with all three chains launched together).
+                with torch.cuda.stream(s_audio):
+                    audio_emb = self.a_emb(embedded_audio)
+                    audio_emb_done = torch.cuda.Event()
+                    audio_emb_done.record(s_audio)
+                    branch["audio"] = self.audio_enc(audio_emb, original_audio_lengths)[0]
+                with torch.cuda.stream(s_text):
+                    if self.stagger_encoders:
+                        s_text.wait_event(audio_emb_done)
+                    branch["text"] = text_branch()[1]
+                    text_done = torch.cuda.Event()
+                    text_done.record(s_text)
+                with torch.cuda.stream(s_image):
+                    if self.stagger_encoders:
+                        s_image.wait_event(audio_emb_done)
+                    branch["image"] = image_branch()[1]
+                make_masks()                          # on the main stream, beside the encoders: needs only the lengths
+                # ... and so do the keep-masks of the two BiDAF blocks (shapes only): two mask draws less between the audio recurrence and
+                # the fused kernel, on the critical path
+                d2 = 2 * self.text_enc.rnn.hidden_size
+                dev = embedded_text.device
+                self.bidaf_att_audio.predraw_dropout((B, Lt, d2), (B, embedded_audio.size(1), d2), dev)
+                self.bidaf_att_image.predraw_dropout((B, Lt, d2), (B, transformed_images.size(1), d2), dev)
+                for att, st in ((self.bidaf_att_audio, s_audio), (self.bidaf_att_image, s_image)):
+                    for t in (getattr(att, "_predrawn", None) or ()):
+                        keep(t, st)
+                masks_done = torch.cuda.Event()
+                masks_done.record(main)
+                with torch.cuda.stream(s_image):
+                    s_image.wait_event(text_done)
+                    s_image.wait_event(masks_done)
+                    mod_text_image, text_img_hidden = image_aware()
+                with torch.cuda.stream(s_audio):
+                    s_audio.wait_event(text_done)
+                    s_audio.wait_event(masks_done)
+                    mod_text_audio, text_audio_hidden = audio_aware()
+                decoder_start()                       # on the main stream, beside the recurrences
+                for st in self._streams:
+                    main.wait_stream(st)
+                keep(branch["text"], s_audio)
+                keep(branch["text"], s_image)
+                for m in masks.values():
+                    keep(m, s_audio)
+                    keep(m, s_image)
+                for t in (mod_text_audio, text_audio_hidden, mod_text_image, text_img_hidden, branch["text"], branch["audio"], branch["image"],
+                          *side.values()):
+                    keep(t, main)
         decoder_mask = masks["decoder"]
 
         # models.py:143-149 (the hidden-state rows are in descending-length order: reference quirk Q3)

@@ -6,6 +6,7 @@ this module (bench.py reports it as ``gpu_launches``).
 """
 from __future__ import annotations
 
+import contextlib
 import os
 from typing import Optional, Tuple
 
@@ -161,25 +162,48 @@ def rng_seed(seed: int, device=None) -> None:
             st.fill_(int(seed) & 0x7FFFFFFFFFFFFFFF)
 
 
+_key_stream = {"stream": None}
+
+
+@contextlib.contextmanager
+def keys_drawn_on(stream: torch.cuda.Stream):
+    """Inside, :func:`rng_next_keys` draws on ``stream`` whatever the current stream is, and the current stream waits for the keys.
+    The key state is one device word that every draw reads and advances: draws issued from concurrent streams would advance it
+    in whatever order the GPU runs them, so which layer gets which key (and whether two get the same one) would change from run to
+    run.  On one stream the draws run in the order they are issued."""
+    saved, _key_stream["stream"] = _key_stream["stream"], stream
+    try:
+        yield
+    finally:
+        _key_stream["stream"] = saved
+
+
 def rng_next_keys(device, n: int) -> torch.Tensor:
     """``n`` fresh dropout keys (int64, on ``device``), drawn ON the device from a resident state: one tiny launch, capturable (a graph
     replay draws new keys).  The state is seeded from torch's seed at first use."""
     device = torch.device(device)
-    st = _rng_state.get(device)
-    if st is None:
-        if torch.cuda.is_current_stream_capturing():
-            # created inside a capture, the state's initial fill would be replayed too: the same masks on every replay
-            raise RuntimeError("mmbidaf_b200: the dropout key state must exist before a CUDA-graph capture (run one eager step, as "
-                               "Trainer.capture does, or call ops.rng_next_keys once)")
-        # (every rank of a data-parallel job draws its own masks: the rank is mixed into the seed)
-        import torch.distributed as dist
-        rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
-        st = _rng_state[device] = torch.full((1,), (((torch.initial_seed() if _rng_seed_override["seed"] is None else _rng_seed_override["seed"]) + 0x51ED27 * rank)
-                                              * 0x9E3779B97F4A7C15 + 0x1234567)
-                                             & 0x7FFFFFFFFFFFFFFF, dtype=torch.int64, device=device)
-    keys = torch.empty(n, dtype=torch.int64, device=device)
-    _lib.check(_lib.lib().mmb_rng_next(_lib.ptr(st), _lib.ptr(keys), n, _lib.stream()), "mmb_rng_next")
+    cur = torch.cuda.current_stream(device)
+    draw = _key_stream["stream"] if _key_stream["stream"] is not None and _key_stream["stream"].device == cur.device else cur
+    with torch.cuda.stream(draw):
+        st = _rng_state.get(device)
+        if st is None:
+            if torch.cuda.is_current_stream_capturing():
+                # created inside a capture, the state's initial fill would be replayed too: the same masks on every replay
+                raise RuntimeError("mmbidaf_b200: the dropout key state must exist before a CUDA-graph capture (run one eager step, as "
+                                   "Trainer.capture does, or call ops.rng_next_keys once)")
+            # (every rank of a data-parallel job draws its own masks: the rank is mixed into the seed)
+            import torch.distributed as dist
+            rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+            st = _rng_state[device] = torch.full((1,), (((torch.initial_seed() if _rng_seed_override["seed"] is None else _rng_seed_override["seed"]) + 0x51ED27 * rank)
+                                                  * 0x9E3779B97F4A7C15 + 0x1234567)
+                                                 & 0x7FFFFFFFFFFFFFFF, dtype=torch.int64, device=device)
+        keys = torch.empty(n, dtype=torch.int64, device=device)
+        _lib.check(_lib.lib().mmb_rng_next(_lib.ptr(st), _lib.ptr(keys), n, _lib.stream()), "mmb_rng_next")
     _count(1)
+    if draw != cur:
+        cur.wait_stream(draw)
+        if not torch.cuda.is_current_stream_capturing():
+            keys.record_stream(cur)                      # allocated on the draw stream, read on this one
     return keys
 
 

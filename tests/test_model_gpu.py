@@ -109,6 +109,30 @@ def test_streams_do_not_change_results():
         assert torch.equal(a, b)
 
 
+def test_dropout_keys_do_not_depend_on_stream_timing():
+    """Training with dropout: the encoder chains run on side streams, but which layer gets which dropout key must not depend on
+    when the GPU gets to each chain.  Holding the text chain's stream back (so that the image chain draws its keys first when the
+    draws follow the GPU's order) leaves the output and the loss bit for bit the same."""
+    from mmbidaf_b200 import ops
+    from mmbidaf_b200.models import MMBiDAF
+    torch.manual_seed(3)
+    model = MMBiDAF(100, 300, 128, 1000, torch.device("cuda"), drop_prob=0.2, max_transcript_length=64).cuda()
+    batch = make_batch(4, 40, 90, 11, 5, seed=31)
+
+    def run(delay_text):
+        ops.rng_seed(11)
+        if delay_text:
+            with torch.cuda.stream(model._streams[1]):                 # (audio, text, image)
+                torch.cuda._sleep(50_000_000)                          # ~25 ms
+        out, loss = _call(model, batch, True)
+        torch.cuda.synchronize()
+        return out.detach().clone(), loss.detach().clone()
+
+    want = run(False)
+    got = run(True)
+    assert torch.equal(got[0], want[0]) and torch.equal(got[1], want[1])
+
+
 def test_tf32_library_gemms_stay_inside_the_reduced_precision_tier():
     """north_star: rel <= 2e-2 on the TF32/bf16 path.  Only the plain library GEMMs change here."""
     g = load_golden("model_readme.pt")
