@@ -184,6 +184,33 @@ MMB_API int mmb_decoder_step_fused_fwd(const float* proj_a, const float* proj_i,
                                        float* cell_out, float* att_cov, float* cov_out, long long* argmax, float* nll,
                                        float* cov_loss, float* hw, float* alpha, float* beta, float* ctx12, float* pb, float* xcat,
                                        float* gates, int B, int Lt, int D, int H, int E, int M, mmb_stream_t stream);
+/*
+ * Greedy summary roll-out: all S = max_dec_len decoder steps of evaluation mode in ONE launch.  Replaces the decode loop of
+ * models.py:156-199 in eval mode (the `else` branches: each step's arg-max row of the text is the next input, models.py:184,193)
+ * -- S calls of attention.py:145-186, S arg-maxes and gathers, the torch.stack of the distributions.  Same cluster kernel as
+ * mmb_decoder_step_fused_fwd (same weight layouts, stages, reduction order and shape limits: the per-step values are bit for bit the
+ * step kernel's); the state between the steps (h', the cell, the coverage, the arg-max) stays on chip.  Start state as
+ * models.py:145-149: h0 (B,H) = the sum of the two modality encoders' h_n (models.py:143), zero cell, coverage and input row.
+ *   emb_text (B,Lt,E)  the embedded text (the next inputs are its rows)     mask (B,M)
+ *   probs (B,S,M)      every step's distribution, in the layout MMBiDAF.forward returns
+ *   argmax (B,S)       every step's first maximal index
+ *   target (B,T) with T >= S, or NULL; then loss_terms (S,2,B) = per step [nll | coverage term] (models.py:168-170, :177), else unused.
+ * Nothing the backward pass would need is written.
+ */
+MMB_API int mmb_decoder_greedy_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                     const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                     const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                     const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                     const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                     const uint8_t* mask, const long long* target, float* probs, long long* argmax, float* loss_terms,
+                                     int B, int Lt, int D, int H, int E, int M, int S, int T, mmb_stream_t stream);
+/*
+ * Greedy sentence selection (evaluate.py:185-202, decode.greedy_search) on the device.  Per video, in step order over argmax (B,S):
+ * the EOS row text_len[b] - 1 ends the summary, an index past it is skipped, any other is kept (repeats too).
+ *   sel (B,S) int32 = the kept indices, then -1;  count (B) int32 = how many were kept.
+ */
+MMB_API int mmb_greedy_select(const long long* argmax, const int32_t* text_len, int32_t* sel, int32_t* count, int B, int S,
+                              mmb_stream_t stream);
 
 MMB_API int mmb_decoder_attn_fwd(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
                                  const float* hw, const float* coverage, const float* v1, const float* wc1,

@@ -207,7 +207,18 @@ __device__ __forceinline__ float block_max(float v, float* red) {
   return warp_max(r);
 }
 
-__global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
+// The greedy roll-out (mmb_decoder_greedy_fused): the same stages, `steps` times in one launch, in eval mode (models.py:156-199, the
+// `else` branches).  The step inputs come from on chip instead of global memory: h = the gathered h' of the previous step (s_hn), the
+// cell of a rank's own hidden units (a register of the thread that owns the unit), the coverage of its own text rows (s_cov += att),
+// sent = emb_text[b, the previous step's arg-max] (every rank reduces the arg-max candidates itself).  Step 0 starts from h0 and a
+// zero cell, coverage and input row (models.py:145-149).  Nothing the backward pass would want is written.
+struct GreedyArgs {
+  const float *emb_text, *h0;                               // (B, Lt, E), (B, H)
+  int steps, T;                                             // roll-out length S; row stride of the target (B, T), T >= S
+};
+
+template <bool kGreedy>
+__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int b = blockIdx.x / CL;
@@ -252,16 +263,31 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
     }
   }
   DEC_STAMP(0);
+  const int S = kGreedy ? g.steps : 1;
+  float cell_own = 0.f;                    // greedy: the cell of hidden unit j0 + tid (stage D), carried between the steps
+  int pick = 0;                            // greedy: the previous step's arg-max
+  for (int s = 0; s < S; ++s) {
+  const uint32_t parity = kGreedy ? (uint32_t)(s & 1) : 0u;      // each row-stage barrier completes once per step
   // ---- stage 0: this video's step inputs -----------------------------------------------------------------------------------
-  for (int i = tid; i < n; i += NT) s_cov[i] = a.cov[(size_t)b * Lt + t0 + i];      // (read per row by the energies: not a global load there)
-  for (int i = tid; i < H; i += NT) s_x[D + E + i] = a.h[(size_t)b * H + i];
-  for (int i = tid; i < E; i += NT) s_x[D + i] = a.sent[(size_t)b * E + i];
-  for (int i = tid; i < D; i += NT) {
-    s_vec[i] = a.v1[i];
-    s_vec[D + i] = a.wc1[i];
-    s_vec[2 * D + i] = a.v2[i];
-    s_vec[3 * D + i] = a.wc2[i];
+  if constexpr (!kGreedy) {
+    for (int i = tid; i < n; i += NT) s_cov[i] = a.cov[(size_t)b * Lt + t0 + i];      // (read per row by the energies: not a global load there)
+    for (int i = tid; i < H; i += NT) s_x[D + E + i] = a.h[(size_t)b * H + i];
+    for (int i = tid; i < E; i += NT) s_x[D + i] = a.sent[(size_t)b * E + i];
+  } else {
+    if (s == 0)
+      for (int i = tid; i < n; i += NT) s_cov[i] = 0.f;
+    for (int i = tid; i < H; i += NT) s_x[D + E + i] = s == 0 ? g.h0[(size_t)b * H + i] : s_hn[i];
+    // (the pick is below Lt whenever the mask is the text mask; a mask wider than the text could point past it: its last row is read)
+    const float* row = g.emb_text + ((size_t)b * Lt + min(pick, Lt - 1)) * E;
+    for (int i = tid; i < E; i += NT) s_x[D + i] = s == 0 ? 0.f : row[i];
   }
+  if (!kGreedy || s == 0)
+    for (int i = tid; i < D; i += NT) {
+      s_vec[i] = a.v1[i];
+      s_vec[D + i] = a.wc1[i];
+      s_vec[2 * D + i] = a.v2[i];
+      s_vec[3 * D + i] = a.wc2[i];
+    }
   __syncthreads();
 
   DEC_STAMP(1);
@@ -271,7 +297,7 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
     block_matvec_t(a.Wh4t, 4 * D, a.bh4, s_x + D + E, H, o1 - o0, s_scr, SCR, (o0 & 3) == 0, [&](int i) { return o0 + i; }, [&](int i, float v) {
       const int o = o0 + i;
       for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_hw, r)[o] = v;
-      a.hw[(size_t)b * 4 * D + o] = v;
+      if constexpr (!kGreedy) a.hw[(size_t)b * 4 * D + o] = v;
     });
   }
   DEC_STAMP(2);
@@ -352,7 +378,7 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
     using R4 = std::integral_constant<int, 4>;
     const bool nj7 = D > 192 && D <= 224;      // the model's D = 2 H = 200; any other D <= 256 takes the zero-padded eight
     if (staged) {
-      if (n > 0) tc::mbar_wait(bar_proj, 0);
+      if (n > 0) tc::mbar_wait(bar_proj, parity);
       if (nj7) energies(s_st0, s_st1, N7{}, R2{});
       else energies(s_st0, s_st1, N8{}, R2{});
     } else {
@@ -387,7 +413,7 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
     __syncthreads();
     DEC_STAMP(5);
     // weighted contexts of this rank's rows
-    if (staged && n > 0) tc::mbar_wait(bar_enc, 0);
+    if (staged && n > 0) tc::mbar_wait(bar_enc, parity);
     const float* ea = staged ? s_st0 : a.enc_a + ((size_t)b * Lt + t0) * D;
     const float* ei = staged ? s_st1 : a.enc_i + ((size_t)b * Lt + t0) * D;
     const bool vec4 = (D & 3) == 0;
@@ -421,6 +447,16 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
       }
     }
     __syncthreads();
+    if constexpr (kGreedy) {
+      // every read of the enc rows is behind the barrier: the buffers take the NEXT step's proj rows, which then arrive while
+      // stages C - E and the next stage A run
+      if (staged && tid == 0 && n > 0 && s + 1 < S) {
+        tc::fence_proxy_async();
+        tc::mbar_expect_tx(bar_proj, 2 * stage_bytes, 1);
+        tc::tma_bulk_g2s(tc::smem_u32(s_st0), a.proj_a + ((size_t)b * Lt + t0) * D, stage_bytes, bar_proj, 1);
+        tc::tma_bulk_g2s(tc::smem_u32(s_st1), a.proj_i + ((size_t)b * Lt + t0) * D, stage_bytes, bar_proj, 1);
+      }
+    }
     // this rank's partials -> slot R of every rank
     for (int d = tid; d < 2 * D; d += NT) {
       const int k = d / D, dd = d - k * D;
@@ -464,7 +500,7 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
       float sum = 0.f;
       for (int r = 0; r < CL; ++r) sum = fmaf(s_w[k * MAXC + r], s_part[r * (4 + 2 * D) + 4 + i], sum);
       s_ctx[i] = sum;
-      if (R == 0) a.ctx12[((size_t)k * a.B + b) * D + (i - k * D)] = sum;
+      if (!kGreedy && R == 0) a.ctx12[((size_t)k * a.B + b) * D + (i - k * D)] = sum;
     }
   }
   __syncthreads();
@@ -481,7 +517,7 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
                      [&](int i, float v) {
                        const int o = lo + i;
                        for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_pb, r)[o] = v;
-                       a.pb[((size_t)k * a.B + b) * D + (o - k * D)] = v;
+                       if constexpr (!kGreedy) a.pb[((size_t)k * a.B + b) * D + (o - k * D)] = v;
                      });
     }
   }
@@ -506,23 +542,31 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
     for (int i = tid; i < n; i += NT) {
       const int t = t0 + i;
       const float a1 = s_e[i] * scale_own[0], a2 = s_e[a.chunk + i] * scale_own[1];
-      a.alpha[((size_t)b * 2 + 0) * Lt + t] = a1;
-      a.alpha[((size_t)b * 2 + 1) * Lt + t] = a2;
+      if constexpr (!kGreedy) {
+        a.alpha[((size_t)b * 2 + 0) * Lt + t] = a1;
+        a.alpha[((size_t)b * 2 + 1) * Lt + t] = a2;
+      }
       const float att = a1 * beta1 + a2 * beta2;                 // bmm([a1 a2], beta), attention.py:167
-      const float cnew = a.cov[(size_t)b * Lt + t] + att;
-      a.att_cov[(size_t)b * Lt + t] = att;
-      a.cov_out[(size_t)b * Lt + t] = cnew;
-      closs += fminf(att, cnew);
+      if constexpr (kGreedy) {
+        const float cnew = s_cov[i] + att;                       // (the energies of this step have read s_cov: barriers since)
+        s_cov[i] = cnew;
+        closs += fminf(att, cnew);
+      } else {
+        const float cnew = a.cov[(size_t)b * Lt + t] + att;
+        a.att_cov[(size_t)b * Lt + t] = att;
+        a.cov_out[(size_t)b * Lt + t] = cnew;
+        closs += fminf(att, cnew);
+      }
     }
     closs = block_sum(closs, s_red);
     if (tid == 0) cluster.map_shared_rank(s_ex, 0)[R * 8 + 0] = closs;      // summed by rank 0 after the next cluster barrier
-    if (R == 0 && tid == 0) {
+    if (!kGreedy && R == 0 && tid == 0) {
       a.beta[b * 2 + 0] = beta1;
       a.beta[b * 2 + 1] = beta2;
     }
   }
   __syncthreads();
-  if (R == 0)
+  if (!kGreedy && R == 0)
     for (int i = tid; i < K; i += NT) a.xcat[(size_t)b * K + i] = s_x[i];
 
   DEC_STAMP(11);
@@ -537,22 +581,29 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
       const int j = j0 + tid;
       const float gi = gate_act(s_g[tid], 1.f), gf = gate_act(s_g[(per + 1) + tid], 1.f), gg = tanh_fast(s_g[2 * (per + 1) + tid]),
                   go = gate_act(s_g[3 * (per + 1) + tid], 1.f);
-      const float c = fmaf(gf, a.cell[(size_t)b * H + j], gi * gg);
+      const float c = fmaf(gf, kGreedy ? cell_own : a.cell[(size_t)b * H + j], gi * gg);
       const float hn = go * tanh_fast(c);
-      a.cell_out[(size_t)b * H + j] = c;
-      a.h_out[(size_t)b * H + j] = hn;
-      float* gs = a.gates + (size_t)b * 4 * H;                  // activated gates, kept for the backward pass
-      gs[j] = gi; gs[H + j] = gf; gs[2 * H + j] = gg; gs[3 * H + j] = go;
+      if constexpr (kGreedy) {
+        cell_own = c;
+      } else {
+        a.cell_out[(size_t)b * H + j] = c;
+        a.h_out[(size_t)b * H + j] = hn;
+        float* gs = a.gates + (size_t)b * 4 * H;                // activated gates, kept for the backward pass
+        gs[j] = gi; gs[H + j] = gf; gs[2 * H + j] = gg; gs[3 * H + j] = go;
+      }
       for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_hn, r)[j] = hn;
     }
   }
   DEC_STAMP(12);
   cluster.sync();
   DEC_STAMP(13);
+  // greedy: the probabilities / arg-max of step s go to row (b, s) of (B, S, M) / (B, S); the loss terms (S, 2, B) to row s
+  const size_t prow = kGreedy ? (size_t)b * S + s : (size_t)b;
+  const int lrow = kGreedy ? s * 2 * a.B + b : b;
   if (R == 0 && tid == 0 && a.cov_loss) {
-    float s = 0.f;
-    for (int r = 0; r < CL; ++r) s += s_ex[r * 8 + 0];
-    a.cov_loss[b] = s;
+    float cs = 0.f;
+    for (int r = 0; r < CL; ++r) cs += s_ex[r * 8 + 0];
+    a.cov_loss[lrow] = cs;
   }
 
   // ---- stage E: logits of this rank's sentences, masked soft-max over M, arg-max, NLL ---------------------------------------
@@ -587,14 +638,14 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
     const float inv = 1.f / gsum;
     float best = -INFINITY;
     int best_i = M;
-    const int tg = a.target ? (int)a.target[b] : -1;
+    const int tg = a.target ? (int)a.target[kGreedy ? b * g.T + s : b] : -1;
     for (int m = m0 + tid; m < m1; m += NT) {
       const float p = expf(lg[m - m0] - gmx) * inv;
-      a.probs[(size_t)b * M + m] = p;
+      a.probs[prow * M + m] = p;
       if (p > best) { best = p; best_i = m; }
-      if (m == tg && a.nll) a.nll[b] = -logf(p + 1e-12f);         // models.py:168-170
+      if (m == tg && a.nll) a.nll[lrow] = -logf(p + 1e-12f);      // models.py:168-170
     }
-    if (a.argmax) {                                               // first maximal index, as torch.max(dim) documents
+    if (kGreedy || a.argmax) {                                    // first maximal index, as torch.max(dim) documents
       const float bbest = block_max(best, s_red);
       int cand = best == bbest ? best_i : M;
 #pragma unroll
@@ -606,12 +657,16 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
       if (tid == 0) {
         int r = M;
         for (int w = 0; w < NW; ++w) r = min(r, redi[w]);
-        float* dst = cluster.map_shared_rank(s_ex, 0) + R * 8;
-        dst[3] = bbest;
-        dst[4] = __int_as_float(r);
+        // (greedy: to every rank, each of which needs the pick for its next step's input row)
+        for (int q = 0; q < (kGreedy ? CL : 1); ++q) {
+          float* dst = cluster.map_shared_rank(s_ex, q) + R * 8;
+          dst[3] = bbest;
+          dst[4] = __int_as_float(r);
+        }
       }
       cluster.sync();
-      if (R == 0 && tid == 0) {
+      // (the step kernel: rank 0 alone; the roll-out: every thread of every rank, for the next step's input row)
+      if (kGreedy || (R == 0 && tid == 0)) {
         float gb = -INFINITY;
         int gi = M;
         for (int r = 0; r < CL; ++r) {
@@ -620,15 +675,27 @@ __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
           const int ib = __float_as_int(s_ex[r * 8 + 4]);
           if (pb_ > gb || (pb_ == gb && ib < gi)) { gb = pb_; gi = ib; }
         }
-        a.argmax[b] = gi;
+        if constexpr (kGreedy) {
+          if (R == 0 && tid == 0) a.argmax[prow] = gi;
+          pick = gi;
+        } else {
+          a.argmax[b] = gi;
+        }
       }
     }
   }
+  }  // steps (the loop body keeps the step kernel's indentation)
   DEC_STAMP(16);
   // (No barrier before the exit: every rank's LAST store into another rank's shared memory -- the soft-max statistics or the arg-max
-  // candidates -- lies before a cluster barrier it has passed, so nothing can still be written into a rank that leaves here.)
+  // candidates -- lies before a cluster barrier it has passed, so nothing can still be written into a rank that leaves here.  In the
+  // greedy loop the same holds between the steps: a store of step s + 1 into another rank lies behind at least one cluster barrier
+  // that the other rank reaches only after its last read of what step s stored there.)
   DEC_STAMP(17);
 }
+
+__global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) { dec_fused_body<false>(a, GreedyArgs{}); }
+
+__global__ void __launch_bounds__(NT) dec_greedy_fused_kernel(const FusedArgs a, const GreedyArgs g) { dec_fused_body<true>(a, g); }
 
 }  // namespace
 
@@ -1162,50 +1229,35 @@ static size_t fused_smem_bytes(int Lt, int D, int H, int E, int M, int CL, int* 
   return floats * sizeof(float) + 64;
 }
 
-}  // namespace mmb
-
-extern "C" int mmb_decoder_step_fused_fwd(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
-                                          const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
-                                          const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
-                                          const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt,
-                                          const float* bcat, const float* out_wt, const float* out_b, const float* sent,
-                                          const float* h, const float* cell, const float* cov, const uint8_t* mask,
-                                          const long long* target, float* probs, float* h_out, float* cell_out, float* att_cov,
-                                          float* cov_out, long long* argmax, float* nll, float* cov_loss, float* hw, float* alpha,
-                                          float* beta, float* ctx12, float* pb, float* xcat, float* gates, int B, int Lt, int D,
-                                          int H, int E, int M, mmb_stream_t stream) {
-  using namespace mmb;
-  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
-                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && sent && h && cell && cov && mask && probs && h_out &&
-                  cell_out && att_cov && cov_out && hw && alpha && beta && ctx12 && pb && xcat && gates,
-              MMB_ERR_INVALID, "mmb_decoder_step_fused_fwd: null pointer");
+// Shape checks, cluster size, shared memory and row stage of the forward cluster kernels, then the launch: `g` null launches one step
+// (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel).
+static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream) {
+  const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
-              "mmb_decoder_step_fused_fwd: B=%d Lt=%d D=%d H=%d E=%d M=%d", B, Lt, D, H, E, M);
-  MMB_REQUIRE(D <= 256, MMB_ERR_UNSUPPORTED, "mmb_decoder_step_fused_fwd: D=%d > 256", D);
+              "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
+  MMB_REQUIRE(D <= 256, MMB_ERR_UNSUPPORTED, "%s: D=%d > 256", who, D);
   // few videos: eight CTAs per video keep more of the chip busy on the text sweep
   const int CL = (long long)B * 4 * 2 <= 160 ? 8 : 4;
-  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
-              sent, h, cell, cov, mask, target, probs, h_out, cell_out, att_cov, cov_out, argmax, nll, cov_loss, hw, alpha, beta,
-              ctx12, pb, xcat, gates, B, Lt, D, H, E, M, 0, 0};
   size_t smem = fused_smem_bytes(Lt, D, H, E, M, CL, &a.chunk);
-  MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "mmb_decoder_step_fused_fwd: %zu B of shared memory (Lt=%d)", smem, Lt);
+  MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "%s: %zu B of shared memory (Lt=%d)", who, smem, Lt);
   {
     // the row stage (see the kernel): two buffers of chunk x D floats behind two mbarriers, when they fit and bulk copies apply
     // (16-byte row granularity).  MMB_DEC_STAGE=0 turns it off (A/B measurements, cross-check in tests/test_decoder_gpu.py).
     static const char* stage_env = getenv("MMB_DEC_STAGE");
     const size_t base_floats = (smem + 15) / 16 * 4;
     const size_t stage_floats = 4 + 2 * (((size_t)a.chunk * D + 3) & ~(size_t)3);
-    const bool aligned = ((reinterpret_cast<uintptr_t>(proj_a) | reinterpret_cast<uintptr_t>(proj_i) | reinterpret_cast<uintptr_t>(enc_a) |
-                           reinterpret_cast<uintptr_t>(enc_i)) & 15) == 0;
+    const bool aligned = ((reinterpret_cast<uintptr_t>(a.proj_a) | reinterpret_cast<uintptr_t>(a.proj_i) |
+                           reinterpret_cast<uintptr_t>(a.enc_a) | reinterpret_cast<uintptr_t>(a.enc_i)) & 15) == 0;
     if ((D & 3) == 0 && aligned && (base_floats + stage_floats) * 4 <= 227 * 1024 && !(stage_env && atoi(stage_env) == 0)) {
       a.stage_off = (int)base_floats;
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set = 0;
-  if (smem > smem_set) {
-    MMB_CUDA(cudaFuncSetAttribute(dec_step_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    smem_set = smem;
+  static size_t smem_set[2] = {0, 0};
+  if (smem > smem_set[g != nullptr]) {
+    if (g) MMB_CUDA(cudaFuncSetAttribute(dec_greedy_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    else MMB_CUDA(cudaFuncSetAttribute(dec_step_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    smem_set[g != nullptr] = smem;
   }
   static const char* trace_env = getenv("MMB_DEC_TRACE");
   static bool trace_set = false;
@@ -1226,8 +1278,58 @@ extern "C" int mmb_decoder_step_fused_fwd(const float* proj_a, const float* proj
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (g) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_greedy_fused_kernel, a, *g));
+    return check_launch("dec_greedy_fused_kernel");
+  }
   MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_step_fused_kernel, a));
   return check_launch("dec_step_fused_kernel");
+}
+
+}  // namespace mmb
+
+extern "C" int mmb_decoder_step_fused_fwd(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                          const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                          const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                          const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt,
+                                          const float* bcat, const float* out_wt, const float* out_b, const float* sent,
+                                          const float* h, const float* cell, const float* cov, const uint8_t* mask,
+                                          const long long* target, float* probs, float* h_out, float* cell_out, float* att_cov,
+                                          float* cov_out, long long* argmax, float* nll, float* cov_loss, float* hw, float* alpha,
+                                          float* beta, float* ctx12, float* pb, float* xcat, float* gates, int B, int Lt, int D,
+                                          int H, int E, int M, mmb_stream_t stream) {
+  using namespace mmb;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && sent && h && cell && cov && mask && probs && h_out &&
+                  cell_out && att_cov && cov_out && hw && alpha && beta && ctx12 && pb && xcat && gates,
+              MMB_ERR_INVALID, "mmb_decoder_step_fused_fwd: null pointer");
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              sent, h, cell, cov, mask, target, probs, h_out, cell_out, att_cov, cov_out, argmax, nll, cov_loss, hw, alpha, beta,
+              ctx12, pb, xcat, gates, B, Lt, D, H, E, M, 0, 0};
+  return launch_fused(a, nullptr, "mmb_decoder_step_fused_fwd", stream);
+}
+
+extern "C" int mmb_decoder_greedy_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                        const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                        const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                        const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                        const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                        const uint8_t* mask, const long long* target, float* probs, long long* argmax,
+                                        float* loss_terms, int B, int Lt, int D, int H, int E, int M, int S, int T,
+                                        mmb_stream_t stream) {
+  using namespace mmb;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && probs && argmax,
+              MMB_ERR_INVALID, "mmb_decoder_greedy_fused: null pointer");
+  MMB_REQUIRE(S > 0 && (!target || (loss_terms && T >= S)), MMB_ERR_INVALID, "mmb_decoder_greedy_fused: S=%d T=%d, target %s, loss_terms %s",
+              S, T, target ? "set" : "null", loss_terms ? "set" : "null");
+  // (the per-step inputs and the saved arrays of the step kernel stay null: the roll-out keeps its state on chip)
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, target, probs, nullptr, nullptr, nullptr, nullptr, argmax,
+              target ? loss_terms : nullptr, target ? loss_terms + B : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+              nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, target ? T : 0};
+  return launch_fused(a, &g, "mmb_decoder_greedy_fused", stream);
 }
 
 extern "C" int mmb_decoder_bwd_head(const float* probs, const float* d_probs, const long long* target, const float* g_nll,

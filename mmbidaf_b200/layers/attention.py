@@ -207,6 +207,42 @@ class MultimodalAttentionDecoder(nn.Module):
         return self.step(sent_embed, decoder_hidden, decoder_cell_state, text_audio_enc_out, text_img_enc_out,
                          coverage_vec, mask)[:5]
 
+    def greedy(self, emb_text, h0, enc_a, enc_i, mask, steps, target=None):
+        """The greedy decode of ``steps`` steps in eval mode (models.py:145-199, the ``else`` branches), batched: start from h0
+        (B, H) or (B, 1, H), a zero cell, coverage and input row; each step's arg-max row of ``emb_text`` (B, Lt, E) is the next
+        input.  ``target`` (B, T) with T >= steps is optional.  No autograd.  Returns (out_distributions (B, steps, M), argmax
+        (B, steps) int64, loss_terms (steps, 2, B) = per step [nll | coverage term] or None) -- bit for bit what ``steps`` calls of
+        :meth:`step` with an arg-max and a gather in between give.  Where the decoder step runs as one cluster kernel
+        (``ops.decoder_cut``) the whole roll-out is one launch; long lectures run the chunk-parallel cut step by step."""
+        if not enc_a.is_cuda:
+            raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
+        if self.num_layers != 1:
+            raise RuntimeError("MultimodalAttentionDecoder: only num_layers=1 is supported (the reference model uses 1)")
+        with torch.no_grad():
+            seq = self._sequence(enc_a, enc_i)["seq"]
+            B, Lt = seq.B, seq.Lt
+            emb = emb_text.contiguous()
+            h = h0.reshape(B, -1).contiguous()
+            mask_u8 = ops._u8(mask)
+            tgt = None if target is None else target.reshape(B, -1).to(torch.int64).contiguous()
+            if ops.decoder_cut(B, Lt) != "chunks":
+                return ops.decoder_greedy_fwd(seq, emb, h, mask_u8, steps, tgt)
+            if tgt is not None and tgt.shape[1] < steps:
+                raise ValueError(f"greedy: {tgt.shape[1]} targets for {steps} steps")
+            rows = torch.arange(B, device=h.device)
+            sent = emb.new_zeros(B, emb.shape[2])
+            cell = h.new_zeros(B, seq.H)
+            cov = h.new_zeros(B, Lt)
+            probs, picks, terms = [], [], []
+            for s in range(steps):
+                p, h, cell, _, cov, am, _, lossvec = ops.decoder_step_fwd(
+                    seq, sent, h, cell, cov, mask_u8, want_argmax=True, target=None if tgt is None else tgt[:, s].contiguous())
+                sent = emb[rows, am]                                           # models.py:184,:193
+                probs.append(p)
+                picks.append(am)
+                terms.append(lossvec)
+            return torch.stack(probs, 1), torch.stack(picks, 1), (torch.stack(terms) if tgt is not None else None)
+
     def step(self, sent_embed, decoder_hidden, decoder_cell_state, text_audio_enc_out, text_img_enc_out, coverage_vec,
              mask, target=None):
         """``forward`` plus, when ``target`` (B) int64 is given, the step's fused loss terms as a sixth result:

@@ -98,6 +98,88 @@ class MMBiDAF(nn.Module):
     def forward(self, embedded_text, original_text_lengths, embedded_audio, original_audio_lengths, transformed_images,
                 original_image_lengths, batch_target_indices, original_target_len, max_dec_len):
         B, Lt = embedded_text.size(0), embedded_text.size(1)
+        steps = batch_target_indices.size(1) if self.training else max_dec_len
+        start = {}
+
+        def decoder_start():                     # everything the decode loop needs that does not depend on the encoders' output
+            start["cell"] = embedded_text.new_zeros(1, B, self.mod_t_a.rnn.hidden_size)
+            start["input"] = embedded_text.new_zeros(B, 1, embedded_text.size(-1))
+            start["cov"] = embedded_text.new_zeros(B, Lt, 1)
+            start["rows"] = torch.arange(B, device=embedded_text.device)
+            start["targets"] = batch_target_indices.reshape(B, -1).to(embedded_text.device).long()   # int(tensor), models.py:168
+            # (steps, B): a step's targets are one contiguous row (a column of (B, T) cost a strided-copy launch between every two
+            # decoder steps -- ~2 us on the serial chain, 12 times)
+            start["targets_t"] = start["targets"].t().contiguous()
+            if self.training:
+                # teacher forcing (models.py:173): every step's next input is known up front -- one gather for the whole
+                # sequence, laid out (steps, B, E) so that a step's slice is contiguous, instead of a gather per step
+                start["next"] = embedded_text[start["rows"].unsqueeze(0), start["targets"][:, :steps].t()]
+            self.multimodal_att_decoder.prepare()          # this step's weight layouts of the decoder's batched GEMMs
+
+        mod_text_audio, mod_text_image, decoder_hidden, decoder_mask = self._encode(
+            embedded_text, original_text_lengths, embedded_audio, original_audio_lengths, transformed_images, original_image_lengths,
+            decoder_start)
+        decoder_cell_state, decoder_input, coverage_vec = start["cell"], start["input"], start["cov"]
+        rows, targets, targets_t = start["rows"], start["targets"], start["targets_t"]
+        out_distributions, step_losses = [], []
+        if self.training:
+            next_inputs = start["next"]
+        for idx in range(steps):
+            tgt = targets_t[idx] if idx < targets_t.size(0) else targets[:, idx]
+            # the decoder kernels also emit this step's loss terms: -log(p[target] + 1e-12) (models.py:168-170)
+            # and sum(min(att_cov_dist, coverage_vec)) (models.py:177), one value per video
+            out_distribution, decoder_hidden, decoder_cell_state, att_cov_dist, coverage_vec, step_loss = \
+                self.multimodal_att_decoder.step(decoder_input, decoder_hidden, decoder_cell_state, mod_text_audio,
+                                                 mod_text_image, coverage_vec, decoder_mask, target=tgt)
+            if self.training:
+                decoder_input = next_inputs[idx].unsqueeze(1)                               # models.py:173
+            else:
+                decoder_input = embedded_text[rows, out_distribution.max(dim=1)[1]].unsqueeze(1)   # models.py:184,:193
+            out_distributions.append(out_distribution)
+            step_losses.append(step_loss)
+        # training adds the coverage loss at every step (models.py:177-178), evaluation once after the loop (:197-198);
+        # loss = (sum of the steps' nll + cov_loss_wt * coverage) / steps (models.py:179 / :199)
+        cov_loss_wt = 1.0
+        loss = Fn.decode_loss(step_losses, steps, cov_loss_wt, self.training)
+        return torch.stack(out_distributions).transpose(0, 1), loss
+
+    def summarize(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, targets=None):
+        """Extractive summaries of a batch (evaluate.py:107-126, :167-202 with method='greedy'): the eval-mode forward pass with the
+        whole greedy decode roll-out on the device, then the greedy sentence selection on the device.  Runs under ``no_grad`` in eval
+        mode and gives the caller's ``training`` flag back.  ``targets`` (B, T, 1) or (B, T) with T >= max_dec_len is optional (the
+        videos need no labels); with it ``loss`` is the eval loss of ``forward`` (models.py:197-199), else None.
+        Returns ``Summary(out_distributions (B, S, M), loss, indices (B, S) int32, counts (B) int32)`` -- the same distributions and
+        loss as ``forward`` in eval mode, the same picks as ``decode.get_generated_indices`` (``Summary.to_lists``)."""
+        from .layers.encoding import length_plan
+        from .summarize import Summary
+        was_training = self.training
+        self.eval()
+        try:
+            with torch.no_grad():
+                B = text.size(0)
+                dec = self.multimodal_att_decoder
+                start = {}
+
+                def decoder_start():
+                    if targets is not None:
+                        start["targets"] = targets.reshape(B, -1).to(text.device).long()
+                    dec.prepare()
+
+                enc_a, enc_i, h0, mask = self._encode(text, text_len, audio, audio_len, images, image_len, decoder_start)
+                probs, argmax, terms = dec.greedy(text, h0, enc_a, enc_i, mask, max_dec_len, target=start.get("targets"))
+                # the eval loss exactly as forward forms it: every step's nll, the last step's coverage term, over the steps
+                loss = None if terms is None else Fn.decode_loss(list(terms.unbind(0)), max_dec_len, 1.0, False)
+                indices, counts = ops.greedy_select(argmax, length_plan(text_len, text.device).len_i32)
+        finally:
+            self.train(was_training)
+        return Summary(probs, loss, indices, counts)
+
+    def _encode(self, embedded_text, original_text_lengths, embedded_audio, original_audio_lengths, transformed_images,
+                original_image_lengths, decoder_start):
+        """The encoder half of the model (models.py:95-143): embeddings, encoders, masks, both BiDAF blocks, the modality LSTMs and
+        the decoder's start state h0.  ``decoder_start()`` is issued on the main stream beside the recurrences (glue that needs no
+        encoder output).  Returns (text x audio encoding (B, Lt, 2H), text x image encoding, h0 (B, 1, H), decoder mask (B, M))."""
+        B, Lt = embedded_text.size(0), embedded_text.size(1)
 
         def text_branch():
             emb = self.emb(embedded_text)
@@ -138,24 +220,6 @@ class MMBiDAF(nn.Module):
                 side["proj_i"] = self.multimodal_att_decoder.hoist("i", out[0])      # ... W3 enc_i: this chain ends ~200 us earlier
                 side["hid_i"] = out[1].sum(1)
             return out
-
-        steps = batch_target_indices.size(1) if self.training else max_dec_len
-        start = {}
-
-        def decoder_start():                     # everything the decode loop needs that does not depend on the encoders' output
-            start["cell"] = embedded_text.new_zeros(1, B, self.mod_t_a.rnn.hidden_size)
-            start["input"] = embedded_text.new_zeros(B, 1, embedded_text.size(-1))
-            start["cov"] = embedded_text.new_zeros(B, Lt, 1)
-            start["rows"] = torch.arange(B, device=embedded_text.device)
-            start["targets"] = batch_target_indices.reshape(B, -1).to(embedded_text.device).long()   # int(tensor), models.py:168
-            # (steps, B): a step's targets are one contiguous row (a column of (B, T) cost a strided-copy launch between every two
-            # decoder steps -- ~2 us on the serial chain, 12 times)
-            start["targets_t"] = start["targets"].t().contiguous()
-            if self.training:
-                # teacher forcing (models.py:173): every step's next input is known up front -- one gather for the whole
-                # sequence, laid out (steps, B, E) so that a step's slice is contiguous, instead of a gather per step
-                start["next"] = embedded_text[start["rows"].unsqueeze(0), start["targets"][:, :steps].t()]
-            self.multimodal_att_decoder.prepare()          # this step's weight layouts of the decoder's batched GEMMs
 
         branch = {}
         if not (self.use_streams and torch.cuda.is_available()):
@@ -246,26 +310,4 @@ class MMBiDAF(nn.Module):
             decoder_hidden = (side["hid_a"] + side["hid_i"]).unsqueeze(1)
         else:
             decoder_hidden = (text_audio_hidden.sum(1) + text_img_hidden.sum(1)).unsqueeze(1)
-        decoder_cell_state, decoder_input, coverage_vec = start["cell"], start["input"], start["cov"]
-        rows, targets, targets_t = start["rows"], start["targets"], start["targets_t"]
-        out_distributions, step_losses = [], []
-        if self.training:
-            next_inputs = start["next"]
-        for idx in range(steps):
-            tgt = targets_t[idx] if idx < targets_t.size(0) else targets[:, idx]
-            # the decoder kernels also emit this step's loss terms: -log(p[target] + 1e-12) (models.py:168-170)
-            # and sum(min(att_cov_dist, coverage_vec)) (models.py:177), one value per video
-            out_distribution, decoder_hidden, decoder_cell_state, att_cov_dist, coverage_vec, step_loss = \
-                self.multimodal_att_decoder.step(decoder_input, decoder_hidden, decoder_cell_state, mod_text_audio,
-                                                 mod_text_image, coverage_vec, decoder_mask, target=tgt)
-            if self.training:
-                decoder_input = next_inputs[idx].unsqueeze(1)                               # models.py:173
-            else:
-                decoder_input = embedded_text[rows, out_distribution.max(dim=1)[1]].unsqueeze(1)   # models.py:184,:193
-            out_distributions.append(out_distribution)
-            step_losses.append(step_loss)
-        # training adds the coverage loss at every step (models.py:177-178), evaluation once after the loop (:197-198);
-        # loss = (sum of the steps' nll + cov_loss_wt * coverage) / steps (models.py:179 / :199)
-        cov_loss_wt = 1.0
-        loss = Fn.decode_loss(step_losses, steps, cov_loss_wt, self.training)
-        return torch.stack(out_distributions).transpose(0, 1), loss
+        return mod_text_audio, mod_text_image, decoder_hidden, decoder_mask

@@ -285,6 +285,18 @@ class DecoderSeq:
         self.counters = torch.zeros(2, self.B, device=self.enc_a.device, dtype=torch.int32)
 
 
+def decoder_cut(B: int, Lt: int) -> str:
+    """Which cut of the decoder step runs for B videos of Lt text rows: "fused" (one cluster kernel per step, or the whole greedy
+    roll-out in one launch) or "chunks" (the five-kernel chunk-parallel cut); MMB_DECODER_CUT overrides ("head" is a backward-only
+    cross-check; the forward treats anything but "chunks" as "fused")."""
+    cut = os.environ.get("MMB_DECODER_CUT")
+    if cut is None:
+        # a cluster (4 or 8 CTAs) per video: at most ~1000 CTAs worth of text rows per launch keeps every CTA's share of the text sweep
+        # short; long lectures (config 5: 16 x 4096 rows) are better spread over the (chunks x B) grid of the five-kernel cut
+        cut = "fused" if B * Lt <= 20000 else "chunks"
+    return cut
+
+
 def decoder_step_fwd(seq: DecoderSeq, sent, h, cell, coverage, mask_u8, want_argmax: bool = False, target=None):
     """One decoder step.  sent (B,E), h/cell (B,H), coverage (B,Lt), mask_u8 (B,M) uint8 -- contiguous fp32 CUDA.
     With ``target`` (B) int64 the kernels also emit the step's loss terms ``lossvec`` (B,2) =
@@ -296,11 +308,7 @@ def decoder_step_fwd(seq: DecoderSeq, sent, h, cell, coverage, mask_u8, want_arg
     f32 = dict(device=h.device, dtype=torch.float32)
     p = _lib.ptr
     st = _lib.stream()
-    cut = os.environ.get("MMB_DECODER_CUT")
-    if cut is None:
-        # a cluster (4 or 8 CTAs) per video: at most ~1000 CTAs worth of text rows per launch keeps every CTA's share of the text sweep
-        # short; long lectures (config 5: 16 x 4096 rows) are better spread over the (chunks x B) grid of the five-kernel cut
-        cut = "fused" if B * Lt <= 20000 else "chunks"
+    cut = decoder_cut(B, Lt)
     if cut != "chunks":
         # the whole step as one cluster kernel (csrc/decoder_fused.cu); MMB_DECODER_CUT=chunks forces the five-kernel cut below
         hw, alpha, beta = torch.empty(B, 4 * D, **f32), torch.empty(B, 2, Lt, **f32), torch.empty(B, 2, **f32)
@@ -346,6 +354,49 @@ def decoder_step_fwd(seq: DecoderSeq, sent, h, cell, coverage, mask_u8, want_arg
     return probs, h_out, cell_out, att_cov, cov_out, argmax, (hw, alpha, beta, ctx12, pb, xcat, gates), lossvec
 
 
+def decoder_greedy_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, steps: int, target=None):
+    """The greedy roll-out of ``steps`` decoder steps in eval mode as ONE launch (csrc/decoder_fused.cu, models.py:156-199).
+    emb_text (B,Lt,E) fp32, h0 (B,H) fp32, mask_u8 (B,M) uint8, target (B,T) int64 with T >= steps or None.
+    Returns (probs (B,steps,M), argmax (B,steps) int64, loss_terms (steps,2,B) = per step [nll | coverage term] or None)."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M):
+        raise ValueError(f"decoder_greedy_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask {tuple(mask_u8.shape)} "
+                         f"for B={B} Lt={Lt} E={E} H={H} M={M}")
+    T = 0
+    if target is not None:
+        T = target.shape[1]
+        if target.dtype != torch.int64 or target.shape[0] != B or T < steps:
+            raise ValueError(f"decoder_greedy_fwd: target {tuple(target.shape)} {target.dtype} for B={B}, {steps} steps")
+    probs = torch.empty(B, steps, M, device=dev, dtype=torch.float32)
+    argmax = torch.empty(B, steps, device=dev, dtype=torch.int64)
+    terms = torch.empty(steps, 2, B, device=dev, dtype=torch.float32) if target is not None else None
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_greedy_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(target), p(probs), p(argmax), p(terms),
+        B, Lt, D, H, E, M, int(steps), int(T), _lib.stream()), "mmb_decoder_greedy_fused")
+    _count(1)
+    return probs, argmax, terms
+
+
+def greedy_select(argmax: torch.Tensor, text_len: torch.Tensor):
+    """decode.greedy_search for a batch on the device: argmax (B,S) int64, text_len (B) int32 -> (sel (B,S) int32 = the chosen
+    sentence indices padded with -1, count (B) int32)."""
+    assert argmax.dtype == torch.int64 and text_len.dtype == torch.int32 and argmax.dim() == 2
+    B, S = argmax.shape
+    if text_len.numel() != B:
+        raise ValueError(f"greedy_select: {text_len.numel()} lengths for {B} videos")
+    sel = torch.empty(B, S, device=argmax.device, dtype=torch.int32)
+    count = torch.empty(B, device=argmax.device, dtype=torch.int32)
+    _lib.check(_lib.lib().mmb_greedy_select(_lib.ptr(argmax.contiguous()), _lib.ptr(text_len.contiguous()), _lib.ptr(sel),
+                                            _lib.ptr(count), B, S, _lib.stream()), "mmb_greedy_select")
+    _count(1)
+    return sel, count
+
+
 def decoder_step_bwd(seq: DecoderSeq, h, cell, coverage, probs, cell_out, saved, d_probs, d_h_out, d_cell_out,
                      d_att_cov, d_cov_out, d_proj_a, d_proj_i, vec_acc, scal_acc, target=None, d_lossvec=None,
                      att_cov=None, cov_out=None):
@@ -367,9 +418,7 @@ def decoder_step_bwd(seq: DecoderSeq, h, cell, coverage, probs, cell_out, saved,
     d_cell = torch.empty(B, H, **f32)
     datt, d_pre_b, d_ctx12 = torch.empty(B, Lt, **f32), torch.empty(2, B, D, **f32), torch.empty(2, B, D, **f32)
     dcov_tot = torch.empty(B, Lt, **f32)
-    cut = os.environ.get("MMB_DECODER_CUT")
-    if cut is None:
-        cut = "fused" if B * Lt <= 20000 else "chunks"
+    cut = decoder_cut(B, Lt)
     if cut == "fused":
         # the WHOLE backward step as one cluster kernel (csrc/decoder_fused.cu): head, both text sweeps, d h.  "head" keeps the
         # round-2 cut (head kernel + chunk-parallel sweeps + library GEMM) as a cross-check.

@@ -1,0 +1,134 @@
+"""Extractive summarisation (reference evaluate.py:107-126, :167-202, method='greedy') on the device.
+
+``MMBiDAF.summarize`` runs the encoder half of the model, the whole greedy decode roll-out and the greedy sentence selection
+without a host round trip; its result is a :class:`Summary`.  :class:`Summarizer` replays ``summarize`` from CUDA graphs, one
+capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
+"""
+from __future__ import annotations
+
+from typing import Dict, List, NamedTuple, Optional
+
+import torch
+import torch.distributed as dist
+
+from .synth import Batch
+
+__all__ = ["Summary", "Summarizer", "gather_summaries"]
+
+
+class Summary(NamedTuple):
+    out_distributions: torch.Tensor        # (B, S, M) fp32: every step's distribution over the sentences, as MMBiDAF.forward returns
+    loss: Optional[torch.Tensor]           # the eval loss (models.py:197-199) when targets were given, else None
+    indices: torch.Tensor                  # (B, S) int32: the chosen sentence indices of every video, padded with -1
+    counts: torch.Tensor                   # (B) int32: how many of them are valid
+
+    def to_lists(self) -> List[List[int]]:
+        """The chosen sentence indices per video as host lists (copies only ``indices`` and ``counts``):
+        equal to ``decode.get_generated_indices(out_distributions, text_len)``."""
+        idx, cnt = self.indices.cpu(), self.counts.cpu().tolist()
+        return [idx[b, :c].tolist() for b, c in enumerate(cnt)]
+
+
+def _bucket_key(batch: Batch, with_targets: bool):
+    return (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), int(batch.max_dec_len),
+            tuple(batch.targets.shape) if with_targets else None)
+
+
+class _Bucket:
+    """One captured ``summarize``: static inputs, static length plans, the graph and its (static) result."""
+
+    def __init__(self, model, batch: Batch, with_targets: bool, warmup: int):
+        import gc
+        from .layers.encoding import pin_lengths
+        dev = batch.text.device
+        # private copies: the captured kernels read the inputs and the lengths from these fixed addresses
+        self.batch = Batch(batch.text.clone(), list(batch.text_len), batch.audio.clone(), list(batch.audio_len), batch.images.clone(),
+                           list(batch.image_len), batch.targets.clone(), list(batch.target_len), batch.max_dec_len)
+        self.with_targets = with_targets
+        self.plans = [pin_lengths(lst, dev) for lst in (self.batch.text_len, self.batch.audio_len, self.batch.image_len)]
+        for m in model.modules():          # per-sequence caches of eager calls still own tensors (see Trainer.capture)
+            if hasattr(m, "_cache"):
+                m._cache = None
+        gc.collect()
+        torch.cuda.synchronize()
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            for _ in range(warmup):        # module loads, per-shape constants (decode_loss weights), the plans' masks
+                self._run(model)
+        torch.cuda.current_stream().wait_stream(side)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self.result = self._run(model)
+
+    def _run(self, model) -> Summary:
+        for plan in self.plans:            # inside the captured region: lengths -> int32, order, masks
+            plan.refresh()
+        b = self.batch
+        return model.summarize(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, b.max_dec_len,
+                               b.targets if self.with_targets else None)
+
+    def load(self, batch: Batch) -> None:
+        if batch is self.batch:
+            return
+        for plan, lens in zip(self.plans, (batch.text_len, batch.audio_len, batch.image_len)):
+            plan.update(lens)
+        s = self.batch
+        s.text.copy_(batch.text, non_blocking=True)
+        s.audio.copy_(batch.audio, non_blocking=True)
+        s.images.copy_(batch.images, non_blocking=True)
+        if self.with_targets:
+            s.targets.copy_(batch.targets, non_blocking=True)
+
+
+class Summarizer:
+    """``model.summarize`` replayed from CUDA graphs.  A batch of a padded-shape bucket seen before (text, audio and key-frame widths,
+    the batch size, ``max_dec_len`` and, with targets, their width) is copied into that bucket's static inputs, its lengths into the
+    bucket's static length plans, and the bucket's graph is replayed; a new bucket is captured first (after ``warmup`` eager runs).
+    The decoder's weight layouts are rebuilt inside the graph, so in-place parameter updates (an optimiser step) show up on the next
+    replay.  The returned :class:`Summary` holds the bucket's static output tensors: the next replay of the same bucket overwrites them."""
+
+    def __init__(self, model, warmup: int = 2):
+        self.model = model
+        self.warmup = warmup
+        self.buckets: Dict[tuple, _Bucket] = {}
+
+    def __call__(self, batch: Batch, with_targets: bool = False) -> Summary:
+        """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``."""
+        key = _bucket_key(batch, with_targets)
+        bucket = self.buckets.get(key)
+        if bucket is None:
+            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup)
+        else:
+            bucket.load(batch)
+        bucket.graph.replay()
+        return bucket.result
+
+
+def gather_summaries(summary: Summary, group=None) -> Optional[List[List[int]]]:
+    """The summaries of a data-parallel job on rank 0: every rank holds the summary of its contiguous shard of the batch
+    (``trainer.shard_batch``, which keeps the global text padding -- the decoder's attention runs over every padded text position,
+    quirk Q2, so a narrower shard would change the picks).  Rank 0 gets the chosen indices of every video in batch order, as
+    ``Summary.to_lists`` of the whole batch would give them; the other ranks get None.  One all-gather of the shard sizes, then one
+    all-gather of the (count, indices) rows padded to the largest shard, as int32 tensors on the summary's device."""
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return summary.to_lists()
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    idx, cnt = summary.indices, summary.counts
+    B, S = idx.shape
+    size = torch.tensor([B], dtype=torch.int32, device=idx.device)
+    sizes = [torch.empty_like(size) for _ in range(world)]
+    dist.all_gather(sizes, size, group=group)
+    sizes = [int(t) for t in sizes]
+    rows = torch.full((max(sizes), S + 1), -1, dtype=torch.int32, device=idx.device)
+    rows[:B, 0] = cnt
+    rows[:B, 1:] = idx
+    parts = [torch.empty_like(rows) for _ in range(world)]
+    dist.all_gather(parts, rows, group=group)
+    if rank != 0:
+        return None
+    out = []
+    for n, part in zip(sizes, parts):
+        host = part[:n].cpu()
+        out += [host[b, 1:1 + int(host[b, 0])].tolist() for b in range(n)]
+    return out
