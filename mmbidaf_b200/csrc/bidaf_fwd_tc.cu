@@ -2,7 +2,7 @@
 // bf16 operands, fp32 accumulation / soft-max; rel <= 2e-2 tier of north_star.
 //
 // Same three streaming-soft-max contractions as the fp32 tier (bidaf_fwd_f32.cu), reorganised for the
-// 5th-generation tensor cores:
+// 5th-generation tensor cores.  Two launches:
 //
 //  1. bidaf_pack_kernel   converts c, q (optionally dropped) to bf16 ONCE, in the UMMA "core matrix" order
 //       pack[b][row/8][chunk 0..25][row%8][8 x bf16]      (8 rows x 16 bytes = one 128-byte core matrix)
@@ -12,34 +12,15 @@
 //     MN-major operand (O = P V: LBO 3328, SBO 128).  Chunk 25 is K padding (200 -> 208); it carries the
 //     additive terms of the trilinear form split into bf16 hi/lo halves: text rows hold
 //     [t_hi, t_lo, 1, 1, 0..] and modality rows [1, 1, m_hi, m_lo, 0..], so the GEMM itself adds
-//     c~.w_c + q~.w_q to every logit.  w_cq is folded into the text-side S operand.
-//  2. Q2C blocks             X = 128 modality rows, streams 64-row text tiles:   T = softmax_i(S)^T c
-//  3. C2Q blocks             X = 128 text rows, streams 64-row modality tiles:   a = softmax_j(S) q,
-//                                                                              b = softmax_j(S) T
-//     Per tile: thread 0 issues 13 MMAs (128 x 64 x 208) into TMEM, commits to an mbarrier; each of the 128
-//     threads owns one row of S (tcgen05.ld 32x32b.x64), does the masked streaming soft-max in registers
-//     (no shuffles: a thread holds its whole row), writes P as bf16 in core-matrix order, and thread 0 issues
-//     the P V MMAs (N = 208, K = 64) into the TMEM accumulators.  Accumulators are rescaled lazily (only
-//     when a row's running max moves by more than TAU), as in FlashAttention-4.
-//     The epilogue drains TMEM through shared memory so that the 4-way concat is written with coalesced
-//     128-bit stores; Q2C also emits T in packed bf16 form for pass 3.
-#include <stdlib.h>
+//     c~.w_c + q~.w_q to every logit.  w_cq is folded into the text-side S operand.  It also writes block 0 of
+//     the output (the text itself) and zeroes the dependency counters and work-queue head of launch 2.
+//  2. bidaf_tc5_kernel (bidaf_fwd_tc5.cu)   one persistent, warp-specialised CTA per SM runs the Q2C items
+//     (T = softmax_i(S)^T c) and the C2Q items (a = softmax_j(S) q, b = softmax_j(S) T) and writes blocks 1 - 3.
 #include "tc_common.cuh"
 
 namespace mmb {
 using namespace tc;
 namespace {
-
-constexpr int TX = 128, TY = 64;
-constexpr int X_BYTES = TX / 8 * GROUP_BYTES;   // 53248
-constexpr int Y_BYTES = TY / 8 * GROUP_BYTES;   // 26624
-constexpr int P_BYTES = TX * TY * 2;            // 16384
-constexpr int MAX_STAGES = 3;
-constexpr int MMA_WARP = 0, TMA_WARP = 1;  // issuing warps (one elected lane each, see tc_common.cuh)
-constexpr int COL_S = 0, COL_O0 = 64, COL_O1 = 64 + DPAD;
-constexpr int STG_STRIDE = 204;           // fp32 staging row stride (conflict-free 128-bit stores)
-
-enum Kind { Q2C = 0, C2Q = 1 };
 
 // ---------------------------------------------------------------------------------------------------------
 // 1. pack: fp32 (B, L, d) -> bf16 core-matrix order (+ folded weights, additive terms, mask words)
@@ -57,8 +38,6 @@ struct PackArgs {
   float keep_scale;
   int L, LP, d, text_side;
 };
-
-constexpr int PACK_CHUNK_STRIDE = 144;   // 128-byte core matrix + 16 bytes: spreads the staging stores over banks
 
 struct PackPair { PackArgs side[2]; };
 
@@ -253,395 +232,8 @@ __global__ void __launch_bounds__(128, 4) bidaf_pack_kernel(const PackPair pp, c
   }
 }
 
-// ---------------------------------------------------------------------------------------------------------
-// 2./3. tensor-core passes
-// ---------------------------------------------------------------------------------------------------------
-struct TcArgs {
-  const __nv_bfloat16* x_pack;       // (B, LXP/8, 26, 8, 8) S operand of the X side
-  const __nv_bfloat16* y_pack;       // S operand of the Y side
-  const __nv_bfloat16* v0_pack;      // value operand 0 (plain Y rows); may equal y_pack
-  const __nv_bfloat16* v1_pack;      // value operand 1 (C2Q: packed T); null for Q2C
-  const unsigned long long* y_words; // (B, LYP/64, 2)
-  const float* bias;
-  float* out;                        // Q2C: T fp32 (B, LX, d);   C2Q: out (B, LX, 4d)
-  __nv_bfloat16* t_pack;             // Q2C: packed T for pass 3
-  float* lse;                        // (B, LX)
-  float* bm;                         // C2Q: optional (B, LX, d) copy of b = s1 T for the backward pass
-  long long* trace;                  // debugging aid: clock64() stamps of CTA (0,0), or null
-  int LX, LXP, LY, LYP, d;
-};
-
-constexpr int NTHREADS = 256;            // two threads per X row: warps 0-3 take S columns 0-31, warps 4-7 columns 32-63
-constexpr float TAU2 = 11.0f;            // lazy-rescale threshold in log2 units (factor 2048)
-
-// One X block of one pass.  `ready` (per batch row) orders the two passes inside ONE launch: a Q2C block bumps
-// ready[b] once its T rows are in memory, a C2Q block of the same batch row waits for all of them.
-template <int KIND>
-__device__ __forceinline__ void bidaf_tc_block(const TcArgs& a, const int b, const int xblk, int* ready, const int ready_target,
-                                               long long* cta_times = nullptr) {
-  constexpr int NACC = KIND == C2Q ? 2 : 1;
-  constexpr int HALF = TY / 2;
-  extern __shared__ __align__(128) unsigned char smem[];
-  const bool sep_v0 = a.v0_pack != a.y_pack;
-  const int nparts = 1 + (sep_v0 ? 1 : 0) + (KIND == C2Q ? 1 : 0);
-  const int stage_bytes = nparts * Y_BYTES;
-  const int STAGES = nparts == 2 ? 3 : 2;                        // what fits in 227 KB next to X and P
-  unsigned char* Xs = smem;
-  unsigned char* Ps = Xs + X_BYTES;
-  unsigned char* St = Ps + P_BYTES;                               // STAGES x stage_bytes
-  uint64_t* bars = reinterpret_cast<uint64_t*>(St + STAGES * stage_bytes);   // [0] x, [1] mma, [2..4] full, [5..7] free
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 8);
-  float* xbuf = reinterpret_cast<float*>(bars + 10);              // [2][TX] cross-half exchange (max, then sum)
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int half = warp >> 2, wq = warp & 3;
-  const int warp_u = uniform_warp_idx();
-  const uint32_t leader = elect_one();                   // one lane per warp: the issuer in the MMA / TMA warps
-  const int row = wq * 32 + lane;
-  const int x0 = xblk * TX;
-  const uint32_t bar_x = smem_u32(bars), bar_mma = smem_u32(bars + 1), bar_full0 = smem_u32(bars + 2);
-  const uint32_t bar_free0 = smem_u32(bars + 2 + MAX_STAGES);
-
-  if (tid == 0) {
-    mbar_init(bar_x, 1);
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(bar_full0 + 8 * s, 1);
-      mbar_init(bar_free0 + 8 * s, 1);
-    }
-    mbar_init(bar_mma, 1);
-    fence_barrier_init();
-  }
-  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), TMEM_COLS);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, *tmem_slot, 0);
-
-  // Tiles past the last un-masked Y row contribute exp(-1e30 - m) = 0 to every soft-max: stop there.  (If nothing at
-  // all is un-masked the soft-max is uniform over the whole range, attention.py:94, and every tile is needed.)
-  int nty = (a.LY + TY - 1) / TY;
-  {
-    int last = 0;
-    for (int t = lane; t < nty; t += 32)
-      if (a.y_words[((size_t)b * (a.LYP / 64) + t) * 2 + 1] != 0ull) last = t + 1;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
-    if (last > 0) nty = last;
-  }
-  const size_t x_off = ((size_t)b * (a.LXP / 8) + x0 / 8) * GROUP_BYTES;
-  const size_t y_batch = (size_t)b * (a.LYP / 8) * GROUP_BYTES;
-  auto issue_stage = [&](int t) {
-    const int s = t % STAGES;
-    const uint32_t bar = bar_full0 + 8 * s;
-    const uint32_t dst = smem_u32(St + s * stage_bytes);
-    const size_t off = y_batch + (size_t)t * Y_BYTES;
-    mbar_expect_tx(bar, stage_bytes, leader);
-    tma_bulk_g2s(dst, reinterpret_cast<const char*>(a.y_pack) + off, Y_BYTES, bar, leader);
-    int part = 1;
-    if (sep_v0) tma_bulk_g2s(dst + (part++) * Y_BYTES, reinterpret_cast<const char*>(a.v0_pack) + off, Y_BYTES, bar, leader);
-    if (KIND == C2Q) tma_bulk_g2s(dst + part * Y_BYTES, reinterpret_cast<const char*>(a.v1_pack) + off, Y_BYTES, bar, leader);
-  };
-  if (warp_u == TMA_WARP) {
-    mbar_expect_tx(bar_x, X_BYTES, leader);
-    tma_bulk_g2s(smem_u32(Xs), reinterpret_cast<const char*>(a.x_pack) + x_off, X_BYTES, bar_x, leader);
-    if (KIND == C2Q && ready) {                                   // the stages carry T: wait for this batch row's Q2C blocks
-      wait_counter(ready + b, ready_target);
-      fence_proxy_async_all();                                    // their generic-proxy stores -> our async-proxy (TMA) loads
-    }
-    for (int t = 0; t < STAGES && t < nty; ++t) issue_stage(t);
-  }
-
-  const float bias2 = a.bias[0] * LOG2E;
-  const uint32_t lane_base = tmem + ((uint32_t)(wq * 32) << 16);     // this warp's 32 TMEM lanes
-  float m_ref = -INFINITY, l_part = 0.f;                             // log2 domain; l over this thread's columns
-  uint32_t mma_phase = 0;
-  constexpr uint32_t IDESC_S = idesc_bf16(TY, 0), IDESC_PV = idesc_bf16(DPAD, 1);
-  const uint32_t xs_addr = smem_u32(Xs);
-  const uint32_t xs_lo = desc_lo(xs_addr, 128), ps_lo = desc_lo(smem_u32(Ps), 2048);
-
-  const bool tracing = a.trace != nullptr && b == 0 && xblk == 0 && tid == 0;
-  int ntrace = 0;
-  auto stamp = [&]() {
-    if (tracing && ntrace < 250) a.trace[ntrace++] = clock64();
-  };
-  stamp();
-  if (warp_u == MMA_WARP) mbar_wait(bar_x, 0);
-  stamp();
-  for (int t = 0; t < nty; ++t) {
-    const int s = t % STAGES;
-    const uint32_t st_addr = smem_u32(St + s * stage_bytes);
-    if (warp_u == MMA_WARP) {
-      mbar_wait(bar_full0 + 8 * s, (t / STAGES) & 1);
-      stamp();
-      tc_fence_after();
-      const uint32_t st_lo = desc_lo(st_addr, 128);
-#pragma unroll
-      for (int k = 0; k < DPAD / 16; ++k)                       // S = X Y^T, both K-major
-        umma_bf16_lh(tmem + COL_S, xs_lo + k * 16, desc_hi(GROUP_BYTES), st_lo + k * 16, desc_hi(GROUP_BYTES), IDESC_S, k > 0,
-                     leader);
-      umma_commit(bar_mma, leader);
-      stamp();
-    }
-    const ulonglong2 words = *reinterpret_cast<const ulonglong2*>(a.y_words + ((size_t)b * (a.LYP / 64) + t) * 2);
-    const uint32_t wvalid = (uint32_t)(words.x >> (HALF * half)), wopen = (uint32_t)(words.y >> (HALF * half));
-    const bool all_open = (words.x & words.y) == ~0ull;         // CTA-uniform: interior tile, nothing masked
-    // the previous tile's P V MMAs commit to the "free" barrier of their stage: refill it while this tile's S MMAs
-    // run, so the load has a whole tile of tensor-core + soft-max time to land
-    if (warp_u == TMA_WARP && t >= 1 && t - 1 + STAGES < nty) {
-      mbar_wait(bar_free0 + 8 * ((t - 1) % STAGES), ((t - 1) / STAGES) & 1);
-      issue_stage(t - 1 + STAGES);
-    }
-    mbar_wait(bar_mma, mma_phase);
-    mma_phase ^= 1;
-    tc_fence_after();
-    stamp();
-
-    // ---- this thread's half row of S: masked streaming soft-max (base-2) -------------------------------------
-    float sv[HALF];
-    tmem_ld16(lane_base + COL_S + half * HALF, sv);
-    tmem_ld16(lane_base + COL_S + half * HALF + 16, sv + 16);
-    float tile_max = -INFINITY;
-    if (all_open) {
-#pragma unroll
-      for (int c = 0; c < HALF; ++c) {
-        sv[c] = fmaf(sv[c], LOG2E, bias2);
-        tile_max = fmaxf(tile_max, sv[c]);
-      }
-    } else {
-#pragma unroll
-      for (int c = 0; c < HALF; ++c) {
-        const float v = ((wopen >> c) & 1u) ? fmaf(sv[c], LOG2E, bias2) : kNegFill * LOG2E;   // attention.py:94
-        sv[c] = v;
-        if ((wvalid >> c) & 1u) tile_max = fmaxf(tile_max, v);
-      }
-    }
-    xbuf[half * TX + row] = tile_max;
-    __syncthreads();
-    stamp();
-    tile_max = fmaxf(tile_max, xbuf[(half ^ 1) * TX + row]);    // both threads of the row now agree
-    float alpha = 1.f;
-    const bool bump = tile_max > m_ref + TAU2;                  // first tile: m_ref = -inf -> always
-    if (bump) {
-      alpha = fast_exp2(m_ref - tile_max);                          // 0 on the first tile
-      m_ref = tile_max;
-    }
-    float psum = 0.f;
-    uint32_t packed[HALF / 2];
-    if (all_open) {
-#pragma unroll
-      for (int c = 0; c < HALF; c += 2) {
-        const float p0 = fast_exp2(sv[c] - m_ref), p1 = fast_exp2(sv[c + 1] - m_ref);
-        psum += p0 + p1;
-        const __nv_bfloat162 pk = __floats2bfloat162_rn(p0, p1);
-        packed[c / 2] = *reinterpret_cast<const uint32_t*>(&pk);
-      }
-    } else {
-#pragma unroll
-      for (int c = 0; c < HALF; c += 2) {
-        const float p0 = ((wvalid >> c) & 1u) ? fast_exp2(sv[c] - m_ref) : 0.f;
-        const float p1 = ((wvalid >> (c + 1)) & 1u) ? fast_exp2(sv[c + 1] - m_ref) : 0.f;
-        psum += p0 + p1;
-        const __nv_bfloat162 pk = __floats2bfloat162_rn(p0, p1);
-        packed[c / 2] = *reinterpret_cast<const uint32_t*>(&pk);
-      }
-    }
-    l_part = l_part * alpha + psum;
-    // P in core-matrix order: chunk c8 (8 columns) at c8*2048 + row*16  (LBO 2048, SBO 128)
-    {
-      unsigned char* prow = Ps + row * 16 + (half * (HALF / 8)) * 2048;
-#pragma unroll
-      for (int c8 = 0; c8 < HALF / 8; ++c8)
-        *reinterpret_cast<uint4*>(prow + c8 * 2048) =
-            make_uint4(packed[c8 * 4], packed[c8 * 4 + 1], packed[c8 * 4 + 2], packed[c8 * 4 + 3]);
-    }
-    fence_proxy_async();                                        // st.shared P -> visible to the tensor core
-    tc_fence_before();
-    const int any_bump = __syncthreads_or(bump && t > 0);
-    stamp();
-    if (any_bump) {                                             // lazy rescale: the two threads of a row split the columns
-      tc_fence_after();
-#pragma unroll 1
-      for (int acc = 0; acc < NACC; ++acc)
-#pragma unroll 1
-        for (int q = half; q < DPAD / 16; q += 2) {
-          float o[16];
-          const uint32_t addr = lane_base + (acc == 0 ? COL_O0 : COL_O1) + q * 16;
-          tmem_ld16(addr, o);
-#pragma unroll
-          for (int i = 0; i < 16; ++i) o[i] *= alpha;
-          tmem_st16(addr, o);
-        }
-      tmem_wait_st();
-      tc_fence_before();
-      __syncthreads();
-    }
-    stamp();
-    if (warp_u == MMA_WARP) {
-      tc_fence_after();
-      const uint32_t v0_lo = desc_lo(sep_v0 ? st_addr + Y_BYTES : st_addr, GROUP_BYTES);
-#pragma unroll
-      for (int k = 0; k < TY / 16; ++k)                         // O0 += P V0 (V MN-major: LBO = group stride)
-        umma_bf16_lh(tmem + COL_O0, ps_lo + k * 256, desc_hi(128), v0_lo + k * 2 * GROUP_BYTES / 16, desc_hi(128), IDESC_PV,
-                     (t > 0) || (k > 0), leader);
-      if (KIND == C2Q) {
-        const uint32_t v1_lo = desc_lo(st_addr + (nparts - 1) * Y_BYTES, GROUP_BYTES);
-#pragma unroll
-        for (int k = 0; k < TY / 16; ++k)
-          umma_bf16_lh(tmem + COL_O1, ps_lo + k * 256, desc_hi(128), v1_lo + k * 2 * GROUP_BYTES / 16, desc_hi(128), IDESC_PV,
-                       (t > 0) || (k > 0), leader);
-      }
-      umma_commit(t == nty - 1 ? bar_mma : bar_free0 + 8 * s, leader);
-    }
-  }
-  // ---- epilogue: TMEM -> registers -> fp32 staging in smem -> coalesced global stores -----------------------------
-  xbuf[half * TX + row] = l_part;                               // combine the two half-row sums
-  mbar_wait(bar_mma, mma_phase);
-  tc_fence_after();
-  __syncthreads();
-  stamp();
-  if (cta_times && tid == 0) cta_times[1] = globaltimer_ns();          // main loop done
-  const float l_run = xbuf[row] + xbuf[TX + row];
-  const int gx = x0 + row;
-  const float inv_l = 1.f / l_run;
-  if (half == 0 && gx < a.LX && a.lse) a.lse[(size_t)b * a.LX + gx] = (m_ref + log2f(l_run)) * LN2;
-  float* stg = reinterpret_cast<float*>(St);                    // 128 x 204 fp32 = 104448 B <= 2 stages
-  const int d = a.d, dv4 = d >> 2;
-  stamp();
-#pragma unroll 1
-  for (int acc = 0; acc < NACC; ++acc) {
-    if (acc > 0) __syncthreads();
-    stamp();
-#pragma unroll 1
-    for (int q = half; q < DPAD / 16; q += 2) {
-      float o[16];
-      tmem_ld16(lane_base + (acc == 0 ? COL_O0 : COL_O1) + q * 16, o);
-#pragma unroll
-      for (int i = 0; i < 16; i += 4)
-        if (q * 16 + i < STG_STRIDE)
-          *reinterpret_cast<float4*>(stg + row * STG_STRIDE + q * 16 + i) =
-              make_float4(o[i] * inv_l, o[i + 1] * inv_l, o[i + 2] * inv_l, o[i + 3] * inv_l);
-    }
-    __syncthreads();
-    stamp();
-    if (KIND == Q2C) {
-      for (int i = tid; i < TX * dv4; i += NTHREADS) {          // fp32 T rows, coalesced
-        const int r = i / dv4, c4 = i - r * dv4;
-        if (x0 + r < a.LX)
-          *reinterpret_cast<float4*>(a.out + ((size_t)b * a.LX + x0 + r) * d + c4 * 4) =
-              *reinterpret_cast<const float4*>(stg + r * STG_STRIDE + c4 * 4);
-      }
-      // packed bf16 T (value operand of pass 3): one 16-byte chunk per (row, chunk), contiguous per 8-row group
-      char* tp = reinterpret_cast<char*>(a.t_pack) + x_off;
-      for (int i = tid; i < TX * CHUNKS; i += NTHREADS) {
-        const int g8 = i / (CHUNKS * 8), rem = i - g8 * CHUNKS * 8, ch = rem >> 3, r8 = rem & 7;
-        const int r = g8 * 8 + r8;
-        __nv_bfloat162 v[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const int col = ch * 8 + 2 * e;
-          const bool ok = (x0 + r < a.LX) && col < d;
-          v[e] = __floats2bfloat162_rn(ok ? stg[r * STG_STRIDE + col] : 0.f, ok ? stg[r * STG_STRIDE + col + 1] : 0.f);
-        }
-        *reinterpret_cast<uint4*>(tp + (size_t)i * 16) = *reinterpret_cast<uint4*>(v);
-      }
-    } else {
-      // blocks 1..3 of the concat (attention.py:52); block 0 (the text itself, exact fp32) was written by the pack
-      // kernel and is read back here for the products.  A warp instruction stores 512 contiguous bytes of ONE row:
-      // measured 30 B/clk/SM against 15 for 64-byte runs over 8 rows (tools/micro/store_rate.cu).
-      constexpr int NW = NTHREADS / 32, RB = 4;
-#pragma unroll 1
-      for (int r0 = warp; r0 < TX; r0 += NW * RB) {
-        float4 cv[RB][2];
-#pragma unroll
-        for (int u = 0; u < RB; ++u) {
-          const int r = r0 + u * NW;
-          const float* crow = a.out + ((size_t)b * a.LX + min(x0 + r, a.LX - 1)) * 4 * d;
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const int c4 = lane + 32 * h;
-            if (c4 < dv4) cv[u][h] = *reinterpret_cast<const float4*>(crow + c4 * 4);
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < RB; ++u) {
-          const int r = r0 + u * NW;
-          if (x0 + r >= a.LX) continue;
-          float* orow = a.out + ((size_t)b * a.LX + x0 + r) * 4 * d;
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const int c4 = lane + 32 * h;
-            if (c4 >= dv4) continue;
-            const float4 v = *reinterpret_cast<const float4*>(stg + r * STG_STRIDE + c4 * 4);
-            const float4 c = cv[u][h];
-            const float4 p = make_float4(c.x * v.x, c.y * v.y, c.z * v.z, c.w * v.w);
-            if (acc == 0) {
-              *reinterpret_cast<float4*>(orow + d + c4 * 4) = v;
-              *reinterpret_cast<float4*>(orow + 2 * d + c4 * 4) = p;
-            } else {
-              *reinterpret_cast<float4*>(orow + 3 * d + c4 * 4) = p;
-              if (a.bm) *reinterpret_cast<float4*>(a.bm + ((size_t)b * a.LX + x0 + r) * d + c4 * 4) = v;
-            }
-          }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  stamp();
-  if (tracing) a.trace[255] = ntrace;
-  if (warp == 0) tmem_dealloc(tmem, TMEM_COLS);
-  if (KIND == Q2C && ready && tid == 0) signal_counter(ready + b);   // after the barrier: every thread's T stores are ordered before it
-}
-
-// Both passes in one launch: the Q2C blocks come first in block order (so they are resident or done before any C2Q
-// block that waits for them is scheduled), then the C2Q blocks.  A C2Q block starts as soon as ITS batch row's Q2C
-// blocks are done, on whichever SM frees up: no launch boundary between the passes, and the store-bound C2Q epilogues
-// (the chip writes ~3.5 TB/s) spread over time instead of hitting memory together.
-struct FusedArgs {
-  TcArgs q2c, c2q;
-  int* ready;            // (B) zeroed before the launch
-  int nq, nc;            // X blocks per batch row of each pass
-  int n_q2c;             // B * nq
-  long long* cta_times;  // debugging aid (MMB_BIDAF_FWD_CTA_TIMES: a device pointer, 12 x int64 per block) or null
-};
-
-// (separate launches: debugging aid, MMB_BIDAF_FWD_SPLIT=1)
-template <int KIND>
-__global__ void __launch_bounds__(NTHREADS, 1) bidaf_tc_kernel(const TcArgs a) {
-  bidaf_tc_block<KIND>(a, blockIdx.y, blockIdx.x, nullptr, 0);
-}
-
-__global__ void __launch_bounds__(NTHREADS, 1) bidaf_tc_fused_kernel(const FusedArgs f) {
-  const int blk = blockIdx.x;
-  long long* times = f.cta_times ? f.cta_times + 12 * (size_t)blk : nullptr;   // debugging aid: [start, loop end, end, SM id, ...]
-  if (times && threadIdx.x == 0) {
-    times[0] = globaltimer_ns();
-    uint32_t smid;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    times[3] = smid;
-  }
-  if (blk < f.n_q2c) {
-    bidaf_tc_block<Q2C>(f.q2c, blk / f.nq, blk % f.nq, f.ready, 0, times);
-  } else {
-    const int i = blk - f.n_q2c;
-    bidaf_tc_block<C2Q>(f.c2q, i / f.nc, i % f.nc, f.ready, f.nq, times);
-  }
-  if (times && threadIdx.x == 0) times[2] = globaltimer_ns();
-}
-
-size_t tc_smem_bytes(int nparts) {
-  return (size_t)X_BYTES + P_BYTES + (size_t)(nparts == 2 ? 3 : 2) * nparts * Y_BYTES + 80 + 2 * TX * 4;
-}
-
 }  // namespace
 
-int bidaf_fwd_tc2_launch(const BidafPacks& pk, const float* bias, float* out, float* q2c, float* bm, float* lse_row,
-                         float* lse_col, int B, int Lc, int Lq, int d, cudaStream_t stream);
-int bidaf_fwd_tc3_launch(const BidafPacks& pk, const float* bias, float* out, float* q2c, float* bm, float* lse_row,
-                         float* lse_col, int B, int Lc, int Lq, int d, cudaStream_t stream);
-int bidaf_fwd_tc4_launch(const BidafPacks& pk, const float* text, const float* bias, float* out, float* q2c, float* bm,
-                         float* lse_row, float* lse_col, int B, int Lc, int Lq, int d, cudaStream_t stream);
 int bidaf_fwd_tc5_launch(const BidafPacks& pk, const float* text, const float* bias, float* out, float* q2c, float* bm,
                          float* lse_row, float* lse_col, int B, int Lc, int Lq, int d, cudaStream_t stream);
 
@@ -654,16 +246,12 @@ int bidaf_fwd_tc(const float* text, const float* modality, const uint8_t* text_m
                  float* bm, float* lse_row, float* lse_col, void* workspace, int B, int Lc, int Lq, int d, cudaStream_t stream) {
   MMB_REQUIRE(d % 8 == 0 && d <= 200, MMB_ERR_UNSUPPORTED, "mmb_bidaf_fwd (bf16 tier): d=%d (need d %% 8 == 0, d <= 200)", d);
   MMB_REQUIRE(workspace, MMB_ERR_INVALID, "mmb_bidaf_fwd (bf16 tier): workspace is null");
-  static_assert(PACK_ROWS == TX, "pack padding must match the X tile");
   const BidafPacks pk = bidaf_packs(workspace, B, Lc, Lq, keep_modality != nullptr);
   const int LcP = pk.LcP, LqP = pk.LqP;
-  __nv_bfloat16 *cw = pk.cw, *cp = pk.cp, *qs = pk.qs, *qp = pk.qp, *tp = pk.tp;
-  unsigned long long *c_words = pk.c_words, *q_words = pk.q_words;
-  long long* trace = getenv("MMB_BIDAF_FWD_TRACE") ? pk.trace : nullptr;   // debugging aid (tools/bidaf_trace.py)
 
   PackPair pp;
-  pp.side[0] = PackArgs{text, keep_text, text_mask, w_text, w_cross, cw, cp, c_words, out, keep_scale, Lc, LcP, d, 1};
-  pp.side[1] = PackArgs{modality, keep_modality, modality_mask, w_modality, nullptr, qs, qp, q_words, nullptr, keep_scale,
+  pp.side[0] = PackArgs{text, keep_text, text_mask, w_text, w_cross, pk.cw, pk.cp, pk.c_words, out, keep_scale, Lc, LcP, d, 1};
+  pp.side[1] = PackArgs{modality, keep_modality, modality_mask, w_modality, nullptr, pk.qs, pk.qp, pk.q_words, nullptr, keep_scale,
                         Lq, LqP, d, 0};
   {
     static int num_sms = 0;
@@ -678,40 +266,7 @@ int bidaf_fwd_tc(const float* text, const float* modality, const uint8_t* text_m
   }
   if (int rc = check_launch("bidaf_pack_kernel")) return rc;
 
-  // Cuts of the same algorithm (profiles/r02_bidaf_fwd.md).  The default is cut 5 (csrc/bidaf_fwd_tc5.cu: one persistent warp-
-  // specialised CTA per SM, 64-column tiles, P through TMEM, split accumulator): the fastest on every shape measured (config 2:
-  // 94 vs 98 us; text x audio of config 3: 97 vs 109; config 5: 329 vs 431).  MMB_BIDAF_FWD_CUT=1..4 forces an earlier cut (kept
-  // as cross-checks of each other in tests/test_bidaf_gpu.py): 1 one block per SM, 2 two blocks per SM, 3 X operand in TMEM,
-  // 4 persistent with 32-column tiles.
-  const char* cut = getenv("MMB_BIDAF_FWD_CUT");
-  const bool two_per_sm = cut && atoi(cut) == 2;
-  if (!cut || atoi(cut) == 5) return bidaf_fwd_tc5_launch(pk, text, bias, out, q2c, bm, lse_row, lse_col, B, Lc, Lq, d, stream);
-  MMB_REQUIRE(q2c && lse_row && lse_col, MMB_ERR_INVALID, "mmb_bidaf_fwd: forward cuts 1 - 4 need q2c / lse_row / lse_col");
-  if (cut && atoi(cut) == 4) return bidaf_fwd_tc4_launch(pk, text, bias, out, q2c, bm, lse_row, lse_col, B, Lc, Lq, d, stream);
-  if (cut && atoi(cut) == 3) return bidaf_fwd_tc3_launch(pk, bias, out, q2c, bm, lse_row, lse_col, B, Lc, Lq, d, stream);
-  if (two_per_sm) return bidaf_fwd_tc2_launch(pk, bias, out, q2c, bm, lse_row, lse_col, B, Lc, Lq, d, stream);
-  // Q2C: X = modality rows, Y = text rows (S operand cw, values cp)
-  const TcArgs aq{qs, cw, cp, nullptr, c_words, bias, q2c, tp, lse_col, nullptr, trace, Lq, LqP, Lc, LcP, d};
-  // C2Q: X = text rows, Y = modality rows (S operand qs, values qp and packed T)
-  const TcArgs ac{cw, qs, qp, tp, q_words, bias, out, nullptr, lse_row, bm, trace ? trace + 256 : nullptr, Lc, LcP, Lq, LqP, d};
-  const size_t smem_q = tc_smem_bytes(2), smem_c = tc_smem_bytes(2 + (qp != qs ? 1 : 0));
-  MMB_REQUIRE(smem_c <= 227 * 1024 && smem_q <= 227 * 1024, MMB_ERR_UNSUPPORTED, "bidaf bf16 tier: %zu B of shared memory", smem_c);
-  if (getenv("MMB_BIDAF_FWD_SPLIT")) {
-    MMB_CUDA(cudaFuncSetAttribute(bidaf_tc_kernel<Q2C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q));
-    bidaf_tc_kernel<Q2C><<<dim3(LqP / TX, B), NTHREADS, smem_q, stream>>>(aq);
-    if (int rc = check_launch("bidaf_tc_kernel<Q2C>")) return rc;
-    MMB_CUDA(cudaFuncSetAttribute(bidaf_tc_kernel<C2Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
-    bidaf_tc_kernel<C2Q><<<dim3(LcP / TX, B), NTHREADS, smem_c, stream>>>(ac);
-    return check_launch("bidaf_tc_kernel<C2Q>");
-  }
-  const size_t smem = smem_q > smem_c ? smem_q : smem_c;
-  MMB_CUDA(cudaMemsetAsync(pk.ready, 0, sizeof(int) * (size_t)B, stream));
-  const char* ct = getenv("MMB_BIDAF_FWD_CTA_TIMES");
-  FusedArgs f{aq, ac, pk.ready, LqP / TX, LcP / TX, B * (LqP / TX), ct ? reinterpret_cast<long long*>(strtoull(ct, nullptr, 0)) : nullptr};
-  MMB_CUDA(cudaFuncSetAttribute(bidaf_tc_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  bidaf_tc_fused_kernel<<<B * (LqP / TX + LcP / TX), NTHREADS, smem, stream>>>(f);
-  if (int rc = check_launch("bidaf_tc_fused_kernel")) return rc;
-  return MMB_OK;
+  return bidaf_fwd_tc5_launch(pk, text, bias, out, q2c, bm, lse_row, lse_col, B, Lc, Lq, d, stream);
 }
 
 }  // namespace mmb

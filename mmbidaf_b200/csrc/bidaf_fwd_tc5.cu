@@ -726,17 +726,16 @@ int bidaf_fwd_tc5_launch(const BidafPacks& pk, const float* text, const float* b
   }
   // (pk.ready[0 .. B] -- the counters and the queue head -- are zeroed by bidaf_pack_kernel)
   const int n_items = f.n_q2c + 2 * f.n_c2q;
-  static const char* pdl_env = getenv("MMB_BIDAF_PDL");                  // 0: plain stream order (A/B switch)
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)(n_items < num_sms ? n_items : num_sms));
   cfg.blockDim = dim3(NTHREADS);
   cfg.dynamicSmemBytes = SMEM_BYTES;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
+  cudaLaunchAttribute attr[1];                                           // programmatic dependent launch (griddepcontrol.wait)
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl_env && atoi(pdl_env) == 0) ? 0 : 1;
+  cfg.numAttrs = 1;
   MMB_CUDA(cudaLaunchKernelEx(&cfg, bidaf_tc5_kernel, f));
   return check_launch("bidaf_tc5_kernel");
 }

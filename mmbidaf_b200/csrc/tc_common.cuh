@@ -116,18 +116,7 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
 }
 // D[tmem] (+)= A[smem] * B[smem], bf16 inputs, fp32 accumulate.  Executed by a converged warp, issued by its leader.
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc,
-                                          uint32_t leader) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p, q;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "setp.ne.b32 q, %5, 0;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}" ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc), "r"(leader)
-      : "memory");
-}
-// Same with the descriptors given as (low word, high word): the high word (SBO, version) is a constant and the low
+// The descriptors are given as (low word, high word): the high word (SBO, version) is a constant and the low
 // word (address >> 4 | LBO) advances by a constant per K step, so the issue loop is one integer add per operand.
 __device__ __forceinline__ void umma_bf16_lh(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
                                              uint32_t idesc, uint32_t acc, uint32_t leader) {
@@ -179,11 +168,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const float* v) {
       : "memory");
 }
 
-// Shared-memory matrix descriptor, no swizzle ("interleave"), Blackwell version field = 1.
-__device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  return (uint64_t)((addr & 0x3FFFFu) >> 4) | ((uint64_t)(lbo_bytes >> 4) << 16) | ((uint64_t)(sbo_bytes >> 4) << 32) |
-         (1ull << 46);
-}
 // Instruction descriptor: D = F32, A = B = BF16.  M = 128: accumulator row i is TMEM lane i.  M = 64: row i is lane
 // (i / 16) * 32 + i % 16 -- sixteen rows in the low half of each 32-lane quarter (tools/micro/umma_m64_layout.cu).
 constexpr uint32_t idesc_bf16(int n, int b_mn_major, int m = 128) {
@@ -208,8 +192,7 @@ struct BidafPacks {
   __nv_bfloat16 *qs, *qp;            // modality: S operand (dropped, term chunk) / plain values (== qs without dropout)
   __nv_bfloat16* tp;                 // packed T = s2^T c
   unsigned long long *c_words, *q_words;   // (B, LP/64, 2): [in-range bits, un-masked bits] per 64 rows
-  int* ready;                        // (B) Q2C -> C2Q dependency counters of the fused launch, then the work-queue head of cut 4
-  long long* trace;                  // 2 x 256 clock stamps (debugging aid), the last 4096 bytes
+  int* ready;                        // (B) Q2C -> C2Q dependency counters of the main launch, then its work-queue head
   int LcP, LqP;
   size_t c_pack, q_pack, bytes;
 };
@@ -234,9 +217,7 @@ inline BidafPacks bidaf_packs(void* workspace, int B, int Lc, int Lq, bool modal
   p.q_words = p.c_words + (size_t)B * (p.LcP / 64) * 2;
   const size_t used = ((size_t)(next - ws) + 16 * (size_t)B * (p.LcP / 64 + p.LqP / 64) + 255) / 256 * 256;
   p.ready = reinterpret_cast<int*>(ws + used);
-  const size_t used2 = used + ((size_t)(B + 1) * 4 + 255) / 256 * 256;
-  p.trace = reinterpret_cast<long long*>(ws + used2);
-  p.bytes = used2 + 4096;
+  p.bytes = used + ((size_t)(B + 1) * 4 + 255) / 256 * 256;
   return p;
 }
 

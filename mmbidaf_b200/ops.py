@@ -37,7 +37,7 @@ def bidaf_fwd(text: torch.Tensor, modality: torch.Tensor, text_mask: torch.Tenso
               keep_scale: float = 1.0, precision: int = PREC_FP32, save: bool = False, aux: bool = True):
     """Fused BiDAF forward (attention.py:37-75).  Returns (out (B,Lc,4d), q2c (B,Lq,d), lse_row (B,Lc),
     lse_col (B,Lq)); with ``save`` also (bm (B,Lc,d), workspace) -- everything the backward pass needs.  ``aux=False`` (bf16 tier,
-    default kernel cut, no ``save``): only ``out`` is computed and written (inference: the reference's forward returns nothing else);
+    no ``save``): only ``out`` is computed and written (inference: the reference's forward returns nothing else);
     the other three results are None."""
     L = _lib.lib()
     assert text.dtype == torch.float32 and modality.dtype == torch.float32
@@ -48,7 +48,7 @@ def bidaf_fwd(text: torch.Tensor, modality: torch.Tensor, text_mask: torch.Tenso
     kt, km = _u8(keep_text), _u8(keep_modality)
     wt, wm, wc = (w.detach().reshape(-1).contiguous() for w in (w_text, w_modality, w_cross))
     out = torch.empty(B, Lc, 4 * d, device=text.device, dtype=torch.float32)
-    want_aux = aux or save or precision != PREC_BF16 or os.environ.get("MMB_BIDAF_FWD_CUT", "5") != "5"
+    want_aux = aux or save or precision != PREC_BF16
     q2c = torch.empty(B, Lq, d, device=text.device, dtype=torch.float32) if want_aux else None
     bm = torch.empty(B, Lc, d, device=text.device, dtype=torch.float32) if save else None
     lse_row = torch.empty(B, Lc, device=text.device, dtype=torch.float32) if want_aux else None
@@ -60,8 +60,6 @@ def bidaf_fwd(text: torch.Tensor, modality: torch.Tensor, text_mask: torch.Tenso
                                p(kt), p(km), float(keep_scale), p(out), p(q2c), p(bm), p(lse_row), p(lse_col), p(ws),
                                B, Lc, Lq, d, int(precision), _lib.stream()), "mmb_bidaf_fwd")
     _count(2)          # fp32: two pass launches; bf16: pack + one fused tensor-core launch
-    if ws is not None and os.environ.get("MMB_BIDAF_FWD_TRACE"):      # debugging aid: clock stamps
-        bidaf_fwd.last_trace = ws[-4096:].view(torch.int64).view(2, 256)
     if save:
         return out, q2c, lse_row, lse_col, bm, ws
     return out, q2c, lse_row, lse_col

@@ -1,5 +1,5 @@
-"""Event log of CTA 0 of the persistent forward (cut 5, csrc/bidaf_fwd_tc5.cu), debugging aid: per role a list of (code, clock64).
-    MMB_BIDAF_FWD_CUT=5 python tools/bidaf_fwd_events.py [B Lc Lq]
+"""Event log of CTA 0 of the persistent forward (csrc/bidaf_fwd_tc5.cu), debugging aid: per role a list of (code, clock64).
+    python tools/bidaf_fwd_events.py [B Lc Lq]
 MMA warp: kind (0 Q, 1 A, 2 B) pass taken, 10 X tile there, 200+t Y tile there, 300+t S buffer free -> S(t) issued, 400+t P(t) there -> P V(t) issued.
 Soft-max warp 0: 200+t S(t) there, 300+t S(t) in registers, 400+t P computed, 500+t P buffer free, 600+t P(t) written.
 TMA warp: kind published, 100+t slot free -> Y tile t requested."""
@@ -14,7 +14,6 @@ d = 200
 dev = "cuda"
 ev = torch.zeros(4, 2048, dtype=torch.int64, device=dev)
 os.environ["MMB_BIDAF_FWD_EV_TRACE"] = str(ev.data_ptr())
-os.environ.setdefault("MMB_BIDAF_FWD_CUT", "5")
 from mmbidaf_b200 import ops  # noqa: E402
 
 gen = torch.Generator().manual_seed(224)

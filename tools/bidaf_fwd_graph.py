@@ -1,7 +1,7 @@
-"""Graph-replayed timing of the fused BiDAF forward (bf16 tier) at BASELINE config 2 for one cut (MMB_BIDAF_FWD_CUT), plus a
-check of its output against the fp32 tier on the same inputs.  The four calls over four rotating input sets are captured into one
-CUDA graph (a call from Python costs ~40 us of host time, more than the kernels).
-    MMB_BIDAF_FWD_CUT=5 python tools/bidaf_fwd_graph.py [--shape B Lc Lq] [--rounds 20]
+"""Graph-replayed timing of the fused BiDAF forward (bf16 tier) at BASELINE config 2, plus a check of its output against the
+fp32 tier on the same inputs.  The four calls over four rotating input sets are captured into one CUDA graph (a call from Python
+costs ~40 us of host time, more than the kernels).
+    python tools/bidaf_fwd_graph.py [--shape B Lc Lq] [--rounds 20]
 """
 import argparse
 import os
@@ -60,5 +60,5 @@ e1.record()
 torch.cuda.synchronize()
 t = e0.elapsed_time(e1) / a.rounds / 4 * 1e3
 algo = 4 * B * (Lc * d + Lq * d + Lc * 4 * d) + B * (Lc + Lq)
-print(f"cut={os.environ.get('MMB_BIDAF_FWD_CUT', 'default')} B={B} Lc={Lc} Lq={Lq}: {t:.1f} us/forward (graph replay), "
+print(f"B={B} Lc={Lc} Lq={Lq}: {t:.1f} us/forward (graph replay), "
       f"{algo / t / 1e3:.1f} GB/s algorithmic ({algo / t / 1e3 / 6553.3 * 100:.1f}% of 6553 GB/s)")

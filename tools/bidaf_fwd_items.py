@@ -1,6 +1,7 @@
-"""Per-item timeline of the persistent forward (cut 4, csrc/bidaf_fwd_tc4.cu), debugging aid.
-    MMB_BIDAF_FWD_CUT=4 python tools/bidaf_fwd_items.py [B Lc Lq]
-Per item: [0] published by the scheduler, [1] epilogue start (accumulator complete), [2] epilogue end, [3] kind, [4] SM, [5] tiles."""
+"""Per-item timeline of the persistent forward (csrc/bidaf_fwd_tc5.cu), debugging aid.
+    python tools/bidaf_fwd_items.py [B Lc Lq]
+Per item: [0] published by the scheduler, [1] epilogue start (accumulator complete), [2] epilogue end, [3] kind, [4] SM, [5] tiles,
+[7] X tile in shared memory (the MMA warp starts the item)."""
 import os
 import sys
 
@@ -13,8 +14,7 @@ dev = "cuda"
 nq, nc = (Lq + 127) // 128, (Lc + 127) // 128
 n_items = B * (nq + 2 * nc)
 trace = torch.zeros(n_items, 8, dtype=torch.int64, device=dev)
-os.environ["MMB_BIDAF_FWD_ITEM_TRACE"] = str(trace.data_ptr())       # read once, at the first cut-4 launch
-os.environ.setdefault("MMB_BIDAF_FWD_CUT", "4")
+os.environ["MMB_BIDAF_FWD_ITEM_TRACE"] = str(trace.data_ptr())       # read once, at the first launch
 from mmbidaf_b200 import ops  # noqa: E402
 
 gen = torch.Generator().manual_seed(224)
@@ -51,4 +51,4 @@ for smid in set(t[:, 4].tolist()):
         per_tile.append(float(x[i, 1] - x[i - 1, 1]) / max(int(x[i, 5]), 1))
 if per_tile:
     pt = torch.tensor(per_tile)
-    print(f"accumulator-complete to accumulator-complete per tile: mean {pt.mean():.0f} ns, median {pt.median():.0f} ns (32-column tiles)")
+    print(f"accumulator-complete to accumulator-complete per tile: mean {pt.mean():.0f} ns, median {pt.median():.0f} ns (64-column tiles)")

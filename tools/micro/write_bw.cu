@@ -40,7 +40,8 @@ __global__ void __launch_bounds__(256) k_bulk(float* out, long long nrows, int n
     asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
 }
-// mode 4 / 5: the store pattern of the persistent forward's epilogue (csrc/bidaf_fwd_tc4.cu): a warp owns 32 rows and sweeps them in
+// mode 4 / 5: the store pattern of the epilogue of bidaf_tc4_kernel, the persistent forward with 32-column tiles that preceded
+// bidaf_tc5_kernel: a warp owns 32 rows and sweeps them in
 // 32-column chunks; one instruction writes 4 rows x 128 bytes (8 lanes x float4 per row); default (4) or .cs (5) stores.
 template <int CS>
 __global__ void __launch_bounds__(256) k_epi(float* out, long long nrows, int nblk) {
