@@ -205,6 +205,32 @@ MMB_API int mmb_decoder_greedy_fused(const float* proj_a, const float* proj_i, c
                                      const uint8_t* mask, const long long* target, float* probs, long long* argmax, float* loss_terms,
                                      int B, int Lt, int D, int H, int E, int M, int S, int T, mmb_stream_t stream);
 /*
+ * Beam summary roll-out: the decode loop of models.py:156-199 in eval mode with K hypotheses per video instead of one, all S steps
+ * in ONE launch of the same cluster kernel (one cluster per video holds every slot); the beam alternative to evaluate.py:185-202's
+ * greedy pick.  This is the project's own beam rule; it does not claim parity with the reference's evaluate.py::beam_search.
+ *   Slots: K per video, each live, finished (its last token was the EOS row text_len[b] - 1) or empty.  Before step 0 slot 0 is live
+ *   with score 0 and the greedy start state (h0, zero cell, coverage and input row), the others empty with score -inf.
+ *   Step: a live slot runs the decoder step from its own state -- bit for bit what mmb_decoder_step_fused_fwd computes from it -- and
+ *   offers (slot, m) for every m with p[m] > 0, scored score + logf(p[m]) in fp32; a finished slot offers one carry (slot, EOS) with
+ *   its score and step probability 1; empty slots offer nothing.  The candidates rank by score descending, then step probability
+ *   descending, then parent slot ascending, then sentence ascending; the first K become the new slots 0..K-1, the rest stay empty.
+ *   No length normalisation.  With K = 1 this is the greedy roll-out.
+ *   text_len (B) int32   tokens / parents / scores (B,S,K) int64 / int32 / fp32: each new slot's token, previous slot and score
+ *                        (-1, -1, -inf for an empty slot)
+ *   probs (B,S,K,M)      the distribution slot j's parent produced at step s (zero for carries and empty slots)
+ *   best (B,S) int64     the tokens of slot 0's path after the last step;  path (B,S) int32: the slot of that path at every step
+ * 1 <= K <= 8.  Shapes as mmb_decoder_greedy_fused; the per-slot state lives in shared memory, so a width whose state does not fit
+ * beside the step's arrays returns MMB_ERR_UNSUPPORTED with the byte count.
+ */
+MMB_API int mmb_decoder_beam_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                   const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                   const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                   const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                   const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                   const uint8_t* mask, const int32_t* text_len, long long* tokens, int32_t* parents, float* scores,
+                                   float* probs, long long* best, int32_t* path, int B, int Lt, int D, int H, int E, int M, int K,
+                                   int S, mmb_stream_t stream);
+/*
  * Greedy sentence selection (evaluate.py:185-202, decode.greedy_search) on the device.  Per video, in step order over argmax (B,S):
  * the EOS row text_len[b] - 1 ends the summary, an index past it is skipped, any other is kept (repeats too).
  *   sel (B,S) int32 = the kept indices, then -1;  count (B) int32 = how many were kept.

@@ -217,8 +217,44 @@ struct GreedyArgs {
   int steps, T;                                             // roll-out length S; row stride of the target (B, T), T >= S
 };
 
-template <bool kGreedy>
-__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g) {
+// The beam roll-out (mmb_decoder_beam_fused): the greedy roll-out with K slots per video (include/mmbidaf_b200.h states the rule).  The
+// live slots of a step run the stages one after another, each from its own state, so every per-hypothesis value is the step kernel's to
+// the bit; what the slots hold between the steps sits in shared memory behind the base arrays (`off`): the table (score, last token,
+// status), h / cell / coverage of every slot (this step's inputs and outputs), this rank's share of every slot's distribution and the
+// selection exchange.  Each rank ranks its own (slot, sentence) candidates, keeps its best K and publishes them to every rank through
+// DSMEM; every rank merges the CL x K entries and the carries of the finished slots in the same order, so all agree on the new table.
+constexpr int MAXK = 8;
+struct BeamArgs {
+  const int* text_len;                                      // (B): the EOS row of video b is text_len[b] - 1
+  long long* tokens;                                        // (B, S, K)
+  int* parents;                                             // (B, S, K)
+  float *scores, *probs;                                    // (B, S, K), (B, S, K, M)
+  long long* best;                                          // (B, S): the tokens of slot 0's path after the last step
+  int* path;                                                // (B, S): the slot of that path at every step
+  int K, off;                                               // width; float offset of the beam region in dynamic shared memory
+};
+enum : int { kEmpty = 0, kLive = 1, kDone = 2 };
+
+// the ranking of the candidates: score descending, then step probability descending, then parent slot, then sentence ascending
+__device__ __forceinline__ bool cand_better(float sa, float pa, int ka, int ma, float sb, float pb, int kb, int mb) {
+  if (sa != sb) return sa > sb;
+  if (pa != pb) return pa > pb;
+  if (ka != kb) return ka < kb;
+  return ma < mb;
+}
+// the best candidate of the warp, in every lane
+__device__ __forceinline__ void cand_warp_best(float& s, float& p, int& k, int& m) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float s2 = __shfl_xor_sync(0xffffffffu, s, o), p2 = __shfl_xor_sync(0xffffffffu, p, o);
+    const int k2 = __shfl_xor_sync(0xffffffffu, k, o), m2 = __shfl_xor_sync(0xffffffffu, m, o);
+    if (cand_better(s2, p2, k2, m2, s, p, k, m)) { s = s2; p = p2; k = k2; m = m2; }
+  }
+}
+
+// kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one
+template <bool kGreedy, bool kBeam = false>
+__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int b = blockIdx.x / CL;
@@ -266,13 +302,53 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   const int S = kGreedy ? g.steps : 1;
   float cell_own = 0.f;                    // greedy: the cell of hidden unit j0 + tid (stage D), carried between the steps
   int pick = 0;                            // greedy: the previous step's arg-max
+  // beam: the region behind the base arrays (beam_floats)
+  const int KW = kBeam ? bm.K : 1;
+  const int ldh = up4(H), ldc = up4(split4(H, CL)), ldv = up4(a.chunk), ldp = up4((M + CL - 1) / CL);
+  float* const bs_score = smem + bm.off;                                 // [MAXK] the table: score,
+  int* const bs_tok = reinterpret_cast<int*>(bs_score + MAXK);           // [MAXK]   last token,
+  int* const bs_stat = bs_tok + MAXK;                                    // [MAXK]   status
+  float* const nt_score = bs_score + 3 * MAXK;                           // [MAXK] the next table: score,
+  int* const nt_tok = reinterpret_cast<int*>(nt_score + MAXK);           // [MAXK]   token,
+  int* const nt_par = nt_tok + MAXK;                                     // [MAXK]   parent slot (-1: empty),
+  int* const nt_kind = nt_par + MAXK;                                    // [MAXK]   status
+  float* const s_cand = nt_score + 4 * MAXK;    // [MAXC][MAXK][4] every rank's best K (score, p, parent, sentence), written remotely
+  float* const s_wred = s_cand + MAXC * MAXK * 4;                        // [NW][4] per-warp bests
+  float* const s_loc = s_wred + NW * 4;                                  // [MAXK][4] this rank's best K
+  float* const s_bh = s_loc + MAXK * 4;                                  // [K][ldh] h of every slot (the step's input)
+  float* const s_bhn = s_bh + KW * ldh;                                  // [K][ldh] h' of every slot
+  float* const s_bc = s_bhn + KW * ldh;                                  // [K][ldc] cell of this rank's hidden units, in
+  float* const s_bcn = s_bc + KW * ldc;                                  //          and out
+  float* const s_bcv = s_bcn + KW * ldc;                                 // [K][ldv] coverage of this rank's text rows, in
+  float* const s_bcvn = s_bcv + KW * ldv;                                //          and out
+  float* const s_bp = s_bcvn + KW * ldv;                                 // [K][ldp] the distribution over this rank's sentences
+  const int eos = kBeam ? bm.text_len[b] - 1 : 0;
+  int runs = 0;                                                          // beam: slot runs so far (row-stage barrier phases)
+  if constexpr (kBeam) {                   // before step 0: slot 0 live with score 0, h0 and a zero cell and coverage; the rest empty
+    if (tid < MAXK) {
+      bs_score[tid] = tid == 0 ? 0.f : -INFINITY;
+      bs_tok[tid] = -1;
+      bs_stat[tid] = tid == 0 ? kLive : kEmpty;
+    }
+    for (int i = tid; i < H; i += NT) s_bh[i] = g.h0[(size_t)b * H + i];
+    for (int i = tid; i < ldc; i += NT) s_bc[i] = 0.f;
+    for (int i = tid; i < n; i += NT) s_bcv[i] = 0.f;
+    __syncthreads();
+  }
   for (int s = 0; s < S; ++s) {
-  const uint32_t parity = kGreedy ? (uint32_t)(s & 1) : 0u;      // each row-stage barrier completes once per step
+  for (int slot = 0; slot < KW; ++slot) {  // beam: the live slots one after another; otherwise once
+  if (kBeam && bs_stat[slot] != kLive) continue;
+  const uint32_t parity = kBeam ? (uint32_t)(runs & 1) : kGreedy ? (uint32_t)(s & 1) : 0u;   // each row-stage barrier completes once per run
   // ---- stage 0: this video's step inputs -----------------------------------------------------------------------------------
   if constexpr (!kGreedy) {
     for (int i = tid; i < n; i += NT) s_cov[i] = a.cov[(size_t)b * Lt + t0 + i];      // (read per row by the energies: not a global load there)
     for (int i = tid; i < H; i += NT) s_x[D + E + i] = a.h[(size_t)b * H + i];
     for (int i = tid; i < E; i += NT) s_x[D + i] = a.sent[(size_t)b * E + i];
+  } else if constexpr (kBeam) {
+    for (int i = tid; i < n; i += NT) s_cov[i] = s_bcv[slot * ldv + i];
+    for (int i = tid; i < H; i += NT) s_x[D + E + i] = s_bh[slot * ldh + i];
+    const float* row = g.emb_text + ((size_t)b * Lt + min(max(bs_tok[slot], 0), Lt - 1)) * E;
+    for (int i = tid; i < E; i += NT) s_x[D + i] = s == 0 ? 0.f : row[i];
   } else {
     if (s == 0)
       for (int i = tid; i < n; i += NT) s_cov[i] = 0.f;
@@ -450,7 +526,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     if constexpr (kGreedy) {
       // every read of the enc rows is behind the barrier: the buffers take the NEXT step's proj rows, which then arrive while
       // stages C - E and the next stage A run
-      if (staged && tid == 0 && n > 0 && s + 1 < S) {
+      // (beam: whether another run follows is known only after the selection -- the last copy is waited for before the exit)
+      if (staged && tid == 0 && n > 0 && (kBeam || s + 1 < S)) {
         tc::fence_proxy_async();
         tc::mbar_expect_tx(bar_proj, 2 * stage_bytes, 1);
         tc::tma_bulk_g2s(tc::smem_u32(s_st0), a.proj_a + ((size_t)b * Lt + t0) * D, stage_bytes, bar_proj, 1);
@@ -547,7 +624,11 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         a.alpha[((size_t)b * 2 + 1) * Lt + t] = a2;
       }
       const float att = a1 * beta1 + a2 * beta2;                 // bmm([a1 a2], beta), attention.py:167
-      if constexpr (kGreedy) {
+      if constexpr (kBeam) {
+        const float cnew = s_cov[i] + att;
+        s_bcvn[slot * ldv + i] = cnew;
+        closs += fminf(att, cnew);
+      } else if constexpr (kGreedy) {
         const float cnew = s_cov[i] + att;                       // (the energies of this step have read s_cov: barriers since)
         s_cov[i] = cnew;
         closs += fminf(att, cnew);
@@ -581,9 +662,11 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       const int j = j0 + tid;
       const float gi = gate_act(s_g[tid], 1.f), gf = gate_act(s_g[(per + 1) + tid], 1.f), gg = tanh_fast(s_g[2 * (per + 1) + tid]),
                   go = gate_act(s_g[3 * (per + 1) + tid], 1.f);
-      const float c = fmaf(gf, kGreedy ? cell_own : a.cell[(size_t)b * H + j], gi * gg);
+      const float c = fmaf(gf, kBeam ? s_bc[slot * ldc + tid] : kGreedy ? cell_own : a.cell[(size_t)b * H + j], gi * gg);
       const float hn = go * tanh_fast(c);
-      if constexpr (kGreedy) {
+      if constexpr (kBeam) {
+        s_bcn[slot * ldc + tid] = c;
+      } else if constexpr (kGreedy) {
         cell_own = c;
       } else {
         a.cell_out[(size_t)b * H + j] = c;
@@ -597,6 +680,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   DEC_STAMP(12);
   cluster.sync();
   DEC_STAMP(13);
+  if constexpr (kBeam)                     // (s_hn is written again only behind the cluster barriers of the next run)
+    for (int i = tid; i < H; i += NT) s_bhn[slot * ldh + i] = s_hn[i];
   // greedy: the probabilities / arg-max of step s go to row (b, s) of (B, S, M) / (B, S); the loss terms (S, 2, B) to row s
   const size_t prow = kGreedy ? (size_t)b * S + s : (size_t)b;
   const int lrow = kGreedy ? s * 2 * a.B + b : b;
@@ -641,11 +726,12 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     const int tg = a.target ? (int)a.target[kGreedy ? b * g.T + s : b] : -1;
     for (int m = m0 + tid; m < m1; m += NT) {
       const float p = expf(lg[m - m0] - gmx) * inv;
-      a.probs[prow * M + m] = p;
+      if constexpr (kBeam) s_bp[slot * ldp + m - m0] = p;
+      else a.probs[prow * M + m] = p;
       if (p > best) { best = p; best_i = m; }
       if (m == tg && a.nll) a.nll[lrow] = -logf(p + 1e-12f);      // models.py:168-170
     }
-    if (kGreedy || a.argmax) {                                    // first maximal index, as torch.max(dim) documents
+    if (!kBeam && (kGreedy || a.argmax)) {                                  // first maximal index, as torch.max(dim) documents
       const float bbest = block_max(best, s_red);
       int cand = best == bbest ? best_i : M;
 #pragma unroll
@@ -684,7 +770,134 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       }
     }
   }
+  if constexpr (kBeam) ++runs;
+  }  // slots
+  if constexpr (kBeam) {
+    // ---- selection: the new table from the live slots' candidates and the finished slots' carries ---------------------------------
+    constexpr int kNone = 0x7fffffff;
+    const int per = (M + CL - 1) / CL, m0 = min(M, R * per), m1 = min(M, m0 + per), nm = m1 - m0;
+    bool any_live = false;
+    for (int k = 0; k < KW; ++k) any_live = any_live || bs_stat[k] == kLive;
+    __syncthreads();                                             // s_bp of the last run
+    if (any_live) {
+      // this rank's best K of its (live slot, sentence) candidates, one block-wide pick per round; each pick ranks below the last
+      float ps = INFINITY, pp = INFINITY;
+      int pk = -1, pm = -1;
+      for (int r = 0; r < KW; ++r) {
+        float cs = -INFINITY, cp = -1.f;
+        int ck = kNone, cm = kNone;
+        for (int c = tid; c < KW * nm; c += NT) {
+          const int k = c / nm, m = m0 + (c - k * nm);
+          if (bs_stat[k] != kLive) continue;
+          const float p = s_bp[k * ldp + m - m0];
+          if (!(p > 0.f)) continue;                              // masked sentences: exactly 0
+          const float sc = bs_score[k] + logf(p);
+          if (cand_better(ps, pp, pk, pm, sc, p, k, m) && cand_better(sc, p, k, m, cs, cp, ck, cm)) { cs = sc; cp = p; ck = k; cm = m; }
+        }
+        cand_warp_best(cs, cp, ck, cm);
+        if (lane == 0) {
+          s_wred[warp * 4 + 0] = cs; s_wred[warp * 4 + 1] = cp;
+          s_wred[warp * 4 + 2] = __int_as_float(ck); s_wred[warp * 4 + 3] = __int_as_float(cm);
+        }
+        __syncthreads();
+        if (warp == 0) {
+          float ws = -INFINITY, wp = -1.f;
+          int wk = kNone, wm = kNone;
+          if (lane < NW) {
+            ws = s_wred[lane * 4 + 0]; wp = s_wred[lane * 4 + 1];
+            wk = __float_as_int(s_wred[lane * 4 + 2]); wm = __float_as_int(s_wred[lane * 4 + 3]);
+          }
+          cand_warp_best(ws, wp, wk, wm);
+          if (lane == 0) {
+            s_loc[r * 4 + 0] = ws; s_loc[r * 4 + 1] = wp;
+            s_loc[r * 4 + 2] = __int_as_float(wk); s_loc[r * 4 + 3] = __int_as_float(wm);
+          }
+        }
+        __syncthreads();
+        ps = s_loc[r * 4 + 0]; pp = s_loc[r * 4 + 1];
+        pk = __float_as_int(s_loc[r * 4 + 2]); pm = __float_as_int(s_loc[r * 4 + 3]);
+      }
+      for (int i = tid; i < CL * KW * 4; i += NT) {              // -> slot R of every rank
+        const int q = i / (KW * 4), e = i - q * KW * 4;
+        cluster.map_shared_rank(s_cand, q)[R * MAXK * 4 + e] = s_loc[e];
+      }
+      cluster.sync();
+    }
+    // every rank merges the same entries in the same order: the ranks' best K (none when no slot is live), then the carries
+    if (warp == 0) {
+      const int npub = any_live ? CL * KW : 0, tot = npub + KW;
+      float ps = INFINITY, pp = INFINITY;
+      int pk = -1, pm = -1;
+      for (int j = 0; j < KW; ++j) {
+        float cs = -INFINITY, cp = -1.f;
+        int ck = kNone, cm = kNone;
+        for (int i = lane; i < tot; i += 32) {
+          float es, ep;
+          int ek, em;
+          if (i < npub) {
+            const float* e = s_cand + ((i / KW) * MAXK + i % KW) * 4;
+            es = e[0]; ep = e[1]; ek = __float_as_int(e[2]); em = __float_as_int(e[3]);
+          } else {
+            const int k = i - npub;
+            if (bs_stat[k] != kDone) continue;
+            es = bs_score[k]; ep = 1.f; ek = k; em = eos;        // a finished slot carries its hypothesis with probability 1
+          }
+          if (ek == kNone) continue;
+          if (cand_better(ps, pp, pk, pm, es, ep, ek, em) && cand_better(es, ep, ek, em, cs, cp, ck, cm)) { cs = es; cp = ep; ck = ek; cm = em; }
+        }
+        cand_warp_best(cs, cp, ck, cm);
+        if (lane == 0) {
+          // kind: 0 empty, 1 live, 2 finished by this step's EOS pick, 3 carried
+          const bool none = ck == kNone;
+          nt_score[j] = none ? -INFINITY : cs;
+          nt_tok[j] = none ? -1 : cm;
+          nt_par[j] = none ? -1 : ck;
+          nt_kind[j] = none ? 0 : bs_stat[ck] == kDone ? 3 : cm == eos ? 2 : 1;
+        }
+        ps = cs; pp = cp; pk = ck; pm = cm;
+      }
+    }
+    __syncthreads();
+    // outputs of step s; the state of the new live slots gathered from their parents' step outputs; the new table
+    const size_t row = ((size_t)b * S + s) * KW;
+    if (R == 0 && tid == 0)
+      for (int j = 0; j < KW; ++j) {
+        bm.tokens[row + j] = nt_tok[j];
+        bm.parents[row + j] = nt_par[j];
+        bm.scores[row + j] = nt_score[j];
+      }
+    for (int i = tid; i < KW * nm; i += NT) {                    // the row the parent produced (zero for carries and empty slots)
+      const int j = i / nm, m = m0 + (i - j * nm), kd = nt_kind[j];
+      bm.probs[(row + j) * M + m] = (kd == 1 || kd == 2) ? s_bp[nt_par[j] * ldp + m - m0] : 0.f;
+    }
+    for (int j = 0; j < KW; ++j) {
+      if (nt_kind[j] != 1) continue;                             // (uniform) only live slots run again
+      const int q = nt_par[j];
+      for (int i = tid; i < H; i += NT) s_bh[j * ldh + i] = s_bhn[q * ldh + i];
+      for (int i = tid; i < ldc; i += NT) s_bc[j * ldc + i] = s_bcn[q * ldc + i];
+      for (int i = tid; i < n; i += NT) s_bcv[j * ldv + i] = s_bcvn[q * ldv + i];
+    }
+    if (tid < KW) {
+      const int kd = nt_kind[tid];
+      bs_score[tid] = nt_score[tid];
+      bs_tok[tid] = nt_tok[tid];
+      bs_stat[tid] = kd == 1 ? kLive : kd == 0 ? kEmpty : kDone;
+    }
+    __syncthreads();
+  }
   }  // steps (the loop body keeps the step kernel's indentation)
+  if constexpr (kBeam) {
+    if (staged && tid == 0 && n > 0) tc::mbar_wait(bar_proj, (uint32_t)(runs & 1));   // the proj rows copied after the last run
+    if (R == 0 && tid == 0) {                                    // backtrack the best hypothesis: slot 0 after the last step
+      int j = 0;
+      for (int s = S - 1; s >= 0; --s) {
+        const size_t row = ((size_t)b * S + s) * KW;
+        bm.path[(size_t)b * S + s] = j;
+        bm.best[(size_t)b * S + s] = j >= 0 ? bm.tokens[row + j] : -1;
+        j = j >= 0 ? bm.parents[row + j] : -1;
+      }
+    }
+  }
   DEC_STAMP(16);
   // (No barrier before the exit: every rank's LAST store into another rank's shared memory -- the soft-max statistics or the arg-max
   // candidates -- lies before a cluster barrier it has passed, so nothing can still be written into a rank that leaves here.  In the
@@ -693,9 +906,13 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   DEC_STAMP(17);
 }
 
-__global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) { dec_fused_body<false>(a, GreedyArgs{}); }
+__global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) { dec_fused_body<false>(a, GreedyArgs{}, BeamArgs{}); }
 
-__global__ void __launch_bounds__(NT) dec_greedy_fused_kernel(const FusedArgs a, const GreedyArgs g) { dec_fused_body<true>(a, g); }
+__global__ void __launch_bounds__(NT) dec_greedy_fused_kernel(const FusedArgs a, const GreedyArgs g) { dec_fused_body<true>(a, g, BeamArgs{}); }
+
+__global__ void __launch_bounds__(NT) dec_beam_fused_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm) {
+  dec_fused_body<true, true>(a, g, bm);
+}
 
 }  // namespace
 
@@ -1229,9 +1446,16 @@ static size_t fused_smem_bytes(int Lt, int D, int H, int E, int M, int CL, int* 
   return floats * sizeof(float) + 64;
 }
 
+// floats of the beam region (see dec_fused_body): the tables, the selection exchange and K slots of state
+static size_t beam_floats(int K, int CL, int chunk, int H, int M) {
+  auto up4 = [](size_t v) { return (v + 3) & ~(size_t)3; };
+  const size_t per_slot = 2 * (up4(H) + up4(split4(H, CL)) + up4(chunk)) + up4((M + CL - 1) / CL);
+  return 7 * MAXK + MAXC * MAXK * 4 + NW * 4 + MAXK * 4 + (size_t)K * per_slot;
+}
+
 // Shape checks, cluster size, shared memory and row stage of the forward cluster kernels, then the launch: `g` null launches one step
-// (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel).
-static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream) {
+// (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel), or with `bm` the beam roll-out (dec_beam_fused_kernel).
+static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
@@ -1240,6 +1464,12 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   const int CL = (long long)B * 4 * 2 <= 160 ? 8 : 4;
   size_t smem = fused_smem_bytes(Lt, D, H, E, M, CL, &a.chunk);
   MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "%s: %zu B of shared memory (Lt=%d)", who, smem, Lt);
+  if (bm) {                                // the beam region behind the base arrays; the row stage follows if it still fits
+    bm->off = (int)((smem + 15) / 16 * 4);
+    smem = ((size_t)bm->off + beam_floats(bm->K, CL, a.chunk, H, M)) * 4 + 64;
+    MMB_REQUIRE(smem <= 227 * 1024, MMB_ERR_UNSUPPORTED, "%s: width %d needs %zu B of shared memory per CTA, more than 232448 (B=%d Lt=%d M=%d)",
+                who, bm->K, smem, B, Lt, M);
+  }
   {
     // the row stage (see the kernel): two buffers of chunk x D floats behind two mbarriers, when they fit and bulk copies apply
     // (16-byte row granularity).  MMB_DEC_STAGE=0 turns it off (A/B measurements, cross-check in tests/test_decoder_gpu.py).
@@ -1253,11 +1483,13 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[2] = {0, 0};
-  if (smem > smem_set[g != nullptr]) {
-    if (g) MMB_CUDA(cudaFuncSetAttribute(dec_greedy_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  static size_t smem_set[3] = {0, 0, 0};
+  const int which = bm ? 2 : g != nullptr;
+  if (smem > smem_set[which]) {
+    if (bm) MMB_CUDA(cudaFuncSetAttribute(dec_beam_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    else if (g) MMB_CUDA(cudaFuncSetAttribute(dec_greedy_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     else MMB_CUDA(cudaFuncSetAttribute(dec_step_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    smem_set[g != nullptr] = smem;
+    smem_set[which] = smem;
   }
   static const char* trace_env = getenv("MMB_DEC_TRACE");
   static bool trace_set = false;
@@ -1278,6 +1510,10 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (bm) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_fused_kernel, a, *g, *bm));
+    return check_launch("dec_beam_fused_kernel");
+  }
   if (g) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_greedy_fused_kernel, a, *g));
     return check_launch("dec_greedy_fused_kernel");
@@ -1330,6 +1566,28 @@ extern "C" int mmb_decoder_greedy_fused(const float* proj_a, const float* proj_i
               nullptr, B, Lt, D, H, E, M, 0, 0};
   const GreedyArgs g{emb_text, h0, S, target ? T : 0};
   return launch_fused(a, &g, "mmb_decoder_greedy_fused", stream);
+}
+
+extern "C" int mmb_decoder_beam_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                      const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                      const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                      const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                      const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                      const uint8_t* mask, const int* text_len, long long* tokens, int* parents, float* scores,
+                                      float* probs, long long* best, int* path, int B, int Lt, int D, int H, int E, int M, int K,
+                                      int S, mmb_stream_t stream) {
+  using namespace mmb;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && text_len && tokens && parents &&
+                  scores && probs && best && path,
+              MMB_ERR_INVALID, "mmb_decoder_beam_fused: null pointer");
+  MMB_REQUIRE(K >= 1 && K <= MAXK && S > 0, MMB_ERR_INVALID, "mmb_decoder_beam_fused: width K=%d (1..%d), S=%d", K, MAXK, S);
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  BeamArgs bm{text_len, tokens, parents, scores, probs, best, path, K, 0};
+  return launch_fused(a, &g, "mmb_decoder_beam_fused", stream, &bm);
 }
 
 extern "C" int mmb_decoder_bwd_head(const float* probs, const float* d_probs, const long long* target, const float* g_nll,

@@ -243,6 +243,21 @@ class MultimodalAttentionDecoder(nn.Module):
                 terms.append(lossvec)
             return torch.stack(probs, 1), torch.stack(picks, 1), (torch.stack(terms) if tgt is not None else None)
 
+    def beam(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, width):
+        """The beam decode of ``steps`` steps in eval mode with ``width`` (1..8) hypotheses per video, as ONE launch of the cluster
+        kernel whatever ``ops.decoder_cut`` says (there is no chunk-cut beam); the rule is documented at mmb_decoder_beam_fused in
+        include/mmbidaf_b200.h.  Same start as :meth:`greedy`; ``text_len`` (B) int32 gives each video's EOS row (text_len - 1).
+        No autograd.  Returns ``ops.decoder_beam_fwd``'s (tokens, parents, scores, probs, best, path)."""
+        if not enc_a.is_cuda:
+            raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
+        if self.num_layers != 1:
+            raise RuntimeError("MultimodalAttentionDecoder: only num_layers=1 is supported (the reference model uses 1)")
+        with torch.no_grad():
+            seq = self._sequence(enc_a, enc_i)["seq"]
+            B = seq.B
+            return ops.decoder_beam_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
+                                        text_len.to(torch.int32).contiguous(), steps, width)
+
     def step(self, sent_embed, decoder_hidden, decoder_cell_state, text_audio_enc_out, text_img_enc_out, coverage_vec,
              mask, target=None):
         """``forward`` plus, when ``target`` (B) int64 is given, the step's fused loss terms as a sixth result:

@@ -380,6 +380,45 @@ def decoder_greedy_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, steps: int, targe
     return probs, argmax, terms
 
 
+BEAM_MAX_WIDTH = 8
+
+
+def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, width: int):
+    """The beam roll-out of ``steps`` decoder steps in eval mode with ``width`` slots per video as ONE launch (csrc/decoder_fused.cu;
+    the rule is documented at mmb_decoder_beam_fused in include/mmbidaf_b200.h).  emb_text (B,Lt,E) fp32, h0 (B,H) fp32, mask_u8
+    (B,M) uint8, text_len_i32 (B) int32 (the EOS row of video b is text_len[b] - 1).  Always the cluster kernel, whatever
+    ``decoder_cut`` says: there is no chunk-cut beam.
+    Returns (tokens (B,S,K) int64, parents (B,S,K) int32, scores (B,S,K) fp32, probs (B,S,K,M) fp32, best (B,S) int64,
+    path (B,S) int32) -- ``best`` is slot 0's path after the last step, ``path`` its slot at every step."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    if not 1 <= int(width) <= BEAM_MAX_WIDTH:
+        raise ValueError(f"decoder_beam_fwd: beam width {width} (1..{BEAM_MAX_WIDTH})")
+    if int(steps) <= 0:
+        raise ValueError(f"decoder_beam_fwd: {steps} steps")
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M) or text_len_i32.shape != (B,):
+        raise ValueError(f"decoder_beam_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask {tuple(mask_u8.shape)}, "
+                         f"text_len {tuple(text_len_i32.shape)} for B={B} Lt={Lt} E={E} H={H} M={M}")
+    if text_len_i32.dtype != torch.int32:
+        raise ValueError(f"decoder_beam_fwd: text_len {text_len_i32.dtype}, not int32")
+    S, K = int(steps), int(width)
+    tokens = torch.empty(B, S, K, device=dev, dtype=torch.int64)
+    parents = torch.empty(B, S, K, device=dev, dtype=torch.int32)
+    scores = torch.empty(B, S, K, device=dev, dtype=torch.float32)
+    probs = torch.empty(B, S, K, M, device=dev, dtype=torch.float32)
+    best = torch.empty(B, S, device=dev, dtype=torch.int64)
+    path = torch.empty(B, S, device=dev, dtype=torch.int32)
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_beam_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(tokens), p(parents), p(scores),
+        p(probs), p(best), p(path), B, Lt, D, H, E, M, K, S, _lib.stream()), "mmb_decoder_beam_fused")
+    _count(1)
+    return tokens, parents, scores, probs, best, path
+
+
 def greedy_select(argmax: torch.Tensor, text_len: torch.Tensor):
     """decode.greedy_search for a batch on the device: argmax (B,S) int64, text_len (B) int32 -> (sel (B,S) int32 = the chosen
     sentence indices padded with -1, count (B) int32)."""

@@ -1,19 +1,66 @@
 """Extractive summarisation (reference evaluate.py:107-126, :167-202, method='greedy') on the device.
 
 ``MMBiDAF.summarize`` runs the encoder half of the model, the whole greedy decode roll-out and the greedy sentence selection
-without a host round trip; its result is a :class:`Summary`.  :class:`Summarizer` replays ``summarize`` from CUDA graphs, one
+without a host round trip; its result is a :class:`Summary`.  With ``beam_width=K`` the roll-out is a beam search over K
+hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  :class:`Summarizer` replays ``summarize`` from CUDA graphs, one
 capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
 """
 from __future__ import annotations
 
-from typing import Dict, List, NamedTuple, Optional
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
 
 from .synth import Batch
 
-__all__ = ["Summary", "Summarizer", "gather_summaries"]
+__all__ = ["Beams", "Summary", "Summarizer", "gather_summaries"]
+
+
+def _select(tokens: Sequence[int], text_len: int) -> List[int]:
+    """The greedy_search rule (decode.greedy_search, evaluate.py:185-202) over a token row: the EOS row text_len - 1 ends the
+    summary, an index past it is skipped, any other is kept."""
+    chosen = []
+    for k in tokens:
+        if k == text_len - 1:
+            break
+        if k > text_len - 1:
+            continue
+        chosen.append(int(k))
+    return chosen
+
+
+class Beams(NamedTuple):
+    """Every slot of a beam roll-out (``MMBiDAF.summarize(..., beam_width=K)``, the rule at mmb_decoder_beam_fused in
+    include/mmbidaf_b200.h).  Slot j of step s holds the j-th best hypothesis after that step."""
+    tokens: torch.Tensor                   # (B, S, K) int64: the slot's last token (-1: empty slot)
+    parents: torch.Tensor                  # (B, S, K) int32: the slot of step s - 1 it extends (-1: empty slot)
+    scores: torch.Tensor                   # (B, S, K) fp32: the sum of logf(p) along its path (-inf: empty slot)
+    probs: torch.Tensor                    # (B, S, K, M) fp32: the distribution its parent produced at step s (zero for carries / empty)
+
+    def paths(self) -> List[List[Tuple[List[int], float]]]:
+        """Per video, the token rows of the non-empty slots after the last step, best first, with their scores (host lists)."""
+        tok, par, sc = self.tokens.cpu(), self.parents.cpu(), self.scores.cpu()
+        B, S, K = tok.shape
+        out = []
+        for b in range(B):
+            hyps = []
+            for j in range(K):
+                if int(par[b, S - 1, j]) < 0:
+                    continue
+                row, k = [], j
+                for s in range(S - 1, -1, -1):
+                    row.append(int(tok[b, s, k]))
+                    k = int(par[b, s, k])
+                hyps.append((row[::-1], float(sc[b, S - 1, j])))
+            out.append(hyps)
+        return out
+
+    def n_best(self, text_len: Sequence[int]) -> List[List[Tuple[List[int], float]]]:
+        """Per video, the hypotheses of the last step's non-empty slots, best first: (chosen sentence indices under the greedy_search
+        rule, score).  ``text_len`` (B) gives each video's EOS row (text_len - 1)."""
+        lens = [int(n) for n in (text_len.tolist() if torch.is_tensor(text_len) else text_len)]
+        return [[(_select(row, lens[b]), score) for row, score in hyps] for b, hyps in enumerate(self.paths())]
 
 
 class Summary(NamedTuple):
@@ -21,6 +68,7 @@ class Summary(NamedTuple):
     loss: Optional[torch.Tensor]           # the eval loss (models.py:197-199) when targets were given, else None
     indices: torch.Tensor                  # (B, S) int32: the chosen sentence indices of every video, padded with -1
     counts: torch.Tensor                   # (B) int32: how many of them are valid
+    beams: Optional[Beams] = None          # a beam summary's every slot (then out_distributions are the best path's rows), else None
 
     def to_lists(self) -> List[List[int]]:
         """The chosen sentence indices per video as host lists (copies only ``indices`` and ``counts``):
@@ -29,15 +77,15 @@ class Summary(NamedTuple):
         return [idx[b, :c].tolist() for b, c in enumerate(cnt)]
 
 
-def _bucket_key(batch: Batch, with_targets: bool):
+def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int]):
     return (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), int(batch.max_dec_len),
-            tuple(batch.targets.shape) if with_targets else None)
+            tuple(batch.targets.shape) if with_targets else None, beam_width)
 
 
 class _Bucket:
     """One captured ``summarize``: static inputs, static length plans, the graph and its (static) result."""
 
-    def __init__(self, model, batch: Batch, with_targets: bool, warmup: int):
+    def __init__(self, model, batch: Batch, with_targets: bool, warmup: int, beam_width: Optional[int] = None):
         import gc
         from .layers.encoding import pin_lengths
         dev = batch.text.device
@@ -45,6 +93,7 @@ class _Bucket:
         self.batch = Batch(batch.text.clone(), list(batch.text_len), batch.audio.clone(), list(batch.audio_len), batch.images.clone(),
                            list(batch.image_len), batch.targets.clone(), list(batch.target_len), batch.max_dec_len)
         self.with_targets = with_targets
+        self.beam_width = beam_width
         self.plans = [pin_lengths(lst, dev) for lst in (self.batch.text_len, self.batch.audio_len, self.batch.image_len)]
         for m in model.modules():          # per-sequence caches of eager calls still own tensors (see Trainer.capture)
             if hasattr(m, "_cache"):
@@ -66,7 +115,7 @@ class _Bucket:
             plan.refresh()
         b = self.batch
         return model.summarize(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, b.max_dec_len,
-                               b.targets if self.with_targets else None)
+                               b.targets if self.with_targets else None, beam_width=self.beam_width)
 
     def load(self, batch: Batch) -> None:
         if batch is self.batch:
@@ -83,8 +132,8 @@ class _Bucket:
 
 class Summarizer:
     """``model.summarize`` replayed from CUDA graphs.  A batch of a padded-shape bucket seen before (text, audio and key-frame widths,
-    the batch size, ``max_dec_len`` and, with targets, their width) is copied into that bucket's static inputs, its lengths into the
-    bucket's static length plans, and the bucket's graph is replayed; a new bucket is captured first (after ``warmup`` eager runs).
+    the batch size, ``max_dec_len``, with targets their width, and the beam width) is copied into that bucket's static inputs, its
+    lengths into the bucket's static length plans, and the bucket's graph is replayed; a new bucket is captured first (after ``warmup`` eager runs).
     The decoder's weight layouts are rebuilt inside the graph, so in-place parameter updates (an optimiser step) show up on the next
     replay.  The returned :class:`Summary` holds the bucket's static output tensors: the next replay of the same bucket overwrites them."""
 
@@ -93,12 +142,13 @@ class Summarizer:
         self.warmup = warmup
         self.buckets: Dict[tuple, _Bucket] = {}
 
-    def __call__(self, batch: Batch, with_targets: bool = False) -> Summary:
-        """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``."""
-        key = _bucket_key(batch, with_targets)
+    def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None) -> Summary:
+        """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``; ``beam_width``
+        decodes by beam search (``MMBiDAF.summarize``), each width in its own bucket."""
+        key = _bucket_key(batch, with_targets, beam_width)
         bucket = self.buckets.get(key)
         if bucket is None:
-            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup)
+            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup, beam_width)
         else:
             bucket.load(batch)
         bucket.graph.replay()
