@@ -231,6 +231,41 @@ MMB_API int mmb_decoder_beam_fused(const float* proj_a, const float* proj_i, con
                                    float* probs, long long* best, int32_t* path, int B, int Lt, int D, int H, int E, int M, int K,
                                    int S, mmb_stream_t stream);
 /*
+ * Constrained summary roll-outs: mmb_decoder_greedy_fused and mmb_decoder_beam_fused with two constraints on the pick, each in ONE
+ * launch of the same cluster kernel.  This is the project's own rule; like the beam rule it claims no parity with the reference.
+ *   Per video b let eos = text_len[b] - 1.  Each hypothesis keeps `kept`, the number of its picks so far with index < eos (repeats
+ *   counted), and used[m], set when m < eos was picked earlier on its path.  Parameters: no_repeat (0 or 1), min_sentences (>= 0).
+ *   avail = eos - (no_repeat ? kept : 0), the non-EOS sentences the hypothesis could still add.  Sentence m is ELIGIBLE when mask[b,m]
+ *   is set and either m < eos and not (no_repeat and used[m]), or m == eos and (kept >= min_sentences or avail == 0).  Rows past eos
+ *   are never eligible.
+ *   Greedy: the pick is the first maximal p[m] over the eligible m; with none eligible (only when the mask hides rows below eos) the
+ *   pick is eos.  The roll-out goes on after EOS with the same rule.
+ *   Beam: a live slot offers (slot, m) for every eligible m with p[m] > 0; everything else is mmb_decoder_beam_fused's rule (scores,
+ *   carries, ranking, empty slots).  A new slot inherits used and kept from its parent, then adds its own token.
+ *   The distributions are not changed: probs are the model's masked soft-max, bit for bit the step kernel's, and scores use that p.
+ *   no_repeat = 0, min_sentences = 0 is exactly the unconstrained rule; the constrained beam with K = 1 is the constrained greedy.
+ *   So: with no_repeat no summary holds a sentence twice, and a summary holds at least min(min_sentences, S, eos) sentences.
+ * Greedy: arguments of mmb_decoder_greedy_fused without target / loss_terms (the eval loss is the unconstrained roll-out's), plus
+ * text_len (B) int32; M / cluster size <= 16384.  Beam: arguments of mmb_decoder_beam_fused; the eligible bits and kept count of every
+ * slot add to its shared memory (MMB_ERR_UNSUPPORTED with the byte count when a width does not fit).
+ */
+MMB_API int mmb_decoder_greedy_constrained_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                                 const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                                 const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                                 const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt,
+                                                 const float* bcat, const float* out_wt, const float* out_b, const float* emb_text,
+                                                 const float* h0, const uint8_t* mask, const int32_t* text_len, float* probs,
+                                                 long long* argmax, int B, int Lt, int D, int H, int E, int M, int S, int no_repeat,
+                                                 int min_sentences, mmb_stream_t stream);
+MMB_API int mmb_decoder_beam_constrained_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                               const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                               const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                               const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                               const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                               const uint8_t* mask, const int32_t* text_len, long long* tokens, int32_t* parents,
+                                               float* scores, float* probs, long long* best, int32_t* path, int B, int Lt, int D, int H,
+                                               int E, int M, int K, int S, int no_repeat, int min_sentences, mmb_stream_t stream);
+/*
  * Greedy sentence selection (evaluate.py:185-202, decode.greedy_search) on the device.  Per video, in step order over argmax (B,S):
  * the EOS row text_len[b] - 1 ends the summary, an index past it is skipped, any other is kept (repeats too).
  *   sel (B,S) int32 = the kept indices, then -1;  count (B) int32 = how many were kept.

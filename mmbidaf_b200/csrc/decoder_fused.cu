@@ -235,6 +235,20 @@ struct BeamArgs {
 };
 enum : int { kEmpty = 0, kLive = 1, kDone = 2 };
 
+// Constrained roll-outs (mmb_decoder_greedy_constrained_fused / mmb_decoder_beam_constrained_fused; include/mmbidaf_b200.h states the
+// rule): the pick of a step -- the greedy arg-max, the beam candidates -- skips sentences that are not eligible.  A hypothesis keeps its
+// eligible-sentence bits of this rank's sentences (set for m <= EOS with the mask set; a pick m < EOS clears its own bit under
+// no_repeat) and `kept`, its picks below EOS so far.  Greedy: one register per thread, bit j for sentence m0 + tid + j NT (every
+// thread learns the pick).  Beam: ceil(ldp / 32) words per slot in shared memory, gathered by parent beside h / cell / coverage.
+struct ConstraintArgs {
+  const int* text_len;                                      // (B): the EOS row of video b is text_len[b] - 1
+  int no_repeat, min_sentences;
+};
+// the EOS row is eligible once the hypothesis holds min_sentences sentences, or has no other sentence left to add
+__device__ __forceinline__ bool eos_allowed(const ConstraintArgs& cn, int eos, int kept) {
+  return kept >= cn.min_sentences || eos - (cn.no_repeat ? kept : 0) == 0;
+}
+
 // the ranking of the candidates: score descending, then step probability descending, then parent slot, then sentence ascending
 __device__ __forceinline__ bool cand_better(float sa, float pa, int ka, int ma, float sb, float pb, int kb, int mb) {
   if (sa != sb) return sa > sb;
@@ -252,9 +266,10 @@ __device__ __forceinline__ void cand_warp_best(float& s, float& p, int& k, int& 
   }
 }
 
-// kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one
-template <bool kGreedy, bool kBeam = false>
-__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm) {
+// kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one; kConstrained (with kGreedy): the pick skips
+// the sentences `cn` makes ineligible
+template <bool kGreedy, bool kBeam = false, bool kConstrained = false>
+__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int b = blockIdx.x / CL;
@@ -322,8 +337,30 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   float* const s_bcv = s_bcn + KW * ldc;                                 // [K][ldv] coverage of this rank's text rows, in
   float* const s_bcvn = s_bcv + KW * ldv;                                //          and out
   float* const s_bp = s_bcvn + KW * ldv;                                 // [K][ldp] the distribution over this rank's sentences
-  const int eos = kBeam ? bm.text_len[b] - 1 : 0;
+  const int eos = kBeam ? bm.text_len[b] - 1 : kConstrained ? cn.text_len[b] - 1 : 0;
   int runs = 0;                                                          // beam: slot runs so far (row-stage barrier phases)
+  // constrained: this rank's sentences [e_m0, e_m1) of stage E; a sentence is eligible to start with when its mask is set and it
+  // is not past EOS
+  const int e_per = (M + CL - 1) / CL, e_m0 = min(M, R * e_per), e_m1 = min(M, e_m0 + e_per);
+  auto allowed0 = [&](int m) { return m < e_m1 && m <= eos && a.mask[(size_t)b * M + m] != 0; };
+  const int ldu = (ldp + 31) / 32;                                       // beam: words of eligible bits per slot
+  uint32_t* bu_cur = reinterpret_cast<uint32_t*>(s_bp + KW * ldp);       // [K][ldu] eligible bits of every slot, in
+  uint32_t* bu_nxt = bu_cur + KW * ldu;                                  //          and out (swapped after each selection)
+  int* bk_cur = reinterpret_cast<int*>(bu_nxt + KW * ldu);               // [MAXK] kept of every slot, in
+  int* bk_nxt = bk_cur + MAXK;                                           //        and out
+  uint32_t allow = 0;                                                    // greedy: eligible bits of this thread's sentences
+  int kept = 0;                                                          // greedy: picks below EOS so far
+  if constexpr (kConstrained && !kBeam) {
+    for (int m = e_m0 + tid, j = 0; m < e_m1; m += NT, ++j)
+      if (allowed0(m)) allow |= 1u << j;
+  }
+  if constexpr (kConstrained && kBeam) {   // slot 0: every sentence allowed to start with, nothing kept
+    for (int w = warp; w < ldu; w += NW) {
+      const uint32_t v = __ballot_sync(0xffffffffu, allowed0(e_m0 + 32 * w + lane));
+      if (lane == 0) bu_cur[w] = v;
+    }
+    if (tid == 0) bk_cur[0] = 0;
+  }
   if constexpr (kBeam) {                   // before step 0: slot 0 live with score 0, h0 and a zero cell and coverage; the rest empty
     if (tid < MAXK) {
       bs_score[tid] = tid == 0 ? 0.f : -INFINITY;
@@ -354,7 +391,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       for (int i = tid; i < n; i += NT) s_cov[i] = 0.f;
     for (int i = tid; i < H; i += NT) s_x[D + E + i] = s == 0 ? g.h0[(size_t)b * H + i] : s_hn[i];
     // (the pick is below Lt whenever the mask is the text mask; a mask wider than the text could point past it: its last row is read)
-    const float* row = g.emb_text + ((size_t)b * Lt + min(pick, Lt - 1)) * E;
+    // (constrained: a pick of EOS = -1, text_len 0, reads row 0)
+    const float* row = g.emb_text + ((size_t)b * Lt + min(kConstrained ? max(pick, 0) : pick, Lt - 1)) * E;
     for (int i = tid; i < E; i += NT) s_x[D + i] = s == 0 ? 0.f : row[i];
   }
   if (!kGreedy || s == 0)
@@ -724,11 +762,14 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     float best = -INFINITY;
     int best_i = M;
     const int tg = a.target ? (int)a.target[kGreedy ? b * g.T + s : b] : -1;
+    const bool eos_ok = kConstrained && !kBeam && eos_allowed(cn, eos, kept);
     for (int m = m0 + tid; m < m1; m += NT) {
       const float p = expf(lg[m - m0] - gmx) * inv;
       if constexpr (kBeam) s_bp[slot * ldp + m - m0] = p;
       else a.probs[prow * M + m] = p;
-      if (p > best) { best = p; best_i = m; }
+      if constexpr (kConstrained && !kBeam) {                    // the first maximum over the eligible sentences
+        if (((allow >> ((unsigned)(m - m0) / NT)) & 1u) && (m != eos || eos_ok) && p > best) { best = p; best_i = m; }
+      } else if (p > best) { best = p; best_i = m; }
       if (m == tg && a.nll) a.nll[lrow] = -logf(p + 1e-12f);      // models.py:168-170
     }
     if (!kBeam && (kGreedy || a.argmax)) {                                  // first maximal index, as torch.max(dim) documents
@@ -762,6 +803,14 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
           if (pb_ > gb || (pb_ == gb && ib < gi)) { gb = pb_; gi = ib; }
         }
         if constexpr (kGreedy) {
+          if constexpr (kConstrained) {
+            if (gi == M) gi = eos;                                 // no eligible sentence (the caller's mask hides rows below EOS)
+            if (gi < eos) {
+              ++kept;
+              const int j = gi - m0;                               // under no_repeat the pick is no longer eligible
+              if (cn.no_repeat && j >= 0 && gi < m1 && j % NT == tid) allow &= ~(1u << (j / NT));
+            }
+          }
           if (R == 0 && tid == 0) a.argmax[prow] = gi;
           pick = gi;
         } else {
@@ -791,6 +840,10 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
           if (bs_stat[k] != kLive) continue;
           const float p = s_bp[k * ldp + m - m0];
           if (!(p > 0.f)) continue;                              // masked sentences: exactly 0
+          if constexpr (kConstrained) {                          // ineligible sentences offer nothing
+            if (!((bu_cur[k * ldu + ((m - m0) >> 5)] >> ((m - m0) & 31)) & 1u)) continue;
+            if (m == eos && !eos_allowed(cn, eos, bk_cur[k])) continue;
+          }
           const float sc = bs_score[k] + logf(p);
           if (cand_better(ps, pp, pk, pm, sc, p, k, m) && cand_better(sc, p, k, m, cs, cp, ck, cm)) { cs = sc; cp = p; ck = k; cm = m; }
         }
@@ -876,6 +929,13 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       for (int i = tid; i < H; i += NT) s_bh[j * ldh + i] = s_bhn[q * ldh + i];
       for (int i = tid; i < ldc; i += NT) s_bc[j * ldc + i] = s_bcn[q * ldc + i];
       for (int i = tid; i < n; i += NT) s_bcv[j * ldv + i] = s_bcvn[q * ldv + i];
+      if constexpr (kConstrained) {          // the parent's eligible bits and kept, then the new slot's own token
+        const int tk = nt_tok[j], rel = tk - m0;
+        const bool clear = cn.no_repeat && tk < eos && rel >= 0 && tk < m1;
+        for (int w = tid; w < ldu; w += NT)
+          bu_nxt[j * ldu + w] = bu_cur[q * ldu + w] & ~(clear && (rel >> 5) == w ? 1u << (rel & 31) : 0u);
+        if (tid == 0) bk_nxt[j] = bk_cur[q] + (tk < eos ? 1 : 0);
+      }
     }
     if (tid < KW) {
       const int kd = nt_kind[tid];
@@ -884,6 +944,10 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       bs_stat[tid] = kd == 1 ? kLive : kd == 0 ? kEmpty : kDone;
     }
     __syncthreads();
+    if constexpr (kConstrained) {            // (uniform) the gathered bits are the next step's input
+      uint32_t* const t = bu_cur; bu_cur = bu_nxt; bu_nxt = t;
+      int* const u = bk_cur; bk_cur = bk_nxt; bk_nxt = u;
+    }
   }
   }  // steps (the loop body keeps the step kernel's indentation)
   if constexpr (kBeam) {
@@ -906,12 +970,25 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   DEC_STAMP(17);
 }
 
-__global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) { dec_fused_body<false>(a, GreedyArgs{}, BeamArgs{}); }
+__global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
+  dec_fused_body<false>(a, GreedyArgs{}, BeamArgs{}, ConstraintArgs{});
+}
 
-__global__ void __launch_bounds__(NT) dec_greedy_fused_kernel(const FusedArgs a, const GreedyArgs g) { dec_fused_body<true>(a, g, BeamArgs{}); }
+__global__ void __launch_bounds__(NT) dec_greedy_fused_kernel(const FusedArgs a, const GreedyArgs g) {
+  dec_fused_body<true>(a, g, BeamArgs{}, ConstraintArgs{});
+}
 
 __global__ void __launch_bounds__(NT) dec_beam_fused_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm) {
-  dec_fused_body<true, true>(a, g, bm);
+  dec_fused_body<true, true>(a, g, bm, ConstraintArgs{});
+}
+
+__global__ void __launch_bounds__(NT) dec_greedy_constrained_kernel(const FusedArgs a, const GreedyArgs g, const ConstraintArgs cn) {
+  dec_fused_body<true, false, true>(a, g, BeamArgs{}, cn);
+}
+
+__global__ void __launch_bounds__(NT) dec_beam_constrained_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm,
+                                                                  const ConstraintArgs cn) {
+  dec_fused_body<true, true, true>(a, g, bm, cn);
 }
 
 }  // namespace
@@ -1446,16 +1523,21 @@ static size_t fused_smem_bytes(int Lt, int D, int H, int E, int M, int CL, int* 
   return floats * sizeof(float) + 64;
 }
 
-// floats of the beam region (see dec_fused_body): the tables, the selection exchange and K slots of state
-static size_t beam_floats(int K, int CL, int chunk, int H, int M) {
+// floats of the beam region (see dec_fused_body): the tables, the selection exchange and K slots of state; constrained, also every
+// slot's eligible bits and kept count, in and out
+static size_t beam_floats(int K, int CL, int chunk, int H, int M, bool constrained = false) {
   auto up4 = [](size_t v) { return (v + 3) & ~(size_t)3; };
-  const size_t per_slot = 2 * (up4(H) + up4(split4(H, CL)) + up4(chunk)) + up4((M + CL - 1) / CL);
-  return 7 * MAXK + MAXC * MAXK * 4 + NW * 4 + MAXK * 4 + (size_t)K * per_slot;
+  const size_t ldp = up4((M + CL - 1) / CL);
+  const size_t per_slot = 2 * (up4(H) + up4(split4(H, CL)) + up4(chunk)) + ldp;
+  const size_t cons = constrained ? 2 * (size_t)K * ((ldp + 31) / 32) + 2 * MAXK : 0;
+  return 7 * MAXK + MAXC * MAXK * 4 + NW * 4 + MAXK * 4 + (size_t)K * per_slot + cons;
 }
 
 // Shape checks, cluster size, shared memory and row stage of the forward cluster kernels, then the launch: `g` null launches one step
-// (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel), or with `bm` the beam roll-out (dec_beam_fused_kernel).
-static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr) {
+// (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel), or with `bm` the beam roll-out (dec_beam_fused_kernel);
+// with `cn` the constrained roll-out of either (dec_greedy_constrained_kernel, dec_beam_constrained_kernel).
+static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr,
+                        const ConstraintArgs* cn = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
@@ -1464,9 +1546,11 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   const int CL = (long long)B * 4 * 2 <= 160 ? 8 : 4;
   size_t smem = fused_smem_bytes(Lt, D, H, E, M, CL, &a.chunk);
   MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "%s: %zu B of shared memory (Lt=%d)", who, smem, Lt);
+  // constrained greedy: a thread keeps the eligible bits of its sentences in one 32-bit register
+  MMB_REQUIRE(!cn || bm || (M + CL - 1) / CL <= 32 * NT, MMB_ERR_UNSUPPORTED, "%s: M=%d > %d sentences per CTA", who, M, 32 * NT);
   if (bm) {                                // the beam region behind the base arrays; the row stage follows if it still fits
     bm->off = (int)((smem + 15) / 16 * 4);
-    smem = ((size_t)bm->off + beam_floats(bm->K, CL, a.chunk, H, M)) * 4 + 64;
+    smem = ((size_t)bm->off + beam_floats(bm->K, CL, a.chunk, H, M, cn != nullptr)) * 4 + 64;
     MMB_REQUIRE(smem <= 227 * 1024, MMB_ERR_UNSUPPORTED, "%s: width %d needs %zu B of shared memory per CTA, more than 232448 (B=%d Lt=%d M=%d)",
                 who, bm->K, smem, B, Lt, M);
   }
@@ -1483,12 +1567,13 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[3] = {0, 0, 0};
-  const int which = bm ? 2 : g != nullptr;
+  static size_t smem_set[5] = {0, 0, 0, 0, 0};
+  const int which = bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
   if (smem > smem_set[which]) {
-    if (bm) MMB_CUDA(cudaFuncSetAttribute(dec_beam_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    else if (g) MMB_CUDA(cudaFuncSetAttribute(dec_greedy_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    else MMB_CUDA(cudaFuncSetAttribute(dec_step_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const void* fn = which == 4 ? (const void*)dec_beam_constrained_kernel : which == 3 ? (const void*)dec_greedy_constrained_kernel
+                   : which == 2 ? (const void*)dec_beam_fused_kernel : which == 1 ? (const void*)dec_greedy_fused_kernel
+                                : (const void*)dec_step_fused_kernel;
+    MMB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     smem_set[which] = smem;
   }
   static const char* trace_env = getenv("MMB_DEC_TRACE");
@@ -1510,6 +1595,14 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (cn && bm) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_constrained_kernel, a, *g, *bm, *cn));
+    return check_launch("dec_beam_constrained_kernel");
+  }
+  if (cn) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_greedy_constrained_kernel, a, *g, *cn));
+    return check_launch("dec_greedy_constrained_kernel");
+  }
   if (bm) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_fused_kernel, a, *g, *bm));
     return check_launch("dec_beam_fused_kernel");
@@ -1588,6 +1681,55 @@ extern "C" int mmb_decoder_beam_fused(const float* proj_a, const float* proj_i, 
   const GreedyArgs g{emb_text, h0, S, 0};
   BeamArgs bm{text_len, tokens, parents, scores, probs, best, path, K, 0};
   return launch_fused(a, &g, "mmb_decoder_beam_fused", stream, &bm);
+}
+
+extern "C" int mmb_decoder_greedy_constrained_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                                    const float* Wh4t, const float* bh4, const float* v1, const float* wc1,
+                                                    const float* v2, const float* wc2, const float* v1b, const float* v2b,
+                                                    const float* Wb13t, const float* vb1, const float* vb2, const float* vb1b,
+                                                    const float* vb2b, const float* Wcatt, const float* bcat, const float* out_wt,
+                                                    const float* out_b, const float* emb_text, const float* h0, const uint8_t* mask,
+                                                    const int* text_len, float* probs, long long* argmax, int B, int Lt, int D,
+                                                    int H, int E, int M, int S, int no_repeat, int min_sentences,
+                                                    mmb_stream_t stream) {
+  using namespace mmb;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && text_len && probs && argmax,
+              MMB_ERR_INVALID, "mmb_decoder_greedy_constrained_fused: null pointer");
+  MMB_REQUIRE(S > 0 && (no_repeat == 0 || no_repeat == 1) && min_sentences >= 0, MMB_ERR_INVALID,
+              "mmb_decoder_greedy_constrained_fused: S=%d no_repeat=%d (0 or 1) min_sentences=%d (>= 0)", S, no_repeat, min_sentences);
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, probs, nullptr, nullptr, nullptr, nullptr, argmax,
+              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  const ConstraintArgs cn{text_len, no_repeat, min_sentences};
+  return launch_fused(a, &g, "mmb_decoder_greedy_constrained_fused", stream, nullptr, &cn);
+}
+
+extern "C" int mmb_decoder_beam_constrained_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                                  const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                                  const float* wc2, const float* v1b, const float* v2b, const float* Wb13t,
+                                                  const float* vb1, const float* vb2, const float* vb1b, const float* vb2b,
+                                                  const float* Wcatt, const float* bcat, const float* out_wt, const float* out_b,
+                                                  const float* emb_text, const float* h0, const uint8_t* mask, const int* text_len,
+                                                  long long* tokens, int* parents, float* scores, float* probs, long long* best,
+                                                  int* path, int B, int Lt, int D, int H, int E, int M, int K, int S, int no_repeat,
+                                                  int min_sentences, mmb_stream_t stream) {
+  using namespace mmb;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && text_len && tokens && parents &&
+                  scores && probs && best && path,
+              MMB_ERR_INVALID, "mmb_decoder_beam_constrained_fused: null pointer");
+  MMB_REQUIRE(K >= 1 && K <= MAXK && S > 0 && (no_repeat == 0 || no_repeat == 1) && min_sentences >= 0, MMB_ERR_INVALID,
+              "mmb_decoder_beam_constrained_fused: width K=%d (1..%d), S=%d, no_repeat=%d (0 or 1), min_sentences=%d (>= 0)", K, MAXK,
+              S, no_repeat, min_sentences);
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  BeamArgs bm{text_len, tokens, parents, scores, probs, best, path, K, 0};
+  const ConstraintArgs cn{text_len, no_repeat, min_sentences};
+  return launch_fused(a, &g, "mmb_decoder_beam_constrained_fused", stream, &bm, &cn);
 }
 
 extern "C" int mmb_decoder_bwd_head(const float* probs, const float* d_probs, const long long* target, const float* g_nll,

@@ -207,23 +207,34 @@ class MultimodalAttentionDecoder(nn.Module):
         return self.step(sent_embed, decoder_hidden, decoder_cell_state, text_audio_enc_out, text_img_enc_out,
                          coverage_vec, mask)[:5]
 
-    def greedy(self, emb_text, h0, enc_a, enc_i, mask, steps, target=None):
+    def greedy(self, emb_text, h0, enc_a, enc_i, mask, steps, target=None, text_len=None, no_repeat=False, min_sentences=0):
         """The greedy decode of ``steps`` steps in eval mode (models.py:145-199, the ``else`` branches), batched: start from h0
         (B, H) or (B, 1, H), a zero cell, coverage and input row; each step's arg-max row of ``emb_text`` (B, Lt, E) is the next
         input.  ``target`` (B, T) with T >= steps is optional.  No autograd.  Returns (out_distributions (B, steps, M), argmax
         (B, steps) int64, loss_terms (steps, 2, B) = per step [nll | coverage term] or None) -- bit for bit what ``steps`` calls of
         :meth:`step` with an arg-max and a gather in between give.  Where the decoder step runs as one cluster kernel
-        (``ops.decoder_cut``) the whole roll-out is one launch; long lectures run the chunk-parallel cut step by step."""
+        (``ops.decoder_cut``) the whole roll-out is one launch; long lectures run the chunk-parallel cut step by step.
+        ``no_repeat`` / ``min_sentences`` constrain the pick (the rule at mmb_decoder_greedy_constrained_fused in
+        include/mmbidaf_b200.h; ``text_len`` (B) gives each video's EOS row, text_len - 1): the roll-out is then always one launch of
+        the cluster kernel, takes no ``target`` and returns None as loss_terms."""
         if not enc_a.is_cuda:
             raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
         if self.num_layers != 1:
             raise RuntimeError("MultimodalAttentionDecoder: only num_layers=1 is supported (the reference model uses 1)")
+        constrained = bool(no_repeat) or min_sentences != 0
+        if constrained and (target is not None or text_len is None):
+            raise ValueError("greedy: a constrained roll-out needs text_len and takes no target (the eval loss is the unconstrained "
+                             "roll-out's)")
         with torch.no_grad():
             seq = self._sequence(enc_a, enc_i)["seq"]
             B, Lt = seq.B, seq.Lt
             emb = emb_text.contiguous()
             h = h0.reshape(B, -1).contiguous()
             mask_u8 = ops._u8(mask)
+            if constrained:
+                probs, picks = ops.decoder_greedy_constrained_fwd(seq, emb, h, mask_u8, text_len.to(torch.int32).contiguous(), steps,
+                                                                  no_repeat, min_sentences)
+                return probs, picks, None
             tgt = None if target is None else target.reshape(B, -1).to(torch.int64).contiguous()
             if ops.decoder_cut(B, Lt) != "chunks":
                 return ops.decoder_greedy_fwd(seq, emb, h, mask_u8, steps, tgt)
@@ -243,10 +254,11 @@ class MultimodalAttentionDecoder(nn.Module):
                 terms.append(lossvec)
             return torch.stack(probs, 1), torch.stack(picks, 1), (torch.stack(terms) if tgt is not None else None)
 
-    def beam(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, width):
+    def beam(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, width, no_repeat=False, min_sentences=0):
         """The beam decode of ``steps`` steps in eval mode with ``width`` (1..8) hypotheses per video, as ONE launch of the cluster
         kernel whatever ``ops.decoder_cut`` says (there is no chunk-cut beam); the rule is documented at mmb_decoder_beam_fused in
-        include/mmbidaf_b200.h.  Same start as :meth:`greedy`; ``text_len`` (B) int32 gives each video's EOS row (text_len - 1).
+        include/mmbidaf_b200.h, and with ``no_repeat`` / ``min_sentences`` at mmb_decoder_beam_constrained_fused.  Same start as
+        :meth:`greedy`; ``text_len`` (B) int32 gives each video's EOS row (text_len - 1).
         No autograd.  Returns ``ops.decoder_beam_fwd``'s (tokens, parents, scores, probs, best, path)."""
         if not enc_a.is_cuda:
             raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
@@ -256,7 +268,7 @@ class MultimodalAttentionDecoder(nn.Module):
             seq = self._sequence(enc_a, enc_i)["seq"]
             B = seq.B
             return ops.decoder_beam_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
-                                        text_len.to(torch.int32).contiguous(), steps, width)
+                                        text_len.to(torch.int32).contiguous(), steps, width, no_repeat, min_sentences)
 
     def step(self, sent_embed, decoder_hidden, decoder_cell_state, text_audio_enc_out, text_img_enc_out, coverage_vec,
              mask, target=None):

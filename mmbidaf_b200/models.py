@@ -143,7 +143,8 @@ class MMBiDAF(nn.Module):
         loss = Fn.decode_loss(step_losses, steps, cov_loss_wt, self.training)
         return torch.stack(out_distributions).transpose(0, 1), loss
 
-    def summarize(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, targets=None, beam_width=None):
+    def summarize(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, targets=None, beam_width=None,
+                  no_repeat=False, min_sentences=0):
         """Extractive summaries of a batch (evaluate.py:107-126, :167-202 with method='greedy'): the eval-mode forward pass with the
         whole greedy decode roll-out on the device, then the greedy sentence selection on the device.  Runs under ``no_grad`` in eval
         mode and gives the caller's ``training`` flag back.  ``targets`` (B, T, 1) or (B, T) with T >= max_dec_len is optional (the
@@ -153,14 +154,15 @@ class MMBiDAF(nn.Module):
         ``beam_width`` K (1..8) decodes by beam search instead (``MultimodalAttentionDecoder.beam``, one launch): the summary is the
         best hypothesis's -- its indices and counts under the greedy_search rule, its distribution rows as ``out_distributions`` --
         ``loss`` is None and ``beams`` holds every slot (``Beams``).  K = 1 gives the greedy summary.  Not with ``targets``: the eval
-        loss is defined by the greedy roll-out."""
+        loss is defined by the greedy roll-out.
+        ``no_repeat`` (bool) keeps a sentence out of the summary once it is in; ``min_sentences`` (int >= 0) keeps the EOS row from
+        ending it before that many sentences (or every sentence of the transcript) are in.  Both constrain the greedy and the beam
+        pick, inside the roll-out kernel (the rule at mmb_decoder_greedy_constrained_fused in include/mmbidaf_b200.h); the
+        distributions stay the model's.  Not with ``targets``.  With the defaults the launches are exactly the unconstrained ones."""
         from .layers.encoding import length_plan
-        from .summarize import Beams, Summary
-        if beam_width is not None:
-            if isinstance(beam_width, bool) or not isinstance(beam_width, int) or not 1 <= beam_width <= ops.BEAM_MAX_WIDTH:
-                raise ValueError(f"summarize: beam_width {beam_width!r}, expected None or an int in 1..{ops.BEAM_MAX_WIDTH}")
-            if targets is not None:
-                raise ValueError("summarize: beam_width with targets -- the eval loss is defined by the greedy roll-out")
+        from .summarize import Beams, Summary, check_options
+        check_options("summarize", targets is not None, beam_width, no_repeat, min_sentences)
+        constrained = no_repeat or min_sentences > 0
         was_training = self.training
         self.eval()
         try:
@@ -177,12 +179,19 @@ class MMBiDAF(nn.Module):
                 enc_a, enc_i, h0, mask = self._encode(text, text_len, audio, audio_len, images, image_len, decoder_start)
                 if beam_width is not None:
                     lens = length_plan(text_len, text.device).len_i32
-                    tokens, parents, scores, rows, best, path = dec.beam(text, h0, enc_a, enc_i, mask, lens, max_dec_len, beam_width)
+                    tokens, parents, scores, rows, best, path = dec.beam(text, h0, enc_a, enc_i, mask, lens, max_dec_len, beam_width,
+                                                                         no_repeat, min_sentences)
                     # the best path's distribution rows: slot path[b, s] of step s
                     M = rows.shape[-1]
                     probs = rows.gather(2, path.long().clamp_min(0)[:, :, None, None].expand(-1, -1, 1, M)).squeeze(2)
                     indices, counts = ops.greedy_select(best, lens)
                     return Summary(probs, None, indices, counts, Beams(tokens, parents, scores, rows))
+                if constrained:
+                    lens = length_plan(text_len, text.device).len_i32
+                    probs, picks, _ = dec.greedy(text, h0, enc_a, enc_i, mask, max_dec_len, text_len=lens, no_repeat=no_repeat,
+                                                 min_sentences=min_sentences)
+                    indices, counts = ops.greedy_select(picks, lens)
+                    return Summary(probs, None, indices, counts)
                 probs, argmax, terms = dec.greedy(text, h0, enc_a, enc_i, mask, max_dec_len, target=start.get("targets"))
                 # the eval loss exactly as forward forms it: every step's nll, the last step's coverage term, over the steps
                 loss = None if terms is None else Fn.decode_loss(list(terms.unbind(0)), max_dec_len, 1.0, False)

@@ -380,14 +380,54 @@ def decoder_greedy_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, steps: int, targe
     return probs, argmax, terms
 
 
+def _check_constraints(who: str, no_repeat, min_sentences) -> None:
+    if not isinstance(no_repeat, int) or no_repeat not in (0, 1):
+        raise ValueError(f"{who}: no_repeat {no_repeat!r}, expected a bool")
+    if isinstance(min_sentences, bool) or not isinstance(min_sentences, int) or min_sentences < 0:
+        raise ValueError(f"{who}: min_sentences {min_sentences!r}, expected an int >= 0")
+
+
+def decoder_greedy_constrained_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, no_repeat: bool = False,
+                                   min_sentences: int = 0):
+    """The constrained greedy roll-out (rule at mmb_decoder_greedy_constrained_fused in include/mmbidaf_b200.h) as ONE launch of the
+    cluster kernel, whatever ``decoder_cut`` says: there is no chunk-cut constrained greedy.  ``no_repeat`` blocks a sentence once
+    picked; the EOS row is not picked before ``min_sentences`` sentences (or every sentence) are in.  Inputs as
+    :func:`decoder_greedy_fwd` without a target, plus text_len_i32 (B) int32 (the EOS row of video b is text_len[b] - 1).
+    Returns (probs (B,steps,M), picks (B,steps) int64) -- the distributions are the unconstrained model's, bit for bit."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    _check_constraints("decoder_greedy_constrained_fwd", no_repeat, min_sentences)
+    if int(steps) <= 0:
+        raise ValueError(f"decoder_greedy_constrained_fwd: {steps} steps")
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M) or text_len_i32.shape != (B,):
+        raise ValueError(f"decoder_greedy_constrained_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, "
+                         f"mask {tuple(mask_u8.shape)}, text_len {tuple(text_len_i32.shape)} for B={B} Lt={Lt} E={E} H={H} M={M}")
+    if text_len_i32.dtype != torch.int32:
+        raise ValueError(f"decoder_greedy_constrained_fwd: text_len {text_len_i32.dtype}, not int32")
+    S = int(steps)
+    probs = torch.empty(B, S, M, device=dev, dtype=torch.float32)
+    picks = torch.empty(B, S, device=dev, dtype=torch.int64)
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_greedy_constrained_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(probs), p(picks),
+        B, Lt, D, H, E, M, S, int(no_repeat), int(min_sentences), _lib.stream()), "mmb_decoder_greedy_constrained_fused")
+    _count(1)
+    return probs, picks
+
+
 BEAM_MAX_WIDTH = 8
 
 
-def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, width: int):
+def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, width: int, no_repeat: bool = False,
+                     min_sentences: int = 0, constrained: Optional[bool] = None):
     """The beam roll-out of ``steps`` decoder steps in eval mode with ``width`` slots per video as ONE launch (csrc/decoder_fused.cu;
     the rule is documented at mmb_decoder_beam_fused in include/mmbidaf_b200.h).  emb_text (B,Lt,E) fp32, h0 (B,H) fp32, mask_u8
     (B,M) uint8, text_len_i32 (B) int32 (the EOS row of video b is text_len[b] - 1).  Always the cluster kernel, whatever
-    ``decoder_cut`` says: there is no chunk-cut beam.
+    ``decoder_cut`` says: there is no chunk-cut beam.  ``no_repeat`` / ``min_sentences`` constrain the candidates (the rule at
+    mmb_decoder_beam_constrained_fused); the constrained kernel runs when either is set, or when ``constrained`` says so.
     Returns (tokens (B,S,K) int64, parents (B,S,K) int32, scores (B,S,K) fp32, probs (B,S,K,M) fp32, best (B,S) int64,
     path (B,S) int32) -- ``best`` is slot 0's path after the last step, ``path`` its slot at every step."""
     lib = _lib.lib()
@@ -397,6 +437,7 @@ def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps
         raise ValueError(f"decoder_beam_fwd: beam width {width} (1..{BEAM_MAX_WIDTH})")
     if int(steps) <= 0:
         raise ValueError(f"decoder_beam_fwd: {steps} steps")
+    _check_constraints("decoder_beam_fwd", no_repeat, min_sentences)
     if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M) or text_len_i32.shape != (B,):
         raise ValueError(f"decoder_beam_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask {tuple(mask_u8.shape)}, "
                          f"text_len {tuple(text_len_i32.shape)} for B={B} Lt={Lt} E={E} H={H} M={M}")
@@ -410,11 +451,17 @@ def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps
     best = torch.empty(B, S, device=dev, dtype=torch.int64)
     path = torch.empty(B, S, device=dev, dtype=torch.int32)
     p = _lib.ptr
-    _lib.check(lib.mmb_decoder_beam_fused(
-        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
-        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
-        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(tokens), p(parents), p(scores),
-        p(probs), p(best), p(path), B, Lt, D, H, E, M, K, S, _lib.stream()), "mmb_decoder_beam_fused")
+    args = (p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+            p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+            p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(tokens), p(parents),
+            p(scores), p(probs), p(best), p(path), B, Lt, D, H, E, M, K, S)
+    if constrained is None:
+        constrained = bool(no_repeat) or min_sentences > 0
+    if constrained:
+        _lib.check(lib.mmb_decoder_beam_constrained_fused(*args, int(no_repeat), int(min_sentences), _lib.stream()),
+                   "mmb_decoder_beam_constrained_fused")
+    else:
+        _lib.check(lib.mmb_decoder_beam_fused(*args, _lib.stream()), "mmb_decoder_beam_fused")
     _count(1)
     return tokens, parents, scores, probs, best, path
 

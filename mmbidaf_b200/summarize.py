@@ -2,7 +2,8 @@
 
 ``MMBiDAF.summarize`` runs the encoder half of the model, the whole greedy decode roll-out and the greedy sentence selection
 without a host round trip; its result is a :class:`Summary`.  With ``beam_width=K`` the roll-out is a beam search over K
-hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  :class:`Summarizer` replays ``summarize`` from CUDA graphs, one
+hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  ``no_repeat`` and
+``min_sentences`` constrain either pick inside the roll-out kernel.  :class:`Summarizer` replays ``summarize`` from CUDA graphs, one
 capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
 """
 from __future__ import annotations
@@ -12,9 +13,27 @@ from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 import torch
 import torch.distributed as dist
 
+from .ops import BEAM_MAX_WIDTH
 from .synth import Batch
 
 __all__ = ["Beams", "Summary", "Summarizer", "gather_summaries"]
+
+
+def check_options(who: str, with_targets: bool, beam_width, no_repeat, min_sentences) -> None:
+    """The decode options of ``MMBiDAF.summarize`` / ``Summarizer``, checked before any device work: ``beam_width`` None or an int
+    in 1..8, ``no_repeat`` a bool, ``min_sentences`` an int >= 0; neither a beam nor a constraint with targets (the eval loss is
+    defined by the unconstrained greedy roll-out)."""
+    if beam_width is not None:
+        if isinstance(beam_width, bool) or not isinstance(beam_width, int) or not 1 <= beam_width <= BEAM_MAX_WIDTH:
+            raise ValueError(f"{who}: beam_width {beam_width!r}, expected None or an int in 1..{BEAM_MAX_WIDTH}")
+        if with_targets:
+            raise ValueError(f"{who}: beam_width with targets -- the eval loss is defined by the greedy roll-out")
+    if not isinstance(no_repeat, bool):
+        raise ValueError(f"{who}: no_repeat {no_repeat!r}, expected a bool")
+    if isinstance(min_sentences, bool) or not isinstance(min_sentences, int) or min_sentences < 0:
+        raise ValueError(f"{who}: min_sentences {min_sentences!r}, expected an int >= 0")
+    if with_targets and (no_repeat or min_sentences > 0):
+        raise ValueError(f"{who}: no_repeat / min_sentences with targets -- the eval loss is defined by the unconstrained roll-out")
 
 
 def _select(tokens: Sequence[int], text_len: int) -> List[int]:
@@ -77,15 +96,16 @@ class Summary(NamedTuple):
         return [idx[b, :c].tolist() for b, c in enumerate(cnt)]
 
 
-def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int]):
+def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int], no_repeat: bool = False, min_sentences: int = 0):
     return (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), int(batch.max_dec_len),
-            tuple(batch.targets.shape) if with_targets else None, beam_width)
+            tuple(batch.targets.shape) if with_targets else None, beam_width, no_repeat, min_sentences)
 
 
 class _Bucket:
     """One captured ``summarize``: static inputs, static length plans, the graph and its (static) result."""
 
-    def __init__(self, model, batch: Batch, with_targets: bool, warmup: int, beam_width: Optional[int] = None):
+    def __init__(self, model, batch: Batch, with_targets: bool, warmup: int, beam_width: Optional[int] = None,
+                 no_repeat: bool = False, min_sentences: int = 0):
         import gc
         from .layers.encoding import pin_lengths
         dev = batch.text.device
@@ -94,6 +114,7 @@ class _Bucket:
                            list(batch.image_len), batch.targets.clone(), list(batch.target_len), batch.max_dec_len)
         self.with_targets = with_targets
         self.beam_width = beam_width
+        self.no_repeat, self.min_sentences = no_repeat, min_sentences
         self.plans = [pin_lengths(lst, dev) for lst in (self.batch.text_len, self.batch.audio_len, self.batch.image_len)]
         for m in model.modules():          # per-sequence caches of eager calls still own tensors (see Trainer.capture)
             if hasattr(m, "_cache"):
@@ -115,7 +136,8 @@ class _Bucket:
             plan.refresh()
         b = self.batch
         return model.summarize(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, b.max_dec_len,
-                               b.targets if self.with_targets else None, beam_width=self.beam_width)
+                               b.targets if self.with_targets else None, beam_width=self.beam_width, no_repeat=self.no_repeat,
+                               min_sentences=self.min_sentences)
 
     def load(self, batch: Batch) -> None:
         if batch is self.batch:
@@ -132,7 +154,7 @@ class _Bucket:
 
 class Summarizer:
     """``model.summarize`` replayed from CUDA graphs.  A batch of a padded-shape bucket seen before (text, audio and key-frame widths,
-    the batch size, ``max_dec_len``, with targets their width, and the beam width) is copied into that bucket's static inputs, its
+    the batch size, ``max_dec_len``, with targets their width, the beam width and the constraints) is copied into that bucket's static inputs, its
     lengths into the bucket's static length plans, and the bucket's graph is replayed; a new bucket is captured first (after ``warmup`` eager runs).
     The decoder's weight layouts are rebuilt inside the graph, so in-place parameter updates (an optimiser step) show up on the next
     replay.  The returned :class:`Summary` holds the bucket's static output tensors: the next replay of the same bucket overwrites them."""
@@ -142,13 +164,16 @@ class Summarizer:
         self.warmup = warmup
         self.buckets: Dict[tuple, _Bucket] = {}
 
-    def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None) -> Summary:
+    def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None, no_repeat: bool = False,
+                 min_sentences: int = 0) -> Summary:
         """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``; ``beam_width``
-        decodes by beam search (``MMBiDAF.summarize``), each width in its own bucket."""
-        key = _bucket_key(batch, with_targets, beam_width)
+        decodes by beam search, ``no_repeat`` / ``min_sentences`` constrain the pick (``MMBiDAF.summarize``); each width and each
+        setting of the constraints in its own bucket.  The options are checked before anything is copied or captured."""
+        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences)
+        key = _bucket_key(batch, with_targets, beam_width, no_repeat, min_sentences)
         bucket = self.buckets.get(key)
         if bucket is None:
-            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup, beam_width)
+            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup, beam_width, no_repeat, min_sentences)
         else:
             bucket.load(batch)
         bucket.graph.replay()
