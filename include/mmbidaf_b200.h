@@ -266,6 +266,42 @@ MMB_API int mmb_decoder_beam_constrained_fused(const float* proj_a, const float*
                                                float* scores, float* probs, long long* best, int32_t* path, int B, int Lt, int D, int H,
                                                int E, int M, int K, int S, int no_repeat, int min_sentences, mmb_stream_t stream);
 /*
+ * Sampled summary roll-outs: N summaries per video, each the greedy roll-out (or the constrained one) with the pick DRAWN, all in ONE
+ * launch of the same cluster kernel (one cluster per (video, sample); the encoder outputs are read per video, not replicated).  This
+ * is the project's own rule.  Inputs: N in 1..64; temperature T finite and > 0; top_k 0 (off) or 1..8; a 64-bit key on the device
+ * (*key, as the dropout entry points take it); no_repeat / min_sentences as above (either set: the constrained candidates).
+ * Roll-out (b, n) runs exactly the greedy roll-out's stages; its distributions are the step kernel's masked soft-max, bit for bit.
+ * Only the pick of step s changes:
+ *   1. Candidates: every sentence 0..M-1; with a constraint set, the eligible sentences of the rule above; with top_k > 0, only the
+ *      top_k of those ranked first by (p descending, m ascending).
+ *   2. Uniform: c = ((b N + n) S + s) M + m as a uint32; u = ((hash32(c, key) >> 9) + 0.5f) 2^-23, exact in fp32 and in
+ *      [2^-24, 1 - 2^-24].  hash32 is the mixing function of the dropout keep bits.
+ *   3. Score: z = logf(p[m]) (1 / T) - logf(-logf(u)) in fp32 (Gumbel-max); p = 0 gives -inf, p > 0 a finite z.
+ *   4. Pick: the candidate with the largest z, ties to the smaller m.  With no candidate (only under a constraint, when the mask hides
+ *      the rows below eos) the pick is eos, as in the constrained greedy.  The roll-out goes on after EOS with the same rule.
+ * So the pick is distributed as p^(1/T) over the candidates; top_k = 1 is the greedy pick (the constrained greedy pick under a
+ * constraint) whatever the key and T; the same key and inputs give the same samples, bit for bit.
+ * Arguments of mmb_decoder_greedy_constrained_fused (text_len may be null without a constraint) plus key, N, T, top_k.  Writes
+ * probs (B,N,S,M) and tokens (B,N,S) int64.  MMB_ERR_INVALID: N, T, top_k or a constraint out of range; MMB_ERR_UNSUPPORTED:
+ * B N S M > 2^32 (the counters of a key), or under a constraint M / cluster size > 16384.
+ */
+MMB_API int mmb_decoder_sample_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                     const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                     const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                     const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                     const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                     const uint8_t* mask, const int32_t* text_len, const unsigned long long* key, float* probs,
+                                     long long* tokens, int B, int Lt, int D, int H, int E, int M, int S, int N, float T, int top_k,
+                                     int no_repeat, int min_sentences, mmb_stream_t stream);
+/*
+ * Steps 1 to 4 of the sampled pick above for given rows, one CTA per row, with the roll-out kernel's score function: the reference
+ * of the tests.  probs (R,M); eligible (R,M) uint8 or null (null: every sentence is a candidate; else the candidates are the rows'
+ * nonzero entries); row r is sample r % N of video row_base[r], i.e. roll-out row_base[r] N + r % N, at step s of S.
+ * picks (R) int64: the pick, or -1 for a row without a candidate.
+ */
+MMB_API int mmb_sample_pick(const float* probs, const uint8_t* eligible, const unsigned long long* key, const int32_t* row_base, int R,
+                            int M, int S, int s, int N, float T, int top_k, long long* picks, mmb_stream_t stream);
+/*
  * Greedy sentence selection (evaluate.py:185-202, decode.greedy_search) on the device.  Per video, in step order over argmax (B,S):
  * the EOS row text_len[b] - 1 ends the summary, an index past it is skipped, any other is kept (repeats too).
  *   sel (B,S) int32 = the kept indices, then -1;  count (B) int32 = how many were kept.

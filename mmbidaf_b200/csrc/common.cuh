@@ -55,7 +55,7 @@ __device__ __forceinline__ float sigmoidf_acc(float x) { return 1.0f / (1.0f + e
 // A 32-bit avalanche hash (two multiplies and three xor-shifts around the two key halves): nine integer instructions, the same bits
 // wherever they are recomputed (the forward store, the backward load, mmb_dropout_mask in the tests).  Not ATen's Philox stream:
 // bit-parity of the random stream with the reference is not a goal (DESIGN.md section 1), parity GIVEN the mask is tested.
-__device__ __forceinline__ bool dropout_keep(uint32_t idx, uint32_t k0, uint32_t k1, uint32_t thresh) {
+__device__ __forceinline__ uint32_t hash32(uint32_t idx, uint32_t k0, uint32_t k1) {
   uint32_t x = idx ^ k0;
   x *= 0x9E3779B1u;
   x ^= x >> 16;
@@ -64,7 +64,18 @@ __device__ __forceinline__ bool dropout_keep(uint32_t idx, uint32_t k0, uint32_t
   x ^= x >> 13;
   x *= 0xC2B2AE35u;
   x ^= x >> 16;
-  return x < thresh;
+  return x;
+}
+__device__ __forceinline__ bool dropout_keep(uint32_t idx, uint32_t k0, uint32_t k1, uint32_t thresh) {
+  return hash32(idx, k0, k1) < thresh;
+}
+// The Gumbel-max score of a sampled pick (the rule at mmb_decoder_sample_fused): z = logf(p) inv_t - logf(-logf(u)) with the uniform
+// u = ((hash32(c, key) >> 9) + 0.5) 2^-23 of counter c.  Every step of u is exact in fp32 (23 bits plus the half), so u lies in
+// [2^-24, 1 - 2^-24] and -logf(-logf(u)) is finite: z is -inf for p = 0 and finite for p > 0.  (With 24 bits the top value would round
+// to u = 1 and give z = +inf.)  The roll-out kernel and mmb_sample_pick both call this one function, so both give the same bits.
+__device__ __forceinline__ float sample_score(float p, float inv_t, uint32_t c, uint32_t k0, uint32_t k1) {
+  const float u = ((float)(hash32(c, k0, k1) >> 9) + 0.5f) * 1.1920928955078125e-7f;
+  return logf(p) * inv_t - logf(-logf(u));
 }
 __host__ __device__ __forceinline__ uint32_t dropout_thresh(float keep_prob) {
   const double t = (double)keep_prob * 4294967296.0;

@@ -265,14 +265,39 @@ __device__ __forceinline__ void cand_warp_best(float& s, float& p, int& k, int& 
     if (cand_better(s2, p2, k2, m2, s, p, k, m)) { s = s2; p = p2; k = k2; m = m2; }
   }
 }
+// Sampled roll-outs (mmb_decoder_sample_fused; include/mmbidaf_b200.h states the rule): the greedy roll-out, or the constrained one,
+// with the pick drawn by Gumbel-max over the candidates instead of the arg-max.  Cluster r runs sample r % N of video r / N.  With
+// top_k > 0 the candidates are the best top_k by (p descending, m ascending), found after stage E by the beam's selection (each rank's
+// best top_k, then the merge of every rank's); the beam region's exchange arrays (`off`) hold them.
+struct SampleArgs {
+  const unsigned long long* key;                            // (1) on the device
+  float T;                                                  // temperature > 0
+  int N, top_k, off;                                        // samples per video; 0 or 1..MAXK; float offset of the exchange arrays
+};
+// The cluster's index in the grid (blockIdx.x / cluster size): in the sampled roll-out, roll-out b N + n.  Read where used (the
+// volatile read is not held in a register over the stages).
+__device__ __forceinline__ int cluster_row() {
+  unsigned r;
+  asm volatile("mov.u32 %0, %%clusterid.x;" : "=r"(r));
+  return (int)r;
+}
+// z of counter c (common.cuh::sample_score) with the key loaded and 1 / T formed where the pick is drawn (the volatile load keeps the
+// compiler from hoisting it into a register held over the step)
+__device__ __forceinline__ float sample_z(const SampleArgs& sp, float p, uint32_t c) {
+  unsigned long long key;
+  asm volatile("ld.global.nc.u64 %0, [%1];" : "=l"(key) : "l"(sp.key));
+  return sample_score(p, 1.f / sp.T, c, (uint32_t)key, (uint32_t)(key >> 32));
+}
 
 // kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one; kConstrained (with kGreedy): the pick skips
-// the sentences `cn` makes ineligible
-template <bool kGreedy, bool kBeam = false, bool kConstrained = false>
-__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn) {
+// the sentences `cn` makes ineligible; kSample (with kGreedy, not kBeam): the pick is drawn (`sp`)
+template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false>
+__device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn,
+                                               const SampleArgs sp) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
-  const int b = blockIdx.x / CL;
+  const int ob = blockIdx.x / CL;                         // the output row: the video (sampled: cluster_row(), the roll-out)
+  const int b = kSample ? cluster_row() / sp.N : ob;      // the video whose inputs the cluster reads
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int D = a.D, H = a.H, E = a.E, M = a.M, Lt = a.Lt, K = D + E + H;
 
@@ -320,7 +345,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   // beam: the region behind the base arrays (beam_floats)
   const int KW = kBeam ? bm.K : 1;
   const int ldh = up4(H), ldc = up4(split4(H, CL)), ldv = up4(a.chunk), ldp = up4((M + CL - 1) / CL);
-  float* const bs_score = smem + bm.off;                                 // [MAXK] the table: score,
+  float* const bs_score = smem + (kSample ? sp.off : bm.off);            // [MAXK] the table: score,
   int* const bs_tok = reinterpret_cast<int*>(bs_score + MAXK);           // [MAXK]   last token,
   int* const bs_stat = bs_tok + MAXK;                                    // [MAXK]   status
   float* const nt_score = bs_score + 3 * MAXK;                           // [MAXK] the next table: score,
@@ -350,6 +375,17 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   int* bk_nxt = bk_cur + MAXK;                                           //        and out
   uint32_t allow = 0;                                                    // greedy: eligible bits of this thread's sentences
   int kept = 0;                                                          // greedy: picks below EOS so far
+  // sampled: the key's halves and 1 / T.  The unconstrained roll-out holds them in registers; the constrained one, which also holds
+  // its eligible bits and kept count, forms them where a pick is drawn (sample_z): held, they take it past the 128 registers of a
+  // 512-thread CTA, and it spills
+  uint32_t key0 = 0, key1 = 0;
+  float inv_t = 1.f;
+  if constexpr (kSample && !kConstrained) {
+    const unsigned long long key = *sp.key;
+    key0 = (uint32_t)key;
+    key1 = (uint32_t)(key >> 32);
+    inv_t = 1.f / sp.T;
+  }
   if constexpr (kConstrained && !kBeam) {
     for (int m = e_m0 + tid, j = 0; m < e_m1; m += NT, ++j)
       if (allowed0(m)) allow |= 1u << j;
@@ -721,7 +757,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   if constexpr (kBeam)                     // (s_hn is written again only behind the cluster barriers of the next run)
     for (int i = tid; i < H; i += NT) s_bhn[slot * ldh + i] = s_hn[i];
   // greedy: the probabilities / arg-max of step s go to row (b, s) of (B, S, M) / (B, S); the loss terms (S, 2, B) to row s
-  const size_t prow = kGreedy ? (size_t)b * S + s : (size_t)b;
+  // (sampled: row (b N + n, s) of (B N, S, M) / (B N, S))
+  const size_t prow = kGreedy ? (size_t)(kSample ? cluster_row() : ob) * S + s : (size_t)b;
   const int lrow = kGreedy ? s * 2 * a.B + b : b;
   if (R == 0 && tid == 0 && a.cov_loss) {
     float cs = 0.f;
@@ -763,16 +800,28 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     int best_i = M;
     const int tg = a.target ? (int)a.target[kGreedy ? b * g.T + s : b] : -1;
     const bool eos_ok = kConstrained && !kBeam && eos_allowed(cn, eos, kept);
+    const uint32_t cbase = ((uint32_t)(kSample ? cluster_row() : 0) * (uint32_t)S + (uint32_t)s) * (uint32_t)M;   // sampled: the counter of sentence 0
     for (int m = m0 + tid; m < m1; m += NT) {
       const float p = expf(lg[m - m0] - gmx) * inv;
       if constexpr (kBeam) s_bp[slot * ldp + m - m0] = p;
       else a.probs[prow * M + m] = p;
-      if constexpr (kConstrained && !kBeam) {                    // the first maximum over the eligible sentences
+      if constexpr (kSample) {
+        // top_k = 0: the first maximum of z over the candidates (the first candidate stands even at z = -inf);
+        // top_k > 0: this rank's p for the selection below
+        const bool cand = !kConstrained || (((allow >> ((unsigned)(m - m0) / NT)) & 1u) && (m != eos || eos_ok));
+        if (sp.top_k > 0) {
+          lg[m - m0] = p;
+        } else if (cand) {
+          const float z = kConstrained ? sample_z(sp, p, cbase + (uint32_t)m) : sample_score(p, inv_t, cbase + (uint32_t)m, key0, key1);
+          if (z > best || best_i == M) { best = z; best_i = m; }
+        }
+      } else if constexpr (kConstrained && !kBeam) {             // the first maximum over the eligible sentences
         if (((allow >> ((unsigned)(m - m0) / NT)) & 1u) && (m != eos || eos_ok) && p > best) { best = p; best_i = m; }
       } else if (p > best) { best = p; best_i = m; }
       if (m == tg && a.nll) a.nll[lrow] = -logf(p + 1e-12f);      // models.py:168-170
     }
-    if (!kBeam && (kGreedy || a.argmax)) {                                  // first maximal index, as torch.max(dim) documents
+    // (sampled with top_k > 0: the pick is made after the step, by the selection)
+    if (!kBeam && (kGreedy || a.argmax) && !(kSample && sp.top_k > 0)) {     // first maximal index, as torch.max(dim) documents
       const float bbest = block_max(best, s_red);
       int cand = best == bbest ? best_i : M;
 #pragma unroll
@@ -821,21 +870,36 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   }
   if constexpr (kBeam) ++runs;
   }  // slots
-  if constexpr (kBeam) {
+  if constexpr (kBeam || kSample) {
     // ---- selection: the new table from the live slots' candidates and the finished slots' carries ---------------------------------
+    // (sampled, top_k > 0: the best top_k of this step's (p, sentence) candidates, and the draw among them)
     constexpr int kNone = 0x7fffffff;
     const int per = (M + CL - 1) / CL, m0 = min(M, R * per), m1 = min(M, m0 + per), nm = m1 - m0;
+    const int KS = kSample ? sp.top_k : KW;                      // the selection's width
+    // the exchange arrays (sampled: formed here from the parameter, so that nothing of them is held over the step's other stages)
+    float* const q_cand = kSample ? smem + sp.off + 7 * MAXK : s_cand;
+    float* const q_wred = kSample ? q_cand + MAXC * MAXK * 4 : s_wred;
+    float* const q_loc = kSample ? q_wred + NW * 4 : s_loc;
     bool any_live = false;
-    for (int k = 0; k < KW; ++k) any_live = any_live || bs_stat[k] == kLive;
-    __syncthreads();                                             // s_bp of the last run
+    if constexpr (kSample) any_live = sp.top_k > 0;             // (uniform)
+    else for (int k = 0; k < KW; ++k) any_live = any_live || bs_stat[k] == kLive;
+    __syncthreads();                                             // s_bp of the last run (sampled: this rank's p in s_cpart)
+    const bool eos_ok = kSample && kConstrained && eos_allowed(cn, eos, kept);
     if (any_live) {
       // this rank's best K of its (live slot, sentence) candidates, one block-wide pick per round; each pick ranks below the last
       float ps = INFINITY, pp = INFINITY;
       int pk = -1, pm = -1;
-      for (int r = 0; r < KW; ++r) {
+      for (int r = 0; r < KS; ++r) {
         float cs = -INFINITY, cp = -1.f;
         int ck = kNone, cm = kNone;
-        for (int c = tid; c < KW * nm; c += NT) {
+        for (int c = tid; c < (kSample ? nm : KW * nm); c += NT) {
+          if constexpr (kSample) {                               // ranked by p (as score and p), then sentence; k = 0
+            const int m = m0 + c;
+            if (kConstrained && (!((allow >> ((unsigned)c / NT)) & 1u) || (m == eos && !eos_ok))) continue;
+            const float p = s_cpart[c];
+            if (cand_better(ps, pp, pk, pm, p, p, 0, m) && cand_better(p, p, 0, m, cs, cp, ck, cm)) { cs = p; cp = p; ck = 0; cm = m; }
+            continue;
+          }
           const int k = c / nm, m = m0 + (c - k * nm);
           if (bs_stat[k] != kLive) continue;
           const float p = s_bp[k * ldp + m - m0];
@@ -849,46 +913,49 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         }
         cand_warp_best(cs, cp, ck, cm);
         if (lane == 0) {
-          s_wred[warp * 4 + 0] = cs; s_wred[warp * 4 + 1] = cp;
-          s_wred[warp * 4 + 2] = __int_as_float(ck); s_wred[warp * 4 + 3] = __int_as_float(cm);
+          q_wred[warp * 4 + 0] = cs; q_wred[warp * 4 + 1] = cp;
+          q_wred[warp * 4 + 2] = __int_as_float(ck); q_wred[warp * 4 + 3] = __int_as_float(cm);
         }
         __syncthreads();
         if (warp == 0) {
           float ws = -INFINITY, wp = -1.f;
           int wk = kNone, wm = kNone;
           if (lane < NW) {
-            ws = s_wred[lane * 4 + 0]; wp = s_wred[lane * 4 + 1];
-            wk = __float_as_int(s_wred[lane * 4 + 2]); wm = __float_as_int(s_wred[lane * 4 + 3]);
+            ws = q_wred[lane * 4 + 0]; wp = q_wred[lane * 4 + 1];
+            wk = __float_as_int(q_wred[lane * 4 + 2]); wm = __float_as_int(q_wred[lane * 4 + 3]);
           }
           cand_warp_best(ws, wp, wk, wm);
           if (lane == 0) {
-            s_loc[r * 4 + 0] = ws; s_loc[r * 4 + 1] = wp;
-            s_loc[r * 4 + 2] = __int_as_float(wk); s_loc[r * 4 + 3] = __int_as_float(wm);
+            q_loc[r * 4 + 0] = ws; q_loc[r * 4 + 1] = wp;
+            q_loc[r * 4 + 2] = __int_as_float(wk); q_loc[r * 4 + 3] = __int_as_float(wm);
           }
         }
         __syncthreads();
-        ps = s_loc[r * 4 + 0]; pp = s_loc[r * 4 + 1];
-        pk = __float_as_int(s_loc[r * 4 + 2]); pm = __float_as_int(s_loc[r * 4 + 3]);
+        ps = q_loc[r * 4 + 0]; pp = q_loc[r * 4 + 1];
+        pk = __float_as_int(q_loc[r * 4 + 2]); pm = __float_as_int(q_loc[r * 4 + 3]);
       }
-      for (int i = tid; i < CL * KW * 4; i += NT) {              // -> slot R of every rank
-        const int q = i / (KW * 4), e = i - q * KW * 4;
-        cluster.map_shared_rank(s_cand, q)[R * MAXK * 4 + e] = s_loc[e];
+      for (int i = tid; i < CL * KS * 4; i += NT) {              // -> slot R of every rank
+        const int q = i / (KS * 4), e = i - q * KS * 4;
+        cluster.map_shared_rank(q_cand, q)[R * MAXK * 4 + e] = q_loc[e];
       }
       cluster.sync();
     }
     // every rank merges the same entries in the same order: the ranks' best K (none when no slot is live), then the carries
-    if (warp == 0) {
-      const int npub = any_live ? CL * KW : 0, tot = npub + KW;
+    // (sampled: every warp, no carries; each of the best top_k is drawn for -- the largest z, ties to the smaller sentence)
+    float bz = -INFINITY;
+    int drawn = M;
+    if (kSample ? any_live : warp == 0) {
+      const int npub = any_live ? CL * KS : 0, tot = npub + (kSample ? 0 : KW);
       float ps = INFINITY, pp = INFINITY;
       int pk = -1, pm = -1;
-      for (int j = 0; j < KW; ++j) {
+      for (int j = 0; j < KS; ++j) {
         float cs = -INFINITY, cp = -1.f;
         int ck = kNone, cm = kNone;
         for (int i = lane; i < tot; i += 32) {
           float es, ep;
           int ek, em;
           if (i < npub) {
-            const float* e = s_cand + ((i / KW) * MAXK + i % KW) * 4;
+            const float* e = q_cand + ((i / KS) * MAXK + i % KS) * 4;
             es = e[0]; ep = e[1]; ek = __float_as_int(e[2]); em = __float_as_int(e[3]);
           } else {
             const int k = i - npub;
@@ -899,7 +966,13 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
           if (cand_better(ps, pp, pk, pm, es, ep, ek, em) && cand_better(es, ep, ek, em, cs, cp, ck, cm)) { cs = es; cp = ep; ck = ek; cm = em; }
         }
         cand_warp_best(cs, cp, ck, cm);
-        if (lane == 0) {
+        if constexpr (kSample) {
+          if (ck != kNone) {
+            const uint32_t c = ((uint32_t)cluster_row() * (uint32_t)S + (uint32_t)s) * (uint32_t)M + (uint32_t)cm;
+            const float z = kConstrained ? sample_z(sp, cp, c) : sample_score(cp, inv_t, c, key0, key1);
+            if (drawn == M || z > bz || (z == bz && cm < drawn)) { bz = z; drawn = cm; }
+          }
+        } else if (lane == 0) {
           // kind: 0 empty, 1 live, 2 finished by this step's EOS pick, 3 carried
           const bool none = ck == kNone;
           nt_score[j] = none ? -INFINITY : cs;
@@ -910,6 +983,21 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         ps = cs; pp = cp; pk = ck; pm = cm;
       }
     }
+    if constexpr (kSample) {
+      if (any_live) {                                            // the pick, as stage E takes it without top_k
+        int gi = drawn;
+        if constexpr (kConstrained) {
+          if (gi == M) gi = eos;                                 // no eligible sentence (the caller's mask hides rows below EOS)
+          if (gi < eos) {
+            ++kept;
+            const int j = gi - m0;                               // under no_repeat the pick is no longer eligible
+            if (cn.no_repeat && j >= 0 && gi < m1 && j % NT == tid) allow &= ~(1u << (j / NT));
+          }
+        }
+        if (R == 0 && tid == 0) a.argmax[(size_t)cluster_row() * S + s] = gi;
+        pick = gi;
+      }
+    } else {
     __syncthreads();
     // outputs of step s; the state of the new live slots gathered from their parents' step outputs; the new table
     const size_t row = ((size_t)b * S + s) * KW;
@@ -948,6 +1036,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       uint32_t* const t = bu_cur; bu_cur = bu_nxt; bu_nxt = t;
       int* const u = bk_cur; bk_cur = bk_nxt; bk_nxt = u;
     }
+    }  // (beam)
   }
   }  // steps (the loop body keeps the step kernel's indentation)
   if constexpr (kBeam) {
@@ -971,24 +1060,33 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
 }
 
 __global__ void __launch_bounds__(NT) dec_step_fused_kernel(const FusedArgs a) {
-  dec_fused_body<false>(a, GreedyArgs{}, BeamArgs{}, ConstraintArgs{});
+  dec_fused_body<false>(a, GreedyArgs{}, BeamArgs{}, ConstraintArgs{}, SampleArgs{});
 }
 
 __global__ void __launch_bounds__(NT) dec_greedy_fused_kernel(const FusedArgs a, const GreedyArgs g) {
-  dec_fused_body<true>(a, g, BeamArgs{}, ConstraintArgs{});
+  dec_fused_body<true>(a, g, BeamArgs{}, ConstraintArgs{}, SampleArgs{});
 }
 
 __global__ void __launch_bounds__(NT) dec_beam_fused_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm) {
-  dec_fused_body<true, true>(a, g, bm, ConstraintArgs{});
+  dec_fused_body<true, true>(a, g, bm, ConstraintArgs{}, SampleArgs{});
 }
 
 __global__ void __launch_bounds__(NT) dec_greedy_constrained_kernel(const FusedArgs a, const GreedyArgs g, const ConstraintArgs cn) {
-  dec_fused_body<true, false, true>(a, g, BeamArgs{}, cn);
+  dec_fused_body<true, false, true>(a, g, BeamArgs{}, cn, SampleArgs{});
 }
 
 __global__ void __launch_bounds__(NT) dec_beam_constrained_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm,
                                                                   const ConstraintArgs cn) {
-  dec_fused_body<true, true, true>(a, g, bm, cn);
+  dec_fused_body<true, true, true>(a, g, bm, cn, SampleArgs{});
+}
+
+__global__ void __launch_bounds__(NT) dec_sample_kernel(const FusedArgs a, const GreedyArgs g, const SampleArgs sp) {
+  dec_fused_body<true, false, false, true>(a, g, BeamArgs{}, ConstraintArgs{}, sp);
+}
+
+__global__ void __launch_bounds__(NT) dec_sample_constrained_kernel(const FusedArgs a, const GreedyArgs g, const ConstraintArgs cn,
+                                                                    const SampleArgs sp) {
+  dec_fused_body<true, false, true, true>(a, g, BeamArgs{}, cn, sp);
 }
 
 }  // namespace
@@ -1535,15 +1633,17 @@ static size_t beam_floats(int K, int CL, int chunk, int H, int M, bool constrain
 
 // Shape checks, cluster size, shared memory and row stage of the forward cluster kernels, then the launch: `g` null launches one step
 // (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel), or with `bm` the beam roll-out (dec_beam_fused_kernel);
-// with `cn` the constrained roll-out of either (dec_greedy_constrained_kernel, dec_beam_constrained_kernel).
+// with `cn` the constrained roll-out of either (dec_greedy_constrained_kernel, dec_beam_constrained_kernel); with `sp` (not `bm`) the
+// sampled roll-out (dec_sample_kernel, with `cn` dec_sample_constrained_kernel), one cluster per (video, sample).
 static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr,
-                        const ConstraintArgs* cn = nullptr) {
+                        const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
   MMB_REQUIRE(D <= 256, MMB_ERR_UNSUPPORTED, "%s: D=%d > 256", who, D);
+  const int rows = sp ? B * sp->N : B;     // clusters: one per video, or per (video, sample)
   // few videos: eight CTAs per video keep more of the chip busy on the text sweep
-  const int CL = (long long)B * 4 * 2 <= 160 ? 8 : 4;
+  const int CL = (long long)rows * 4 * 2 <= 160 ? 8 : 4;
   size_t smem = fused_smem_bytes(Lt, D, H, E, M, CL, &a.chunk);
   MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "%s: %zu B of shared memory (Lt=%d)", who, smem, Lt);
   // constrained greedy: a thread keeps the eligible bits of its sentences in one 32-bit register
@@ -1553,6 +1653,9 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
     smem = ((size_t)bm->off + beam_floats(bm->K, CL, a.chunk, H, M, cn != nullptr)) * 4 + 64;
     MMB_REQUIRE(smem <= 227 * 1024, MMB_ERR_UNSUPPORTED, "%s: width %d needs %zu B of shared memory per CTA, more than 232448 (B=%d Lt=%d M=%d)",
                 who, bm->K, smem, B, Lt, M);
+  } else if (sp) {                         // sampled: the beam region's tables and exchange arrays, no slots
+    sp->off = (int)((smem + 15) / 16 * 4);
+    smem = ((size_t)sp->off + beam_floats(0, CL, a.chunk, H, M)) * 4 + 64;
   }
   {
     // the row stage (see the kernel): two buffers of chunk x D floats behind two mbarriers, when they fit and bulk copies apply
@@ -1567,10 +1670,11 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[5] = {0, 0, 0, 0, 0};
-  const int which = bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
+  static size_t smem_set[7] = {0, 0, 0, 0, 0, 0, 0};
+  const int which = sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
   if (smem > smem_set[which]) {
-    const void* fn = which == 4 ? (const void*)dec_beam_constrained_kernel : which == 3 ? (const void*)dec_greedy_constrained_kernel
+    const void* fn = which == 6 ? (const void*)dec_sample_constrained_kernel : which == 5 ? (const void*)dec_sample_kernel
+                   : which == 4 ? (const void*)dec_beam_constrained_kernel : which == 3 ? (const void*)dec_greedy_constrained_kernel
                    : which == 2 ? (const void*)dec_beam_fused_kernel : which == 1 ? (const void*)dec_greedy_fused_kernel
                                 : (const void*)dec_step_fused_kernel;
     MMB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1584,7 +1688,7 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
     trace_set = true;
   }
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(B * CL));
+  cfg.gridDim = dim3((unsigned)(rows * CL));
   cfg.blockDim = dim3(NT);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = static_cast<cudaStream_t>(stream);
@@ -1595,6 +1699,14 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (sp && cn) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_sample_constrained_kernel, a, *g, *cn, *sp));
+    return check_launch("dec_sample_constrained_kernel");
+  }
+  if (sp) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_sample_kernel, a, *g, *sp));
+    return check_launch("dec_sample_kernel");
+  }
   if (cn && bm) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_constrained_kernel, a, *g, *bm, *cn));
     return check_launch("dec_beam_constrained_kernel");
@@ -1730,6 +1842,37 @@ extern "C" int mmb_decoder_beam_constrained_fused(const float* proj_a, const flo
   BeamArgs bm{text_len, tokens, parents, scores, probs, best, path, K, 0};
   const ConstraintArgs cn{text_len, no_repeat, min_sentences};
   return launch_fused(a, &g, "mmb_decoder_beam_constrained_fused", stream, &bm, &cn);
+}
+
+extern "C" int mmb_decoder_sample_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                        const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                        const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                        const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                        const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                        const uint8_t* mask, const int* text_len, const unsigned long long* key, float* probs,
+                                        long long* tokens, int B, int Lt, int D, int H, int E, int M, int S, int N, float T,
+                                        int top_k, int no_repeat, int min_sentences, mmb_stream_t stream) {
+  using namespace mmb;
+  const bool constrained = no_repeat != 0 || min_sentences != 0;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && key && probs && tokens &&
+                  (text_len || !constrained),
+              MMB_ERR_INVALID, "mmb_decoder_sample_fused: null pointer");
+  MMB_REQUIRE(S > 0 && N >= 1 && N <= 64 && T > 0.f && isfinite(T) && top_k >= 0 && top_k <= MAXK && (no_repeat == 0 || no_repeat == 1) &&
+                  min_sentences >= 0,
+              MMB_ERR_INVALID,
+              "mmb_decoder_sample_fused: S=%d, N=%d (1..64), T=%g (finite, > 0), top_k=%d (0..%d), no_repeat=%d (0 or 1), "
+              "min_sentences=%d (>= 0)", S, N, (double)T, top_k, MAXK, no_repeat, min_sentences);
+  MMB_REQUIRE(B > 0 && M > 0, MMB_ERR_INVALID, "mmb_decoder_sample_fused: B=%d M=%d", B, M);
+  MMB_REQUIRE((unsigned long long)B * N * S * M <= (1ull << 32), MMB_ERR_UNSUPPORTED,
+              "mmb_decoder_sample_fused: B N S M = %d x %d x %d x %d exceeds the 2^32 counters of a key", B, N, S, M);
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, probs, nullptr, nullptr, nullptr, nullptr, tokens,
+              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  const ConstraintArgs cn{text_len, no_repeat, min_sentences};
+  SampleArgs sp{key, T, N, top_k, 0};
+  return launch_fused(a, &g, "mmb_decoder_sample_fused", stream, nullptr, constrained ? &cn : nullptr, &sp);
 }
 
 extern "C" int mmb_decoder_bwd_head(const float* probs, const float* d_probs, const long long* target, const float* g_nll,

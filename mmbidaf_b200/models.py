@@ -144,7 +144,7 @@ class MMBiDAF(nn.Module):
         return torch.stack(out_distributions).transpose(0, 1), loss
 
     def summarize(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, targets=None, beam_width=None,
-                  no_repeat=False, min_sentences=0):
+                  no_repeat=False, min_sentences=0, num_samples=None, temperature=1.0, top_k=0, seed=None):
         """Extractive summaries of a batch (evaluate.py:107-126, :167-202 with method='greedy'): the eval-mode forward pass with the
         whole greedy decode roll-out on the device, then the greedy sentence selection on the device.  Runs under ``no_grad`` in eval
         mode and gives the caller's ``training`` flag back.  ``targets`` (B, T, 1) or (B, T) with T >= max_dec_len is optional (the
@@ -158,10 +158,16 @@ class MMBiDAF(nn.Module):
         ``no_repeat`` (bool) keeps a sentence out of the summary once it is in; ``min_sentences`` (int >= 0) keeps the EOS row from
         ending it before that many sentences (or every sentence of the transcript) are in.  Both constrain the greedy and the beam
         pick, inside the roll-out kernel (the rule at mmb_decoder_greedy_constrained_fused in include/mmbidaf_b200.h); the
-        distributions stay the model's.  Not with ``targets``.  With the defaults the launches are exactly the unconstrained ones."""
+        distributions stay the model's.  Not with ``targets``.  With the defaults the launches are exactly the unconstrained ones.
+        ``num_samples`` N (1..64) draws N summaries per video instead, in one launch (``MultimodalAttentionDecoder.sample``; the rule
+        at mmb_decoder_sample_fused in include/mmbidaf_b200.h): the pick of every step is drawn from p^(1/``temperature``) over the
+        candidates -- the ``top_k`` (0: off, else 1..8) likeliest, after the constraints.  ``seed`` None draws the key from the
+        device key stream (``ops.rng_next_keys``: fresh samples on every call and graph replay); an int seed reproduces its samples.
+        The summary is the likeliest sample's (highest ``Samples.logp``, ties to the lower n); ``samples`` holds all N.  Not with
+        ``beam_width`` or ``targets``."""
         from .layers.encoding import length_plan
-        from .summarize import Beams, Summary, check_options
-        check_options("summarize", targets is not None, beam_width, no_repeat, min_sentences)
+        from .summarize import Beams, Samples, Summary, best_sample, check_options, sample_logp
+        check_options("summarize", targets is not None, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed)
         constrained = no_repeat or min_sentences > 0
         was_training = self.training
         self.eval()
@@ -177,6 +183,15 @@ class MMBiDAF(nn.Module):
                     dec.prepare()
 
                 enc_a, enc_i, h0, mask = self._encode(text, text_len, audio, audio_len, images, image_len, decoder_start)
+                if num_samples is not None:
+                    lens = length_plan(text_len, text.device).len_i32
+                    key = ops.rng_next_keys(text.device, 1) if seed is None else ops.seed_key(seed, text.device)
+                    probs, tokens = dec.sample(text, h0, enc_a, enc_i, mask, lens, max_dec_len, num_samples, key, temperature, top_k,
+                                               no_repeat, min_sentences)
+                    samples = Samples(tokens, probs, sample_logp(probs, tokens, lens))
+                    sel, cnt = ops.greedy_select(tokens.view(B * num_samples, -1), lens.repeat_interleave(num_samples))
+                    best_probs, indices, counts = best_sample(samples, sel, cnt)
+                    return Summary(best_probs, None, indices, counts, None, samples)
                 if beam_width is not None:
                     lens = length_plan(text_len, text.device).len_i32
                     tokens, parents, scores, rows, best, path = dec.beam(text, h0, enc_a, enc_i, mask, lens, max_dec_len, beam_width,

@@ -7,6 +7,7 @@ this module (bench.py reports it as ``gpu_launches``).
 from __future__ import annotations
 
 import contextlib
+import math
 import os
 from typing import Optional, Tuple
 
@@ -464,6 +465,94 @@ def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps
         _lib.check(lib.mmb_decoder_beam_fused(*args, _lib.stream()), "mmb_decoder_beam_fused")
     _count(1)
     return tokens, parents, scores, probs, best, path
+
+
+SAMPLE_MAX_N, SAMPLE_MAX_TOP_K = 64, 8
+
+
+def check_sampling(who: str, num_samples, temperature, top_k) -> None:
+    """``num_samples`` an int in 1..64, ``temperature`` a finite number > 0, ``top_k`` an int in 0..8 (the rule at
+    mmb_decoder_sample_fused in include/mmbidaf_b200.h)."""
+    if isinstance(num_samples, bool) or not isinstance(num_samples, int) or not 1 <= num_samples <= SAMPLE_MAX_N:
+        raise ValueError(f"{who}: num_samples {num_samples!r}, expected an int in 1..{SAMPLE_MAX_N}")
+    if isinstance(temperature, bool) or not isinstance(temperature, (int, float)) or not math.isfinite(temperature) or temperature <= 0:
+        raise ValueError(f"{who}: temperature {temperature!r}, expected a finite number > 0")
+    if isinstance(top_k, bool) or not isinstance(top_k, int) or not 0 <= top_k <= SAMPLE_MAX_TOP_K:
+        raise ValueError(f"{who}: top_k {top_k!r}, expected an int in 0..{SAMPLE_MAX_TOP_K}")
+
+
+def decoder_sample_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, num_samples: int, key: torch.Tensor,
+                       temperature: float = 1.0, top_k: int = 0, no_repeat: bool = False, min_sentences: int = 0):
+    """N sampled roll-outs per video (the rule at mmb_decoder_sample_fused in include/mmbidaf_b200.h) as ONE launch of the cluster
+    kernel, whatever ``decoder_cut`` says.  Inputs as :func:`decoder_greedy_constrained_fwd` (text_len_i32 may be None without a
+    constraint), plus ``key`` (1) int64 on the device (:func:`rng_next_keys`, or a fill).  Returns (probs (B,N,S,M), tokens (B,N,S)
+    int64) -- each roll-out's distributions are the step kernel's, bit for bit."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    check_sampling("decoder_sample_fwd", num_samples, temperature, top_k)
+    _check_constraints("decoder_sample_fwd", no_repeat, min_sentences)
+    if int(steps) <= 0:
+        raise ValueError(f"decoder_sample_fwd: {steps} steps")
+    constrained = bool(no_repeat) or min_sentences > 0
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M) or \
+            (text_len_i32 is None and constrained) or (text_len_i32 is not None and text_len_i32.shape != (B,)):
+        raise ValueError(f"decoder_sample_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask {tuple(mask_u8.shape)}, "
+                         f"text_len {None if text_len_i32 is None else tuple(text_len_i32.shape)} for B={B} Lt={Lt} E={E} H={H} M={M}")
+    if text_len_i32 is not None and text_len_i32.dtype != torch.int32:
+        raise ValueError(f"decoder_sample_fwd: text_len {text_len_i32.dtype}, not int32")
+    if key.dtype != torch.int64 or key.numel() != 1 or key.device != dev:
+        raise ValueError(f"decoder_sample_fwd: key {key.dtype} {tuple(key.shape)} on {key.device}, expected one int64 on {dev}")
+    S, N = int(steps), int(num_samples)
+    probs = torch.empty(B, N, S, M, device=dev, dtype=torch.float32)
+    tokens = torch.empty(B, N, S, device=dev, dtype=torch.int64)
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_sample_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(key.contiguous()), p(probs),
+        p(tokens), B, Lt, D, H, E, M, S, N, float(temperature), int(top_k), int(no_repeat), int(min_sentences), _lib.stream()),
+        "mmb_decoder_sample_fused")
+    _count(1)
+    return probs, tokens
+
+
+def sample_pick(probs: torch.Tensor, key: torch.Tensor, row_base: torch.Tensor, S: int, s: int, N: int = 1, temperature: float = 1.0,
+                top_k: int = 0, eligible: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Steps 1 to 4 of the sampled pick (mmb_sample_pick) for the rows of ``probs`` (R, M) fp32: row r is sample r % N of video
+    ``row_base[r]`` (R int32) at step ``s`` of ``S``; ``eligible`` (R, M) bool / uint8 limits the candidates.  Returns picks (R) int64,
+    -1 for a row without a candidate -- the roll-out kernel's pick, bit for bit."""
+    check_sampling("sample_pick", N, temperature, top_k)
+    if probs.dtype != torch.float32 or probs.dim() != 2 or not probs.is_cuda:
+        raise ValueError(f"sample_pick: probs {probs.dtype} {tuple(probs.shape)} on {probs.device}, expected (R, M) fp32 on a GPU")
+    R, M = probs.shape
+    dev = probs.device
+    if row_base.dtype != torch.int32 or row_base.numel() != R or row_base.device != dev:
+        raise ValueError(f"sample_pick: row_base {row_base.dtype} {tuple(row_base.shape)} on {row_base.device} for {R} rows on {dev}")
+    if key.dtype != torch.int64 or key.numel() != 1 or key.device != dev:
+        raise ValueError(f"sample_pick: key {key.dtype} {tuple(key.shape)} on {key.device}, expected one int64 on {dev}")
+    if eligible is not None and (eligible.shape != (R, M) or eligible.device != dev or
+                                 eligible.dtype not in (torch.bool, torch.uint8)):
+        raise ValueError(f"sample_pick: eligible {eligible.dtype} {tuple(eligible.shape)} on {eligible.device}, expected (R, M) = "
+                         f"({R}, {M}) bool / uint8 on {dev}")
+    if not 0 <= int(s) < int(S):
+        raise ValueError(f"sample_pick: step {s} of {S}")
+    picks = torch.empty(R, device=probs.device, dtype=torch.int64)
+    _lib.check(_lib.lib().mmb_sample_pick(_lib.ptr(probs.contiguous()), _lib.ptr(_u8(eligible)), _lib.ptr(key.contiguous()),
+                                          _lib.ptr(row_base.contiguous()), R, M, int(S), int(s), int(N), float(temperature), int(top_k),
+                                          _lib.ptr(picks), _lib.stream()), "mmb_sample_pick")
+    _count(1)
+    return picks
+
+
+def seed_key(seed: int, device) -> torch.Tensor:
+    """The sampling key of an int seed: splitmix64 of the seed (so that nearby seeds give unrelated streams), written by a device
+    fill -- no host copy, so a CUDA graph captures it and every replay refills the same key."""
+    z = (int(seed) + 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & 0xFFFFFFFFFFFFFFFF
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & 0xFFFFFFFFFFFFFFFF
+    z ^= z >> 31
+    return torch.full((1,), z - (1 << 64) if z >= 1 << 63 else z, dtype=torch.int64, device=device)
 
 
 def greedy_select(argmax: torch.Tensor, text_len: torch.Tensor):

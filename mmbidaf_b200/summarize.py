@@ -2,9 +2,10 @@
 
 ``MMBiDAF.summarize`` runs the encoder half of the model, the whole greedy decode roll-out and the greedy sentence selection
 without a host round trip; its result is a :class:`Summary`.  With ``beam_width=K`` the roll-out is a beam search over K
-hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  ``no_repeat`` and
-``min_sentences`` constrain either pick inside the roll-out kernel.  :class:`Summarizer` replays ``summarize`` from CUDA graphs, one
-capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
+hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  With
+``num_samples=N`` N summaries per video are drawn inside one launch (temperature, top-k); the summary is the likeliest sample's, and
+:class:`Samples` holds all N.  ``no_repeat`` and ``min_sentences`` constrain any pick inside the roll-out kernel.
+:class:`Summarizer` replays ``summarize`` from CUDA graphs, one capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
 """
 from __future__ import annotations
 
@@ -13,16 +14,28 @@ from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 import torch
 import torch.distributed as dist
 
-from .ops import BEAM_MAX_WIDTH
+from .ops import BEAM_MAX_WIDTH, check_sampling
 from .synth import Batch
 
-__all__ = ["Beams", "Summary", "Summarizer", "gather_summaries"]
+__all__ = ["Beams", "Samples", "Summary", "Summarizer", "gather_summaries"]
 
 
-def check_options(who: str, with_targets: bool, beam_width, no_repeat, min_sentences) -> None:
+def check_options(who: str, with_targets: bool, beam_width, no_repeat, min_sentences, num_samples=None, temperature=1.0, top_k=0,
+                  seed=None) -> None:
     """The decode options of ``MMBiDAF.summarize`` / ``Summarizer``, checked before any device work: ``beam_width`` None or an int
     in 1..8, ``no_repeat`` a bool, ``min_sentences`` an int >= 0; neither a beam nor a constraint with targets (the eval loss is
-    defined by the unconstrained greedy roll-out)."""
+    defined by the unconstrained greedy roll-out).  Sampling: ``num_samples`` None or an int in 1..64, not with a beam or targets;
+    ``temperature`` finite and > 0, ``top_k`` an int in 0..8, ``seed`` None or an int -- set only with ``num_samples``."""
+    if num_samples is not None:
+        check_sampling(who, num_samples, temperature, top_k)
+        if beam_width is not None:
+            raise ValueError(f"{who}: num_samples with beam_width -- sampling and beam search are separate decodes")
+        if with_targets:
+            raise ValueError(f"{who}: num_samples with targets -- the eval loss is defined by the greedy roll-out")
+        if seed is not None and (isinstance(seed, bool) or not isinstance(seed, int)):
+            raise ValueError(f"{who}: seed {seed!r}, expected None or an int")
+    elif temperature != 1.0 or top_k != 0 or seed is not None:
+        raise ValueError(f"{who}: temperature / top_k / seed without num_samples")
     if beam_width is not None:
         if isinstance(beam_width, bool) or not isinstance(beam_width, int) or not 1 <= beam_width <= BEAM_MAX_WIDTH:
             raise ValueError(f"{who}: beam_width {beam_width!r}, expected None or an int in 1..{BEAM_MAX_WIDTH}")
@@ -82,12 +95,46 @@ class Beams(NamedTuple):
         return [[(_select(row, lens[b]), score) for row, score in hyps] for b, hyps in enumerate(self.paths())]
 
 
+class Samples(NamedTuple):
+    """Every sampled roll-out (``MMBiDAF.summarize(..., num_samples=N)``, the rule at mmb_decoder_sample_fused in
+    include/mmbidaf_b200.h)."""
+    tokens: torch.Tensor                   # (B, N, S) int64: the picks of sample n of video b
+    probs: torch.Tensor                    # (B, N, S, M) fp32: its distribution at every step
+    logp: torch.Tensor                     # (B, N) fp32: sum of log p_s[tok_s] up to and including its first EOS pick (all S without)
+
+    def summaries(self, text_len: Sequence[int]) -> List[List[Tuple[List[int], float]]]:
+        """Per video, every sample in order: (chosen sentence indices under the greedy_search rule, logp).  ``text_len`` (B) gives
+        each video's EOS row (text_len - 1)."""
+        lens = [int(n) for n in (text_len.tolist() if torch.is_tensor(text_len) else text_len)]
+        tok, lp = self.tokens.cpu().tolist(), self.logp.cpu().tolist()
+        return [[(_select(row, lens[b]), lp[b][n]) for n, row in enumerate(rows)] for b, rows in enumerate(tok)]
+
+
+def sample_logp(probs: torch.Tensor, tokens: torch.Tensor, text_len_i32: torch.Tensor) -> torch.Tensor:
+    """logp (B, N) fp32 of sampled roll-outs: the sum of log p_s[tok_s] over the steps up to and including the first EOS pick
+    (text_len - 1), or over all S without one.  Device ops only (capturable)."""
+    lp = torch.log(probs.gather(3, tokens.clamp_min(0).unsqueeze(3)).squeeze(3))               # (B, N, S)
+    hit = (tokens == (text_len_i32.long() - 1).view(-1, 1, 1)).long()
+    after = (hit.cumsum(2) - hit) > 0                                                          # steps after the first EOS pick
+    return torch.where(after, torch.zeros_like(lp), lp).sum(2)
+
+
+def best_sample(samples: Samples, sel: torch.Tensor, count: torch.Tensor):
+    """The likeliest sample of every video (highest logp, ties to the lower n): (its distributions (B, S, M), its indices (B, S) and
+    count (B) out of ``sel`` (B N, S) / ``count`` (B N), the greedy selection over every sample's tokens)."""
+    B, N, S = samples.tokens.shape
+    best = samples.logp.argmax(1)                          # the first maximal n
+    rows = torch.arange(B, device=best.device)
+    return samples.probs[rows, best], sel.view(B, N, S)[rows, best], count.view(B, N)[rows, best]
+
+
 class Summary(NamedTuple):
     out_distributions: torch.Tensor        # (B, S, M) fp32: every step's distribution over the sentences, as MMBiDAF.forward returns
     loss: Optional[torch.Tensor]           # the eval loss (models.py:197-199) when targets were given, else None
     indices: torch.Tensor                  # (B, S) int32: the chosen sentence indices of every video, padded with -1
     counts: torch.Tensor                   # (B) int32: how many of them are valid
     beams: Optional[Beams] = None          # a beam summary's every slot (then out_distributions are the best path's rows), else None
+    samples: Optional[Samples] = None      # a sampled summary's every sample (then the other fields are the likeliest sample's), else None
 
     def to_lists(self) -> List[List[int]]:
         """The chosen sentence indices per video as host lists (copies only ``indices`` and ``counts``):
@@ -96,16 +143,17 @@ class Summary(NamedTuple):
         return [idx[b, :c].tolist() for b, c in enumerate(cnt)]
 
 
-def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int], no_repeat: bool = False, min_sentences: int = 0):
+def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int], no_repeat: bool = False, min_sentences: int = 0,
+                sampling: tuple = (None, 1.0, 0, None)):
     return (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), int(batch.max_dec_len),
-            tuple(batch.targets.shape) if with_targets else None, beam_width, no_repeat, min_sentences)
+            tuple(batch.targets.shape) if with_targets else None, beam_width, no_repeat, min_sentences, sampling)
 
 
 class _Bucket:
     """One captured ``summarize``: static inputs, static length plans, the graph and its (static) result."""
 
     def __init__(self, model, batch: Batch, with_targets: bool, warmup: int, beam_width: Optional[int] = None,
-                 no_repeat: bool = False, min_sentences: int = 0):
+                 no_repeat: bool = False, min_sentences: int = 0, sampling: tuple = (None, 1.0, 0, None)):
         import gc
         from .layers.encoding import pin_lengths
         dev = batch.text.device
@@ -115,6 +163,7 @@ class _Bucket:
         self.with_targets = with_targets
         self.beam_width = beam_width
         self.no_repeat, self.min_sentences = no_repeat, min_sentences
+        self.sampling = sampling             # (num_samples, temperature, top_k, seed); seed None: the key state exists after warm-up
         self.plans = [pin_lengths(lst, dev) for lst in (self.batch.text_len, self.batch.audio_len, self.batch.image_len)]
         for m in model.modules():          # per-sequence caches of eager calls still own tensors (see Trainer.capture)
             if hasattr(m, "_cache"):
@@ -137,7 +186,8 @@ class _Bucket:
         b = self.batch
         return model.summarize(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, b.max_dec_len,
                                b.targets if self.with_targets else None, beam_width=self.beam_width, no_repeat=self.no_repeat,
-                               min_sentences=self.min_sentences)
+                               min_sentences=self.min_sentences, num_samples=self.sampling[0], temperature=self.sampling[1],
+                               top_k=self.sampling[2], seed=self.sampling[3])
 
     def load(self, batch: Batch) -> None:
         if batch is self.batch:
@@ -165,15 +215,20 @@ class Summarizer:
         self.buckets: Dict[tuple, _Bucket] = {}
 
     def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None, no_repeat: bool = False,
-                 min_sentences: int = 0) -> Summary:
+                 min_sentences: int = 0, num_samples: Optional[int] = None, temperature: float = 1.0, top_k: int = 0,
+                 seed: Optional[int] = None) -> Summary:
         """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``; ``beam_width``
         decodes by beam search, ``no_repeat`` / ``min_sentences`` constrain the pick (``MMBiDAF.summarize``); each width and each
-        setting of the constraints in its own bucket.  The options are checked before anything is copied or captured."""
-        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences)
-        key = _bucket_key(batch, with_targets, beam_width, no_repeat, min_sentences)
+        setting of the constraints in its own bucket.  ``num_samples`` / ``temperature`` / ``top_k`` / ``seed`` sample (each setting,
+        the seed included, in its own bucket): with ``seed=None`` every replay draws a fresh key from the device key stream, with an int
+        seed every replay gives that seed's samples.  The options are checked before anything is copied or captured."""
+        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed)
+        sampling = (num_samples, temperature, top_k, seed)
+        key = _bucket_key(batch, with_targets, beam_width, no_repeat, min_sentences, sampling)
         bucket = self.buckets.get(key)
         if bucket is None:
-            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup, beam_width, no_repeat, min_sentences)
+            bucket = self.buckets[key] = _Bucket(self.model, batch, with_targets, self.warmup, beam_width, no_repeat, min_sentences,
+                                                 sampling)
         else:
             bucket.load(batch)
         bucket.graph.replay()
