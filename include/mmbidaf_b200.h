@@ -172,8 +172,12 @@ MMB_API int mmb_decoder_chunks(int B, int Lt);
  * pb (2,B,D), xcat (B,D+E+H) = [c3 | sent | h], gates (B,4H) activated.  argmax, target / nll and cov_loss may be NULL.
  * When D is a multiple of 4 and proj / enc are 16-byte aligned, each CTA stages its rows of proj_a / proj_i (then enc_a / enc_i) in shared
  * memory by bulk copies issued at kernel start (two buffers of ceil(Lt / cluster) x D floats; skipped when they do not fit in 227 KB, and
- * with MMB_DEC_STAGE=0): same results, fewer L2 round trips.  mmb_decoder_step_fused_bwd stages enc then proj the same way and adds its
- * d z rows into d_proj_a / d_proj_i with one bulk reduction per modality (d_proj_* must then be 16-byte aligned too).
+ * with MMB_DEC_STAGE=0, read once per process): the results of reading the rows from L2 (bit for bit when D >= 86, where the backward's
+ * mat-vecs split K the same way on both), with fewer L2 round trips.
+ * mmb_decoder_step_fused_bwd stages enc then proj the same way and adds its d z rows into d_proj_a / d_proj_i with one bulk reduction
+ * per modality (d_proj_* must then be 16-byte aligned too).  Rows need only 4-byte alignment: when enc_a / enc_i are not 16-byte aligned
+ * (or D is not a multiple of 4) the weighted contexts read them one float at a time, in this kernel and in mmb_decoder_attn_fwd, which
+ * splits the rows over the threads differently: the same values up to fp32 rounding, not bit for bit.
  */
 MMB_API int mmb_decoder_step_fused_fwd(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
                                        const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,

@@ -87,6 +87,7 @@ struct FusedArgs {
   float *hw, *alpha, *beta, *ctx12, *pb, *xcat, *gates;     // (B,4D), (B,2,Lt), (B,2), (2,B,D), (2,B,D), (B,D+E+H), (B,4H)
   int B, Lt, D, H, E, M, chunk;
   int stage_off;   // float offset of the row stage in dynamic shared memory ([2 mbarriers][2][chunk * D]), or 0: rows read from L2
+  int ctx_vec4;    // 1: the weighted contexts read enc_a / enc_i rows as float4 (D % 4 == 0 and both 16-byte aligned), 0: as floats
 };
 
 // y[i] = sum_k Wt[k][col_of(i)] x[k] + bias[col_of(i)] for i < n_out, with the weights TRANSPOSED (Wt (K, ldn): consecutive threads read
@@ -566,7 +567,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     if (staged && n > 0) tc::mbar_wait(bar_enc, parity);
     const float* ea = staged ? s_st0 : a.enc_a + ((size_t)b * Lt + t0) * D;
     const float* ei = staged ? s_st1 : a.enc_i + ((size_t)b * Lt + t0) * D;
-    const bool vec4 = (D & 3) == 0;
+    const bool vec4 = a.ctx_vec4 != 0;       // (staged rows are always aligned; rows read from L2 may not be)
     const int groups = vec4 ? NT / (D >> 2) : NT / D;
     if (vec4) {
       const int dv4 = D >> 2;
@@ -1659,12 +1660,15 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   }
   {
     // the row stage (see the kernel): two buffers of chunk x D floats behind two mbarriers, when they fit and bulk copies apply
-    // (16-byte row granularity).  MMB_DEC_STAGE=0 turns it off (A/B measurements, cross-check in tests/test_decoder_gpu.py).
+    // (16-byte row granularity).  MMB_DEC_STAGE=0 turns it off (A/B measurements; read once per process, on the first launch: the
+    // cross-check in tests/test_decoder_paths_gpu.py sets it in a child process).
     static const char* stage_env = getenv("MMB_DEC_STAGE");
     const size_t base_floats = (smem + 15) / 16 * 4;
     const size_t stage_floats = 4 + 2 * (((size_t)a.chunk * D + 3) & ~(size_t)3);
-    const bool aligned = ((reinterpret_cast<uintptr_t>(a.proj_a) | reinterpret_cast<uintptr_t>(a.proj_i) |
-                           reinterpret_cast<uintptr_t>(a.enc_a) | reinterpret_cast<uintptr_t>(a.enc_i)) & 15) == 0;
+    const bool enc_aligned = ((reinterpret_cast<uintptr_t>(a.enc_a) | reinterpret_cast<uintptr_t>(a.enc_i)) & 15) == 0;
+    const bool aligned = enc_aligned && ((reinterpret_cast<uintptr_t>(a.proj_a) | reinterpret_cast<uintptr_t>(a.proj_i)) & 15) == 0;
+    // with D % 4 == 0 every row start keeps the base pointer's alignment: float4 context loads when the bases are 16-byte aligned
+    a.ctx_vec4 = (D & 3) == 0 && enc_aligned;
     if ((D & 3) == 0 && aligned && (base_floats + stage_floats) * 4 <= 227 * 1024 && !(stage_env && atoi(stage_env) == 0)) {
       a.stage_off = (int)base_floats;
       smem = (base_floats + stage_floats) * 4;
@@ -1949,7 +1953,7 @@ extern "C" int mmb_decoder_step_fused_bwd(const float* probs, const float* d_pro
   MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "mmb_decoder_step_fused_bwd: %zu B of shared memory (Lt=%d)", smem, Lt);
   {
     // the row stage (see the kernel): two buffers of chunk x D floats behind two mbarriers; the column-partial reduction then runs in two
-    // passes over half the buffer.  MMB_DEC_STAGE=0 turns it off.
+    // passes over half the buffer.  MMB_DEC_STAGE=0 turns it off (read once per process, as in launch_fused).
     static const char* stage_env = getenv("MMB_DEC_STAGE");
     const size_t base_floats = (head_smem_bytes(D, H, M, CL, chunk, true, NW / 2) - 64) / 4;
     const size_t stage_floats = 4 + 2 * (((size_t)chunk * D + 3) & ~(size_t)3);

@@ -111,6 +111,7 @@ struct PartialArgs {
   float *ctx12, *scale;      // written by the last chunk block of each video (combine_video)
   int* counters;             // (B) zero on entry, zero on exit
   int B, Lt, D, chunk, nch;
+  int vec4;                  // 1: the weighted contexts read enc_a / enc_i rows as float4 (D % 4 == 0 and both 16-byte aligned)
 };
 
 __global__ void __launch_bounds__(NT) dec_attn_partial_kernel(const PartialArgs a) {
@@ -119,7 +120,7 @@ __global__ void __launch_bounds__(NT) dec_attn_partial_kernel(const PartialArgs 
   const int t0 = c * a.chunk, t1 = min(Lt, t0 + a.chunk), n = t1 - t0;
   extern __shared__ __align__(16) float smem[];
   float* part = smem;                    // [groups][2][D]  (16-byte aligned, float4 path)
-  const bool vec4 = (D & 3) == 0;
+  const bool vec4 = a.vec4 != 0;
   const int groups = vec4 ? NT / (D >> 2) : NT / D;
   float* vec = part + groups * 2 * D;    // [6][D]: v1 | wc1 | hw1 | v2 | wc2 | hw2
   float* red = vec + 6 * D;              // [32]
@@ -715,9 +716,11 @@ extern "C" int mmb_decoder_attn_fwd(const float* proj_a, const float* proj_i, co
   MMB_REQUIRE(D <= NT, MMB_ERR_UNSUPPORTED, "mmb_decoder_attn_fwd: 2H=%d > %d", D, NT);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int chunk = (Lt + nch - 1) / nch;
+  // with D % 4 == 0 every row start keeps the base pointer's alignment: float4 context loads when the bases are 16-byte aligned
+  const int vec4 = D % 4 == 0 && ((reinterpret_cast<uintptr_t>(enc_a) | reinterpret_cast<uintptr_t>(enc_i)) & 15) == 0;
   PartialArgs a{proj_a, proj_i, enc_a, enc_i, hw, coverage, v1, wc1, v2, wc2, v1b, v2b, p, stats, ctxp, ctx12, scale, counters,
-                B, Lt, D, chunk, nch};
-  const int groups = (D % 4 == 0) ? NT / (D / 4) : NT / D;
+                B, Lt, D, chunk, nch, vec4};
+  const int groups = vec4 ? NT / (D / 4) : NT / D;
   const size_t smem = sizeof(float) * ((size_t)groups * 2 * D + 6 * D + 32 + 2 * chunk);
   MMB_REQUIRE(smem <= 227 * 1024, MMB_ERR_UNSUPPORTED, "mmb_decoder_attn_fwd: chunk %d too large", chunk);
   MMB_CUDA(cudaFuncSetAttribute(dec_attn_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
