@@ -722,10 +722,11 @@ int launch(const LstmArgs& a, bool backward, cudaStream_t stream) {
   // Opt-in (MMB_LSTM_PAIR=1).  Measured (B = 32, H = 100): 0.62 instead of 0.67 us per step for ONE layer alone -- the step is bound by
   // its dependent chain (LDS -> 52-deep FMA chains -> shuffles -> activations -> barrier), not by issue slots, so halving the warps per
   // scheduler buys 7 % -- but a pair takes 128 SMs per layer and the training step runs three encoders side by side (384 CTAs on 296
-  // slots): 5 870 instead of 6 186 videos/s.  Kept as a measured alternative, off by default.
+  // slots): 5 870 instead of 6 186 videos/s.  Kept as a measured alternative, off by default.  The pair kernel writes neither the
+  // dropped output `y` nor trace stamps: a layer with output dropout, or a traced launch, takes the single-CTA kernel below.
   const char* pair_env = getenv("MMB_LSTM_PAIR");
   const bool pair_ok = pair_env && atoi(pair_env) != 0;
-  if (!backward && NB == 1 && pair_ok && a.H >= 32 && 2 * a.B * a.ndir <= 2 * 148) {
+  if (!backward && NB == 1 && pair_ok && !a.y && !a.trace && a.H >= 32 && 2 * a.B * a.ndir <= 2 * 148) {
     // two CTAs per (sequence, direction): see bilstm_fwd_pair_kernel
     const int pthr = threads_for(KS / 2 + 1);
     const int UH = (a.H + 1) / 2;
