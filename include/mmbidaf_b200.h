@@ -306,6 +306,42 @@ MMB_API int mmb_decoder_sample_fused(const float* proj_a, const float* proj_i, c
 MMB_API int mmb_sample_pick(const float* probs, const uint8_t* eligible, const unsigned long long* key, const int32_t* row_base, int R,
                             int M, int S, int s, int N, float T, int top_k, long long* picks, mmb_stream_t stream);
 /*
+ * Nucleus (top-p) summary roll-outs: mmb_decoder_sample_fused with the draw limited to the smallest set of the likeliest candidates
+ * that holds top_p of their mass, cut inside the same one-launch cluster kernel.  This is the project's own rule.  Per step of roll-out
+ * (b, n), the candidates C are step 1 of the sampled rule above (every sentence or the eligible ones, cut to the first top_k in
+ * (p descending, m ascending) order when top_k > 0).  Then, for top_p < 1:
+ *   1. Each candidate has the integer mass q[m] = floor(p[m] 2^24), exact from the fp32 p; Q = sum of q over C.
+ *   2. P = rint(top_p 2^24) from the fp32 top_p (round half to even).
+ *   3. The NUCLEUS is the first n candidates in that order, n the smallest n >= 1 with 2^24 (sum of the first n q) >= P Q.  Integer
+ *      sums do not depend on their order: the set is the same however the cluster splits the sentences, and a host recomputes it
+ *      exactly from the probs the kernel writes.
+ *   4. The draw is steps 2 to 4 of the sampled rule over the nucleus: the largest z = logf(p) (1 / T) - logf(-logf(u)), same counter
+ *      and key, ties to the smaller m; no candidate: eos.
+ * The nucleus is cut from the model's p, not from p^(1/T): the set comes from the model and T only shapes the draw inside it.  (This
+ * differs from tempering first and cutting after, when T != 1.)  So P Q <= 2^24 q of the first candidate gives n = 1, and the pick is
+ * the (constrained) greedy pick whatever T and the key; a small enough top_p always gets there.  top_p = 1 is no cut: the call is
+ * mmb_decoder_sample_fused's, with its samples bit for bit (a cut at P = 2^24 would drop candidates whose q is 0).
+ * Arguments of mmb_decoder_sample_fused plus top_p.  MMB_ERR_INVALID: top_p outside (0, 1], or any error of mmb_decoder_sample_fused;
+ * MMB_ERR_UNSUPPORTED: M >= 65536 with top_p < 1 (P Q must fit 64 bits), a row of M floats that does not fit in shared memory beside
+ * the step's arrays, or any reason of mmb_decoder_sample_fused.
+ */
+MMB_API int mmb_decoder_sample_nucleus_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                             const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                             const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                             const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                             const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                             const uint8_t* mask, const int32_t* text_len, const unsigned long long* key, float* probs,
+                                             long long* tokens, int B, int Lt, int D, int H, int E, int M, int S, int N, float T,
+                                             int top_k, int no_repeat, int min_sentences, float top_p, mmb_stream_t stream);
+/*
+ * mmb_sample_pick with the nucleus rule above: the reference of the tests for mmb_decoder_sample_nucleus_fused.  top_p = 1 is
+ * mmb_sample_pick.  MMB_ERR_INVALID: top_p outside (0, 1] or any error of mmb_sample_pick; MMB_ERR_UNSUPPORTED: M >= 65536 with
+ * top_p < 1.
+ */
+MMB_API int mmb_sample_pick_nucleus(const float* probs, const uint8_t* eligible, const unsigned long long* key, const int32_t* row_base,
+                                    int R, int M, int S, int s, int N, float T, int top_k, long long* picks, float top_p,
+                                    mmb_stream_t stream);
+/*
  * Greedy sentence selection (evaluate.py:185-202, decode.greedy_search) on the device.  Per video, in step order over argmax (B,S):
  * the EOS row text_len[b] - 1 ends the summary, an index past it is skipped, any other is kept (repeats too).
  *   sel (B,S) int32 = the kept indices, then -1;  count (B) int32 = how many were kept.

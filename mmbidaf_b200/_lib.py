@@ -44,6 +44,8 @@ SIGNATURES = {
     "mmb_decoder_beam_constrained_fused": [c_void_p] * 31 + [c_int] * 10 + [c_void_p],
     "mmb_decoder_sample_fused": [c_void_p] * 28 + [c_int] * 8 + [c_float] + [c_int] * 3 + [c_void_p],
     "mmb_sample_pick": [c_void_p] * 4 + [c_int] * 5 + [c_float, c_int, c_void_p, c_void_p],
+    "mmb_decoder_sample_nucleus_fused": [c_void_p] * 28 + [c_int] * 8 + [c_float] + [c_int] * 3 + [c_float, c_void_p],
+    "mmb_sample_pick_nucleus": [c_void_p] * 4 + [c_int] * 5 + [c_float, c_int, c_void_p, c_float, c_void_p],
     "mmb_greedy_select": [c_void_p] * 4 + [c_int] * 2 + [c_void_p],
     "mmb_decoder_bwd_head": [c_void_p] * 25 + [c_int] + [c_void_p] + [c_int] + [c_void_p] * 7 + [c_int] * 5 + [c_void_p],
     "mmb_decoder_attn_fwd": [c_void_p] * 18 + [c_int] * 4 + [c_void_p],

@@ -290,11 +290,135 @@ __device__ __forceinline__ float sample_z(const SampleArgs& sp, float p, uint32_
   return sample_score(p, 1.f / sp.T, c, (uint32_t)key, (uint32_t)(key >> 32));
 }
 
+// Nucleus roll-outs (mmb_decoder_sample_nucleus_fused; include/mmbidaf_b200.h states the rule): the sampled roll-out with the draw
+// limited to the nucleus, the first n candidates in (p descending, m ascending) order whose integer masses q = floor(p 2^24) reach
+// need = ceil(P Q / 2^24).  With top_k = 0 every rank writes its candidates' p into every rank's copy of the row (`off`: [M] floats,
+// -1 for a non-candidate) and, after one cluster barrier, each rank cuts the same row by itself (nucleus_cut); with top_k > 0 the
+// cut is a prefix of the merged top_k entries.
+struct NucleusArgs {
+  uint32_t P;                                               // rint(top_p 2^24), below 2^24 (top_p = 1 runs dec_sample_kernel)
+  int off;                                                  // float offset of the nucleus region (nucleus_floats)
+};
+constexpr int kNucBuckets = 256;                            // radix digits of 8 bits, four passes over the bits of p
+
+// The nucleus of row v[0..M) (v[m] = p, or -1 for a non-candidate), in every thread of the block: its boundary p* (as bits) and m*, so
+// that the nucleus is {m : v[m] > p*} + {m : v[m] == p*, m <= m*}.  The masses are integers, so every sum below is exact in any order:
+// each rank of the cluster cuts its copy of the row to the same set.
+//  * need = 0 (P Q < 2^24, Q = 0 included): the first candidate, the largest p with the smallest m (n = 1).
+//  * else p* is radix-selected on the bits of p (monotone for p >= 0), top digit first: a pass histograms the mass q of the candidates
+//    under the prefix found so far by digit, and takes the digit where the mass from above reaches what is still needed (`rem`).
+//    Candidates with q = 0 are never needed: the mass is reached at a candidate with q* > 0.  Then ceil(rem / q*) ties at p* are
+//    needed, and m* is the m of the last of them, found by a block prefix count over contiguous m ranges.
+// hist: kNucBuckets u64; red: 32 u64 (warp totals and broadcasts).  Ends behind a block barrier.
+struct NucleusCut {
+  uint32_t pstar;                                           // bits of p*
+  int mstar;                                                // -1: no candidate
+};
+__device__ __forceinline__ NucleusCut nucleus_cut(const float* __restrict__ v, int M, uint32_t P, unsigned long long* hist,
+                                                  unsigned long long* red) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  uint32_t prefix = 0, pmask = 0;
+  unsigned long long rem = 0;
+  bool first = false;
+  for (int pass = 0; pass < 4; ++pass) {
+    const int shift = 24 - 8 * pass;
+    if (tid < kNucBuckets) hist[tid] = 0ull;
+    __syncthreads();
+    // (flat rows put most candidates under one digit: the lanes of a digit add their masses first, one shared atomic per digit and
+    // warp instead of one per candidate -- a warp's masses stay below 2^29)
+    for (int m0 = 0; m0 < M; m0 += NT) {
+      const int m = m0 + tid;
+      const float p = m < M ? v[m] : -1.f;
+      const uint32_t bits = __float_as_uint(p);
+      uint32_t q = __float2uint_rz(p * 16777216.f);                    // (a non-candidate's -1 gives q = 0)
+      const bool in = q != 0u && (bits & pmask) == prefix;
+      const uint32_t digit = in ? (bits >> shift) & (kNucBuckets - 1) : kNucBuckets;
+      q = in ? q : 0u;
+      const uint32_t peers = __match_any_sync(0xffffffffu, digit);
+      const uint32_t sum = __reduce_add_sync(peers, q);
+      if (in && lane == __ffs(peers) - 1) atomicAdd(hist + digit, (unsigned long long)sum);
+    }
+    __syncthreads();
+    // suffix sums: thread t < 256 holds digit 255 - t, an inclusive scan over the threads
+    const unsigned long long h = tid < kNucBuckets ? hist[kNucBuckets - 1 - tid] : 0ull;
+    unsigned long long s = h;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned long long t = __shfl_up_sync(0xffffffffu, s, o);
+      if (lane >= o) s += t;
+    }
+    if (lane == 31 && warp < kNucBuckets / 32) red[warp] = s;
+    __syncthreads();
+    unsigned long long below = 0, total = 0;
+    for (int w = 0; w < kNucBuckets / 32; ++w) {
+      below += w < warp ? red[w] : 0ull;
+      total += red[w];
+    }
+    s += below;
+    if (pass == 0) {                                         // total = Q, the same in every thread
+      const unsigned long long pq = (unsigned long long)P * total;
+      rem = (pq >> 24) + ((pq & 0xffffffull) != 0ull);       // need
+      if (rem == 0ull) { first = true; break; }
+    }
+    if (tid < kNucBuckets && s - h < rem && rem <= s) {     // the one digit where the mass from above reaches rem
+      red[8] = (unsigned long long)(kNucBuckets - 1 - tid);
+      red[9] = rem - (s - h);
+    }
+    __syncthreads();
+    prefix |= (uint32_t)red[8] << shift;
+    pmask |= (uint32_t)(kNucBuckets - 1) << shift;
+    rem = red[9];
+  }
+  unsigned long long ties = 1;
+  if (first) {                                               // the largest p over the candidates (0 bits also when there is none)
+    uint32_t mx = 0;
+    for (int m = tid; m < M; m += NT) {
+      const float p = v[m];
+      if (p >= 0.f) mx = max(mx, __float_as_uint(p));
+    }
+    mx = __reduce_max_sync(0xffffffffu, mx);
+    __syncthreads();
+    if (lane == 0) red[warp] = mx;
+    __syncthreads();
+    prefix = 0;
+    for (int w = 0; w < NW; ++w) prefix = max(prefix, (uint32_t)red[w]);
+  } else {
+    const unsigned long long qs = __float2uint_rz(__uint_as_float(prefix) * 16777216.f);
+    ties = (rem + qs - 1) / qs;
+  }
+  // m*: the ties-th m (ascending) with v[m] == p*; thread t counts the ties in its range [t c, t c + c)
+  const int c = (M + NT - 1) / NT, lo = min(M, tid * c), hi = min(M, lo + c);
+  int cnt = 0;
+  for (int m = lo; m < hi; ++m) cnt += __float_as_uint(v[m]) == prefix;
+  int incl = cnt;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int t = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += t;
+  }
+  __syncthreads();                                           // red is read above
+  if (lane == 31) red[warp] = (unsigned long long)incl;
+  if (tid == 0) red[NW] = ~0ull;                             // m* = -1 when there is no candidate at all
+  __syncthreads();
+  unsigned long long excl = (unsigned long long)(incl - cnt);
+  for (int w = 0; w < warp; ++w) excl += red[w];
+  if (excl < ties && ties <= excl + (unsigned long long)cnt) {
+    unsigned long long k = excl;
+    for (int m = lo; m < hi; ++m)
+      if (__float_as_uint(v[m]) == prefix && ++k == ties) red[NW] = (unsigned long long)m;
+  }
+  __syncthreads();
+  const NucleusCut cut{prefix, (int)(long long)red[NW]};
+  __syncthreads();                                           // red is free again
+  return cut;
+}
+
 // kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one; kConstrained (with kGreedy): the pick skips
-// the sentences `cn` makes ineligible; kSample (with kGreedy, not kBeam): the pick is drawn (`sp`)
-template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false>
+// the sentences `cn` makes ineligible; kSample (with kGreedy, not kBeam): the pick is drawn (`sp`); kNucleus (with kSample): drawn
+// from the nucleus (`nu`)
+template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false, bool kNucleus = false>
 __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn,
-                                               const SampleArgs sp) {
+                                               const SampleArgs sp, const NucleusArgs nu = NucleusArgs{}) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int ob = blockIdx.x / CL;                         // the output row: the video (sampled: cluster_row(), the roll-out)
@@ -533,8 +657,11 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       if (nj7) energies(s_st0, s_st1, N7{}, R2{});
       else energies(s_st0, s_st1, N8{}, R2{});
     } else {
-      if (nj7) energies(gpa, gpi, N7{}, R4{});
-      else energies(gpa, gpi, N8{}, R4{});
+      // (the constrained nucleus roll-out holds more across the step: two rows per warp round keep it at 128 registers without a
+      // spill -- four spilled 80 bytes around these loads.  The rows' sums are the same either way)
+      using RL = std::conditional_t<kNucleus && kConstrained, R2, R4>;
+      if (nj7) energies(gpa, gpi, N7{}, RL{});
+      else energies(gpa, gpi, N8{}, RL{});
     }
     __syncthreads();
     if (staged && tid == 0 && n > 0) {       // every read of the proj rows is behind the barrier: the buffers take the enc rows
@@ -812,6 +939,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         const bool cand = !kConstrained || (((allow >> ((unsigned)(m - m0) / NT)) & 1u) && (m != eos || eos_ok));
         if (sp.top_k > 0) {
           lg[m - m0] = p;
+        } else if constexpr (kNucleus) {                         // nucleus: the row of every rank (the draw follows the cut)
+          for (int r = 0; r < CL; ++r) cluster.map_shared_rank(smem + nu.off, r)[m] = cand ? p : -1.f;
         } else if (cand) {
           const float z = kConstrained ? sample_z(sp, p, cbase + (uint32_t)m) : sample_score(p, inv_t, cbase + (uint32_t)m, key0, key1);
           if (z > best || best_i == M) { best = z; best_i = m; }
@@ -820,6 +949,22 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         if (((allow >> ((unsigned)(m - m0) / NT)) & 1u) && (m != eos || eos_ok) && p > best) { best = p; best_i = m; }
       } else if (p > best) { best = p; best_i = m; }
       if (m == tg && a.nll) a.nll[lrow] = -logf(p + 1e-12f);      // models.py:168-170
+    }
+    if constexpr (kNucleus) {
+      if (sp.top_k == 0) {                                       // (uniform) the cut of the whole row, then the draw over this rank's members
+        cluster.sync();
+        const float* const nv = smem + nu.off;
+        const NucleusCut cut = nucleus_cut(nv, M, nu.P, reinterpret_cast<unsigned long long*>(smem + nu.off + up4(M)),
+                                           reinterpret_cast<unsigned long long*>(smem + nu.off + up4(M) + 2 * kNucBuckets));
+        for (int m = m0 + tid; m < m1; m += NT) {
+          const float p = nv[m];
+          const uint32_t bits = __float_as_uint(p);
+          if (p >= 0.f && (bits > cut.pstar || (bits == cut.pstar && m <= cut.mstar))) {
+            const float z = kConstrained ? sample_z(sp, p, cbase + (uint32_t)m) : sample_score(p, inv_t, cbase + (uint32_t)m, key0, key1);
+            if (z > best || best_i == M) { best = z; best_i = m; }
+          }
+        }
+      }
     }
     // (sampled with top_k > 0: the pick is made after the step, by the selection)
     if (!kBeam && (kGreedy || a.argmax) && !(kSample && sp.top_k > 0)) {     // first maximal index, as torch.max(dim) documents
@@ -949,6 +1094,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       const int npub = any_live ? CL * KS : 0, tot = npub + (kSample ? 0 : KW);
       float ps = INFINITY, pp = INFINITY;
       int pk = -1, pm = -1;
+      float nuc_p = 0.f;                                         // nucleus: lane j keeps the j-th entry (nuc_m = M: none)
+      int nuc_m = M;
       for (int j = 0; j < KS; ++j) {
         float cs = -INFINITY, cp = -1.f;
         int ck = kNone, cm = kNone;
@@ -967,7 +1114,9 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
           if (cand_better(ps, pp, pk, pm, es, ep, ek, em) && cand_better(es, ep, ek, em, cs, cp, ck, cm)) { cs = es; cp = ep; ck = ek; cm = em; }
         }
         cand_warp_best(cs, cp, ck, cm);
-        if constexpr (kSample) {
+        if constexpr (kNucleus) {
+          if (ck != kNone && lane == j) { nuc_p = cp; nuc_m = cm; }
+        } else if constexpr (kSample) {
           if (ck != kNone) {
             const uint32_t c = ((uint32_t)cluster_row() * (uint32_t)S + (uint32_t)s) * (uint32_t)M + (uint32_t)cm;
             const float z = kConstrained ? sample_z(sp, cp, c) : sample_score(cp, inv_t, c, key0, key1);
@@ -982,6 +1131,30 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
           nt_kind[j] = none ? 0 : bs_stat[ck] == kDone ? 3 : cm == eos ? 2 : 1;
         }
         ps = cs; pp = cp; pk = ck; pm = cm;
+      }
+      if constexpr (kNucleus) {
+        // the nucleus is the first n entries: lane j is in when the mass before it is below need (lane 0 always).  At most 8
+        // masses of at most 2^24: the sums fit 32 bits
+        const uint32_t q = nuc_m < M ? __float2uint_rz(nuc_p * 16777216.f) : 0u;
+        uint32_t incl = q;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+          if (lane >= o) incl += t;
+        }
+        const unsigned long long pq = (unsigned long long)nu.P * __shfl_sync(0xffffffffu, incl, 31);
+        const unsigned long long need = (pq >> 24) + ((pq & 0xffffffull) != 0ull);
+        if (nuc_m < M && (lane == 0 || (unsigned long long)(incl - q) < need)) {
+          const uint32_t c = ((uint32_t)cluster_row() * (uint32_t)S + (uint32_t)s) * (uint32_t)M + (uint32_t)nuc_m;
+          bz = kConstrained ? sample_z(sp, nuc_p, c) : sample_score(nuc_p, inv_t, c, key0, key1);
+          drawn = nuc_m;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {                       // the largest z, ties to the smaller sentence
+          const float z2 = __shfl_xor_sync(0xffffffffu, bz, o);
+          const int d2 = __shfl_xor_sync(0xffffffffu, drawn, o);
+          if (d2 != M && (drawn == M || z2 > bz || (z2 == bz && d2 < drawn))) { bz = z2; drawn = d2; }
+        }
       }
     }
     if constexpr (kSample) {
@@ -1088,6 +1261,17 @@ __global__ void __launch_bounds__(NT) dec_sample_kernel(const FusedArgs a, const
 __global__ void __launch_bounds__(NT) dec_sample_constrained_kernel(const FusedArgs a, const GreedyArgs g, const ConstraintArgs cn,
                                                                     const SampleArgs sp) {
   dec_fused_body<true, false, true, true>(a, g, BeamArgs{}, cn, sp);
+}
+
+__global__ void __launch_bounds__(NT) dec_sample_nucleus_kernel(const FusedArgs a, const GreedyArgs g, const SampleArgs sp,
+                                                                const NucleusArgs nu) {
+  dec_fused_body<true, false, false, true, true>(a, g, BeamArgs{}, ConstraintArgs{}, sp, nu);
+}
+
+__global__ void __launch_bounds__(NT) dec_sample_nucleus_constrained_kernel(const FusedArgs a, const GreedyArgs g,
+                                                                            const ConstraintArgs cn, const SampleArgs sp,
+                                                                            const NucleusArgs nu) {
+  dec_fused_body<true, false, true, true, true>(a, g, BeamArgs{}, cn, sp, nu);
 }
 
 }  // namespace
@@ -1632,12 +1816,16 @@ static size_t beam_floats(int K, int CL, int chunk, int H, int M, bool constrain
   return 7 * MAXK + MAXC * MAXK * 4 + NW * 4 + MAXK * 4 + (size_t)K * per_slot + cons;
 }
 
+// floats of the nucleus region (see nucleus_cut): every rank's copy of the row, the histogram (u64) and the block exchanges (u64)
+static size_t nucleus_floats(int M) { return (((size_t)M + 3) & ~(size_t)3) + 2 * kNucBuckets + 2 * 32; }
+
 // Shape checks, cluster size, shared memory and row stage of the forward cluster kernels, then the launch: `g` null launches one step
 // (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel), or with `bm` the beam roll-out (dec_beam_fused_kernel);
 // with `cn` the constrained roll-out of either (dec_greedy_constrained_kernel, dec_beam_constrained_kernel); with `sp` (not `bm`) the
-// sampled roll-out (dec_sample_kernel, with `cn` dec_sample_constrained_kernel), one cluster per (video, sample).
+// sampled roll-out (dec_sample_kernel, with `cn` dec_sample_constrained_kernel), one cluster per (video, sample); with `sp` and `nu`
+// the nucleus roll-out (dec_sample_nucleus_kernel, with `cn` dec_sample_nucleus_constrained_kernel).
 static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr,
-                        const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr) {
+                        const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr, NucleusArgs* nu = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
@@ -1657,6 +1845,12 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   } else if (sp) {                         // sampled: the beam region's tables and exchange arrays, no slots
     sp->off = (int)((smem + 15) / 16 * 4);
     smem = ((size_t)sp->off + beam_floats(0, CL, a.chunk, H, M)) * 4 + 64;
+    if (nu) {                              // nucleus: its region behind the exchange arrays
+      nu->off = (int)((smem + 15) / 16 * 4);
+      smem = ((size_t)nu->off + nucleus_floats(M)) * 4 + 64;
+      MMB_REQUIRE(smem <= 227 * 1024, MMB_ERR_UNSUPPORTED, "%s: the nucleus row of M=%d needs %zu B of shared memory per CTA, more than "
+                  "232448 (Lt=%d)", who, M, smem, Lt);
+    }
   }
   {
     // the row stage (see the kernel): two buffers of chunk x D floats behind two mbarriers, when they fit and bulk copies apply
@@ -1674,10 +1868,11 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[7] = {0, 0, 0, 0, 0, 0, 0};
-  const int which = sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
+  static size_t smem_set[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  const int which = nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
   if (smem > smem_set[which]) {
-    const void* fn = which == 6 ? (const void*)dec_sample_constrained_kernel : which == 5 ? (const void*)dec_sample_kernel
+    const void* fn = which == 8 ? (const void*)dec_sample_nucleus_constrained_kernel : which == 7 ? (const void*)dec_sample_nucleus_kernel
+                   : which == 6 ? (const void*)dec_sample_constrained_kernel : which == 5 ? (const void*)dec_sample_kernel
                    : which == 4 ? (const void*)dec_beam_constrained_kernel : which == 3 ? (const void*)dec_greedy_constrained_kernel
                    : which == 2 ? (const void*)dec_beam_fused_kernel : which == 1 ? (const void*)dec_greedy_fused_kernel
                                 : (const void*)dec_step_fused_kernel;
@@ -1703,6 +1898,14 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (nu && cn) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_sample_nucleus_constrained_kernel, a, *g, *cn, *sp, *nu));
+    return check_launch("dec_sample_nucleus_constrained_kernel");
+  }
+  if (nu) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_sample_nucleus_kernel, a, *g, *sp, *nu));
+    return check_launch("dec_sample_nucleus_kernel");
+  }
   if (sp && cn) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_sample_constrained_kernel, a, *g, *cn, *sp));
     return check_launch("dec_sample_constrained_kernel");
@@ -1848,6 +2051,39 @@ extern "C" int mmb_decoder_beam_constrained_fused(const float* proj_a, const flo
   return launch_fused(a, &g, "mmb_decoder_beam_constrained_fused", stream, &bm, &cn);
 }
 
+namespace mmb {
+// the sampled roll-out (nu null) or the nucleus roll-out: argument checks, then launch_fused
+static int sample_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                        const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                        const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                        const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                        const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                        const uint8_t* mask, const int* text_len, const unsigned long long* key, float* probs,
+                        long long* tokens, int B, int Lt, int D, int H, int E, int M, int S, int N, float T,
+                        int top_k, int no_repeat, int min_sentences, mmb_stream_t stream, NucleusArgs* nu, const char* who) {
+  const bool constrained = no_repeat != 0 || min_sentences != 0;
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && key && probs && tokens &&
+                  (text_len || !constrained),
+              MMB_ERR_INVALID, "%s: null pointer", who);
+  MMB_REQUIRE(S > 0 && N >= 1 && N <= 64 && T > 0.f && isfinite(T) && top_k >= 0 && top_k <= MAXK && (no_repeat == 0 || no_repeat == 1) &&
+                  min_sentences >= 0,
+              MMB_ERR_INVALID,
+              "%s: S=%d, N=%d (1..64), T=%g (finite, > 0), top_k=%d (0..%d), no_repeat=%d (0 or 1), "
+              "min_sentences=%d (>= 0)", who, S, N, (double)T, top_k, MAXK, no_repeat, min_sentences);
+  MMB_REQUIRE(B > 0 && M > 0, MMB_ERR_INVALID, "%s: B=%d M=%d", who, B, M);
+  MMB_REQUIRE((unsigned long long)B * N * S * M <= (1ull << 32), MMB_ERR_UNSUPPORTED,
+              "%s: B N S M = %d x %d x %d x %d exceeds the 2^32 counters of a key", who, B, N, S, M);
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, probs, nullptr, nullptr, nullptr, nullptr, tokens,
+              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  const ConstraintArgs cn{text_len, no_repeat, min_sentences};
+  SampleArgs sp{key, T, N, top_k, 0};
+  return launch_fused(a, &g, who, stream, nullptr, constrained ? &cn : nullptr, &sp, nu);
+}
+}  // namespace mmb
+
 extern "C" int mmb_decoder_sample_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
                                         const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
                                         const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
@@ -1856,27 +2092,28 @@ extern "C" int mmb_decoder_sample_fused(const float* proj_a, const float* proj_i
                                         const uint8_t* mask, const int* text_len, const unsigned long long* key, float* probs,
                                         long long* tokens, int B, int Lt, int D, int H, int E, int M, int S, int N, float T,
                                         int top_k, int no_repeat, int min_sentences, mmb_stream_t stream) {
+  return mmb::sample_fused(proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt,
+                           bcat, out_wt, out_b, emb_text, h0, mask, text_len, key, probs, tokens, B, Lt, D, H, E, M, S, N, T, top_k,
+                           no_repeat, min_sentences, stream, nullptr, "mmb_decoder_sample_fused");
+}
+
+extern "C" int mmb_decoder_sample_nucleus_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                                const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                                const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                                const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                                const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                                const uint8_t* mask, const int* text_len, const unsigned long long* key, float* probs,
+                                                long long* tokens, int B, int Lt, int D, int H, int E, int M, int S, int N, float T,
+                                                int top_k, int no_repeat, int min_sentences, float top_p,
+                                                mmb_stream_t stream) {
   using namespace mmb;
-  const bool constrained = no_repeat != 0 || min_sentences != 0;
-  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
-                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && key && probs && tokens &&
-                  (text_len || !constrained),
-              MMB_ERR_INVALID, "mmb_decoder_sample_fused: null pointer");
-  MMB_REQUIRE(S > 0 && N >= 1 && N <= 64 && T > 0.f && isfinite(T) && top_k >= 0 && top_k <= MAXK && (no_repeat == 0 || no_repeat == 1) &&
-                  min_sentences >= 0,
-              MMB_ERR_INVALID,
-              "mmb_decoder_sample_fused: S=%d, N=%d (1..64), T=%g (finite, > 0), top_k=%d (0..%d), no_repeat=%d (0 or 1), "
-              "min_sentences=%d (>= 0)", S, N, (double)T, top_k, MAXK, no_repeat, min_sentences);
-  MMB_REQUIRE(B > 0 && M > 0, MMB_ERR_INVALID, "mmb_decoder_sample_fused: B=%d M=%d", B, M);
-  MMB_REQUIRE((unsigned long long)B * N * S * M <= (1ull << 32), MMB_ERR_UNSUPPORTED,
-              "mmb_decoder_sample_fused: B N S M = %d x %d x %d x %d exceeds the 2^32 counters of a key", B, N, S, M);
-  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
-              nullptr, nullptr, nullptr, nullptr, mask, nullptr, probs, nullptr, nullptr, nullptr, nullptr, tokens,
-              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
-  const GreedyArgs g{emb_text, h0, S, 0};
-  const ConstraintArgs cn{text_len, no_repeat, min_sentences};
-  SampleArgs sp{key, T, N, top_k, 0};
-  return launch_fused(a, &g, "mmb_decoder_sample_fused", stream, nullptr, constrained ? &cn : nullptr, &sp);
+  MMB_REQUIRE(top_p > 0.f && top_p <= 1.f, MMB_ERR_INVALID, "mmb_decoder_sample_nucleus_fused: top_p=%g (in (0, 1])", (double)top_p);
+  // the integer masses of the rule: P Q < 2^24 2^24 M fits 64 bits
+  MMB_REQUIRE(top_p == 1.f || M < 65536, MMB_ERR_UNSUPPORTED, "mmb_decoder_sample_nucleus_fused: M=%d (below 65536 with top_p < 1)", M);
+  NucleusArgs nu{(uint32_t)rintf(top_p * 16777216.f), 0};
+  return sample_fused(proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat,
+                      out_wt, out_b, emb_text, h0, mask, text_len, key, probs, tokens, B, Lt, D, H, E, M, S, N, T, top_k, no_repeat,
+                      min_sentences, stream, top_p == 1.f ? nullptr : &nu, "mmb_decoder_sample_nucleus_fused");   // (1: no cut, the sampled roll-out)
 }
 
 extern "C" int mmb_decoder_bwd_head(const float* probs, const float* d_probs, const long long* target, const float* g_nll,

@@ -3,6 +3,7 @@ from __future__ import annotations
 
 from typing import List, Sequence
 
+import numpy as np
 import torch
 
 
@@ -20,6 +21,31 @@ def greedy_search(out_distributions: torch.Tensor, original_text_length: int) ->
             continue
         chosen.append(int(k))
     return chosen
+
+
+def nucleus(p, eligible=None, top_k: int = 0, top_p: float = 1.0) -> List[int]:
+    """The candidates a sampled pick draws from (the rules at mmb_decoder_sample_fused / mmb_decoder_sample_nucleus_fused in
+    include/mmbidaf_b200.h), in (p descending, m ascending) order, from one row ``p`` (M) of fp32 probabilities as the kernels write
+    them: every m (or those with ``eligible[m]`` set), cut to the first ``top_k`` when ``top_k > 0``, then for ``top_p < 1`` to the
+    first n whose integer masses q = floor(p 2^24) reach P Q (P = rint(top_p 2^24) in fp32, Q the candidates' mass), n >= 1.
+    Integers only after the fp32 inputs, so the set is the kernels' exactly.  A verification helper (O(M log M) on the host, one row
+    at a time): the tests check the kernels' picks against it, and a user can check a returned sample the same way."""
+    row = np.asarray(p.detach().cpu() if torch.is_tensor(p) else p, dtype=np.float32).reshape(-1)
+    ok = np.ones(row.shape, dtype=bool) if eligible is None else np.asarray(
+        eligible.detach().cpu() if torch.is_tensor(eligible) else eligible, dtype=bool).reshape(-1)
+    cand = sorted((m for m in range(row.size) if ok[m]), key=lambda m: (-float(row[m]), m))
+    if top_k > 0:
+        cand = cand[:top_k]
+    if np.float32(top_p) == np.float32(1.0):
+        return cand
+    q = [int(np.floor(np.float64(row[m]) * 2 ** 24)) for m in cand]     # exact: p 2^24 is a scaled fp32 value
+    P = int(np.rint(np.float64(np.float32(top_p)) * 2 ** 24))           # half to even, as rintf
+    need, acc = P * sum(q), 0
+    for n, qm in enumerate(q, 1):
+        acc += qm
+        if (acc << 24) >= need:
+            return cand[:n]
+    return cand                                                          # (no candidate)
 
 
 def get_generated_indices(batch_out_distributions: torch.Tensor, original_text_lengths: Sequence[int]) -> List[List[int]]:

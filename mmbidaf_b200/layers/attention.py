@@ -271,11 +271,12 @@ class MultimodalAttentionDecoder(nn.Module):
                                         text_len.to(torch.int32).contiguous(), steps, width, no_repeat, min_sentences)
 
     def sample(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, num_samples, key, temperature=1.0, top_k=0, no_repeat=False,
-               min_sentences=0):
+               min_sentences=0, *, top_p=1.0):
         """``num_samples`` sampled decodes of ``steps`` steps per video in eval mode, as ONE launch of the cluster kernel whatever
         ``ops.decoder_cut`` says; the rule (temperature, top_k, the constraints, the counter of ``key``) is documented at
-        mmb_decoder_sample_fused in include/mmbidaf_b200.h.  Same start as :meth:`greedy`; ``text_len`` (B) int32 gives each video's
-        EOS row; ``key`` (1) int64 on the device.  No autograd.  Returns ``ops.decoder_sample_fwd``'s (probs (B,N,S,M), tokens (B,N,S))."""
+        mmb_decoder_sample_fused in include/mmbidaf_b200.h, and ``top_p`` < 1 (the nucleus) at mmb_decoder_sample_nucleus_fused.  Same
+        start as :meth:`greedy`; ``text_len`` (B) int32 gives each video's EOS row; ``key`` (1) int64 on the device.  No autograd.
+        Returns ``ops.decoder_sample_fwd``'s (probs (B,N,S,M), tokens (B,N,S))."""
         if not enc_a.is_cuda:
             raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
         if self.num_layers != 1:
@@ -285,7 +286,7 @@ class MultimodalAttentionDecoder(nn.Module):
             B = seq.B
             return ops.decoder_sample_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
                                           text_len.to(torch.int32).contiguous(), steps, num_samples, key, temperature, top_k,
-                                          no_repeat, min_sentences)
+                                          no_repeat, min_sentences, top_p)
 
     def step(self, sent_embed, decoder_hidden, decoder_cell_state, text_audio_enc_out, text_img_enc_out, coverage_vec,
              mask, target=None):

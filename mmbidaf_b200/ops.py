@@ -7,6 +7,7 @@ this module (bench.py reports it as ``gpu_launches``).
 from __future__ import annotations
 
 import contextlib
+import ctypes
 import math
 import os
 from typing import Optional, Tuple
@@ -470,27 +471,31 @@ def decoder_beam_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps
 SAMPLE_MAX_N, SAMPLE_MAX_TOP_K = 64, 8
 
 
-def check_sampling(who: str, num_samples, temperature, top_k) -> None:
+def check_sampling(who: str, num_samples, temperature, top_k, top_p=1.0) -> None:
     """``num_samples`` an int in 1..64, ``temperature`` a finite number > 0, ``top_k`` an int in 0..8 (the rule at
-    mmb_decoder_sample_fused in include/mmbidaf_b200.h)."""
+    mmb_decoder_sample_fused in include/mmbidaf_b200.h), ``top_p`` a real in (0, 1] that stays above 0 in fp32 (the rule at
+    mmb_decoder_sample_nucleus_fused)."""
     if isinstance(num_samples, bool) or not isinstance(num_samples, int) or not 1 <= num_samples <= SAMPLE_MAX_N:
         raise ValueError(f"{who}: num_samples {num_samples!r}, expected an int in 1..{SAMPLE_MAX_N}")
     if isinstance(temperature, bool) or not isinstance(temperature, (int, float)) or not math.isfinite(temperature) or temperature <= 0:
         raise ValueError(f"{who}: temperature {temperature!r}, expected a finite number > 0")
     if isinstance(top_k, bool) or not isinstance(top_k, int) or not 0 <= top_k <= SAMPLE_MAX_TOP_K:
         raise ValueError(f"{who}: top_k {top_k!r}, expected an int in 0..{SAMPLE_MAX_TOP_K}")
+    if isinstance(top_p, bool) or not isinstance(top_p, (int, float)) or not 0 < top_p <= 1 or ctypes.c_float(top_p).value <= 0:
+        raise ValueError(f"{who}: top_p {top_p!r}, expected a real in (0, 1]")
 
 
 def decoder_sample_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, num_samples: int, key: torch.Tensor,
-                       temperature: float = 1.0, top_k: int = 0, no_repeat: bool = False, min_sentences: int = 0):
+                       temperature: float = 1.0, top_k: int = 0, no_repeat: bool = False, min_sentences: int = 0, top_p: float = 1.0):
     """N sampled roll-outs per video (the rule at mmb_decoder_sample_fused in include/mmbidaf_b200.h) as ONE launch of the cluster
     kernel, whatever ``decoder_cut`` says.  Inputs as :func:`decoder_greedy_constrained_fwd` (text_len_i32 may be None without a
-    constraint), plus ``key`` (1) int64 on the device (:func:`rng_next_keys`, or a fill).  Returns (probs (B,N,S,M), tokens (B,N,S)
-    int64) -- each roll-out's distributions are the step kernel's, bit for bit."""
+    constraint), plus ``key`` (1) int64 on the device (:func:`rng_next_keys`, or a fill).  ``top_p`` < 1 draws from the nucleus
+    (mmb_decoder_sample_nucleus_fused); 1 is the plain sampled launch.  Returns (probs (B,N,S,M), tokens (B,N,S) int64) -- each
+    roll-out's distributions are the step kernel's, bit for bit."""
     lib = _lib.lib()
     B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
     dev = h0.device
-    check_sampling("decoder_sample_fwd", num_samples, temperature, top_k)
+    check_sampling("decoder_sample_fwd", num_samples, temperature, top_k, top_p)
     _check_constraints("decoder_sample_fwd", no_repeat, min_sentences)
     if int(steps) <= 0:
         raise ValueError(f"decoder_sample_fwd: {steps} steps")
@@ -507,22 +512,25 @@ def decoder_sample_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, ste
     probs = torch.empty(B, N, S, M, device=dev, dtype=torch.float32)
     tokens = torch.empty(B, N, S, device=dev, dtype=torch.int64)
     p = _lib.ptr
-    _lib.check(lib.mmb_decoder_sample_fused(
-        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
-        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
-        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(key.contiguous()), p(probs),
-        p(tokens), B, Lt, D, H, E, M, S, N, float(temperature), int(top_k), int(no_repeat), int(min_sentences), _lib.stream()),
-        "mmb_decoder_sample_fused")
+    args = (p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+            p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+            p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(key.contiguous()), p(probs),
+            p(tokens), B, Lt, D, H, E, M, S, N, float(temperature), int(top_k), int(no_repeat), int(min_sentences))
+    if top_p == 1.0:
+        _lib.check(lib.mmb_decoder_sample_fused(*args, _lib.stream()), "mmb_decoder_sample_fused")
+    else:
+        _lib.check(lib.mmb_decoder_sample_nucleus_fused(*args, float(top_p), _lib.stream()), "mmb_decoder_sample_nucleus_fused")
     _count(1)
     return probs, tokens
 
 
 def sample_pick(probs: torch.Tensor, key: torch.Tensor, row_base: torch.Tensor, S: int, s: int, N: int = 1, temperature: float = 1.0,
-                top_k: int = 0, eligible: Optional[torch.Tensor] = None) -> torch.Tensor:
+                top_k: int = 0, eligible: Optional[torch.Tensor] = None, top_p: float = 1.0) -> torch.Tensor:
     """Steps 1 to 4 of the sampled pick (mmb_sample_pick) for the rows of ``probs`` (R, M) fp32: row r is sample r % N of video
-    ``row_base[r]`` (R int32) at step ``s`` of ``S``; ``eligible`` (R, M) bool / uint8 limits the candidates.  Returns picks (R) int64,
-    -1 for a row without a candidate -- the roll-out kernel's pick, bit for bit."""
-    check_sampling("sample_pick", N, temperature, top_k)
+    ``row_base[r]`` (R int32) at step ``s`` of ``S``; ``eligible`` (R, M) bool / uint8 limits the candidates; ``top_p`` < 1 draws
+    from the nucleus (mmb_sample_pick_nucleus).  Returns picks (R) int64, -1 for a row without a candidate -- the roll-out kernel's
+    pick, bit for bit."""
+    check_sampling("sample_pick", N, temperature, top_k, top_p)
     if probs.dtype != torch.float32 or probs.dim() != 2 or not probs.is_cuda:
         raise ValueError(f"sample_pick: probs {probs.dtype} {tuple(probs.shape)} on {probs.device}, expected (R, M) fp32 on a GPU")
     R, M = probs.shape
@@ -538,9 +546,12 @@ def sample_pick(probs: torch.Tensor, key: torch.Tensor, row_base: torch.Tensor, 
     if not 0 <= int(s) < int(S):
         raise ValueError(f"sample_pick: step {s} of {S}")
     picks = torch.empty(R, device=probs.device, dtype=torch.int64)
-    _lib.check(_lib.lib().mmb_sample_pick(_lib.ptr(probs.contiguous()), _lib.ptr(_u8(eligible)), _lib.ptr(key.contiguous()),
-                                          _lib.ptr(row_base.contiguous()), R, M, int(S), int(s), int(N), float(temperature), int(top_k),
-                                          _lib.ptr(picks), _lib.stream()), "mmb_sample_pick")
+    args = (_lib.ptr(probs.contiguous()), _lib.ptr(_u8(eligible)), _lib.ptr(key.contiguous()), _lib.ptr(row_base.contiguous()), R, M,
+            int(S), int(s), int(N), float(temperature), int(top_k), _lib.ptr(picks))
+    if top_p == 1.0:
+        _lib.check(_lib.lib().mmb_sample_pick(*args, _lib.stream()), "mmb_sample_pick")
+    else:
+        _lib.check(_lib.lib().mmb_sample_pick_nucleus(*args, float(top_p), _lib.stream()), "mmb_sample_pick_nucleus")
     _count(1)
     return picks
 

@@ -3,7 +3,7 @@
 ``MMBiDAF.summarize`` runs the encoder half of the model, the whole greedy decode roll-out and the greedy sentence selection
 without a host round trip; its result is a :class:`Summary`.  With ``beam_width=K`` the roll-out is a beam search over K
 hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  With
-``num_samples=N`` N summaries per video are drawn inside one launch (temperature, top-k); the summary is the likeliest sample's, and
+``num_samples=N`` N summaries per video are drawn inside one launch (temperature, top-k, top-p); the summary is the likeliest sample's, and
 :class:`Samples` holds all N.  ``no_repeat`` and ``min_sentences`` constrain any pick inside the roll-out kernel.
 :class:`Summarizer` replays ``summarize`` from CUDA graphs, one capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
 """
@@ -21,21 +21,22 @@ __all__ = ["Beams", "Samples", "Summary", "Summarizer", "gather_summaries"]
 
 
 def check_options(who: str, with_targets: bool, beam_width, no_repeat, min_sentences, num_samples=None, temperature=1.0, top_k=0,
-                  seed=None) -> None:
+                  seed=None, top_p=1.0) -> None:
     """The decode options of ``MMBiDAF.summarize`` / ``Summarizer``, checked before any device work: ``beam_width`` None or an int
     in 1..8, ``no_repeat`` a bool, ``min_sentences`` an int >= 0; neither a beam nor a constraint with targets (the eval loss is
     defined by the unconstrained greedy roll-out).  Sampling: ``num_samples`` None or an int in 1..64, not with a beam or targets;
-    ``temperature`` finite and > 0, ``top_k`` an int in 0..8, ``seed`` None or an int -- set only with ``num_samples``."""
+    ``temperature`` finite and > 0, ``top_k`` an int in 0..8, ``seed`` None or an int, ``top_p`` a real in (0, 1] -- set only with
+    ``num_samples``."""
     if num_samples is not None:
-        check_sampling(who, num_samples, temperature, top_k)
+        check_sampling(who, num_samples, temperature, top_k, top_p)
         if beam_width is not None:
             raise ValueError(f"{who}: num_samples with beam_width -- sampling and beam search are separate decodes")
         if with_targets:
             raise ValueError(f"{who}: num_samples with targets -- the eval loss is defined by the greedy roll-out")
         if seed is not None and (isinstance(seed, bool) or not isinstance(seed, int)):
             raise ValueError(f"{who}: seed {seed!r}, expected None or an int")
-    elif temperature != 1.0 or top_k != 0 or seed is not None:
-        raise ValueError(f"{who}: temperature / top_k / seed without num_samples")
+    elif temperature != 1.0 or top_k != 0 or seed is not None or isinstance(top_p, bool) or top_p != 1.0:
+        raise ValueError(f"{who}: temperature / top_k / top_p / seed without num_samples")
     if beam_width is not None:
         if isinstance(beam_width, bool) or not isinstance(beam_width, int) or not 1 <= beam_width <= BEAM_MAX_WIDTH:
             raise ValueError(f"{who}: beam_width {beam_width!r}, expected None or an int in 1..{BEAM_MAX_WIDTH}")
@@ -144,7 +145,7 @@ class Summary(NamedTuple):
 
 
 def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int], no_repeat: bool = False, min_sentences: int = 0,
-                sampling: tuple = (None, 1.0, 0, None)):
+                sampling: tuple = (None, 1.0, 0, None, 1.0)):
     return (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), int(batch.max_dec_len),
             tuple(batch.targets.shape) if with_targets else None, beam_width, no_repeat, min_sentences, sampling)
 
@@ -153,7 +154,7 @@ class _Bucket:
     """One captured ``summarize``: static inputs, static length plans, the graph and its (static) result."""
 
     def __init__(self, model, batch: Batch, with_targets: bool, warmup: int, beam_width: Optional[int] = None,
-                 no_repeat: bool = False, min_sentences: int = 0, sampling: tuple = (None, 1.0, 0, None)):
+                 no_repeat: bool = False, min_sentences: int = 0, sampling: tuple = (None, 1.0, 0, None, 1.0)):
         import gc
         from .layers.encoding import pin_lengths
         dev = batch.text.device
@@ -163,7 +164,7 @@ class _Bucket:
         self.with_targets = with_targets
         self.beam_width = beam_width
         self.no_repeat, self.min_sentences = no_repeat, min_sentences
-        self.sampling = sampling             # (num_samples, temperature, top_k, seed); seed None: the key state exists after warm-up
+        self.sampling = sampling             # (num_samples, temperature, top_k, seed, top_p); seed None: the key state exists after warm-up
         self.plans = [pin_lengths(lst, dev) for lst in (self.batch.text_len, self.batch.audio_len, self.batch.image_len)]
         for m in model.modules():          # per-sequence caches of eager calls still own tensors (see Trainer.capture)
             if hasattr(m, "_cache"):
@@ -187,7 +188,7 @@ class _Bucket:
         return model.summarize(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, b.max_dec_len,
                                b.targets if self.with_targets else None, beam_width=self.beam_width, no_repeat=self.no_repeat,
                                min_sentences=self.min_sentences, num_samples=self.sampling[0], temperature=self.sampling[1],
-                               top_k=self.sampling[2], seed=self.sampling[3])
+                               top_k=self.sampling[2], seed=self.sampling[3], top_p=self.sampling[4])
 
     def load(self, batch: Batch) -> None:
         if batch is self.batch:
@@ -216,14 +217,14 @@ class Summarizer:
 
     def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None, no_repeat: bool = False,
                  min_sentences: int = 0, num_samples: Optional[int] = None, temperature: float = 1.0, top_k: int = 0,
-                 seed: Optional[int] = None) -> Summary:
+                 seed: Optional[int] = None, top_p: float = 1.0) -> Summary:
         """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``; ``beam_width``
         decodes by beam search, ``no_repeat`` / ``min_sentences`` constrain the pick (``MMBiDAF.summarize``); each width and each
-        setting of the constraints in its own bucket.  ``num_samples`` / ``temperature`` / ``top_k`` / ``seed`` sample (each setting,
+        setting of the constraints in its own bucket.  ``num_samples`` / ``temperature`` / ``top_k`` / ``seed`` / ``top_p`` sample (each setting,
         the seed included, in its own bucket): with ``seed=None`` every replay draws a fresh key from the device key stream, with an int
         seed every replay gives that seed's samples.  The options are checked before anything is copied or captured."""
-        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed)
-        sampling = (num_samples, temperature, top_k, seed)
+        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed, top_p)
+        sampling = (num_samples, temperature, top_k, seed, top_p)
         key = _bucket_key(batch, with_targets, beam_width, no_repeat, min_sentences, sampling)
         bucket = self.buckets.get(key)
         if bucket is None:
