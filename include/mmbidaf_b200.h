@@ -270,6 +270,52 @@ MMB_API int mmb_decoder_beam_constrained_fused(const float* proj_a, const float*
                                                float* scores, float* probs, long long* best, int32_t* path, int B, int Lt, int D, int H,
                                                int E, int M, int K, int S, int no_repeat, int min_sentences, mmb_stream_t stream);
 /*
+ * Stochastic beam summary roll-outs: K DISTINCT summaries per video, an exact sample without replacement from the model's tempered,
+ * renormalised sequence distribution, in ONE launch of the beam's cluster kernel (Kool, van Hoof and Welling, "Stochastic Beams and
+ * Where to Find Them", ICML 2019).  This is the project's own rule; no reference parity is claimed.  Per video b: eos = text_len[b] - 1,
+ * K slots, S steps, temperature T, a 64-bit key on the device (*key, as mmb_decoder_sample_fused takes it).
+ *   Slots: the beam's (token, parent, status live / finished / empty, score = the sum of logf(p) along the path), plus two fp32 values:
+ *   phi, the path's log-probability under the sampling distribution, and key, its perturbed log-probability.  Before step 0 slot 0 is
+ *   live with score = phi = 0, key = -logf(-logf(u)) (a Gumbel(0) draw, u as below with the counter B S K M + b) and the greedy start
+ *   state; the others are empty with all three -inf.  (The root's key must be a draw, not 0: with the root fixed, the final keys are
+ *   conditioned on their maximum and the inclusion probabilities below would be wrong; the sample itself does not depend on it.)
+ *   Candidates of a live slot k: the beam's -- every m with p[m] > 0, or under no_repeat / min_sentences the eligible m with p[m] > 0
+ *   (the constrained beam's rule); p is the step kernel's distribution, bit for bit.
+ *   Sampling distribution, exact and independent of how the cluster splits M:
+ *     1. l[m] = logf(p[m]) * (1 / T) in fp32;  mu = the max of l over the candidates.
+ *     2. q[m] = floor(expf(l[m] - mu) 2^24), Q = the sum of q as a uint64 (exact in any order; the max candidate has q = 2^24).
+ *     3. lam = mu + logf((float)Q * 2^-24); the child's phi' = phi_k + (l[m] - lam).
+ *   Perturbation: u as the sampled rule's step 2 with the counter c = ((b S + s) K + k) M + m (uint32; K = 1 is the counter of
+ *   mmb_decoder_sample_fused with N = 1); G = phi' + -logf(-logf(u)); Z_k = the max of G over slot k's candidates.
+ *   Child key: G truncated to at most the parent's key, key' = (key_k - fmaxf(v, 0)) - log1pf(expf(-fabsf(v))) with
+ *   v = (key_k - G) + log1mexp(G - Z_k), log1mexp(a) = a > -ln 2 ? logf(-expm1f(a)) : log1pf(-expf(a)) (all fp32).  The child with
+ *   G = Z_k gets exactly key_k.
+ *   A finished slot offers one carry (slot, eos) with its score, phi and key and step probability 1; empty slots offer nothing.
+ *   Selection: key descending, then step probability descending, then parent ascending, then sentence ascending (the beam's order with
+ *   key in place of score); the first K become the new slots, the rest stay empty.  A new slot's score is score_k + logf(p[m]), its
+ *   phi phi', its key key' (a carry keeps all three).
+ *   Threshold: kappa[b] = the largest key, over the steps, of the (K + 1)-th entry of that step's ranking (the best candidate the
+ *   step prunes), -inf when no step ranks more than K.  A pruned candidate's subtree holds a sequence with exactly its key and none
+ *   with a larger one, so kappa is the (K + 1)-th largest key of all sequences.
+ * So the K final slots are distinct token rows; the inclusion probability of final slot i is 1 - exp(-exp(phi_i - kappa)), and
+ * exp(phi_i) over it is an unbiased importance weight.
+ * Arguments of mmb_decoder_beam_constrained_fused (text_len required; no_repeat = min_sentences = 0 is the unconstrained rule) plus key
+ * and T.  Writes the beam's tokens / parents / scores (B,S,K) and probs (B,S,K,M), plus phi and keys (B,S,K) fp32, paths (B,K,S) int64
+ * (every final slot's tokens, step order), path_slots (B,K,S) int32 (its slot at every step) and kappa (B) fp32.  An empty final slot's
+ * path is eos at every step and its path_slots -1; its phi, key and score are -inf.  MMB_ERR_INVALID: K outside 1..8, S <= 0, T not
+ * finite and > 0, or a constraint out of range; MMB_ERR_UNSUPPORTED: B S K M + B > 2^32 (the counters of a key), or the shared memory of
+ * the width (with the byte count), as for the beam.
+ */
+MMB_API int mmb_decoder_beam_sample_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                          const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                          const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                          const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                          const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                          const uint8_t* mask, const int32_t* text_len, const unsigned long long* key, long long* tokens,
+                                          int32_t* parents, float* scores, float* probs, float* phi, float* keys, long long* paths,
+                                          int32_t* path_slots, float* kappa, int B, int Lt, int D, int H, int E, int M, int K, int S,
+                                          float T, int no_repeat, int min_sentences, mmb_stream_t stream);
+/*
  * Sampled summary roll-outs: N summaries per video, each the greedy roll-out (or the constrained one) with the pick DRAWN, all in ONE
  * launch of the same cluster kernel (one cluster per (video, sample); the encoder outputs are read per video, not replicated).  This
  * is the project's own rule.  Inputs: N in 1..64; temperature T finite and > 0; top_k 0 (off) or 1..8; a 64-bit key on the device

@@ -42,7 +42,8 @@ SIGNATURES = {
     "mmb_decoder_beam_fused": [c_void_p] * 31 + [c_int] * 8 + [c_void_p],
     "mmb_decoder_greedy_constrained_fused": [c_void_p] * 27 + [c_int] * 9 + [c_void_p],
     "mmb_decoder_beam_constrained_fused": [c_void_p] * 31 + [c_int] * 10 + [c_void_p],
-    "mmb_decoder_sample_fused": [c_void_p] * 28 + [c_int] * 8 + [c_float] + [c_int] * 3 + [c_void_p],
+    "mmb_decoder_beam_sample_fused": [c_void_p] * 35 + [c_int] * 8 + [c_float] + [c_int] * 2 + [c_void_p],
+    "mmb_decoder_sample_fused":[c_void_p] * 28 + [c_int] * 8 + [c_float] + [c_int] * 3 + [c_void_p],
     "mmb_sample_pick": [c_void_p] * 4 + [c_int] * 5 + [c_float, c_int, c_void_p, c_void_p],
     "mmb_decoder_sample_nucleus_fused": [c_void_p] * 28 + [c_int] * 8 + [c_float] + [c_int] * 3 + [c_float, c_void_p],
     "mmb_sample_pick_nucleus": [c_void_p] * 4 + [c_int] * 5 + [c_float, c_int, c_void_p, c_float, c_void_p],

@@ -301,6 +301,43 @@ struct NucleusArgs {
 };
 constexpr int kNucBuckets = 256;                            // radix digits of 8 bits, four passes over the bits of p
 
+// Stochastic beam roll-outs (mmb_decoder_beam_sample_fused; include/mmbidaf_b200.h states the rule): the beam roll-out with every
+// candidate ranked by its key -- its Gumbel-perturbed log-probability under the renormalised, tempered step distribution, truncated
+// below its parent's key -- instead of its score.  Per slot the table also keeps phi (the path's log-probability under that
+// distribution) and its key.  Before the selection three cluster exchanges per step give every live slot k its normaliser (mu_k, then
+// the integer mass Q_k) and the largest perturbed child Z_k; each rank then writes its candidates' keys into `off` and the beam's
+// selection runs on them.  The selection keeps K + 1 entries: the (K + 1)-th is the best key pruned at that step, and the threshold
+// kappa is the largest of them over the steps (every pruned subtree holds a sequence with exactly its root's key, and no larger one).
+struct StochArgs {
+  const unsigned long long* key;                            // (1) on the device
+  float T;                                                  // temperature > 0
+  float *phi, *keys;                                        // (B, S, K)
+  long long* paths;                                         // (B, K, S): every final slot's tokens (eos for an empty slot)
+  int* path_slots;                                          // (B, K, S): its slot at every step (-1 for an empty slot)
+  float* kappa;                                             // (B)
+  int off;                                                  // float offset of the stochastic region (stoch_floats)
+};
+__device__ __forceinline__ unsigned long long block_sum_u64(unsigned long long v, float* red) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  unsigned long long* r = reinterpret_cast<unsigned long long*>(red);   // (NW words: 32 floats)
+  __syncthreads();
+  if (lane == 0) r[warp] = v;
+  __syncthreads();
+  unsigned long long t = lane < NW ? r[lane] : 0ull;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+  return t;
+}
+// log(1 - e^a) for a <= 0, and the key of a child whose perturbed log-probability is G, under its parent's key kp and the largest
+// perturbed child Z (Kool et al. 2019, appendix B.3): at G = Z, v = -inf and the key is kp exactly
+__device__ __forceinline__ float log1mexpf(float a) { return a > -0.693147182f ? logf(-expm1f(a)) : log1pf(-expf(a)); }
+__device__ __forceinline__ float truncated_key(float kp, float G, float Z) {
+  const float v = (kp - G) + log1mexpf(G - Z);
+  return (kp - fmaxf(v, 0.f)) - log1pf(expf(-fabsf(v)));
+}
+
 // The nucleus of row v[0..M) (v[m] = p, or -1 for a non-candidate), in every thread of the block: its boundary p* (as bits) and m*, so
 // that the nucleus is {m : v[m] > p*} + {m : v[m] == p*, m <= m*}.  The masses are integers, so every sum below is exact in any order:
 // each rank of the cluster cuts its copy of the row to the same set.
@@ -415,10 +452,10 @@ __device__ __forceinline__ NucleusCut nucleus_cut(const float* __restrict__ v, i
 
 // kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one; kConstrained (with kGreedy): the pick skips
 // the sentences `cn` makes ineligible; kSample (with kGreedy, not kBeam): the pick is drawn (`sp`); kNucleus (with kSample): drawn
-// from the nucleus (`nu`)
-template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false, bool kNucleus = false>
+// from the nucleus (`nu`); kStoch (with kBeam): the stochastic beam (`st`)
+template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false, bool kNucleus = false, bool kStoch = false>
 __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn,
-                                               const SampleArgs sp, const NucleusArgs nu = NucleusArgs{}) {
+                                               const SampleArgs sp, const NucleusArgs nu = NucleusArgs{}, const StochArgs st = StochArgs{}) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int ob = blockIdx.x / CL;                         // the output row: the video (sampled: cluster_row(), the roll-out)
@@ -477,10 +514,11 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   int* const nt_tok = reinterpret_cast<int*>(nt_score + MAXK);           // [MAXK]   token,
   int* const nt_par = nt_tok + MAXK;                                     // [MAXK]   parent slot (-1: empty),
   int* const nt_kind = nt_par + MAXK;                                    // [MAXK]   status
-  float* const s_cand = nt_score + 4 * MAXK;    // [MAXC][MAXK][4] every rank's best K (score, p, parent, sentence), written remotely
-  float* const s_wred = s_cand + MAXC * MAXK * 4;                        // [NW][4] per-warp bests
-  float* const s_loc = s_wred + NW * 4;                                  // [MAXK][4] this rank's best K
-  float* const s_bh = s_loc + MAXK * 4;                                  // [K][ldh] h of every slot (the step's input)
+  constexpr int CS = kStoch ? MAXK + 1 : MAXK;  // exchange entries per rank (stochastic: K + 1, the best pruned key)
+  float* const s_cand = nt_score + 4 * MAXK;    // [MAXC][CS][4] every rank's best K (score, p, parent, sentence), written remotely
+  float* const s_wred = s_cand + MAXC * CS * 4;                          // [NW][4] per-warp bests
+  float* const s_loc = s_wred + NW * 4;                                  // [CS][4] this rank's best K
+  float* const s_bh = s_loc + CS * 4;                                    // [K][ldh] h of every slot (the step's input)
   float* const s_bhn = s_bh + KW * ldh;                                  // [K][ldh] h' of every slot
   float* const s_bc = s_bhn + KW * ldh;                                  // [K][ldc] cell of this rank's hidden units, in
   float* const s_bcn = s_bc + KW * ldc;                                  //          and out
@@ -527,6 +565,17 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       bs_score[tid] = tid == 0 ? 0.f : -INFINITY;
       bs_tok[tid] = -1;
       bs_stat[tid] = tid == 0 ? kLive : kEmpty;
+      if constexpr (kStoch) {              // slot 0: phi 0 and the key G_0 ~ Gumbel(0), of the counter B S K M + b
+        float k0 = -INFINITY;
+        if (tid == 0) {
+          const unsigned long long key = *st.key;
+          const uint32_t c = (uint32_t)a.B * (uint32_t)S * (uint32_t)KW * (uint32_t)M + (uint32_t)b;
+          const float u = ((float)(hash32(c, (uint32_t)key, (uint32_t)(key >> 32)) >> 9) + 0.5f) * 1.1920928955078125e-7f;
+          k0 = -logf(-logf(u));
+        }
+        smem[st.off + tid] = tid == 0 ? 0.f : -INFINITY;
+        smem[st.off + MAXK + tid] = k0;
+      }
     }
     for (int i = tid; i < H; i += NT) s_bh[i] = g.h0[(size_t)b * H + i];
     for (int i = tid; i < ldc; i += NT) s_bc[i] = 0.f;
@@ -1021,7 +1070,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     // (sampled, top_k > 0: the best top_k of this step's (p, sentence) candidates, and the draw among them)
     constexpr int kNone = 0x7fffffff;
     const int per = (M + CL - 1) / CL, m0 = min(M, R * per), m1 = min(M, m0 + per), nm = m1 - m0;
-    const int KS = kSample ? sp.top_k : KW;                      // the selection's width
+    // the selection's width (stochastic: one more, the best pruned key)
+    const int KS = kSample ? sp.top_k : kStoch ? KW + 1 : KW;
     // the exchange arrays (sampled: formed here from the parameter, so that nothing of them is held over the step's other stages)
     float* const q_cand = kSample ? smem + sp.off + 7 * MAXK : s_cand;
     float* const q_wred = kSample ? q_cand + MAXC * MAXK * 4 : s_wred;
@@ -1031,6 +1081,95 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     else for (int k = 0; k < KW; ++k) any_live = any_live || bs_stat[k] == kLive;
     __syncthreads();                                             // s_bp of the last run (sampled: this rank's p in s_cpart)
     const bool eos_ok = kSample && kConstrained && eos_allowed(cn, eos, kept);
+    // stochastic: the stochastic region (see StochArgs), formed here like the sampled exchange arrays
+    float* const x_phi = smem + st.off;                          // [MAXK] phi of every slot,
+    float* const x_key = x_phi + MAXK;                           // [MAXK]   key,
+    float* const x_nphi = x_key + MAXK;                          // [MAXK]   of the next table,
+    float* const x_nkey = x_nphi + MAXK;                         // [MAXK]
+    float* const x_lam = x_nkey + MAXK;                          // [MAXK] lam of every slot this step
+    unsigned long long* const x_q = reinterpret_cast<unsigned long long*>(x_lam + MAXK);   // [MAXC][MAXK] every rank's mass, remote
+    float* const x_mu = reinterpret_cast<float*>(x_q + MAXC * MAXK);                     // [MAXC][MAXK] every rank's max l, remote
+    float* const x_z = x_mu + MAXC * MAXK;                                               // [MAXC][MAXK] every rank's max G, remote
+    float* const s_key = x_z + MAXC * MAXK;                      // [K][ldp] the key of every (slot, sentence) of this rank
+    if constexpr (kStoch) {
+      if (any_live) {                                            // (uniform) the keys of every live slot's candidates
+        unsigned long long key;
+        asm volatile("ld.global.nc.u64 %0, [%1];" : "=l"(key) : "l"(st.key));
+        const float it = 1.f / st.T;                             // (l = logf(p) it is rounded before it is used: never an FMA)
+        auto cand = [&](int k, int m, float p) {                 // the beam's candidates (p > 0, eligible)
+          if (!(p > 0.f)) return false;
+          if constexpr (kConstrained) {
+            if (!((bu_cur[k * ldu + ((m - m0) >> 5)] >> ((m - m0) & 31)) & 1u)) return false;
+            if (m == eos && !eos_allowed(cn, eos, bk_cur[k])) return false;
+          }
+          return true;
+        };
+        auto rank_max = [&](const float* x, int k) {             // over the ranks (a rank without candidates gives -inf)
+          float v = -INFINITY;
+          for (int r = 0; r < CL; ++r) v = fmaxf(v, x[r * MAXK + k]);
+          return v;
+        };
+        // mu: the largest l = logf(p) / T of the candidates
+        for (int k = 0; k < KW; ++k) {
+          if (bs_stat[k] != kLive) continue;
+          float mx = -INFINITY;
+          for (int m = m0 + tid; m < m1; m += NT) {
+            const float p = s_bp[k * ldp + m - m0];
+            if (cand(k, m, p)) mx = fmaxf(mx, __fmul_rn(logf(p), it));
+          }
+          mx = block_max(mx, s_red);
+          if (tid < CL) cluster.map_shared_rank(x_mu, tid)[R * MAXK + k] = mx;
+        }
+        cluster.sync();
+        // Q: the integer masses floor(e^(l - mu) 2^24), summed exactly
+        for (int k = 0; k < KW; ++k) {
+          if (bs_stat[k] != kLive) continue;
+          const float mu = rank_max(x_mu, k);
+          unsigned long long q = 0;
+          for (int m = m0 + tid; m < m1; m += NT) {
+            const float p = s_bp[k * ldp + m - m0];
+            if (cand(k, m, p)) q += __float2ull_rz(expf(__fmul_rn(logf(p), it) - mu) * 16777216.f);
+          }
+          q = block_sum_u64(q, s_red);
+          if (tid < CL) cluster.map_shared_rank(x_q, tid)[R * MAXK + k] = q;
+        }
+        cluster.sync();
+        // lam, the perturbed log-probabilities G of the children and their largest, Z
+        for (int k = 0; k < KW; ++k) {
+          if (bs_stat[k] != kLive) continue;
+          unsigned long long Q = 0;
+          for (int r = 0; r < CL; ++r) Q += x_q[r * MAXK + k];
+          const float lam = rank_max(x_mu, k) + logf((float)Q * 5.9604644775390625e-8f);
+          if (tid == 0) x_lam[k] = lam;
+          const float phk = x_phi[k];
+          const uint32_t cb = (((uint32_t)b * (uint32_t)S + (uint32_t)s) * (uint32_t)KW + (uint32_t)k) * (uint32_t)M;
+          float mx = -INFINITY;
+          for (int m = m0 + tid; m < m1; m += NT) {
+            const float p = s_bp[k * ldp + m - m0];
+            float G = -INFINITY;
+            if (cand(k, m, p)) {
+              const float u = ((float)(hash32(cb + (uint32_t)m, (uint32_t)key, (uint32_t)(key >> 32)) >> 9) + 0.5f) * 1.1920928955078125e-7f;
+              G = (phk + (__fmul_rn(logf(p), it) - lam)) + -logf(-logf(u));
+              mx = fmaxf(mx, G);
+            }
+            s_key[k * ldp + m - m0] = G;
+          }
+          mx = block_max(mx, s_red);
+          if (tid < CL) cluster.map_shared_rank(x_z, tid)[R * MAXK + k] = mx;
+        }
+        cluster.sync();
+        // the keys: G truncated below the parent's key at Z
+        for (int k = 0; k < KW; ++k) {
+          if (bs_stat[k] != kLive) continue;
+          const float Z = rank_max(x_z, k), kp = x_key[k];
+          for (int m = m0 + tid; m < m1; m += NT) {
+            const float G = s_key[k * ldp + m - m0];
+            if (G != -INFINITY) s_key[k * ldp + m - m0] = truncated_key(kp, G, Z);
+          }
+        }
+        __syncthreads();
+      }
+    }
     if (any_live) {
       // this rank's best K of its (live slot, sentence) candidates, one block-wide pick per round; each pick ranks below the last
       float ps = INFINITY, pp = INFINITY;
@@ -1054,7 +1193,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
             if (!((bu_cur[k * ldu + ((m - m0) >> 5)] >> ((m - m0) & 31)) & 1u)) continue;
             if (m == eos && !eos_allowed(cn, eos, bk_cur[k])) continue;
           }
-          const float sc = bs_score[k] + logf(p);
+          const float sc = kStoch ? s_key[k * ldp + m - m0] : bs_score[k] + logf(p);      // (stochastic: ranked by key)
           if (cand_better(ps, pp, pk, pm, sc, p, k, m) && cand_better(sc, p, k, m, cs, cp, ck, cm)) { cs = sc; cp = p; ck = k; cm = m; }
         }
         cand_warp_best(cs, cp, ck, cm);
@@ -1082,7 +1221,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       }
       for (int i = tid; i < CL * KS * 4; i += NT) {              // -> slot R of every rank
         const int q = i / (KS * 4), e = i - q * KS * 4;
-        cluster.map_shared_rank(q_cand, q)[R * MAXK * 4 + e] = q_loc[e];
+        cluster.map_shared_rank(q_cand, q)[R * CS * 4 + e] = q_loc[e];
       }
       cluster.sync();
     }
@@ -1103,12 +1242,13 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
           float es, ep;
           int ek, em;
           if (i < npub) {
-            const float* e = q_cand + ((i / KS) * MAXK + i % KS) * 4;
+            const float* e = q_cand + ((i / KS) * CS + i % KS) * 4;
             es = e[0]; ep = e[1]; ek = __float_as_int(e[2]); em = __float_as_int(e[3]);
           } else {
             const int k = i - npub;
             if (bs_stat[k] != kDone) continue;
-            es = bs_score[k]; ep = 1.f; ek = k; em = eos;        // a finished slot carries its hypothesis with probability 1
+            // a finished slot carries its hypothesis with probability 1 (stochastic: its key)
+            es = kStoch ? x_key[k] : bs_score[k]; ep = 1.f; ek = k; em = eos;
           }
           if (ek == kNone) continue;
           if (cand_better(ps, pp, pk, pm, es, ep, ek, em) && cand_better(es, ep, ek, em, cs, cp, ck, cm)) { cs = es; cp = ep; ck = ek; cm = em; }
@@ -1121,6 +1261,22 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
             const uint32_t c = ((uint32_t)cluster_row() * (uint32_t)S + (uint32_t)s) * (uint32_t)M + (uint32_t)cm;
             const float z = kConstrained ? sample_z(sp, cp, c) : sample_score(cp, inv_t, c, key0, key1);
             if (drawn == M || z > bz || (z == bz && cm < drawn)) { bz = z; drawn = cm; }
+          }
+        } else if constexpr (kStoch) {
+          if (lane == 0) {
+            // the table as the beam's, with the score, phi and key of the new slot; the (K + 1)-th entry is the best pruned key,
+            // and the threshold the largest of them so far
+            const bool none = ck == kNone, carry = !none && bs_stat[ck] == kDone;
+            if (j == KW) {
+              if (R == 0) st.kappa[b] = fmaxf(s == 0 ? -INFINITY : st.kappa[b], none ? -INFINITY : cs);
+            } else {
+              nt_score[j] = none ? -INFINITY : carry ? bs_score[ck] : bs_score[ck] + logf(cp);
+              x_nphi[j] = none ? -INFINITY : carry ? x_phi[ck] : x_phi[ck] + (__fmul_rn(logf(cp), 1.f / st.T) - x_lam[ck]);
+              x_nkey[j] = none ? -INFINITY : cs;
+              nt_tok[j] = none ? -1 : cm;
+              nt_par[j] = none ? -1 : ck;
+              nt_kind[j] = none ? 0 : carry ? 3 : cm == eos ? 2 : 1;
+            }
           }
         } else if (lane == 0) {
           // kind: 0 empty, 1 live, 2 finished by this step's EOS pick, 3 carried
@@ -1180,6 +1336,10 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         bm.tokens[row + j] = nt_tok[j];
         bm.parents[row + j] = nt_par[j];
         bm.scores[row + j] = nt_score[j];
+        if constexpr (kStoch) {
+          st.phi[row + j] = x_nphi[j];
+          st.keys[row + j] = x_nkey[j];
+        }
       }
     for (int i = tid; i < KW * nm; i += NT) {                    // the row the parent produced (zero for carries and empty slots)
       const int j = i / nm, m = m0 + (i - j * nm), kd = nt_kind[j];
@@ -1204,6 +1364,10 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       bs_score[tid] = nt_score[tid];
       bs_tok[tid] = nt_tok[tid];
       bs_stat[tid] = kd == 1 ? kLive : kd == 0 ? kEmpty : kDone;
+      if constexpr (kStoch) {
+        x_phi[tid] = x_nphi[tid];
+        x_key[tid] = x_nkey[tid];
+      }
     }
     __syncthreads();
     if constexpr (kConstrained) {            // (uniform) the gathered bits are the next step's input
@@ -1215,7 +1379,18 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   }  // steps (the loop body keeps the step kernel's indentation)
   if constexpr (kBeam) {
     if (staged && tid == 0 && n > 0) tc::mbar_wait(bar_proj, (uint32_t)(runs & 1));   // the proj rows copied after the last run
-    if (R == 0 && tid == 0) {                                    // backtrack the best hypothesis: slot 0 after the last step
+    if constexpr (kStoch) {
+      if (R == 0 && tid < KW) {                                  // backtrack every final slot (an empty one: eos, slot -1)
+        const size_t o = ((size_t)b * KW + tid) * S;
+        int j = bm.parents[((size_t)b * S + S - 1) * KW + tid] < 0 ? -1 : tid;
+        for (int s = S - 1; s >= 0; --s) {
+          const size_t row = ((size_t)b * S + s) * KW;
+          st.path_slots[o + s] = j;
+          st.paths[o + s] = j >= 0 ? bm.tokens[row + j] : eos;
+          j = j >= 0 ? bm.parents[row + j] : -1;
+        }
+      }
+    } else if (R == 0 && tid == 0) {                             // backtrack the best hypothesis: slot 0 after the last step
       int j = 0;
       for (int s = S - 1; s >= 0; --s) {
         const size_t row = ((size_t)b * S + s) * KW;
@@ -1272,6 +1447,16 @@ __global__ void __launch_bounds__(NT) dec_sample_nucleus_constrained_kernel(cons
                                                                             const ConstraintArgs cn, const SampleArgs sp,
                                                                             const NucleusArgs nu) {
   dec_fused_body<true, false, true, true, true>(a, g, BeamArgs{}, cn, sp, nu);
+}
+
+__global__ void __launch_bounds__(NT) dec_beam_sample_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm,
+                                                             const StochArgs st) {
+  dec_fused_body<true, true, false, false, false, true>(a, g, bm, ConstraintArgs{}, SampleArgs{}, NucleusArgs{}, st);
+}
+
+__global__ void __launch_bounds__(NT) dec_beam_sample_constrained_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm,
+                                                                         const ConstraintArgs cn, const StochArgs st) {
+  dec_fused_body<true, true, true, false, false, true>(a, g, bm, cn, SampleArgs{}, NucleusArgs{}, st);
 }
 
 }  // namespace
@@ -1819,13 +2004,23 @@ static size_t beam_floats(int K, int CL, int chunk, int H, int M, bool constrain
 // floats of the nucleus region (see nucleus_cut): every rank's copy of the row, the histogram (u64) and the block exchanges (u64)
 static size_t nucleus_floats(int M) { return (((size_t)M + 3) & ~(size_t)3) + 2 * kNucBuckets + 2 * 32; }
 
+// floats the stochastic beam adds: the ninth exchange entry of every rank and of this rank's list (they lengthen the beam region),
+// then the stochastic region (phi / key tables, lam, the three exchanges of the normaliser and Z, every candidate's key)
+constexpr size_t kStochBeamExtra = MAXC * 4 + 4;
+static size_t stoch_floats(int K, int CL, int M) {
+  const size_t ldp = (((size_t)M + CL - 1) / CL + 3) & ~(size_t)3;
+  return 5 * MAXK + 2 * MAXC * MAXK + 2 * MAXC * MAXK + (size_t)K * ldp;
+}
+
 // Shape checks, cluster size, shared memory and row stage of the forward cluster kernels, then the launch: `g` null launches one step
 // (dec_step_fused_kernel), else the greedy roll-out (dec_greedy_fused_kernel), or with `bm` the beam roll-out (dec_beam_fused_kernel);
 // with `cn` the constrained roll-out of either (dec_greedy_constrained_kernel, dec_beam_constrained_kernel); with `sp` (not `bm`) the
 // sampled roll-out (dec_sample_kernel, with `cn` dec_sample_constrained_kernel), one cluster per (video, sample); with `sp` and `nu`
-// the nucleus roll-out (dec_sample_nucleus_kernel, with `cn` dec_sample_nucleus_constrained_kernel).
+// the nucleus roll-out (dec_sample_nucleus_kernel, with `cn` dec_sample_nucleus_constrained_kernel); with `bm` and `sb` the
+// stochastic beam (dec_beam_sample_kernel, with `cn` dec_beam_sample_constrained_kernel).
 static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr,
-                        const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr, NucleusArgs* nu = nullptr) {
+                        const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr, NucleusArgs* nu = nullptr,
+                        StochArgs* sb = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
@@ -1840,6 +2035,10 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   if (bm) {                                // the beam region behind the base arrays; the row stage follows if it still fits
     bm->off = (int)((smem + 15) / 16 * 4);
     smem = ((size_t)bm->off + beam_floats(bm->K, CL, a.chunk, H, M, cn != nullptr)) * 4 + 64;
+    if (sb) {                              // stochastic: the longer exchange, then its region
+      sb->off = (int)(((size_t)bm->off + beam_floats(bm->K, CL, a.chunk, H, M, cn != nullptr) + kStochBeamExtra + 3) & ~(size_t)3);
+      smem = ((size_t)sb->off + stoch_floats(bm->K, CL, M)) * 4 + 64;
+    }
     MMB_REQUIRE(smem <= 227 * 1024, MMB_ERR_UNSUPPORTED, "%s: width %d needs %zu B of shared memory per CTA, more than 232448 (B=%d Lt=%d M=%d)",
                 who, bm->K, smem, B, Lt, M);
   } else if (sp) {                         // sampled: the beam region's tables and exchange arrays, no slots
@@ -1868,10 +2067,11 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-  const int which = nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
+  static size_t smem_set[11] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  const int which = sb ? (cn ? 10 : 9) : nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
   if (smem > smem_set[which]) {
-    const void* fn = which == 8 ? (const void*)dec_sample_nucleus_constrained_kernel : which == 7 ? (const void*)dec_sample_nucleus_kernel
+    const void* fn = which == 10 ? (const void*)dec_beam_sample_constrained_kernel : which == 9 ? (const void*)dec_beam_sample_kernel
+                   : which == 8 ? (const void*)dec_sample_nucleus_constrained_kernel : which == 7 ? (const void*)dec_sample_nucleus_kernel
                    : which == 6 ? (const void*)dec_sample_constrained_kernel : which == 5 ? (const void*)dec_sample_kernel
                    : which == 4 ? (const void*)dec_beam_constrained_kernel : which == 3 ? (const void*)dec_greedy_constrained_kernel
                    : which == 2 ? (const void*)dec_beam_fused_kernel : which == 1 ? (const void*)dec_greedy_fused_kernel
@@ -1898,6 +2098,14 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (sb && cn) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_sample_constrained_kernel, a, *g, *bm, *cn, *sb));
+    return check_launch("dec_beam_sample_constrained_kernel");
+  }
+  if (sb) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_sample_kernel, a, *g, *bm, *sb));
+    return check_launch("dec_beam_sample_kernel");
+  }
   if (nu && cn) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_sample_nucleus_constrained_kernel, a, *g, *cn, *sp, *nu));
     return check_launch("dec_sample_nucleus_constrained_kernel");
@@ -2049,6 +2257,38 @@ extern "C" int mmb_decoder_beam_constrained_fused(const float* proj_a, const flo
   BeamArgs bm{text_len, tokens, parents, scores, probs, best, path, K, 0};
   const ConstraintArgs cn{text_len, no_repeat, min_sentences};
   return launch_fused(a, &g, "mmb_decoder_beam_constrained_fused", stream, &bm, &cn);
+}
+
+extern "C" int mmb_decoder_beam_sample_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                             const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                             const float* wc2, const float* v1b, const float* v2b, const float* Wb13t,
+                                             const float* vb1, const float* vb2, const float* vb1b, const float* vb2b,
+                                             const float* Wcatt, const float* bcat, const float* out_wt, const float* out_b,
+                                             const float* emb_text, const float* h0, const uint8_t* mask, const int* text_len,
+                                             const unsigned long long* key, long long* tokens, int* parents, float* scores,
+                                             float* probs, float* phi, float* keys, long long* paths, int* path_slots, float* kappa,
+                                             int B, int Lt, int D, int H, int E, int M, int K, int S, float T, int no_repeat,
+                                             int min_sentences, mmb_stream_t stream) {
+  using namespace mmb;
+  const char* who = "mmb_decoder_beam_sample_fused";
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && text_len && key && tokens &&
+                  parents && scores && probs && phi && keys && paths && path_slots && kappa,
+              MMB_ERR_INVALID, "%s: null pointer", who);
+  MMB_REQUIRE(K >= 1 && K <= MAXK && S > 0 && T > 0.f && isfinite(T) && (no_repeat == 0 || no_repeat == 1) && min_sentences >= 0,
+              MMB_ERR_INVALID, "%s: width K=%d (1..%d), S=%d, T=%g (finite, > 0), no_repeat=%d (0 or 1), min_sentences=%d (>= 0)", who,
+              K, MAXK, S, (double)T, no_repeat, min_sentences);
+  MMB_REQUIRE(B > 0 && M > 0, MMB_ERR_INVALID, "%s: B=%d M=%d", who, B, M);
+  MMB_REQUIRE((unsigned long long)B * S * K * M + B <= (1ull << 32), MMB_ERR_UNSUPPORTED,
+              "%s: B S K M + B = %d x %d x %d x %d + %d exceeds the 2^32 counters of a key", who, B, S, K, M, B);
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+              nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  BeamArgs bm{text_len, tokens, parents, scores, probs, nullptr, nullptr, K, 0};
+  const ConstraintArgs cn{text_len, no_repeat, min_sentences};
+  StochArgs sb{key, T, phi, keys, paths, path_slots, kappa, 0};
+  return launch_fused(a, &g, who, stream, &bm, no_repeat != 0 || min_sentences != 0 ? &cn : nullptr, nullptr, nullptr, &sb);
 }
 
 namespace mmb {

@@ -48,6 +48,21 @@ def nucleus(p, eligible=None, top_k: int = 0, top_p: float = 1.0) -> List[int]:
     return cand                                                          # (no candidate)
 
 
+def truncated_key(parent_key, g, z):
+    """The child key of the stochastic beam rule (mmb_decoder_beam_sample_fused in include/mmbidaf_b200.h) in numpy fp32: the
+    perturbed log-probability ``g`` of a child truncated to at most its parent's key ``parent_key``, given ``z``, the largest ``g`` of
+    the parent's children -- key' = (parent_key - max(v, 0)) - log1p(exp(-|v|)), v = (parent_key - g) + log1mexp(g - z),
+    log1mexp(a) = log(-expm1(a)) above -ln 2, else log1p(-exp(a)).  The child with g = z keeps parent_key exactly; the result is
+    monotone in g.  ``g`` may be an array.  (numpy's log1p / expm1 may round differently from the device's in the last bit.)"""
+    f = np.float32
+    kp, gv, zv = f(parent_key), np.asarray(g, dtype=f), f(z)
+    a = gv - zv
+    with np.errstate(divide="ignore", invalid="ignore"):
+        l1 = np.where(a > f(-0.6931472), np.log(-np.expm1(a)), np.log1p(-np.exp(a))).astype(f)
+        v = (kp - gv) + l1
+        return ((kp - np.maximum(v, f(0))) - np.log1p(np.exp(-np.abs(v)))).astype(f)
+
+
 def get_generated_indices(batch_out_distributions: torch.Tensor, original_text_lengths: Sequence[int]) -> List[List[int]]:
     """Greedy indices for a batch (B, T, M) (evaluate.py:167-183, method='greedy')."""
     host = batch_out_distributions.detach().cpu()

@@ -270,6 +270,25 @@ class MultimodalAttentionDecoder(nn.Module):
             return ops.decoder_beam_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
                                         text_len.to(torch.int32).contiguous(), steps, width, no_repeat, min_sentences)
 
+    def beam_sample(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, width, key, temperature=1.0, no_repeat=False,
+                    min_sentences=0):
+        """The stochastic beam decode of ``steps`` steps in eval mode: ``width`` (1..8) distinct sequences per video, a sample without
+        replacement from p^(1/``temperature``) renormalised over the candidates (the constraints included), as ONE launch of the
+        cluster kernel whatever ``ops.decoder_cut`` says; the rule (the keys, the counter of ``key``, the threshold) is documented at
+        mmb_decoder_beam_sample_fused in include/mmbidaf_b200.h.  Same start as :meth:`greedy`; ``text_len`` (B) int32 gives each
+        video's EOS row; ``key`` (1) int64 on the device.  No autograd.  Returns ``ops.decoder_beam_sample_fwd``'s (tokens, parents,
+        scores, probs, phi, keys, paths, path_slots, kappa)."""
+        if not enc_a.is_cuda:
+            raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
+        if self.num_layers != 1:
+            raise RuntimeError("MultimodalAttentionDecoder: only num_layers=1 is supported (the reference model uses 1)")
+        with torch.no_grad():
+            seq = self._sequence(enc_a, enc_i)["seq"]
+            B = seq.B
+            return ops.decoder_beam_sample_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
+                                               text_len.to(torch.int32).contiguous(), steps, width, key, temperature, no_repeat,
+                                               min_sentences)
+
     def sample(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, num_samples, key, temperature=1.0, top_k=0, no_repeat=False,
                min_sentences=0, *, top_p=1.0):
         """``num_samples`` sampled decodes of ``steps`` steps per video in eval mode, as ONE launch of the cluster kernel whatever

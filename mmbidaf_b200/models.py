@@ -144,7 +144,7 @@ class MMBiDAF(nn.Module):
         return torch.stack(out_distributions).transpose(0, 1), loss
 
     def summarize(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, targets=None, beam_width=None,
-                  no_repeat=False, min_sentences=0, num_samples=None, temperature=1.0, top_k=0, seed=None, top_p=1.0):
+                  no_repeat=False, min_sentences=0, num_samples=None, temperature=1.0, top_k=0, seed=None, top_p=1.0, replacement=True):
         """Extractive summaries of a batch (evaluate.py:107-126, :167-202 with method='greedy'): the eval-mode forward pass with the
         whole greedy decode roll-out on the device, then the greedy sentence selection on the device.  Runs under ``no_grad`` in eval
         mode and gives the caller's ``training`` flag back.  ``targets`` (B, T, 1) or (B, T) with T >= max_dec_len is optional (the
@@ -166,11 +166,17 @@ class MMBiDAF(nn.Module):
         The summary is the likeliest sample's (highest ``Samples.logp``, ties to the lower n); ``samples`` holds all N.  Not with
         ``beam_width`` or ``targets``.  ``top_p`` (in (0, 1], with ``num_samples``) draws each pick from the nucleus, the smallest
         prefix of the candidates (likeliest first) that holds ``top_p`` of their mass, cut from the model's p inside the same launch
-        (the rule at mmb_decoder_sample_nucleus_fused in include/mmbidaf_b200.h); 1 is no cut, the same launch as without it."""
+        (the rule at mmb_decoder_sample_nucleus_fused in include/mmbidaf_b200.h); 1 is no cut, the same launch as without it.
+        ``replacement=False`` (with ``num_samples`` K in 1..8, not with ``top_k`` or ``top_p``) draws K DISTINCT summaries per video, a
+        sample without replacement from the tempered, renormalised sequence distribution, by one stochastic beam roll-out
+        (``MultimodalAttentionDecoder.beam_sample``; the rule at mmb_decoder_beam_sample_fused in include/mmbidaf_b200.h).
+        ``samples`` then holds the K final slots in slot order (``logp`` their scores; an empty slot, when fewer than K sequences
+        exist, has an empty summary and logp -inf) and ``inclusion`` (``Inclusion``) their inclusion probabilities and importance
+        weights; the summary is the likeliest sample's."""
         from .layers.encoding import length_plan
-        from .summarize import Beams, Samples, Summary, best_sample, check_options, sample_logp
+        from .summarize import Beams, Inclusion, Samples, Summary, best_sample, check_options, sample_logp
         check_options("summarize", targets is not None, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed,
-                      top_p)
+                      top_p, replacement)
         constrained = no_repeat or min_sentences > 0
         was_training = self.training
         self.eval()
@@ -189,6 +195,17 @@ class MMBiDAF(nn.Module):
                 if num_samples is not None:
                     lens = length_plan(text_len, text.device).len_i32
                     key = ops.rng_next_keys(text.device, 1) if seed is None else ops.seed_key(seed, text.device)
+                    if not replacement:
+                        _, _, scores, rows, phi, keys, paths, slots, kappa = dec.beam_sample(
+                            text, h0, enc_a, enc_i, mask, lens, max_dec_len, num_samples, key, temperature, no_repeat, min_sentences)
+                        # every final slot's distribution rows: slot path_slots[b, k, s] of step s (zero rows for an empty slot)
+                        M = rows.shape[-1]
+                        idx = slots.long().clamp_min(0).unsqueeze(3).expand(-1, -1, -1, M)
+                        probs = rows.transpose(1, 2).gather(1, idx) * (slots >= 0).unsqueeze(3)
+                        samples = Samples(paths, probs, scores[:, -1])
+                        sel, cnt = ops.greedy_select(paths.view(B * num_samples, -1), lens.repeat_interleave(num_samples))
+                        best_probs, indices, counts = best_sample(samples, sel, cnt)
+                        return Summary(best_probs, None, indices, counts, None, samples, Inclusion(phi[:, -1], keys[:, -1], kappa))
                     probs, tokens = dec.sample(text, h0, enc_a, enc_i, mask, lens, max_dec_len, num_samples, key, temperature, top_k,
                                                no_repeat, min_sentences, top_p=top_p)
                     samples = Samples(tokens, probs, sample_logp(probs, tokens, lens))

@@ -524,6 +524,52 @@ def decoder_sample_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, ste
     return probs, tokens
 
 
+def decoder_beam_sample_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, text_len_i32, steps: int, width: int, key: torch.Tensor,
+                            temperature: float = 1.0, no_repeat: bool = False, min_sentences: int = 0):
+    """The stochastic beam roll-out (the rule at mmb_decoder_beam_sample_fused in include/mmbidaf_b200.h): ``width`` (1..8) distinct
+    sequences per video, sampled without replacement, as ONE launch of the cluster kernel whatever ``decoder_cut`` says.  Inputs as
+    :func:`decoder_beam_fwd`, plus ``key`` (1) int64 on the device (:func:`rng_next_keys` or :func:`seed_key`) and ``temperature``.
+    Returns (tokens (B,S,K) int64, parents (B,S,K) int32, scores (B,S,K) fp32, probs (B,S,K,M) fp32, phi (B,S,K) fp32, keys (B,S,K)
+    fp32, paths (B,K,S) int64, path_slots (B,K,S) int32, kappa (B) fp32) -- ``paths`` / ``path_slots`` are every final slot's tokens
+    and slots (eos / -1 for an empty slot), ``kappa`` the threshold of the inclusion probabilities."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    if not 1 <= int(width) <= BEAM_MAX_WIDTH:
+        raise ValueError(f"decoder_beam_sample_fwd: width {width} (1..{BEAM_MAX_WIDTH})")
+    if int(steps) <= 0:
+        raise ValueError(f"decoder_beam_sample_fwd: {steps} steps")
+    if isinstance(temperature, bool) or not isinstance(temperature, (int, float)) or not math.isfinite(temperature) or temperature <= 0:
+        raise ValueError(f"decoder_beam_sample_fwd: temperature {temperature!r}, expected a finite number > 0")
+    _check_constraints("decoder_beam_sample_fwd", no_repeat, min_sentences)
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M) or text_len_i32.shape != (B,):
+        raise ValueError(f"decoder_beam_sample_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask {tuple(mask_u8.shape)}, "
+                         f"text_len {tuple(text_len_i32.shape)} for B={B} Lt={Lt} E={E} H={H} M={M}")
+    if text_len_i32.dtype != torch.int32:
+        raise ValueError(f"decoder_beam_sample_fwd: text_len {text_len_i32.dtype}, not int32")
+    if key.dtype != torch.int64 or key.numel() != 1 or key.device != dev:
+        raise ValueError(f"decoder_beam_sample_fwd: key {key.dtype} {tuple(key.shape)} on {key.device}, expected one int64 on {dev}")
+    S, K = int(steps), int(width)
+    tokens = torch.empty(B, S, K, device=dev, dtype=torch.int64)
+    parents = torch.empty(B, S, K, device=dev, dtype=torch.int32)
+    scores = torch.empty(B, S, K, device=dev, dtype=torch.float32)
+    probs = torch.empty(B, S, K, M, device=dev, dtype=torch.float32)
+    phi = torch.empty(B, S, K, device=dev, dtype=torch.float32)
+    keys = torch.empty(B, S, K, device=dev, dtype=torch.float32)
+    paths = torch.empty(B, K, S, device=dev, dtype=torch.int64)
+    path_slots = torch.empty(B, K, S, device=dev, dtype=torch.int32)
+    kappa = torch.empty(B, device=dev, dtype=torch.float32)
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_beam_sample_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(text_len_i32), p(key.contiguous()), p(tokens),
+        p(parents), p(scores), p(probs), p(phi), p(keys), p(paths), p(path_slots), p(kappa), B, Lt, D, H, E, M, K, S,
+        float(temperature), int(no_repeat), int(min_sentences), _lib.stream()), "mmb_decoder_beam_sample_fused")
+    _count(1)
+    return tokens, parents, scores, probs, phi, keys, paths, path_slots, kappa
+
+
 def sample_pick(probs: torch.Tensor, key: torch.Tensor, row_base: torch.Tensor, S: int, s: int, N: int = 1, temperature: float = 1.0,
                 top_k: int = 0, eligible: Optional[torch.Tensor] = None, top_p: float = 1.0) -> torch.Tensor:
     """Steps 1 to 4 of the sampled pick (mmb_sample_pick) for the rows of ``probs`` (R, M) fp32: row r is sample r % N of video

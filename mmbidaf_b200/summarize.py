@@ -9,6 +9,7 @@ hypotheses per video (one launch too); the summary is the best hypothesis's, and
 """
 from __future__ import annotations
 
+import math
 from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
@@ -17,16 +18,26 @@ import torch.distributed as dist
 from .ops import BEAM_MAX_WIDTH, check_sampling
 from .synth import Batch
 
-__all__ = ["Beams", "Samples", "Summary", "Summarizer", "gather_summaries"]
+__all__ = ["Beams", "Inclusion", "Samples", "Summary", "Summarizer", "gather_summaries"]
 
 
 def check_options(who: str, with_targets: bool, beam_width, no_repeat, min_sentences, num_samples=None, temperature=1.0, top_k=0,
-                  seed=None, top_p=1.0) -> None:
+                  seed=None, top_p=1.0, replacement=True) -> None:
     """The decode options of ``MMBiDAF.summarize`` / ``Summarizer``, checked before any device work: ``beam_width`` None or an int
     in 1..8, ``no_repeat`` a bool, ``min_sentences`` an int >= 0; neither a beam nor a constraint with targets (the eval loss is
     defined by the unconstrained greedy roll-out).  Sampling: ``num_samples`` None or an int in 1..64, not with a beam or targets;
     ``temperature`` finite and > 0, ``top_k`` an int in 0..8, ``seed`` None or an int, ``top_p`` a real in (0, 1] -- set only with
-    ``num_samples``."""
+    ``num_samples``.  ``replacement`` a bool; False (the stochastic beam) needs ``num_samples`` in 1..8 and takes neither ``top_k``
+    nor ``top_p``."""
+    if not isinstance(replacement, bool):
+        raise ValueError(f"{who}: replacement {replacement!r}, expected a bool")
+    if not replacement:
+        if num_samples is None:
+            raise ValueError(f"{who}: replacement=False without num_samples")
+        if isinstance(num_samples, bool) or not isinstance(num_samples, int) or not 1 <= num_samples <= BEAM_MAX_WIDTH:
+            raise ValueError(f"{who}: num_samples {num_samples!r} with replacement=False, expected an int in 1..{BEAM_MAX_WIDTH}")
+        if isinstance(top_k, bool) or top_k != 0 or isinstance(top_p, bool) or top_p != 1.0:
+            raise ValueError(f"{who}: top_k / top_p with replacement=False -- the stochastic beam draws from every candidate")
     if num_samples is not None:
         check_sampling(who, num_samples, temperature, top_k, top_p)
         if beam_width is not None:
@@ -129,6 +140,31 @@ def best_sample(samples: Samples, sel: torch.Tensor, count: torch.Tensor):
     return samples.probs[rows, best], sel.view(B, N, S)[rows, best], count.view(B, N)[rows, best]
 
 
+class Inclusion(NamedTuple):
+    """What a sample without replacement (``MMBiDAF.summarize(..., num_samples=K, replacement=False)``, the rule at
+    mmb_decoder_beam_sample_fused in include/mmbidaf_b200.h) needs for estimates under the model: per final slot its log-probability
+    under the sampling distribution and its key, and per video the threshold.  Empty slots have logq = keys = -inf."""
+    logq: torch.Tensor                     # (B, K) fp32: phi of every final slot, the log-probability of its sequence
+    keys: torch.Tensor                     # (B, K) fp32: its perturbed log-probability (descending over the slots)
+    threshold: torch.Tensor                # (B) fp32: kappa, the (K + 1)-th key of all sequences (-inf when at most K exist)
+
+    def probabilities(self) -> torch.Tensor:
+        """(B, K) fp64: the probability that each sample is in a sample of K, 1 - exp(-exp(logq - threshold)); 1 where the threshold
+        is -inf (every sequence is in), 0 for empty slots.  Device ops only (capturable)."""
+        lq, th = self.logq.double(), self.threshold.double().unsqueeze(1)
+        p = -torch.expm1(-torch.exp(lq - th))
+        p = torch.where(th == -math.inf, torch.ones_like(p), p)
+        return torch.where(lq == -math.inf, torch.zeros_like(p), p)
+
+    def weights(self, normalise: bool = True) -> torch.Tensor:
+        """(B, K) fp64 importance weights exp(logq) / probabilities() (0 for empty slots): sum_i w_i f(y_i) is an unbiased estimate
+        of the expectation of f under the sampling distribution; ``normalise`` divides each video's weights by their sum (a
+        consistent estimate with lower variance).  Device ops only (capturable)."""
+        q = self.probabilities()
+        w = torch.where(q > 0, torch.exp(self.logq.double()) / q, torch.zeros_like(q))
+        return w / w.sum(1, keepdim=True) if normalise else w
+
+
 class Summary(NamedTuple):
     out_distributions: torch.Tensor        # (B, S, M) fp32: every step's distribution over the sentences, as MMBiDAF.forward returns
     loss: Optional[torch.Tensor]           # the eval loss (models.py:197-199) when targets were given, else None
@@ -136,6 +172,7 @@ class Summary(NamedTuple):
     counts: torch.Tensor                   # (B) int32: how many of them are valid
     beams: Optional[Beams] = None          # a beam summary's every slot (then out_distributions are the best path's rows), else None
     samples: Optional[Samples] = None      # a sampled summary's every sample (then the other fields are the likeliest sample's), else None
+    inclusion: Optional[Inclusion] = None  # a sample without replacement's inclusion probabilities and weights, else None
 
     def to_lists(self) -> List[List[int]]:
         """The chosen sentence indices per video as host lists (copies only ``indices`` and ``counts``):
@@ -145,7 +182,7 @@ class Summary(NamedTuple):
 
 
 def _bucket_key(batch: Batch, with_targets: bool, beam_width: Optional[int], no_repeat: bool = False, min_sentences: int = 0,
-                sampling: tuple = (None, 1.0, 0, None, 1.0)):
+                sampling: tuple = (None, 1.0, 0, None, 1.0, True)):
     return (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), int(batch.max_dec_len),
             tuple(batch.targets.shape) if with_targets else None, beam_width, no_repeat, min_sentences, sampling)
 
@@ -154,7 +191,7 @@ class _Bucket:
     """One captured ``summarize``: static inputs, static length plans, the graph and its (static) result."""
 
     def __init__(self, model, batch: Batch, with_targets: bool, warmup: int, beam_width: Optional[int] = None,
-                 no_repeat: bool = False, min_sentences: int = 0, sampling: tuple = (None, 1.0, 0, None, 1.0)):
+                 no_repeat: bool = False, min_sentences: int = 0, sampling: tuple = (None, 1.0, 0, None, 1.0, True)):
         import gc
         from .layers.encoding import pin_lengths
         dev = batch.text.device
@@ -164,7 +201,7 @@ class _Bucket:
         self.with_targets = with_targets
         self.beam_width = beam_width
         self.no_repeat, self.min_sentences = no_repeat, min_sentences
-        self.sampling = sampling             # (num_samples, temperature, top_k, seed, top_p); seed None: the key state exists after warm-up
+        self.sampling = sampling             # (num_samples, temperature, top_k, seed, top_p, replacement); seed None: the key state exists after warm-up
         self.plans = [pin_lengths(lst, dev) for lst in (self.batch.text_len, self.batch.audio_len, self.batch.image_len)]
         for m in model.modules():          # per-sequence caches of eager calls still own tensors (see Trainer.capture)
             if hasattr(m, "_cache"):
@@ -188,7 +225,7 @@ class _Bucket:
         return model.summarize(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, b.max_dec_len,
                                b.targets if self.with_targets else None, beam_width=self.beam_width, no_repeat=self.no_repeat,
                                min_sentences=self.min_sentences, num_samples=self.sampling[0], temperature=self.sampling[1],
-                               top_k=self.sampling[2], seed=self.sampling[3], top_p=self.sampling[4])
+                               top_k=self.sampling[2], seed=self.sampling[3], top_p=self.sampling[4], replacement=self.sampling[5])
 
     def load(self, batch: Batch) -> None:
         if batch is self.batch:
@@ -217,14 +254,16 @@ class Summarizer:
 
     def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None, no_repeat: bool = False,
                  min_sentences: int = 0, num_samples: Optional[int] = None, temperature: float = 1.0, top_k: int = 0,
-                 seed: Optional[int] = None, top_p: float = 1.0) -> Summary:
+                 seed: Optional[int] = None, top_p: float = 1.0, replacement: bool = True) -> Summary:
         """``batch`` resident on the device; ``with_targets`` also computes the eval loss from ``batch.targets``; ``beam_width``
         decodes by beam search, ``no_repeat`` / ``min_sentences`` constrain the pick (``MMBiDAF.summarize``); each width and each
         setting of the constraints in its own bucket.  ``num_samples`` / ``temperature`` / ``top_k`` / ``seed`` / ``top_p`` sample (each setting,
         the seed included, in its own bucket): with ``seed=None`` every replay draws a fresh key from the device key stream, with an int
-        seed every replay gives that seed's samples.  The options are checked before anything is copied or captured."""
-        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed, top_p)
-        sampling = (num_samples, temperature, top_k, seed, top_p)
+        seed every replay gives that seed's samples.  ``replacement=False`` samples without replacement (the stochastic beam, its own
+        buckets).  The options are checked before anything is copied or captured."""
+        check_options("Summarizer", with_targets, beam_width, no_repeat, min_sentences, num_samples, temperature, top_k, seed, top_p,
+                      replacement)
+        sampling = (num_samples, temperature, top_k, seed, top_p, replacement)
         key = _bucket_key(batch, with_targets, beam_width, no_repeat, min_sentences, sampling)
         bucket = self.buckets.get(key)
         if bucket is None:
