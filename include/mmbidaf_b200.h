@@ -209,6 +209,32 @@ MMB_API int mmb_decoder_greedy_fused(const float* proj_a, const float* proj_i, c
                                      const uint8_t* mask, const long long* target, float* probs, long long* argmax, float* loss_terms,
                                      int B, int Lt, int D, int H, int E, int M, int S, int T, mmb_stream_t stream);
 /*
+ * Forced summary roll-out: the model's likelihood of GIVEN sentence sequences, N candidates per video, all S steps in ONE launch of
+ * the same cluster kernel (one cluster per (video, candidate); the encoder outputs are read per video, not replicated).  This is the
+ * teacher-forced decode loop of models.py:156-179 (the training branches) without dropout or autograd.  Row r = b N + n, step s,
+ * t = tokens[b, n, s]:
+ *   The stages are the greedy roll-out's, bit for bit: its distribution is the step kernel's masked soft-max from the row's state.
+ *   Next input: emb_text[b, min(max(t, 0), Lt - 1)] (the greedy roll-out's clamp).  Step 0 starts from h0 with a zero cell,
+ *   coverage and input row, as the greedy roll-out does.
+ *   p_tok[b, n, s] = p[t] when 0 <= t < M, else 0 (an out-of-range token still feeds the clamped row to the next step).
+ *   loss_terms[s, 0, r] = -logf(p_tok + 1e-12f) for EVERY token (models.py:168-170), loss_terms[s, 1, r] = the coverage term
+ *   (models.py:177): the greedy roll-out's (S,2,B) layout with rows in place of videos.
+ * So the teacher-forced loss of row r is (sum_s nll + sum_s coverage) / S (models.py:179), and the p_tok and probs of a row whose
+ * tokens are another launch's picks (greedy arg-max, samples) are that launch's, bit for bit, where the cluster size is the same.
+ * There is no arg-max exchange: every CTA reads the next token from memory.
+ *   tokens (B,N,S) int64   probs (B,N,S,M) fp32 or NULL (the full rows, written only when set)   p_tok (B,N,S) fp32
+ *   loss_terms (S,2,B N) fp32
+ * Arguments of mmb_decoder_greedy_fused without target / argmax / T, plus tokens and N.  MMB_ERR_INVALID: N outside 1..64, S <= 0, or a
+ * null pointer other than probs; MMB_ERR_UNSUPPORTED: the shared-memory limits of mmb_decoder_greedy_fused.
+ */
+MMB_API int mmb_decoder_forced_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                     const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                     const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                     const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                     const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                     const uint8_t* mask, const long long* tokens, float* probs, float* p_tok, float* loss_terms,
+                                     int B, int Lt, int D, int H, int E, int M, int S, int N, mmb_stream_t stream);
+/*
  * Beam summary roll-out: the decode loop of models.py:156-199 in eval mode with K hypotheses per video instead of one, all S steps
  * in ONE launch of the same cluster kernel (one cluster per video holds every slot); the beam alternative to evaluate.py:185-202's
  * greedy pick.  This is the project's own beam rule; it does not claim parity with the reference's evaluate.py::beam_search.

@@ -317,6 +317,14 @@ struct StochArgs {
   float* kappa;                                             // (B)
   int off;                                                  // float offset of the stochastic region (stoch_floats)
 };
+// Forced roll-outs (mmb_decoder_forced_fused; include/mmbidaf_b200.h states the rule): the greedy roll-out with the token of every step
+// read from memory instead of reduced over the cluster -- the teacher-forced scoring of given candidates.  Cluster r runs candidate
+// r % N of video r / N; step s writes p[t] of its token t = tokens[r, s] and the loss terms of row r.  There is no arg-max exchange.
+struct ForcedArgs {
+  const long long* tokens;                                  // (B N, S)
+  float* p_tok;                                             // (B N, S)
+  int N;                                                    // candidates per video
+};
 __device__ __forceinline__ unsigned long long block_sum_u64(unsigned long long v, float* red) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
@@ -452,14 +460,17 @@ __device__ __forceinline__ NucleusCut nucleus_cut(const float* __restrict__ v, i
 
 // kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one; kConstrained (with kGreedy): the pick skips
 // the sentences `cn` makes ineligible; kSample (with kGreedy, not kBeam): the pick is drawn (`sp`); kNucleus (with kSample): drawn
-// from the nucleus (`nu`); kStoch (with kBeam): the stochastic beam (`st`)
-template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false, bool kNucleus = false, bool kStoch = false>
+// from the nucleus (`nu`); kStoch (with kBeam): the stochastic beam (`st`); kForced (with kGreedy alone): the tokens are given (`fo`)
+template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false, bool kNucleus = false, bool kStoch = false,
+          bool kForced = false>
 __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn,
-                                               const SampleArgs sp, const NucleusArgs nu = NucleusArgs{}, const StochArgs st = StochArgs{}) {
+                                               const SampleArgs sp, const NucleusArgs nu = NucleusArgs{}, const StochArgs st = StochArgs{},
+                                               const ForcedArgs fo = ForcedArgs{}) {
+  static_assert(!kForced || (kGreedy && !kBeam && !kConstrained && !kSample), "the forced roll-out is the greedy one's");
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
-  const int ob = blockIdx.x / CL;                         // the output row: the video (sampled: cluster_row(), the roll-out)
-  const int b = kSample ? cluster_row() / sp.N : ob;      // the video whose inputs the cluster reads
+  const int ob = blockIdx.x / CL;                         // the output row: the video (sampled / forced: cluster_row(), the roll-out)
+  const int b = kSample ? cluster_row() / sp.N : kForced ? cluster_row() / fo.N : ob;   // the video whose inputs the cluster reads
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int D = a.D, H = a.H, E = a.E, M = a.M, Lt = a.Lt, K = D + E + H;
 
@@ -503,7 +514,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   DEC_STAMP(0);
   const int S = kGreedy ? g.steps : 1;
   float cell_own = 0.f;                    // greedy: the cell of hidden unit j0 + tid (stage D), carried between the steps
-  int pick = 0;                            // greedy: the previous step's arg-max
+  int pick = 0;                            // greedy: the previous step's arg-max (forced: its token, clamped to 0..Lt-1)
   // beam: the region behind the base arrays (beam_floats)
   const int KW = kBeam ? bm.K : 1;
   const int ldh = up4(H), ldc = up4(split4(H, CL)), ldv = up4(a.chunk), ldp = up4((M + CL - 1) / CL);
@@ -707,8 +718,9 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       else energies(s_st0, s_st1, N8{}, R2{});
     } else {
       // (the constrained nucleus roll-out holds more across the step: two rows per warp round keep it at 128 registers without a
-      // spill -- four spilled 80 bytes around these loads.  The rows' sums are the same either way)
-      using RL = std::conditional_t<kNucleus && kConstrained, R2, R4>;
+      // spill -- four spilled 80 bytes around these loads; so does the forced roll-out, where four spilled 24 bytes of the state it
+      // carries over the step.  The rows' sums are the same either way)
+      using RL = std::conditional_t<(kNucleus && kConstrained) || kForced, R2, R4>;
       if (nj7) energies(gpa, gpi, N7{}, RL{});
       else energies(gpa, gpi, N8{}, RL{});
     }
@@ -934,9 +946,9 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   if constexpr (kBeam)                     // (s_hn is written again only behind the cluster barriers of the next run)
     for (int i = tid; i < H; i += NT) s_bhn[slot * ldh + i] = s_hn[i];
   // greedy: the probabilities / arg-max of step s go to row (b, s) of (B, S, M) / (B, S); the loss terms (S, 2, B) to row s
-  // (sampled: row (b N + n, s) of (B N, S, M) / (B N, S))
-  const size_t prow = kGreedy ? (size_t)(kSample ? cluster_row() : ob) * S + s : (size_t)b;
-  const int lrow = kGreedy ? s * 2 * a.B + b : b;
+  // (sampled: row (b N + n, s) of (B N, S, M) / (B N, S); forced: the same rows, and the loss terms (S, 2, B N) to row (s, b N + n))
+  const size_t prow = kGreedy ? (size_t)(kSample || kForced ? cluster_row() : ob) * S + s : (size_t)b;
+  const int lrow = kForced ? s * 2 * a.B * fo.N + cluster_row() : kGreedy ? s * 2 * a.B + b : b;
   if (R == 0 && tid == 0 && a.cov_loss) {
     float cs = 0.f;
     for (int r = 0; r < CL; ++r) cs += s_ex[r * 8 + 0];
@@ -981,7 +993,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     for (int m = m0 + tid; m < m1; m += NT) {
       const float p = expf(lg[m - m0] - gmx) * inv;
       if constexpr (kBeam) s_bp[slot * ldp + m - m0] = p;
-      else a.probs[prow * M + m] = p;
+      else if (!kForced || a.probs) a.probs[prow * M + m] = p;   // (forced: the rows are optional)
+      if constexpr (kForced) continue;                           // (its token's p follows the loop)
       if constexpr (kSample) {
         // top_k = 0: the first maximum of z over the candidates (the first candidate stands even at z = -inf);
         // top_k > 0: this rank's p for the selection below
@@ -1015,8 +1028,20 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         }
       }
     }
+    if constexpr (kForced) {
+      // this step's token t (compared whole: any int64 is a token).  Thread 0 of the rank that owns t writes p[t] -- the loop's
+      // expression over the same logit, so the loop's bits -- and its nll (models.py:168-170); a token no rank owns has p = 0 and
+      // nll -logf(0 + 1e-12f), written by rank 0
+      const long long t = fo.tokens[prow];
+      if (tid == 0 && (t >= m0 && t < m1 || R == 0 && (t < 0 || t >= M))) {
+        const float p = t >= m0 && t < m1 ? expf(lg[t - m0] - gmx) * inv : 0.f;
+        fo.p_tok[prow] = p;
+        a.nll[lrow] = -logf(p + 1e-12f);
+      }
+      pick = (int)min(max(t, 0ll), (long long)(Lt - 1));        // the next input row, clamped as the greedy roll-out's
+    }
     // (sampled with top_k > 0: the pick is made after the step, by the selection)
-    if (!kBeam && (kGreedy || a.argmax) && !(kSample && sp.top_k > 0)) {     // first maximal index, as torch.max(dim) documents
+    if (!kBeam && !kForced && (kGreedy || a.argmax) && !(kSample && sp.top_k > 0)) {     // first maximal index, as torch.max(dim) documents
       const float bbest = block_max(best, s_red);
       int cand = best == bbest ? best_i : M;
 #pragma unroll
@@ -1405,6 +1430,18 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
   // candidates -- lies before a cluster barrier it has passed, so nothing can still be written into a rank that leaves here.  In the
   // greedy loop the same holds between the steps: a store of step s + 1 into another rank lies behind at least one cluster barrier
   // that the other rank reaches only after its last read of what step s stored there.)
+  // The forced roll-out drops the arg-max exchange and the cluster barrier behind it (#6 below), so a step has five: #1 after stage A,
+  // #2 after the partials of stage B, #3 after stage C, #4 after stage D, #5 after the soft-max statistics of stage E.  Every remote
+  // store of step s + 1 still lies behind a barrier that every rank passes after its last read of the same words in step s:
+  //   s_hw     stored in A (s + 1), before #1 (s + 1); last read in C (s), before #4 (s)         -- the writer has passed #4 (s), #5 (s)
+  //   s_part   stored in B (s + 1), after #1 (s + 1); last read in the merge (s), before #3 (s)   -- #3 (s) and on
+  //   s_pb     stored in C (s + 1), after #2 (s + 1); last read in C (s), before #4 (s)           -- #4 (s) and on
+  //   s_ex[0]  stored in C (s + 1), after #3 (s + 1); rank 0 reads it between #4 (s) and #5 (s)   -- #5 (s) and on
+  //   s_hn     stored in D (s + 1), after #3 (s + 1); last read by stage 0 (s + 1), before #1 (s + 1)
+  //   s_ex[1..2] stored in E (s + 1), after #4 (s + 1); last read in E (s), after #5 (s), before #1 (s + 1)
+  // and no rank reads another's shared memory (DSMEM is written only).  At the exit the last remote store of every rank is the
+  // soft-max statistics of the last step, before #5 of that step: every rank has passed #5 before it leaves, so nothing can still be
+  // written into a rank that has left.
   DEC_STAMP(17);
 }
 
@@ -1457,6 +1494,11 @@ __global__ void __launch_bounds__(NT) dec_beam_sample_kernel(const FusedArgs a, 
 __global__ void __launch_bounds__(NT) dec_beam_sample_constrained_kernel(const FusedArgs a, const GreedyArgs g, const BeamArgs bm,
                                                                          const ConstraintArgs cn, const StochArgs st) {
   dec_fused_body<true, true, true, false, false, true>(a, g, bm, cn, SampleArgs{}, NucleusArgs{}, st);
+}
+
+__global__ void __launch_bounds__(NT) dec_forced_kernel(const FusedArgs a, const GreedyArgs g, const ForcedArgs fo) {
+  dec_fused_body<true, false, false, false, false, false, true>(a, g, BeamArgs{}, ConstraintArgs{}, SampleArgs{}, NucleusArgs{},
+                                                                StochArgs{}, fo);
 }
 
 }  // namespace
@@ -2017,15 +2059,17 @@ static size_t stoch_floats(int K, int CL, int M) {
 // with `cn` the constrained roll-out of either (dec_greedy_constrained_kernel, dec_beam_constrained_kernel); with `sp` (not `bm`) the
 // sampled roll-out (dec_sample_kernel, with `cn` dec_sample_constrained_kernel), one cluster per (video, sample); with `sp` and `nu`
 // the nucleus roll-out (dec_sample_nucleus_kernel, with `cn` dec_sample_nucleus_constrained_kernel); with `bm` and `sb` the
-// stochastic beam (dec_beam_sample_kernel, with `cn` dec_beam_sample_constrained_kernel).
+// stochastic beam (dec_beam_sample_kernel, with `cn` dec_beam_sample_constrained_kernel); with `fo` (and `g` alone) the forced roll-out
+// (dec_forced_kernel), one cluster per (video, candidate).
 static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr,
                         const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr, NucleusArgs* nu = nullptr,
-                        StochArgs* sb = nullptr) {
+                        StochArgs* sb = nullptr, const ForcedArgs* fo = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
   MMB_REQUIRE(D <= 256, MMB_ERR_UNSUPPORTED, "%s: D=%d > 256", who, D);
-  const int rows = sp ? B * sp->N : B;     // clusters: one per video, or per (video, sample)
+  // clusters: one per video, or per (video, sample), or per (video, candidate)
+  const int rows = sp ? B * sp->N : fo ? B * fo->N : B;
   // few videos: eight CTAs per video keep more of the chip busy on the text sweep
   const int CL = (long long)rows * 4 * 2 <= 160 ? 8 : 4;
   size_t smem = fused_smem_bytes(Lt, D, H, E, M, CL, &a.chunk);
@@ -2067,10 +2111,11 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[11] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  const int which = sb ? (cn ? 10 : 9) : nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
+  static size_t smem_set[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  const int which = fo ? 11 : sb ? (cn ? 10 : 9) : nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
   if (smem > smem_set[which]) {
-    const void* fn = which == 10 ? (const void*)dec_beam_sample_constrained_kernel : which == 9 ? (const void*)dec_beam_sample_kernel
+    const void* fn = which == 11 ? (const void*)dec_forced_kernel
+                   : which == 10 ? (const void*)dec_beam_sample_constrained_kernel : which == 9 ? (const void*)dec_beam_sample_kernel
                    : which == 8 ? (const void*)dec_sample_nucleus_constrained_kernel : which == 7 ? (const void*)dec_sample_nucleus_kernel
                    : which == 6 ? (const void*)dec_sample_constrained_kernel : which == 5 ? (const void*)dec_sample_kernel
                    : which == 4 ? (const void*)dec_beam_constrained_kernel : which == 3 ? (const void*)dec_greedy_constrained_kernel
@@ -2098,6 +2143,10 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (fo) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_forced_kernel, a, *g, *fo));
+    return check_launch("dec_forced_kernel");
+  }
   if (sb && cn) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_beam_sample_constrained_kernel, a, *g, *bm, *cn, *sb));
     return check_launch("dec_beam_sample_constrained_kernel");
@@ -2186,6 +2235,30 @@ extern "C" int mmb_decoder_greedy_fused(const float* proj_a, const float* proj_i
               nullptr, B, Lt, D, H, E, M, 0, 0};
   const GreedyArgs g{emb_text, h0, S, target ? T : 0};
   return launch_fused(a, &g, "mmb_decoder_greedy_fused", stream);
+}
+
+extern "C" int mmb_decoder_forced_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                        const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                        const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                        const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                        const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                        const uint8_t* mask, const long long* tokens, float* probs, float* p_tok, float* loss_terms,
+                                        int B, int Lt, int D, int H, int E, int M, int S, int N, mmb_stream_t stream) {
+  using namespace mmb;
+  const char* who = "mmb_decoder_forced_fused";
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && tokens && p_tok && loss_terms,
+              MMB_ERR_INVALID, "%s: null pointer", who);
+  MMB_REQUIRE(S > 0 && N >= 1 && N <= 64, MMB_ERR_INVALID, "%s: S=%d, N=%d (1..64)", who, S, N);
+  MMB_REQUIRE(B > 0, MMB_ERR_INVALID, "%s: B=%d", who, B);
+  // (probs may be null: the full rows are written only when asked for)
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, probs, nullptr, nullptr, nullptr, nullptr, nullptr,
+              loss_terms, loss_terms + (size_t)B * N, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+              B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  const ForcedArgs fo{tokens, p_tok, N};
+  return launch_fused(a, &g, who, stream, nullptr, nullptr, nullptr, nullptr, nullptr, &fo);
 }
 
 extern "C" int mmb_decoder_beam_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,

@@ -254,6 +254,21 @@ class MultimodalAttentionDecoder(nn.Module):
                 terms.append(lossvec)
             return torch.stack(probs, 1), torch.stack(picks, 1), (torch.stack(terms) if tgt is not None else None)
 
+    def force(self, emb_text, h0, enc_a, enc_i, mask, tokens, want_probs=False):
+        """The teacher-forced decode of given token rows in eval mode: ``tokens`` (B, N, S) int64, N (1..64) candidates per video,
+        each run as :meth:`greedy` runs with its own tokens as the picks (the rule at mmb_decoder_forced_fused in
+        include/mmbidaf_b200.h), as ONE launch of the cluster kernel whatever ``ops.decoder_cut`` says.  Same start as :meth:`greedy`.
+        No autograd.  Returns ``ops.decoder_forced_fwd``'s (probs (B,N,S,M) or None, p_tok (B,N,S), loss_terms (S,2,B N))."""
+        if not enc_a.is_cuda:
+            raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
+        if self.num_layers != 1:
+            raise RuntimeError("MultimodalAttentionDecoder: only num_layers=1 is supported (the reference model uses 1)")
+        with torch.no_grad():
+            seq = self._sequence(enc_a, enc_i)["seq"]
+            B = seq.B
+            return ops.decoder_forced_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
+                                          tokens.contiguous(), want_probs)
+
     def beam(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, width, no_repeat=False, min_sentences=0):
         """The beam decode of ``steps`` steps in eval mode with ``width`` (1..8) hypotheses per video, as ONE launch of the cluster
         kernel whatever ``ops.decoder_cut`` says (there is no chunk-cut beam); the rule is documented at mmb_decoder_beam_fused in

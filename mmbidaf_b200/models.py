@@ -235,6 +235,47 @@ class MMBiDAF(nn.Module):
             self.train(was_training)
         return Summary(probs, loss, indices, counts)
 
+    def score(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, candidates, probs=False):
+        """The model's likelihood of given summaries of a batch: every candidate's teacher-forced roll-out of ``max_dec_len`` steps
+        (models.py:156-179 in training mode, without dropout), N candidates per video in ONE launch of the cluster kernel
+        (``MultimodalAttentionDecoder.force``; the rule at mmb_decoder_forced_fused in include/mmbidaf_b200.h).  Runs like
+        :meth:`summarize`: eval mode, ``no_grad``, the encoder half once per video, the caller's ``training`` flag given back.
+        ``candidates`` is either a device tensor (B, N, max_dec_len) int64 of token rows with N in 1..64, used as is with every row
+        valid (capturable: ``Samples.tokens`` or beam paths go in directly), or host lists, per video, of candidate summaries as
+        sentence-index lists, turned into rows by ``summarize.candidate_tokens`` (ValueError, before any device work, for a bad
+        candidate).  ``probs`` also returns every step's distribution.  Returns ``Scores(tokens, step_p, logp, loss, valid, probs)``:
+        ``logp`` by the rule of ``Samples.logp``, ``loss`` the teacher-forced loss of each row (the training loss of ``forward`` per
+        video), -inf / +inf on invalid rows."""
+        from .layers.encoding import length_plan
+        from .ops import FORCED_MAX_N
+        from .summarize import candidate_tokens, forced_scores
+        if not isinstance(probs, bool):
+            raise ValueError(f"score: probs {probs!r}, expected a bool")
+        B, S = text.size(0), int(max_dec_len)
+        if torch.is_tensor(candidates):
+            if candidates.dtype != torch.int64 or candidates.dim() != 3 or candidates.shape[0] != B or \
+                    not 1 <= candidates.shape[1] <= FORCED_MAX_N or candidates.shape[2] != S or candidates.device != text.device:
+                raise ValueError(f"score: candidates {candidates.dtype} {tuple(candidates.shape)} on {candidates.device}, expected "
+                                 f"(B={B}, N in 1..{FORCED_MAX_N}, max_dec_len={S}) int64 on {text.device}")
+            tokens, valid = candidates, None
+        else:
+            tokens, valid = candidate_tokens(candidates, text_len, S)
+            if tokens.shape[0] != B:
+                raise ValueError(f"score: candidates for {tokens.shape[0]} videos, the batch holds {B}")
+            tokens, valid = tokens.to(text.device), valid.to(text.device)
+        was_training = self.training
+        self.eval()
+        try:
+            with torch.no_grad():
+                dec = self.multimodal_att_decoder
+                enc_a, enc_i, h0, mask = self._encode(text, text_len, audio, audio_len, images, image_len, dec.prepare)
+                rows, p_tok, terms = dec.force(text, h0, enc_a, enc_i, mask, tokens, want_probs=probs)
+                if valid is None:
+                    valid = torch.ones(tokens.shape[:2], dtype=torch.bool, device=text.device)
+                return forced_scores(tokens, p_tok, terms, valid, length_plan(text_len, text.device).len_i32, rows)
+        finally:
+            self.train(was_training)
+
     def _encode(self, embedded_text, original_text_lengths, embedded_audio, original_audio_lengths, transformed_images,
                 original_image_lengths, decoder_start):
         """The encoder half of the model (models.py:95-143): embeddings, encoders, masks, both BiDAF blocks, the modality LSTMs and

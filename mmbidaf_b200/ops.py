@@ -382,6 +382,39 @@ def decoder_greedy_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, steps: int, targe
     return probs, argmax, terms
 
 
+FORCED_MAX_N = 64
+
+
+def decoder_forced_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, tokens, want_probs: bool = False):
+    """The teacher-forced roll-out of given token rows (the rule at mmb_decoder_forced_fused in include/mmbidaf_b200.h) as ONE launch
+    of the cluster kernel, whatever ``decoder_cut`` says: N candidates per video, each the greedy roll-out with its own tokens as the
+    picks.  emb_text (B,Lt,E) fp32, h0 (B,H) fp32, mask_u8 (B,M) uint8, tokens (B,N,S) int64 with N in 1..64 -- contiguous, on the
+    device.  A token outside 0..M-1 scores p = 0 and feeds the clamped row.  Returns (probs (B,N,S,M) fp32 or None without
+    ``want_probs``, p_tok (B,N,S) fp32 = each step's p of its token, loss_terms (S,2,B N) = per step [nll | coverage term])."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M):
+        raise ValueError(f"decoder_forced_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask {tuple(mask_u8.shape)} "
+                         f"for B={B} Lt={Lt} E={E} H={H} M={M}")
+    if tokens.dtype != torch.int64 or tokens.dim() != 3 or tokens.shape[0] != B or tokens.device != dev or \
+            not 1 <= tokens.shape[1] <= FORCED_MAX_N or tokens.shape[2] <= 0:
+        raise ValueError(f"decoder_forced_fwd: tokens {tokens.dtype} {tuple(tokens.shape)} on {tokens.device}, expected (B={B}, "
+                         f"N in 1..{FORCED_MAX_N}, S > 0) int64 on {dev}")
+    N, S = int(tokens.shape[1]), int(tokens.shape[2])
+    probs = torch.empty(B, N, S, M, device=dev, dtype=torch.float32) if want_probs else None
+    p_tok = torch.empty(B, N, S, device=dev, dtype=torch.float32)
+    terms = torch.empty(S, 2, B * N, device=dev, dtype=torch.float32)
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_forced_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(tokens.contiguous()), p(probs), p(p_tok),
+        p(terms), B, Lt, D, H, E, M, S, N, _lib.stream()), "mmb_decoder_forced_fused")
+    _count(1)
+    return probs, p_tok, terms
+
+
 def _check_constraints(who: str, no_repeat, min_sentences) -> None:
     if not isinstance(no_repeat, int) or no_repeat not in (0, 1):
         raise ValueError(f"{who}: no_repeat {no_repeat!r}, expected a bool")

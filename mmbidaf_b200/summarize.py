@@ -5,11 +5,13 @@ without a host round trip; its result is a :class:`Summary`.  With ``beam_width=
 hypotheses per video (one launch too); the summary is the best hypothesis's, and :class:`Beams` holds all K.  With
 ``num_samples=N`` N summaries per video are drawn inside one launch (temperature, top-k, top-p); the summary is the likeliest sample's, and
 :class:`Samples` holds all N.  ``no_repeat`` and ``min_sentences`` constrain any pick inside the roll-out kernel.
-:class:`Summarizer` replays ``summarize`` from CUDA graphs, one capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
+``MMBiDAF.score`` evaluates given candidate summaries instead: their teacher-forced likelihood under the model (:class:`Scores`).
+:class:`Summarizer` replays ``summarize`` (and ``score``) from CUDA graphs, one capture per padded-shape bucket.  :func:`gather_summaries` collects the summaries of a data-parallel job on rank 0.
 """
 from __future__ import annotations
 
 import math
+import numbers
 from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
@@ -18,7 +20,7 @@ import torch.distributed as dist
 from .ops import BEAM_MAX_WIDTH, check_sampling
 from .synth import Batch
 
-__all__ = ["Beams", "Inclusion", "Samples", "Summary", "Summarizer", "gather_summaries"]
+__all__ = ["Beams", "Inclusion", "Samples", "Scores", "Summary", "Summarizer", "candidate_tokens", "gather_summaries"]
 
 
 def check_options(who: str, with_targets: bool, beam_width, no_repeat, min_sentences, num_samples=None, temperature=1.0, top_k=0,
@@ -122,13 +124,88 @@ class Samples(NamedTuple):
         return [[(_select(row, lens[b]), lp[b][n]) for n, row in enumerate(rows)] for b, rows in enumerate(tok)]
 
 
-def sample_logp(probs: torch.Tensor, tokens: torch.Tensor, text_len_i32: torch.Tensor) -> torch.Tensor:
-    """logp (B, N) fp32 of sampled roll-outs: the sum of log p_s[tok_s] over the steps up to and including the first EOS pick
-    (text_len - 1), or over all S without one.  Device ops only (capturable)."""
-    lp = torch.log(probs.gather(3, tokens.clamp_min(0).unsqueeze(3)).squeeze(3))               # (B, N, S)
+def path_logp(step_p: torch.Tensor, tokens: torch.Tensor, text_len_i32: torch.Tensor) -> torch.Tensor:
+    """logp (B, N) fp32 of token rows (B, N, S) from the probability of each step's token ``step_p`` (B, N, S): the sum of
+    log step_p over the steps up to and including the first EOS token (text_len - 1), or over all S without one.  The rule of
+    ``Samples.logp`` and ``Scores.logp``.  Device ops only (capturable)."""
+    lp = torch.log(step_p)
     hit = (tokens == (text_len_i32.long() - 1).view(-1, 1, 1)).long()
     after = (hit.cumsum(2) - hit) > 0                                                          # steps after the first EOS pick
     return torch.where(after, torch.zeros_like(lp), lp).sum(2)
+
+
+def sample_logp(probs: torch.Tensor, tokens: torch.Tensor, text_len_i32: torch.Tensor) -> torch.Tensor:
+    """logp (B, N) fp32 of sampled roll-outs: :func:`path_logp` of each pick's p in ``probs`` (B, N, S, M).  Device ops only
+    (capturable)."""
+    return path_logp(probs.gather(3, tokens.clamp_min(0).unsqueeze(3)).squeeze(3), tokens, text_len_i32)
+
+
+class Scores(NamedTuple):
+    """The model's teacher-forced likelihood of given candidates (``MMBiDAF.score``, the rule at mmb_decoder_forced_fused in
+    include/mmbidaf_b200.h).  Rows that hold no candidate (``valid`` False: padding of a video with fewer candidates) have
+    logp -inf and loss +inf."""
+    tokens: torch.Tensor                   # (B, N, S) int64: the forced token rows
+    step_p: torch.Tensor                   # (B, N, S) fp32: the p of each step's token (0 for a token outside 0..M-1)
+    logp: torch.Tensor                     # (B, N) fp32: sum of log step_p up to and including the first EOS token (all S without)
+    loss: torch.Tensor                     # (B, N) fp32: the teacher-forced loss (sum_s nll_s + sum_s coverage_s) / S (models.py:168-179)
+    valid: torch.Tensor                    # (B, N) bool: whether the row holds a real candidate
+    probs: Optional[torch.Tensor] = None   # (B, N, S, M) fp32: every step's distribution, when asked for
+
+
+def candidate_tokens(candidates, text_len, steps: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Token rows of candidate summaries given as host lists: ``candidates[b]`` is video b's list of candidates, each a list of
+    sentence indices (``Summary.to_lists()[b]``) or an (indices, score) pair (``Samples.summaries`` / ``Beams.n_best``).  With
+    eos = text_len[b] - 1, a candidate's row is its indices, then eos up to ``steps`` (a candidate of exactly ``steps`` indices has no
+    EOS).  Videos with fewer candidates than the most are padded with invalid rows (eos throughout).  Returns (tokens (B, N, steps)
+    int64, valid (B, N) bool) on the host.  ValueError for an index outside 0..eos-1, more than ``steps`` indices, more than 64
+    candidates for a video, or no candidate at all."""
+    from .ops import FORCED_MAX_N
+    lens = [int(n) for n in (text_len.tolist() if torch.is_tensor(text_len) else text_len)]
+    S = int(steps)
+    if S <= 0:
+        raise ValueError(f"candidate_tokens: {steps} steps")
+    if len(candidates) != len(lens):
+        raise ValueError(f"candidate_tokens: candidates for {len(candidates)} videos, text_len for {len(lens)}")
+    rows: List[List[List[int]]] = []
+    for b, cands in enumerate(candidates):
+        eos = lens[b] - 1
+        if len(cands) > FORCED_MAX_N:
+            raise ValueError(f"candidate_tokens: video {b} has {len(cands)} candidates, at most {FORCED_MAX_N}")
+        vid = []
+        for c in cands:
+            if isinstance(c, tuple) and len(c) == 2 and isinstance(c[0], (list, tuple)):
+                c = c[0]                                   # an (indices, score) pair
+            if any(isinstance(k, bool) or not isinstance(k, numbers.Integral) for k in c):
+                raise ValueError(f"candidate_tokens: video {b}: candidate {list(c)!r} holds a non-integer index")
+            idx = [int(k) for k in c]
+            if len(idx) > S:
+                raise ValueError(f"candidate_tokens: video {b}: a candidate of {len(idx)} sentences for {S} steps")
+            if any(not 0 <= k < eos for k in idx):
+                raise ValueError(f"candidate_tokens: video {b}: candidate {idx} has an index outside 0..{eos - 1} (EOS row {eos})")
+            vid.append(idx + [eos] * (S - len(idx)))
+        rows.append(vid)
+    N = max(len(v) for v in rows) if rows else 0
+    if N == 0:
+        raise ValueError("candidate_tokens: no candidate at all")
+    tokens = torch.empty(len(rows), N, S, dtype=torch.int64)
+    valid = torch.zeros(len(rows), N, dtype=torch.bool)
+    for b, vid in enumerate(rows):
+        tokens[b] = lens[b] - 1
+        if vid:
+            tokens[b, :len(vid)] = torch.tensor(vid, dtype=torch.int64)
+            valid[b, :len(vid)] = True
+    return tokens, valid
+
+
+def forced_scores(tokens: torch.Tensor, p_tok: torch.Tensor, terms: torch.Tensor, valid: torch.Tensor, text_len_i32: torch.Tensor,
+                  probs: Optional[torch.Tensor] = None) -> Scores:
+    """:class:`Scores` from the outputs of one forced roll-out (``ops.decoder_forced_fwd``).  Device ops only (capturable)."""
+    B, N, S = tokens.shape
+    logp = path_logp(p_tok, tokens, text_len_i32)
+    loss = ((terms[:, 0].sum(0) + terms[:, 1].sum(0)) / S).view(B, N)                           # models.py:179, per row
+    logp = torch.where(valid, logp, torch.full_like(logp, -math.inf))
+    loss = torch.where(valid, loss, torch.full_like(loss, math.inf))
+    return Scores(tokens, p_tok, logp, loss, valid, probs)
 
 
 def best_sample(samples: Samples, sel: torch.Tensor, count: torch.Tensor):
@@ -240,6 +317,26 @@ class _Bucket:
             s.targets.copy_(batch.targets, non_blocking=True)
 
 
+class _ScoreBucket(_Bucket):
+    """One captured ``score``: a summarize bucket's static inputs plus a static token buffer."""
+
+    def __init__(self, model, batch: Batch, tokens: torch.Tensor, probs: bool, warmup: int):
+        self.tokens = tokens.clone()        # (read by the captured kernel from this fixed address)
+        self.probs = probs
+        super().__init__(model, batch, False, warmup)
+
+    def _run(self, model) -> Scores:
+        for plan in self.plans:
+            plan.refresh()
+        b = self.batch
+        return model.score(b.text, b.text_len, b.audio, b.audio_len, b.images, b.image_len, self.tokens.shape[2], self.tokens,
+                           probs=self.probs)
+
+    def load(self, batch: Batch, tokens: torch.Tensor) -> None:
+        super().load(batch)
+        self.tokens.copy_(tokens, non_blocking=True)
+
+
 class Summarizer:
     """``model.summarize`` replayed from CUDA graphs.  A batch of a padded-shape bucket seen before (text, audio and key-frame widths,
     the batch size, ``max_dec_len``, with targets their width, the beam width and the constraints) is copied into that bucket's static inputs, its
@@ -251,6 +348,7 @@ class Summarizer:
         self.model = model
         self.warmup = warmup
         self.buckets: Dict[tuple, _Bucket] = {}
+        self.score_buckets: Dict[tuple, _ScoreBucket] = {}
 
     def __call__(self, batch: Batch, with_targets: bool = False, beam_width: Optional[int] = None, no_repeat: bool = False,
                  min_sentences: int = 0, num_samples: Optional[int] = None, temperature: float = 1.0, top_k: int = 0,
@@ -271,6 +369,27 @@ class Summarizer:
                                                  sampling)
         else:
             bucket.load(batch)
+        bucket.graph.replay()
+        return bucket.result
+
+    def score(self, batch: Batch, tokens: torch.Tensor, probs: bool = False) -> Scores:
+        """``model.score`` of the token rows ``tokens`` (B, N, S) int64 on the device (N in 1..64, S steps) replayed from CUDA graphs:
+        buckets of their own, keyed by the batch's padded shapes, the tokens' shape and ``probs``.  The batch and the tokens are copied
+        into the bucket's static inputs before the replay; as for ``__call__``, in-place parameter updates show up on the next replay
+        and the returned :class:`Scores` holds the bucket's static outputs."""
+        from .ops import FORCED_MAX_N
+        if not isinstance(probs, bool):
+            raise ValueError(f"Summarizer.score: probs {probs!r}, expected a bool")
+        if not torch.is_tensor(tokens) or tokens.dtype != torch.int64 or tokens.dim() != 3 or tokens.device != batch.text.device or \
+                tokens.shape[0] != batch.text.shape[0] or not 1 <= tokens.shape[1] <= FORCED_MAX_N or tokens.shape[2] <= 0:
+            raise ValueError(f"Summarizer.score: tokens {getattr(tokens, 'dtype', type(tokens))} {tuple(getattr(tokens, 'shape', ()))}, "
+                             f"expected (B={batch.text.shape[0]}, N in 1..{FORCED_MAX_N}, S > 0) int64 on {batch.text.device}")
+        key = (tuple(batch.text.shape), tuple(batch.audio.shape), tuple(batch.images.shape), tuple(tokens.shape), probs)
+        bucket = self.score_buckets.get(key)
+        if bucket is None:
+            bucket = self.score_buckets[key] = _ScoreBucket(self.model, batch, tokens, probs, self.warmup)
+        else:
+            bucket.load(batch, tokens)
         bucket.graph.replay()
         return bucket.result
 
