@@ -235,6 +235,24 @@ MMB_API int mmb_decoder_forced_fused(const float* proj_a, const float* proj_i, c
                                      const uint8_t* mask, const long long* tokens, float* probs, float* p_tok, float* loss_terms,
                                      int B, int Lt, int D, int H, int E, int M, int S, int N, mmb_stream_t stream);
 /*
+ * Forced roll-out for training: mmb_decoder_forced_fused (same arguments, same p_tok, probs and loss_terms bit for bit; probs is
+ * required here) that also writes, for every step, what mmb_decoder_forced_bwd_fused reads.  The saved arrays are step-major with rows
+ * r = b N + n; step s's slice of each is exactly what mmb_decoder_step_fused_fwd writes for those B N rows at step s:
+ *   probs (S,B N,M)  hw (S,B N,4D)  alpha (S,B N,2,Lt)  beta (S,B N,2)  ctx12 / pb (S,2,B N,D)  xcat (S,B N,D+E+H)  gates (S,B N,4H)
+ *   att_cov (S,B N,Lt)  cell (S+1,B N,H) and cov (S+1,B N,Lt): row 0 the start state (zero), row s + 1 step s's output
+ *   h_last (B N,H): h' of the last step (step s's h' for s < S - 1 is the h part of step s + 1's xcat)
+ * MMB_ERR_INVALID / MMB_ERR_UNSUPPORTED as mmb_decoder_forced_fused (every pointer is required).
+ */
+MMB_API int mmb_decoder_forced_train_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                           const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                           const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                           const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt, const float* bcat,
+                                           const float* out_wt, const float* out_b, const float* emb_text, const float* h0,
+                                           const uint8_t* mask, const long long* tokens, float* probs, float* p_tok, float* loss_terms,
+                                           float* hw, float* alpha, float* beta, float* ctx12, float* pb, float* xcat, float* gates,
+                                           float* att_cov, float* cell, float* cov, float* h_last, int B, int Lt, int D, int H, int E,
+                                           int M, int S, int N, mmb_stream_t stream);
+/*
  * Beam summary roll-out: the decode loop of models.py:156-199 in eval mode with K hypotheses per video instead of one, all S steps
  * in ONE launch of the same cluster kernel (one cluster per video holds every slot); the beam alternative to evaluate.py:185-202's
  * greedy pick.  This is the project's own beam rule; it does not claim parity with the reference's evaluate.py::beam_search.
@@ -496,6 +514,32 @@ MMB_API int mmb_decoder_step_fused_bwd(const float* probs, const float* d_probs,
                                        const float* enc_a, const float* enc_i, const float* coverage, const float* v1, const float* wc1,
                                        const float* v2, const float* wc2, float* d_proj_a, float* d_proj_i, float* d_cov,
                                        const float* Wh_stack, float* d_h, int B, int Lt, int D, int H, int M, mmb_stream_t stream);
+/*
+ * Reverse forced roll-out: the backward of mmb_decoder_forced_train_fused for s = S - 1 .. 0 in ONE launch, one cluster per row
+ * r = b N + n (b = r / N).  Each step is the whole-step backward of mmb_decoder_step_fused_bwd over the B N rows -- the head, both text
+ * sweeps and d h -- from step s's slices of the saved arrays; proj_* / enc_* of video b are read per video, never replicated.  What a
+ * step takes from the next one stays on chip: d h, d cell and each rank's rows of d coverage (zero after the last step).
+ *   g_terms (S,2,B N)   d objective / d loss_terms[s, 0, r] (the nll term) and [s, 1, r] (the coverage term), the step kernel's
+ *                       g_nll / g_cov per step.  A token outside 0..M-1 has a constant nll term: its entry adds nothing.
+ *   d_logits (S,B N,ldd) columns M..ldd-1 zeroed;  d_gates (S,B N,ldg) = [d_gates | d_hw4], ldg >= 4H + 4D;  d_pre_b / d_ctx12
+ *   (S,2,B N,D);  vec_acc (B N,6,D) and scal_acc (B N,4) accumulated in place;  d_h0 (B N,H) = d h of step 0's input;
+ *   d_proj_a / d_proj_i (B,Lt,D) accumulated per video over its N rows and S steps (the step kernel's bulk reduction or L2
+ *   reductions: at N > 1 the order of the rows' additions is not fixed).
+ * Cluster size, chunk and row stage follow the step kernel's rules with B N rows (8 CTAs when 8 B N <= 160, else 4), so every per-row
+ * output is the step kernel's, bit for bit.  Shared memory is the whole-step backward's plus 2H floats of carried d h / d cell; at
+ * config 3 (Lt = 409, D = 200, H = 100, 4 CTAs) that is 222.75 KB with the row stage, which fits: the staged arm.
+ * MMB_ERR_INVALID for N outside 1..64, S <= 0, a null pointer or the shape limits of mmb_decoder_step_fused_bwd; MMB_ERR_UNSUPPORTED
+ * for D > 256 or shapes whose arrays do not fit in shared memory, with the byte count.
+ */
+MMB_API int mmb_decoder_forced_bwd_fused(const float* probs, const long long* tokens, const float* g_terms, const float* out_w,
+                                         const float* gates, const float* cell, const float* Wcat_ctx, const float* alpha,
+                                         const float* beta, const float* ctx12, const float* pb, const float* hw, const float* vb1,
+                                         const float* vb2, const float* att_cov, const float* cov, const float* Wb13,
+                                         const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                         const float* v1, const float* wc1, const float* v2, const float* wc2, const float* Wh_stack,
+                                         float* d_logits, int ldd, float* d_gates, int ldg, float* d_pre_b, float* d_ctx12,
+                                         float* vec_acc, float* scal_acc, float* d_proj_a, float* d_proj_i, float* d_h0, int B,
+                                         int Lt, int D, int H, int M, int S, int N, mmb_stream_t stream);
 
 MMB_API int mmb_decoder_attn_bwd(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
                                  const float* hw, const float* coverage, const float* alpha, const float* beta,

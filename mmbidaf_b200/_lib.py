@@ -40,6 +40,8 @@ SIGNATURES = {
     "mmb_decoder_step_fused_fwd": [c_void_p] * 42 + [c_int] * 6 + [c_void_p],
     "mmb_decoder_greedy_fused": [c_void_p] * 28 + [c_int] * 8 + [c_void_p],
     "mmb_decoder_forced_fused": [c_void_p] * 28 + [c_int] * 8 + [c_void_p],
+    "mmb_decoder_forced_train_fused": [c_void_p] * 39 + [c_int] * 8 + [c_void_p],
+    "mmb_decoder_forced_bwd_fused": [c_void_p] * 27 + [c_int] + [c_void_p] + [c_int] + [c_void_p] * 7 + [c_int] * 7 + [c_void_p],
     "mmb_decoder_beam_fused": [c_void_p] * 31 + [c_int] * 8 + [c_void_p],
     "mmb_decoder_greedy_constrained_fused": [c_void_p] * 27 + [c_int] * 9 + [c_void_p],
     "mmb_decoder_beam_constrained_fused": [c_void_p] * 31 + [c_int] * 10 + [c_void_p],

@@ -325,6 +325,13 @@ struct ForcedArgs {
   float* p_tok;                                             // (B N, S)
   int N;                                                    // candidates per video
 };
+// The forced roll-out for training (mmb_decoder_forced_train_fused; kSave): the same stages, and every step also writes what
+// mmb_decoder_step_fused_bwd reads, step-major with rows r = b N + n -- the saved arrays of FusedArgs (hw, alpha, beta, ctx12, pb,
+// xcat, gates, att_cov) as (S, B N, ...) / (S, 2, B N, D), cell_out / cov_out as the (S + 1, B N, ...) states (row 0 the start state)
+// -- and h' of the last step here (the other steps' h' is the h part of the next step's xcat).
+struct TrainArgs {
+  float* h_last;                                            // (B N, H)
+};
 __device__ __forceinline__ unsigned long long block_sum_u64(unsigned long long v, float* red) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
@@ -460,13 +467,15 @@ __device__ __forceinline__ NucleusCut nucleus_cut(const float* __restrict__ v, i
 
 // kGreedy: the roll-out; kBeam (with kGreedy): the beam roll-out instead of the greedy one; kConstrained (with kGreedy): the pick skips
 // the sentences `cn` makes ineligible; kSample (with kGreedy, not kBeam): the pick is drawn (`sp`); kNucleus (with kSample): drawn
-// from the nucleus (`nu`); kStoch (with kBeam): the stochastic beam (`st`); kForced (with kGreedy alone): the tokens are given (`fo`)
+// from the nucleus (`nu`); kStoch (with kBeam): the stochastic beam (`st`); kForced (with kGreedy alone): the tokens are given (`fo`);
+// kSave (with kForced): every step's saved arrays are written (`tr`, TrainArgs)
 template <bool kGreedy, bool kBeam = false, bool kConstrained = false, bool kSample = false, bool kNucleus = false, bool kStoch = false,
-          bool kForced = false>
+          bool kForced = false, bool kSave = false>
 __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyArgs& g, const BeamArgs& bm, const ConstraintArgs& cn,
                                                const SampleArgs sp, const NucleusArgs nu = NucleusArgs{}, const StochArgs st = StochArgs{},
-                                               const ForcedArgs fo = ForcedArgs{}) {
+                                               const ForcedArgs fo = ForcedArgs{}, const TrainArgs tr = TrainArgs{}) {
   static_assert(!kForced || (kGreedy && !kBeam && !kConstrained && !kSample), "the forced roll-out is the greedy one's");
+  static_assert(!kSave || kForced, "the saved arrays are the forced roll-out's");
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int ob = blockIdx.x / CL;                         // the output row: the video (sampled / forced: cluster_row(), the roll-out)
@@ -593,6 +602,8 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     for (int i = tid; i < n; i += NT) s_bcv[i] = 0.f;
     __syncthreads();
   }
+  // kSave: rows of the (S, B N, ...) saved arrays (RBn = B N rows per step); read where used, as cluster_row()
+  const size_t RBn = kSave ? (size_t)a.B * fo.N : 0;
   for (int s = 0; s < S; ++s) {
   for (int slot = 0; slot < KW; ++slot) {  // beam: the live slots one after another; otherwise once
   if (kBeam && bs_stat[slot] != kLive) continue;
@@ -633,6 +644,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       const int o = o0 + i;
       for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_hw, r)[o] = v;
       if constexpr (!kGreedy) a.hw[(size_t)b * 4 * D + o] = v;
+      if constexpr (kSave) a.hw[((size_t)s * RBn + cluster_row()) * 4 * D + o] = v;
     });
   }
   DEC_STAMP(2);
@@ -841,6 +853,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       for (int r = 0; r < CL; ++r) sum = fmaf(s_w[k * MAXC + r], s_part[r * (4 + 2 * D) + 4 + i], sum);
       s_ctx[i] = sum;
       if (!kGreedy && R == 0) a.ctx12[((size_t)k * a.B + b) * D + (i - k * D)] = sum;
+      if (kSave && R == 0) a.ctx12[(((size_t)s * 2 + k) * RBn + cluster_row()) * D + (i - k * D)] = sum;
     }
   }
   __syncthreads();
@@ -858,6 +871,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
                        const int o = lo + i;
                        for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_pb, r)[o] = v;
                        if constexpr (!kGreedy) a.pb[((size_t)k * a.B + b) * D + (o - k * D)] = v;
+                       if constexpr (kSave) a.pb[(((size_t)s * 2 + k) * RBn + cluster_row()) * D + (o - k * D)] = v;
                      });
     }
   }
@@ -893,6 +907,14 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
         closs += fminf(att, cnew);
       } else if constexpr (kGreedy) {
         const float cnew = s_cov[i] + att;                       // (the energies of this step have read s_cov: barriers since)
+        if constexpr (kSave) {
+          const size_t row = (size_t)s * RBn + cluster_row();
+          a.alpha[(row * 2 + 0) * Lt + t] = a1;
+          a.alpha[(row * 2 + 1) * Lt + t] = a2;
+          a.att_cov[row * Lt + t] = att;
+          if (s == 0) a.cov_out[row * Lt + t] = s_cov[i];        // the start state, row 0
+          a.cov_out[(row + RBn) * Lt + t] = cnew;
+        }
         s_cov[i] = cnew;
         closs += fminf(att, cnew);
       } else {
@@ -908,10 +930,17 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       a.beta[b * 2 + 0] = beta1;
       a.beta[b * 2 + 1] = beta2;
     }
+    if (kSave && R == 0 && tid == 0) {
+      const size_t row = (size_t)s * RBn + cluster_row();
+      a.beta[row * 2 + 0] = beta1;
+      a.beta[row * 2 + 1] = beta2;
+    }
   }
   __syncthreads();
   if (!kGreedy && R == 0)
     for (int i = tid; i < K; i += NT) a.xcat[(size_t)b * K + i] = s_x[i];
+  if (kSave && R == 0)
+    for (int i = tid; i < K; i += NT) a.xcat[((size_t)s * RBn + cluster_row()) * K + i] = s_x[i];
 
   DEC_STAMP(11);
   // ---- stage D: LSTM gates of this rank's hidden units, cell update; h' gathered -------------------------------------------
@@ -930,6 +959,14 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
       if constexpr (kBeam) {
         s_bcn[slot * ldc + tid] = c;
       } else if constexpr (kGreedy) {
+        if constexpr (kSave) {
+          const size_t row = (size_t)s * RBn + cluster_row();
+          float* gs = a.gates + row * 4 * H;
+          gs[j] = gi; gs[H + j] = gf; gs[2 * H + j] = gg; gs[3 * H + j] = go;
+          if (s == 0) a.cell_out[row * H + j] = cell_own;       // the start state, row 0
+          a.cell_out[(row + RBn) * H + j] = c;
+          if (s == S - 1) tr.h_last[(size_t)cluster_row() * H + j] = hn;
+        }
         cell_own = c;
       } else {
         a.cell_out[(size_t)b * H + j] = c;
@@ -993,7 +1030,7 @@ __device__ __forceinline__ void dec_fused_body(const FusedArgs& a, const GreedyA
     for (int m = m0 + tid; m < m1; m += NT) {
       const float p = expf(lg[m - m0] - gmx) * inv;
       if constexpr (kBeam) s_bp[slot * ldp + m - m0] = p;
-      else if (!kForced || a.probs) a.probs[prow * M + m] = p;   // (forced: the rows are optional)
+      else if (!kForced || a.probs) a.probs[(kSave ? (size_t)s * RBn + cluster_row() : prow) * M + m] = p;   // (forced: the rows are optional; saved: step-major)
       if constexpr (kForced) continue;                           // (its token's p follows the loop)
       if constexpr (kSample) {
         // top_k = 0: the first maximum of z over the candidates (the first candidate stands even at z = -inf);
@@ -1501,6 +1538,12 @@ __global__ void __launch_bounds__(NT) dec_forced_kernel(const FusedArgs a, const
                                                                 StochArgs{}, fo);
 }
 
+__global__ void __launch_bounds__(NT) dec_forced_train_kernel(const FusedArgs a, const GreedyArgs g, const ForcedArgs fo,
+                                                              const TrainArgs tr) {
+  dec_fused_body<true, false, false, false, false, false, true, true>(a, g, BeamArgs{}, ConstraintArgs{}, SampleArgs{}, NucleusArgs{},
+                                                                      StochArgs{}, fo, tr);
+}
+
 }  // namespace
 
 // ----------------------------------------------------------------------------------------------------------------------------------
@@ -1539,10 +1582,24 @@ struct HeadArgs {
   int stage_off;   // whole step: float offset of the row stage ([2 mbarriers][2][chunk * D]) in dynamic shared memory, or 0
 };
 
-__global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
+// The reverse forced roll-out (mmb_decoder_forced_bwd_fused): the whole-step backward once per step, s = S - 1 .. 0, in one launch,
+// one cluster per row r = b N + n of the forced roll-out.  HeadArgs then hold step s's slices of the saved arrays (B = the B N rows);
+// the step's token comes from `tokens`; proj / enc / d_proj are the video's (b = r / N).  What the step kernel takes from the next step's
+// backward stays on chip: d h (gathered into every rank at the end of a step), d cell (every rank holds all H) and this rank's rows
+// of d cov (the d cov accumulation of sweep 8 is the next step's d coverage').
+struct RollBwdArgs {
+  const long long* tokens;                                  // (B N, S)
+  float* d_h0;                                              // (B N, H): d h of step 0's input
+  int N, S;                                                 // candidates per video, steps
+  int s, it;                                                // this step, and S - 1 - s (the row-stage barriers' phase)
+};
+
+template <bool kRoll>
+__device__ __forceinline__ void dec_bwd_body(const HeadArgs& a, const RollBwdArgs& ro) {
   cg::cluster_group cluster = cg::this_cluster();
   const int CL = (int)cluster.num_blocks(), R = (int)cluster.block_rank();
   const int b = blockIdx.x / CL;
+  const int bv = kRoll ? b / ro.N : b;                  // the video whose proj / enc / d_proj rows the row reads (roll-out: b is the row)
   const int tid = threadIdx.x;
   const int D = a.D, H = a.H, M = a.M, Lt = a.Lt;
 
@@ -1561,6 +1618,19 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
   const int mv_cap = a.sweeps ? (a.stage_off != 0 ? NW / 2 : NW) * 3 * D : NT;
   float* const mv_scr = a.sweeps ? s_scr + NT + up4(2 * D) + up4(2 * a.chunk) + up4(4 * a.chunk) + up4(6 * D) : s_scr;
   const bool mv_quads = a.sweeps != 0;
+  // roll-out: the sweeps' row scalars (s_rowc, s_row below: stage 5 writes them in place) and, behind the sweeps' region, the carried
+  // d h / d cell.  (Set up here for the roll-out only: the step kernel keeps its code.)
+  float *r_rowc = nullptr, *r_row = nullptr, *s_dhc = nullptr, *s_dcell = nullptr;
+  if constexpr (kRoll) {
+    r_rowc = s_scr + NT + up4(2 * D) + up4(2 * a.chunk);                                      // = s_rowc
+    r_row = r_rowc + up4(4 * a.chunk) + up4(6 * D) + up4((a.stage_off != 0 ? NW / 2 : NW) * 3 * D);   // = s_row
+    s_dhc = r_row + up4(a.chunk) + up4(CL * 6 * D) + up4(4 * H + 4 * D);     // [H]  d h of the next step's backward (written remotely)
+    s_dcell = s_dhc + up4(H);                                                 // [H]  d cell of the next step's backward
+    if (ro.it == 0) {                                   // (every carry is read behind a cluster barrier; the remote d h behind several)
+      for (int i = tid; i < H; i += NT) s_dhc[i] = s_dcell[i] = 0.f;
+      for (int i = tid; i < a.chunk; i += NT) r_row[i] = 0.f;
+    }
+  }
 
   // Row stage of the whole-step launch (see dec_step_fused_kernel): this rank's rows of enc_a / enc_i come in by two bulk copies issued
   // NOW, six head stages before sweep 7 reads them; when sweep 7 is done the same buffers take the rows of proj_a / proj_i for sweep 8
@@ -1572,21 +1642,38 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
   float* const s_st1 = s_st0 + up4(a.chunk * D);
   const uint32_t bar_enc = tc::smem_u32(smem + a.stage_off), bar_proj = bar_enc + 8;
   const uint32_t stage_bytes = (uint32_t)(n * D) * 4u;
+  // (roll-out: each barrier completes once per step; the previous step's bulk reductions out of the buffers have completed)
+  const uint32_t parity = kRoll ? (uint32_t)(ro.it & 1) : 0u;
   if (staged && tid == 0) {
-    tc::mbar_init(bar_enc, 1);
-    tc::mbar_init(bar_proj, 1);
-    tc::fence_barrier_init();
+    if (!kRoll || ro.it == 0) {
+      tc::mbar_init(bar_enc, 1);
+      tc::mbar_init(bar_proj, 1);
+      tc::fence_barrier_init();
+    } else {
+      tc::fence_proxy_async();
+    }
     if (n > 0) {
       tc::mbar_expect_tx(bar_enc, 2 * stage_bytes, 1);
-      tc::tma_bulk_g2s(tc::smem_u32(s_st0), a.enc_a + ((size_t)b * Lt + t0) * D, stage_bytes, bar_enc, 1);
-      tc::tma_bulk_g2s(tc::smem_u32(s_st1), a.enc_i + ((size_t)b * Lt + t0) * D, stage_bytes, bar_enc, 1);
+      tc::tma_bulk_g2s(tc::smem_u32(s_st0), a.enc_a + ((size_t)bv * Lt + t0) * D, stage_bytes, bar_enc, 1);
+      tc::tma_bulk_g2s(tc::smem_u32(s_st1), a.enc_i + ((size_t)bv * Lt + t0) * D, stage_bytes, bar_enc, 1);
     }
   }
   DEC_STAMP(18);
   // ---- 1: masked soft-max backward: d_logit = p (dp - sum p dp); masked entries have p = 0 ---------------------------------
   const int m0 = min(M, R * per_m), m1 = min(M, m0 + per_m);
-  const int tg = a.target ? (int)a.target[b] : -1;
-  const float dp_t = a.target ? -a.g_nll[b] / (a.probs[(size_t)b * M + tg] + 1e-12f) : 0.f;   // d(-log(p_tgt + eps)) at the target column
+  // (roll-out: the row's token of this step; one outside 0..M-1 has a constant nll term and adds nothing)
+  bool has_t = false;
+  int tg;
+  float dp_t;
+  if constexpr (kRoll) {
+    const long long tk = ro.tokens[(size_t)b * ro.S + ro.s];
+    has_t = tk >= 0 && tk < M;
+    tg = has_t ? (int)tk : -1;
+    dp_t = has_t ? -a.g_nll[b] / (a.probs[(size_t)b * M + tg] + 1e-12f) : 0.f;
+  } else {
+    tg = a.target ? (int)a.target[b] : -1;
+    dp_t = a.target ? -a.g_nll[b] / (a.probs[(size_t)b * M + tg] + 1e-12f) : 0.f;   // d(-log(p_tgt + eps)) at the target column
+  }
   if (a.d_probs) {      // (uniform over the cluster.  With the fused loss terms alone -- a training step -- sum p dp has the target's term
                         // only, which every rank forms by itself: no exchange, no cluster barrier)
     float dot = 0.f;
@@ -1599,7 +1686,7 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
     float dot = 0.f;
     if (a.d_probs)
       for (int r = 0; r < CL; ++r) dot += s_ex[r * 4 + 0];
-    if (a.target) dot = fmaf(a.probs[(size_t)b * M + tg], dp_t, dot);
+    if (kRoll ? has_t : a.target != nullptr) dot = fmaf(a.probs[(size_t)b * M + tg], dp_t, dot);
     for (int m = m0 + tid; m < m1; m += NT) {
       const float dp = (a.d_probs ? a.d_probs[(size_t)b * M + m] : 0.f) + (m == tg ? dp_t : 0.f);
       const float v = a.probs[(size_t)b * M + m] * (dp - dot);
@@ -1624,19 +1711,21 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
     const int j = tid;
     float dh = 0.f;
     for (int r = 0; r < CL; ++r) dh += s_dhp[r * H + j];
-    if (a.d_h_out) dh += a.d_h_out[(size_t)b * H + j];
+    if constexpr (kRoll) dh += s_dhc[j];
+    else if (a.d_h_out) dh += a.d_h_out[(size_t)b * H + j];
     const float* g = a.gates + (size_t)b * 4 * H;
     const float gi = g[j], gf = g[H + j], gg = g[2 * H + j], go = g[3 * H + j];
     const float tc = tanh_fast(a.cell_out[(size_t)b * H + j]);
-    const float dc = fmaf(dh * go, 1.f - tc * tc, a.d_cell_out ? a.d_cell_out[(size_t)b * H + j] : 0.f);
+    const float dc = fmaf(dh * go, 1.f - tc * tc, kRoll ? s_dcell[j] : a.d_cell_out ? a.d_cell_out[(size_t)b * H + j] : 0.f);
     const float di = dc * gg * gi * (1.f - gi), df = dc * a.cell_in[(size_t)b * H + j] * gf * (1.f - gf);
     const float dg = dc * gi * (1.f - gg * gg), dO = dh * tc * go * (1.f - go);
     s_dg[j] = di; s_dg[H + j] = df; s_dg[2 * H + j] = dg; s_dg[3 * H + j] = dO;
     if (R == 0) {
       float* o = a.d_gates + (size_t)b * a.ldg;
       o[j] = di; o[H + j] = df; o[2 * H + j] = dg; o[3 * H + j] = dO;
-      a.d_cell[(size_t)b * H + j] = dc * gf;
+      if constexpr (!kRoll) a.d_cell[(size_t)b * H + j] = dc * gf;
     }
+    if constexpr (kRoll) s_dcell[j] = dc * gf;
   }
   __syncthreads();
   DEC_STAMP(21);
@@ -1661,17 +1750,22 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
     const float gc = a.g_cov ? a.g_cov[b] : 0.f;
     const int t0 = min(Lt, R * a.chunk), t1 = min(Lt, t0 + a.chunk);
     for (int t = t0 + tid; t < t1; t += NT) {
-      float dcv = a.d_cov_out ? a.d_cov_out[(size_t)b * Lt + t] : 0.f;
-      float g = a.d_att_cov ? a.d_att_cov[(size_t)b * Lt + t] : 0.f;
+      float dcv = kRoll ? r_row[t - t0] : a.d_cov_out ? a.d_cov_out[(size_t)b * Lt + t] : 0.f;
+      float g = !kRoll && a.d_att_cov ? a.d_att_cov[(size_t)b * Lt + t] : 0.f;
       if (a.g_cov) {                                              // d sum min(att, cov'): ties split evenly (torch.minimum)
         const float av = a.att[(size_t)b * Lt + t], cv = a.cov_out[(size_t)b * Lt + t];
         const float tie = av == cv ? 0.5f * gc : 0.f;
         g += av < cv ? gc : tie;
         dcv += cv < av ? gc : tie;
       }
-      a.dcov_tot[(size_t)b * Lt + t] = dcv;
       g += dcv;                                                   // coverage' = coverage + att
-      a.datt[(size_t)b * Lt + t] = g;
+      if constexpr (kRoll) {                                      // (the sweeps' per-row scalars, kept on chip)
+        r_row[t - t0] = dcv;
+        r_rowc[2 * a.chunk + t - t0] = g;
+      } else {
+        a.dcov_tot[(size_t)b * Lt + t] = dcv;
+        a.datt[(size_t)b * Lt + t] = g;
+      }
       db1 = fmaf(a.alpha[((size_t)b * 2 + 0) * Lt + t], g, db1);
       db2 = fmaf(a.alpha[((size_t)b * 2 + 1) * Lt + t], g, db2);
     }
@@ -1741,7 +1835,7 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
   float* s_vec = s_rowc + up4s(4 * a.chunk);            // [6][D]  v1 | wc1 | hw1 | v2 | wc2 | hw2
   const int PW = staged ? NW / 2 : NW;                  // warps per pass of the column-partial reduction (staged: half the buffer, two passes)
   float* s_part = s_vec + up4s(6 * D);                  // [PW][3][D]
-  float* s_row = s_part + up4s(PW * 3 * D);             // [chunk]  d cov accumulation
+  float* s_row = s_part + up4s(PW * 3 * D);             // [chunk]  d cov accumulation (roll-out: carried to the next step as its d cov')
   float* s_colp = s_row + up4s(a.chunk);                // [CL][2][3][D]  column partials of every rank (written remotely)
   float* s_in = s_colp + up4s(CL * 6 * D);              // [4H + 4D]  d_gates | d (W2 h) | d (W4 h) | d_pre_b
   // Both sweeps are written like stage B of the forward kernel (see there): a lane's per-column constants live in registers for the
@@ -1762,10 +1856,10 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
   // the per-row scalars of both sweeps come in ONCE, here: read inside the sweeps they were dependent global loads at the end (sweep
   // 7) or in the middle (sweep 8) of every warp iteration -- ~800 exposed cycles each (tools/decoder_bwd_trace.py)
   for (int i = tid; i < n; i += NT) {
-    s_row[i] = a.dcov_tot[(size_t)b * Lt + t0 + i];
+    if constexpr (!kRoll) s_row[i] = a.dcov_tot[(size_t)b * Lt + t0 + i];
     s_rowc[i] = a.alpha[((size_t)b * 2 + 0) * Lt + t0 + i];
     s_rowc[a.chunk + i] = a.alpha[((size_t)b * 2 + 1) * Lt + t0 + i];
-    s_rowc[2 * a.chunk + i] = a.datt[(size_t)b * Lt + t0 + i];      // (written by this rank in stage 5)
+    if constexpr (!kRoll) s_rowc[2 * a.chunk + i] = a.datt[(size_t)b * Lt + t0 + i];      // (written by this rank in stage 5)
     s_rowc[3 * a.chunk + i] = a.cov[(size_t)b * Lt + t0 + i];
   }
   __syncthreads();
@@ -1815,11 +1909,11 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
     }
   };
   if (staged) {
-    if (n > 0) tc::mbar_wait(bar_enc, 0);
+    if (n > 0) tc::mbar_wait(bar_enc, parity);
     if (nj7) sweep7(s_st0, s_st1, N7{}); else sweep7(s_st0, s_st1, N8{});
   } else {
-    const float* const gea = a.enc_a + ((size_t)b * Lt + t0) * D;
-    const float* const gei = a.enc_i + ((size_t)b * Lt + t0) * D;
+    const float* const gea = a.enc_a + ((size_t)bv * Lt + t0) * D;
+    const float* const gei = a.enc_i + ((size_t)bv * Lt + t0) * D;
     if (nj7) sweep7(gea, gei, N7{}); else sweep7(gea, gei, N8{});
   }
   {
@@ -1827,8 +1921,8 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
     if (staged && tid == 0 && n > 0) {       // every read of the enc rows is behind block_sum's barriers: the buffers take the proj rows
       tc::fence_proxy_async();
       tc::mbar_expect_tx(bar_proj, 2 * stage_bytes, 1);
-      tc::tma_bulk_g2s(tc::smem_u32(s_st0), a.proj_a + ((size_t)b * Lt + t0) * D, stage_bytes, bar_proj, 1);
-      tc::tma_bulk_g2s(tc::smem_u32(s_st1), a.proj_i + ((size_t)b * Lt + t0) * D, stage_bytes, bar_proj, 1);
+      tc::tma_bulk_g2s(tc::smem_u32(s_st0), a.proj_a + ((size_t)bv * Lt + t0) * D, stage_bytes, bar_proj, 1);
+      tc::tma_bulk_g2s(tc::smem_u32(s_st1), a.proj_i + ((size_t)bv * Lt + t0) * D, stage_bytes, bar_proj, 1);
     }
     s2 = block_sum(s2, s_red);
     if (tid < CL) {
@@ -1859,7 +1953,7 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
   auto sweep8 = [&](const int m, float* proj, auto nj_tag, auto staged_tag) {
     constexpr int NJ = decltype(nj_tag)::value;
     constexpr bool STAGED = decltype(staged_tag)::value;
-    float* dproj = (m == 0 ? a.d_proj_a : a.d_proj_i) + ((size_t)b * Lt + t0) * D;
+    float* dproj = (m == 0 ? a.d_proj_a : a.d_proj_i) + ((size_t)bv * Lt + t0) * D;
     float vvr[NJ], wcr[NJ], hwk[NJ];                    // v, Wc, K2 (W h) of this lane's columns
     float c_dz[NJ], c_cov[NJ], c_v[NJ];
 #pragma unroll
@@ -1950,17 +2044,18 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
         for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_colp, r)[(R * 2 + m) * 3 * D + i] = xacc[q];
     }
   };
-  if (staged && n > 0) tc::mbar_wait(bar_proj, 0);
+  if (staged && n > 0) tc::mbar_wait(bar_proj, parity);
   for (int m = 0; m < 2; ++m) {
     if (staged) {
       float* const sp = m == 0 ? s_st0 : s_st1;
       if (nj7) sweep8(m, sp, N7{}, std::true_type{}); else sweep8(m, sp, N8{}, std::true_type{});
     } else {
-      float* const gp = const_cast<float*>(m == 0 ? a.proj_a : a.proj_i) + ((size_t)b * Lt + t0) * D;      // (read only on this path)
+      float* const gp = const_cast<float*>(m == 0 ? a.proj_a : a.proj_i) + ((size_t)bv * Lt + t0) * D;      // (read only on this path)
       if (nj7) sweep8(m, gp, N7{}, std::false_type{}); else sweep8(m, gp, N8{}, std::false_type{});
     }
   }
-  for (int i = tid; i < n; i += NT) a.d_cov[(size_t)b * Lt + t0 + i] = s_row[i];
+  if constexpr (!kRoll)
+    for (int i = tid; i < n; i += NT) a.d_cov[(size_t)b * Lt + t0 + i] = s_row[i];
   if (tid < CL) {
     float* dst = cluster.map_shared_rank(s_ex, tid) + R * 4;
     dst[2] = se_m0;
@@ -1998,23 +2093,55 @@ __global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) {
   {
     const int per = split4(H, CL), j0 = min(H, R * per), j1 = min(H, j0 + per);
     block_matvec_t(a.Wh_stack, H, nullptr, s_in, 4 * H + 4 * D, j1 - j0, mv_scr, mv_cap, mv_quads, [&](int i) { return j0 + i; },
-                   [&](int i, float v) { a.d_h[(size_t)b * H + j0 + i] = v; });
+                   [&](int i, float v) {
+                     if constexpr (!kRoll) {
+                       a.d_h[(size_t)b * H + j0 + i] = v;
+                     } else if (ro.s > 0) {                 // the next step's d h', read in its stage 3 behind its cluster barriers
+                       for (int r = 0; r < CL; ++r) cluster.map_shared_rank(s_dhc, r)[j0 + i] = v;
+                     } else {
+                       ro.d_h0[(size_t)b * H + j0 + i] = v;
+                     }
+                   });
   }
   if (staged && tid == 0) bulk_wait_all();              // the stage buffers are read by the bulk reductions until here
   DEC_STAMP(27);
   // (No barrier before the exit: the last stores into another rank's shared memory -- the column partials of sweep 8 -- lie before
-  // the cluster barrier in front of stage 9.)
+  // the cluster barrier in front of stage 9.  Roll-out: the d h stores of step s > 0 land behind every read of s_dhc in step s, and
+  // are read in step s - 1 behind its first cluster barrier; step 0 stores d h to memory only.  A rank makes the remote stores of
+  // step s - 1 only after it has passed every cluster barrier of step s, and every rank's reads of the same words in step s lie
+  // before one of those barriers.)
+}
+
+__global__ void __launch_bounds__(NT) dec_bwd_head_kernel(const HeadArgs a) { dec_bwd_body<false>(a, RollBwdArgs{}); }
+
+// a0: the step-0 slices (cell_out / cov_out: row 1 of the (S + 1)-row states; g_nll / g_cov: g_terms / g_terms + B N)
+__global__ void __launch_bounds__(NT) dec_forced_bwd_kernel(const HeadArgs a0, const RollBwdArgs r0) {
+  const size_t RB = (size_t)a0.B;
+  for (int s = r0.S - 1; s >= 0; --s) {
+    const size_t o = (size_t)s * RB;
+    HeadArgs a = a0;
+    a.probs += o * a.M; a.g_nll += o * 2; a.g_cov += o * 2;
+    a.gates += o * 4 * a.H; a.cell_in += o * a.H; a.cell_out += o * a.H;
+    a.alpha += o * 2 * a.Lt; a.beta += o * 2; a.ctx12 += o * 2 * a.D; a.pb += o * 2 * a.D; a.hw += o * 4 * a.D;
+    a.att += o * a.Lt; a.cov_out += o * a.Lt; a.cov += o * a.Lt;
+    a.d_logits += o * a.ldd; a.d_gates += o * a.ldg; a.d_pre_b += o * 2 * a.D; a.d_ctx12 += o * 2 * a.D;
+    RollBwdArgs ro = r0;
+    ro.s = s;
+    ro.it = r0.S - 1 - s;
+    dec_bwd_body<true>(a, ro);
+  }
 }
 
 static size_t g_head_smem_set = 0;   // dynamic shared memory the kernel attribute of dec_bwd_head_kernel allows (both launchers share it)
 
-static size_t head_smem_bytes(int D, int H, int M, int CL, int chunk = 0, bool sweeps = false, int PW = NW) {
+static size_t head_smem_bytes(int D, int H, int M, int CL, int chunk = 0, bool sweeps = false, int PW = NW, bool roll = false) {
   auto up4 = [](size_t v) { return (v + 3) & ~(size_t)3; };
   const size_t per_m = (M + CL - 1) / CL;
   size_t floats = up4(per_m) + up4((size_t)MAXC * H) + up4(4 * H) + up4(D) + up4(2 * D) + MAXC * 4 + 32 + NT;
   if (sweeps)
     floats += up4(2 * D) + up4(2 * (size_t)chunk) + up4(4 * (size_t)chunk) + up4(6 * D) + up4((size_t)PW * 3 * D) + up4(chunk) + up4((size_t)CL * 6 * D) +
               up4(4 * H + 4 * D);
+  if (roll) floats += 2 * up4(H);                       // the roll-out's carried d h and d cell
   return floats * sizeof(float) + 64;
 }
 
@@ -2060,10 +2187,11 @@ static size_t stoch_floats(int K, int CL, int M) {
 // sampled roll-out (dec_sample_kernel, with `cn` dec_sample_constrained_kernel), one cluster per (video, sample); with `sp` and `nu`
 // the nucleus roll-out (dec_sample_nucleus_kernel, with `cn` dec_sample_nucleus_constrained_kernel); with `bm` and `sb` the
 // stochastic beam (dec_beam_sample_kernel, with `cn` dec_beam_sample_constrained_kernel); with `fo` (and `g` alone) the forced roll-out
-// (dec_forced_kernel), one cluster per (video, candidate).
+// (dec_forced_kernel), one cluster per (video, candidate); with `fo` and `tr` the forced roll-out that saves every step
+// (dec_forced_train_kernel).
 static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_stream_t stream, BeamArgs* bm = nullptr,
                         const ConstraintArgs* cn = nullptr, SampleArgs* sp = nullptr, NucleusArgs* nu = nullptr,
-                        StochArgs* sb = nullptr, const ForcedArgs* fo = nullptr) {
+                        StochArgs* sb = nullptr, const ForcedArgs* fo = nullptr, const TrainArgs* tr = nullptr) {
   const int B = a.B, Lt = a.Lt, D = a.D, H = a.H, E = a.E, M = a.M;
   MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && E >= 0 && M > 0, MMB_ERR_INVALID,
               "%s: B=%d Lt=%d D=%d H=%d E=%d M=%d", who, B, Lt, D, H, E, M);
@@ -2111,10 +2239,10 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
       smem = (base_floats + stage_floats) * 4;
     }
   }
-  static size_t smem_set[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  const int which = fo ? 11 : sb ? (cn ? 10 : 9) : nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
+  static size_t smem_set[13] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  const int which = tr ? 12 : fo ? 11 : sb ? (cn ? 10 : 9) : nu ? (cn ? 8 : 7) : sp ? (cn ? 6 : 5) : bm ? (cn ? 4 : 2) : g ? (cn ? 3 : 1) : 0;
   if (smem > smem_set[which]) {
-    const void* fn = which == 11 ? (const void*)dec_forced_kernel
+    const void* fn = which == 12 ? (const void*)dec_forced_train_kernel : which == 11 ? (const void*)dec_forced_kernel
                    : which == 10 ? (const void*)dec_beam_sample_constrained_kernel : which == 9 ? (const void*)dec_beam_sample_kernel
                    : which == 8 ? (const void*)dec_sample_nucleus_constrained_kernel : which == 7 ? (const void*)dec_sample_nucleus_kernel
                    : which == 6 ? (const void*)dec_sample_constrained_kernel : which == 5 ? (const void*)dec_sample_kernel
@@ -2143,6 +2271,10 @@ static int launch_fused(FusedArgs a, const GreedyArgs* g, const char* who, mmb_s
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if (tr) {
+    MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_forced_train_kernel, a, *g, *fo, *tr));
+    return check_launch("dec_forced_train_kernel");
+  }
   if (fo) {
     MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_forced_kernel, a, *g, *fo));
     return check_launch("dec_forced_kernel");
@@ -2259,6 +2391,34 @@ extern "C" int mmb_decoder_forced_fused(const float* proj_a, const float* proj_i
   const GreedyArgs g{emb_text, h0, S, 0};
   const ForcedArgs fo{tokens, p_tok, N};
   return launch_fused(a, &g, who, stream, nullptr, nullptr, nullptr, nullptr, nullptr, &fo);
+}
+
+extern "C" int mmb_decoder_forced_train_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                              const float* Wh4t, const float* bh4, const float* v1, const float* wc1, const float* v2,
+                                              const float* wc2, const float* v1b, const float* v2b, const float* Wb13t, const float* vb1,
+                                              const float* vb2, const float* vb1b, const float* vb2b, const float* Wcatt,
+                                              const float* bcat, const float* out_wt, const float* out_b, const float* emb_text,
+                                              const float* h0, const uint8_t* mask, const long long* tokens, float* probs, float* p_tok,
+                                              float* loss_terms, float* hw, float* alpha, float* beta, float* ctx12, float* pb,
+                                              float* xcat, float* gates, float* att_cov, float* cell, float* cov, float* h_last, int B,
+                                              int Lt, int D, int H, int E, int M, int S, int N, mmb_stream_t stream) {
+  using namespace mmb;
+  const char* who = "mmb_decoder_forced_train_fused";
+  MMB_REQUIRE(proj_a && proj_i && enc_a && enc_i && Wh4t && bh4 && v1 && wc1 && v2 && wc2 && v1b && v2b && Wb13t && vb1 && vb2 &&
+                  vb1b && vb2b && Wcatt && bcat && out_wt && out_b && emb_text && h0 && mask && tokens && probs && p_tok &&
+                  loss_terms && hw && alpha && beta && ctx12 && pb && xcat && gates && att_cov && cell && cov && h_last,
+              MMB_ERR_INVALID, "%s: null pointer", who);
+  MMB_REQUIRE(S > 0 && N >= 1 && N <= 64, MMB_ERR_INVALID, "%s: S=%d, N=%d (1..64)", who, S, N);
+  MMB_REQUIRE(B > 0, MMB_ERR_INVALID, "%s: B=%d", who, B);
+  // (the saved arrays take the places of the step kernel's; cell / cov are the (S + 1)-row states)
+  FusedArgs a{proj_a, proj_i, enc_a, enc_i, Wh4t, bh4, v1, wc1, v2, wc2, v1b, v2b, Wb13t, vb1, vb2, vb1b, vb2b, Wcatt, bcat, out_wt, out_b,
+              nullptr, nullptr, nullptr, nullptr, mask, nullptr, probs, nullptr, cell, att_cov, cov, nullptr,
+              loss_terms, loss_terms + (size_t)B * N, hw, alpha, beta, ctx12, pb, xcat, gates,
+              B, Lt, D, H, E, M, 0, 0};
+  const GreedyArgs g{emb_text, h0, S, 0};
+  const ForcedArgs fo{tokens, p_tok, N};
+  const TrainArgs tr{h_last};
+  return launch_fused(a, &g, who, stream, nullptr, nullptr, nullptr, nullptr, nullptr, &fo, &tr);
 }
 
 extern "C" int mmb_decoder_beam_fused(const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
@@ -2533,4 +2693,71 @@ extern "C" int mmb_decoder_step_fused_bwd(const float* probs, const float* d_pro
   cfg.numAttrs = 1;
   MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_bwd_head_kernel, a));
   return check_launch("dec_bwd_head_kernel (whole step)");
+}
+
+// The reverse forced roll-out: the whole-step backward (mmb_decoder_step_fused_bwd) for s = S - 1 .. 0 in ONE launch, one cluster per row
+// of the forced roll-out, from what mmb_decoder_forced_train_fused saved.  Cluster size, chunk and row stage follow the step kernel's
+// rules for B N rows, so each step is the step kernel's over those rows, bit for bit.
+extern "C" int mmb_decoder_forced_bwd_fused(const float* probs, const long long* tokens, const float* g_terms, const float* out_w,
+                                            const float* gates, const float* cell, const float* Wcat_ctx, const float* alpha,
+                                            const float* beta, const float* ctx12, const float* pb, const float* hw, const float* vb1,
+                                            const float* vb2, const float* att_cov, const float* cov, const float* Wb13,
+                                            const float* proj_a, const float* proj_i, const float* enc_a, const float* enc_i,
+                                            const float* v1, const float* wc1, const float* v2, const float* wc2, const float* Wh_stack,
+                                            float* d_logits, int ldd, float* d_gates, int ldg, float* d_pre_b, float* d_ctx12,
+                                            float* vec_acc, float* scal_acc, float* d_proj_a, float* d_proj_i, float* d_h0, int B,
+                                            int Lt, int D, int H, int M, int S, int N, mmb_stream_t stream) {
+  using namespace mmb;
+  const char* who = "mmb_decoder_forced_bwd_fused";
+  MMB_REQUIRE(probs && tokens && g_terms && out_w && gates && cell && Wcat_ctx && alpha && beta && ctx12 && pb && hw && vb1 && vb2 &&
+                  att_cov && cov && Wb13 && proj_a && proj_i && enc_a && enc_i && v1 && wc1 && v2 && wc2 && Wh_stack && d_logits &&
+                  d_gates && d_pre_b && d_ctx12 && vec_acc && scal_acc && d_proj_a && d_proj_i && d_h0,
+              MMB_ERR_INVALID, "%s: null pointer", who);
+  MMB_REQUIRE(S > 0 && N >= 1 && N <= 64, MMB_ERR_INVALID, "%s: S=%d, N=%d (1..64)", who, S, N);
+  MMB_REQUIRE(B > 0 && Lt > 0 && D > 0 && H > 0 && M > 0 && ldd >= M && ldg >= 4 * H + 4 * D && H <= NT, MMB_ERR_INVALID,
+              "%s: B=%d Lt=%d D=%d H=%d M=%d ldd=%d ldg=%d", who, B, Lt, D, H, M, ldd, ldg);
+  MMB_REQUIRE(D <= 256, MMB_ERR_UNSUPPORTED, "%s: D=%d > 256", who, D);
+  const int rows = B * N;
+  const int CL = (long long)rows * 4 * 2 <= 160 ? 8 : 4;
+  const int chunk = (Lt + CL - 1) / CL;
+  const size_t RB = (size_t)rows;
+  HeadArgs a{probs, nullptr, nullptr, g_terms, g_terms + RB, out_w, gates, cell, cell + RB * H, nullptr, nullptr, Wcat_ctx, nullptr,
+             nullptr, alpha, beta, ctx12, pb, hw, vb1, vb2, att_cov, cov + RB * Lt, Wb13, d_logits, d_gates, nullptr, nullptr, nullptr,
+             d_pre_b, d_ctx12, vec_acc, scal_acc, rows, Lt, D, H, M, ldd, ldg, chunk,
+             1, proj_a, proj_i, enc_a, enc_i, cov, v1, wc1, v2, wc2, d_proj_a, d_proj_i, nullptr, Wh_stack, nullptr, 0};
+  const RollBwdArgs ro{tokens, d_h0, N, S, 0, 0};
+  size_t smem = head_smem_bytes(D, H, M, CL, chunk, true, NW, true);
+  MMB_REQUIRE(smem <= 200 * 1024, MMB_ERR_UNSUPPORTED, "%s: %zu B of shared memory (Lt=%d)", who, smem, Lt);
+  {
+    // the row stage, as mmb_decoder_step_fused_bwd's (MMB_DEC_STAGE=0 turns it off)
+    static const char* stage_env = getenv("MMB_DEC_STAGE");
+    const size_t base_floats = (head_smem_bytes(D, H, M, CL, chunk, true, NW / 2, true) - 64) / 4;
+    const size_t stage_floats = 4 + 2 * (((size_t)chunk * D + 3) & ~(size_t)3);
+    const bool aligned = ((reinterpret_cast<uintptr_t>(proj_a) | reinterpret_cast<uintptr_t>(proj_i) | reinterpret_cast<uintptr_t>(enc_a) |
+                           reinterpret_cast<uintptr_t>(enc_i) | reinterpret_cast<uintptr_t>(d_proj_a) |
+                           reinterpret_cast<uintptr_t>(d_proj_i)) & 15) == 0;
+    if ((D & 3) == 0 && aligned && (base_floats + stage_floats) * 4 + 64 <= 227 * 1024 && !(stage_env && atoi(stage_env) == 0)) {
+      a.stage_off = (int)base_floats;
+      smem = (base_floats + stage_floats) * 4 + 64;
+    }
+  }
+  static size_t smem_set = 0;
+  if (smem > smem_set) {
+    MMB_CUDA(cudaFuncSetAttribute(dec_forced_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    smem_set = smem;
+  }
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3((unsigned)(rows * CL));
+  cfg.blockDim = dim3(NT);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = static_cast<cudaStream_t>(stream);
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = (unsigned)CL;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  MMB_CUDA(cudaLaunchKernelEx(&cfg, dec_forced_bwd_kernel, a, ro));
+  return check_launch("dec_forced_bwd_kernel");
 }

@@ -387,32 +387,39 @@ class _DecoderOpen(torch.autograd.Function):
 
     @staticmethod
     def _param_grads(ctx, tape, r, s):
-        B, D, H, E = s.B, s.D, s.H, s.E
+        B, D = s.B, s.D
         cat = lambda k: torch.cat(r[k], dim=0)
-        h_prev, xcat, h_out, dlog, da, dhw4 = cat("h_prev"), cat("xcat"), cat("h_out"), cat("dlog"), cat("da"), cat("dhw4")
         S = len(r["dlog"])
         kmajor = lambda k: torch.stack(r[k], dim=0).permute(1, 0, 2, 3).reshape(2, S * B, D)   # (S,2,B,D) -> (2,S*B,D)
-        dpre, ctx12 = kmajor("dpre"), kmajor("ctx12")
-        vec, scal = tape.vec_acc.sum(dim=0), tape.scal_acc.sum(dim=0)        # (6, D), (4)
-        d_wh4 = dhw4.t() @ h_prev                                            # (4D, H): W2 | W4 | W_beta_2 | W_beta_4
-        hw_sum = dhw4.sum(dim=0)
-        d_wb13 = torch.bmm(dpre.transpose(1, 2), ctx12)                      # (2, D, D): W_beta_1 | W_beta_3
-        pre_sum = dpre.sum(dim=1)
-        d_wcat = da.t() @ xcat                                               # (4H, D+E+H): W_ih | W_hh
-        gate_sum = da.sum(dim=0)
-        g = {
-            "W2": d_wh4[:D], "b2": hw_sum[:D], "Wc1": vec[0].reshape(D, 1), "bc1": hw_sum[:D],
-            "v1": vec[2].reshape(1, D), "v1b": scal[0:1],
-            "W4": d_wh4[D:2 * D], "b4": hw_sum[D:2 * D], "Wc2": vec[1].reshape(D, 1), "bc2": hw_sum[D:2 * D],
-            "v2": vec[3].reshape(1, D), "v2b": scal[1:2],
-            "Wb1": d_wb13[0], "bb1": pre_sum[0], "Wb2": d_wh4[2 * D:3 * D], "bb2": hw_sum[2 * D:3 * D],
-            "Wb3": d_wb13[1], "bb3": pre_sum[1], "Wb4": d_wh4[3 * D:], "bb4": hw_sum[3 * D:],
-            "vb1": vec[4].reshape(1, D), "vb1b": scal[2:3], "vb2": vec[5].reshape(1, D), "vb2b": scal[3:4],
-            "lstm_w_ih": d_wcat[:, :D + E], "lstm_w_hh": d_wcat[:, D + E:], "lstm_b_ih": gate_sum, "lstm_b_hh": gate_sum,
-            "out_w": dlog.t() @ h_out, "out_b": dlog.sum(dim=0),
-        }
-        from ._lib import DECODER_WEIGHT_FIELDS
-        return [g[name].reshape(shape) for name, shape in zip(DECODER_WEIGHT_FIELDS, ctx.shapes)]
+        return decoder_param_grads(ctx.shapes, s, cat("h_prev"), cat("xcat"), cat("h_out"), cat("dlog"), cat("da"), cat("dhw4"),
+                                   kmajor("dpre"), kmajor("ctx12"), tape.vec_acc, tape.scal_acc)
+
+
+def decoder_param_grads(shapes, s, h_prev, xcat, h_out, dlog, da, dhw4, dpre, ctx12, vec_acc, scal_acc):
+    """The gradients of the 30 decoder parameters (``_lib.DECODER_WEIGHT_FIELDS``, reshaped to ``shapes``) from the rows of every step
+    of a sequence: h_prev / xcat / h_out (rows, .) the steps' h, [c3 | sent | h] and h', dlog / da / dhw4 (rows, .) their d_logits,
+    d_gates and d_hw4, dpre / ctx12 (2, rows, D) d_pre_b and the contexts, vec_acc / scal_acc the kernels' per-row accumulators."""
+    D, H, E = s.D, s.H, s.E
+    vec, scal = vec_acc.sum(dim=0), scal_acc.sum(dim=0)                  # (6, D), (4)
+    d_wh4 = dhw4.t() @ h_prev                                            # (4D, H): W2 | W4 | W_beta_2 | W_beta_4
+    hw_sum = dhw4.sum(dim=0)
+    d_wb13 = torch.bmm(dpre.transpose(1, 2), ctx12)                      # (2, D, D): W_beta_1 | W_beta_3
+    pre_sum = dpre.sum(dim=1)
+    d_wcat = da.t() @ xcat                                               # (4H, D+E+H): W_ih | W_hh
+    gate_sum = da.sum(dim=0)
+    g = {
+        "W2": d_wh4[:D], "b2": hw_sum[:D], "Wc1": vec[0].reshape(D, 1), "bc1": hw_sum[:D],
+        "v1": vec[2].reshape(1, D), "v1b": scal[0:1],
+        "W4": d_wh4[D:2 * D], "b4": hw_sum[D:2 * D], "Wc2": vec[1].reshape(D, 1), "bc2": hw_sum[D:2 * D],
+        "v2": vec[3].reshape(1, D), "v2b": scal[1:2],
+        "Wb1": d_wb13[0], "bb1": pre_sum[0], "Wb2": d_wh4[2 * D:3 * D], "bb2": hw_sum[2 * D:3 * D],
+        "Wb3": d_wb13[1], "bb3": pre_sum[1], "Wb4": d_wh4[3 * D:], "bb4": hw_sum[3 * D:],
+        "vb1": vec[4].reshape(1, D), "vb1b": scal[2:3], "vb2": vec[5].reshape(1, D), "vb2b": scal[3:4],
+        "lstm_w_ih": d_wcat[:, :D + E], "lstm_w_hh": d_wcat[:, D + E:], "lstm_b_ih": gate_sum, "lstm_b_hh": gate_sum,
+        "out_w": dlog.t() @ h_out, "out_b": dlog.sum(dim=0),
+    }
+    from ._lib import DECODER_WEIGHT_FIELDS
+    return [g[name].reshape(shape) for name, shape in zip(DECODER_WEIGHT_FIELDS, shapes)]
 
 
 class _DecoderStep(torch.autograd.Function):
@@ -510,6 +517,67 @@ def decoder_open(tape, proj_a, proj_i, enc_a, enc_i, params):
 
 def decoder_step(tape, token, sent, h, cell, cov, mask_u8, target=None):
     return _DecoderStep.apply(tape, token, sent, h, cell, cov, mask_u8, target)
+
+
+def fold_step_p_grad(g_terms: Optional[torch.Tensor], g_p: Optional[torch.Tensor], p_tok: torch.Tensor) -> torch.Tensor:
+    """The loss-term gradient (S, 2, R) the forced roll-out's backward takes, with the gradient of ``p_tok`` (B, N, S) folded into the
+    nll coefficient.  p_tok reaches the kernel's backward only through nll = -log(p_tok + 1e-12), whose backward forms
+    dp_t = -g_nll / (p_tok + 1e-12): with g_nll -= g_p (p_tok + 1e-12) that is the nll's share plus exactly g_p.  Where p_tok == 0 (a
+    masked or out-of-range token) the p_tok gradient is dropped, so the result is never 0 * inf.  Device ops only (capturable)."""
+    B, N, S = p_tok.shape
+    g = p_tok.new_zeros(S, 2, B * N) if g_terms is None else g_terms.clone(memory_format=torch.contiguous_format)
+    if g_p is not None:
+        gp, pt = g_p.reshape(B * N, S).t(), p_tok.reshape(B * N, S).t()
+        g[:, 0] -= torch.where(pt != 0, gp * (pt + 1e-12), torch.zeros_like(gp))
+    return g
+
+
+class _DecoderForced(torch.autograd.Function):
+    """The teacher-forced roll-out of N candidate rows per video under autograd: ONE launch forward
+    (ops.decoder_forced_train_fwd), ONE launch backward (ops.decoder_forced_bwd), then the parameter gradients by the GEMMs of
+    the per-step path (:func:`decoder_param_grads`) over the S B N rows.  Outputs (p_tok (B,N,S), loss_terms (S,2,B N))."""
+
+    @staticmethod
+    def forward(ctx, seq, emb_text, mask_u8, tokens, proj_a, proj_i, enc_a, enc_i, h0, *params):
+        p_tok, terms, saved = ops.decoder_forced_train_fwd(seq, emb_text, h0.detach().contiguous(), mask_u8, tokens)
+        ctx.seq = seq
+        ctx.shapes = [p.shape for p in params]
+        ctx.save_for_backward(tokens, p_tok, *saved)
+        return p_tok, terms
+
+    @staticmethod
+    def backward(ctx, g_p, g_terms):
+        # the saved rows are handed out below (d_proj accumulates in place): a second backward would double-count -- refuse it
+        if getattr(ctx, "consumed", False):
+            raise RuntimeError("mmbidaf_b200: the forced roll-out's backward ran twice over one forward (retain_graph=True is not "
+                               "supported)")
+        ctx.consumed = True
+        seq = ctx.seq
+        tokens, p_tok, *saved = ctx.saved_tensors
+        B, N, S = tokens.shape
+        R, Lt, D, H, E, M = B * N, seq.Lt, seq.D, seq.H, seq.E, seq.M
+        g = fold_step_p_grad(g_terms, g_p, p_tok)
+        d_proj_a, d_proj_i = torch.zeros_like(seq.proj_a), torch.zeros_like(seq.proj_i)
+        vec_acc, scal_acc = seq.enc_a.new_zeros(R, 6, D), seq.enc_a.new_zeros(R, 4)
+        d_logits, d_gates, d_hw4, d_ctx12, d_pre_b, d_h0 = ops.decoder_forced_bwd(seq, saved, tokens, g, d_proj_a, d_proj_i,
+                                                                                  vec_acc, scal_acc)
+        _, _, alpha, _, ctx12, _, xcat, _, _, _, _, h_last = saved
+        # d enc_k[b] = sum over (s, n) of alpha_k^T d_ctx12_k: one bmm per modality with K = S N
+        d_enc = [torch.bmm(alpha[:, :, k].reshape(S, B, N, Lt).permute(1, 3, 0, 2).reshape(B, Lt, S * N),
+                           d_ctx12[:, k].reshape(S, B, N, D).permute(1, 0, 2, 3).reshape(B, S * N, D)) for k in (0, 1)]
+        h_in = xcat[:, :, D + E:]                                              # each step's h; step s + 1's is step s's h'
+        h_out = torch.cat([h_in[1:], h_last.unsqueeze(0)])
+        kmajor = lambda t: t.permute(1, 0, 2, 3).reshape(2, S * R, D)        # (S,2,R,D) -> (2,S*R,D)
+        grads = decoder_param_grads(ctx.shapes, seq, h_in.reshape(S * R, H), xcat.reshape(S * R, -1), h_out.reshape(S * R, H),
+                                    d_logits.reshape(S * R, M), d_gates.reshape(S * R, 4 * H), d_hw4.reshape(S * R, 4 * D),
+                                    kmajor(d_pre_b), kmajor(ctx12), vec_acc, scal_acc)
+        return (None, None, None, None, d_proj_a, d_proj_i, d_enc[0], d_enc[1], d_h0.view(B, N, H).sum(1), *grads)
+
+
+def decoder_forced(seq, emb_text, mask_u8, tokens, proj_a, proj_i, enc_a, enc_i, h0, params):
+    """(p_tok (B,N,S), loss_terms (S,2,B N)) of the forced roll-out of ``tokens`` (B,N,S), differentiable in proj_a / proj_i / enc_a /
+    enc_i (B,Lt,D), h0 (B,H) and the 30 decoder ``params`` (``_lib.DECODER_WEIGHT_FIELDS`` order)."""
+    return _DecoderForced.apply(seq, emb_text, mask_u8, tokens, proj_a, proj_i, enc_a, enc_i, h0, *params)
 
 
 class _HighwayLayer(torch.autograd.Function):

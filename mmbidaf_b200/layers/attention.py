@@ -269,6 +269,23 @@ class MultimodalAttentionDecoder(nn.Module):
             return ops.decoder_forced_fwd(seq, emb_text.contiguous(), h0.reshape(B, -1).contiguous(), ops._u8(mask),
                                           tokens.contiguous(), want_probs)
 
+    def force_train(self, emb_text, h0, enc_a, enc_i, mask, tokens):
+        """:meth:`force` under autograd: (p_tok (B,N,S), loss_terms (S,2,B N)) with gradients into ``enc_a`` / ``enc_i`` (also through
+        the hoisted W1 / W3 projections), ``h0`` and every decoder parameter -- one launch forward, one launch backward (the rules at
+        mmb_decoder_forced_train_fused / mmb_decoder_forced_bwd_fused in include/mmbidaf_b200.h), whatever ``ops.decoder_cut`` says.
+        No gradient reaches ``emb_text``.  The sequence is its own: the per-step tape of :meth:`step` is not used."""
+        if not enc_a.is_cuda:
+            raise RuntimeError("mmbidaf_b200.layers.MultimodalAttentionDecoder runs on a B200 only (no CPU fallback)")
+        if self.num_layers != 1:
+            raise RuntimeError("MultimodalAttentionDecoder: only num_layers=1 is supported (the reference model uses 1)")
+        proj_a = self._hoisted_or_new("a", enc_a, self.W1)
+        proj_i = self._hoisted_or_new("i", enc_i, self.W3)
+        params = {name: self._param_of(name) for name in _lib_fields()}
+        prepared, self._prepared = self._prepared, None
+        seq = ops.DecoderSeq(params, enc_a, enc_i, proj_a, proj_i, self.output_size, weights=prepared)
+        return Fn.decoder_forced(seq, emb_text.detach().contiguous(), ops._u8(mask), tokens.contiguous(), proj_a, proj_i, enc_a, enc_i,
+                                 h0.reshape(seq.B, -1), list(params.values()))
+
     def beam(self, emb_text, h0, enc_a, enc_i, mask, text_len, steps, width, no_repeat=False, min_sentences=0):
         """The beam decode of ``steps`` steps in eval mode with ``width`` (1..8) hypotheses per video, as ONE launch of the cluster
         kernel whatever ``ops.decoder_cut`` says (there is no chunk-cut beam); the rule is documented at mmb_decoder_beam_fused in

@@ -247,22 +247,10 @@ class MMBiDAF(nn.Module):
         ``logp`` by the rule of ``Samples.logp``, ``loss`` the teacher-forced loss of each row (the training loss of ``forward`` per
         video), -inf / +inf on invalid rows."""
         from .layers.encoding import length_plan
-        from .ops import FORCED_MAX_N
-        from .summarize import candidate_tokens, forced_scores
+        from .summarize import forced_scores
         if not isinstance(probs, bool):
             raise ValueError(f"score: probs {probs!r}, expected a bool")
-        B, S = text.size(0), int(max_dec_len)
-        if torch.is_tensor(candidates):
-            if candidates.dtype != torch.int64 or candidates.dim() != 3 or candidates.shape[0] != B or \
-                    not 1 <= candidates.shape[1] <= FORCED_MAX_N or candidates.shape[2] != S or candidates.device != text.device:
-                raise ValueError(f"score: candidates {candidates.dtype} {tuple(candidates.shape)} on {candidates.device}, expected "
-                                 f"(B={B}, N in 1..{FORCED_MAX_N}, max_dec_len={S}) int64 on {text.device}")
-            tokens, valid = candidates, None
-        else:
-            tokens, valid = candidate_tokens(candidates, text_len, S)
-            if tokens.shape[0] != B:
-                raise ValueError(f"score: candidates for {tokens.shape[0]} videos, the batch holds {B}")
-            tokens, valid = tokens.to(text.device), valid.to(text.device)
+        tokens, valid = self._candidate_rows("score", text, text_len, max_dec_len, candidates)
         was_training = self.training
         self.eval()
         try:
@@ -275,6 +263,51 @@ class MMBiDAF(nn.Module):
                 return forced_scores(tokens, p_tok, terms, valid, length_plan(text_len, text.device).len_i32, rows)
         finally:
             self.train(was_training)
+
+    def sequence_scores(self, text, text_len, audio, audio_len, images, image_len, max_dec_len, candidates):
+        """:meth:`score` for training: the same ``Scores`` (``tokens, step_p, logp, loss, valid``; no ``probs``), but in the caller's
+        mode and grad mode, as ``forward`` runs -- in training mode the encoders' dropout applies -- and differentiable: ``logp``,
+        ``loss`` and ``step_p`` carry gradients to every parameter of the model, so sequence-level objectives (self-critical or
+        REINFORCE with sampled candidates, minimum risk, the estimator of a stochastic beam) train it.  With grad enabled the decoder
+        runs one forced roll-out that saves every step and one reverse roll-out for the backward
+        (``MultimodalAttentionDecoder.force_train``: two launches whatever ``max_dec_len`` is); without, the roll-out of :meth:`score`.
+        ``candidates`` as for :meth:`score`: a device tensor (B, N, max_dec_len) int64 with N in 1..64 (capturable), or host lists
+        through ``summarize.candidate_tokens``; invalid padding rows get zero gradient.  ValueError, before any device work, for bad
+        candidates, and for ``text.requires_grad``: the decoder's next inputs are rows of ``text``, and their gradient is not formed."""
+        from .layers.encoding import length_plan
+        from .summarize import forced_scores
+        if torch.is_tensor(text) and text.requires_grad:
+            raise ValueError("sequence_scores: text requires grad; the decoder's next-input rows are gathered from it and their gradient "
+                             "is not formed (pass text.detach())")
+        tokens, valid = self._candidate_rows("sequence_scores", text, text_len, max_dec_len, candidates)
+        if not text.is_cuda:
+            raise RuntimeError("mmbidaf_b200 MMBiDAF.sequence_scores runs on a B200 only (no CPU fallback)")
+        dec = self.multimodal_att_decoder
+        enc_a, enc_i, h0, mask = self._encode(text, text_len, audio, audio_len, images, image_len, dec.prepare)
+        if torch.is_grad_enabled():
+            p_tok, terms = dec.force_train(text, h0, enc_a, enc_i, mask, tokens)
+        else:
+            _, p_tok, terms = dec.force(text, h0, enc_a, enc_i, mask, tokens)
+        if valid is None:
+            valid = torch.ones(tokens.shape[:2], dtype=torch.bool, device=text.device)
+        return forced_scores(tokens, p_tok, terms, valid, length_plan(text_len, text.device).len_i32)
+
+    def _candidate_rows(self, who, text, text_len, max_dec_len, candidates):
+        """The candidate token rows of :meth:`score` / :meth:`sequence_scores` and their validity (None: every row valid), checked
+        before any device work."""
+        from .ops import FORCED_MAX_N
+        from .summarize import candidate_tokens
+        B, S = text.size(0), int(max_dec_len)
+        if torch.is_tensor(candidates):
+            if candidates.dtype != torch.int64 or candidates.dim() != 3 or candidates.shape[0] != B or \
+                    not 1 <= candidates.shape[1] <= FORCED_MAX_N or candidates.shape[2] != S or candidates.device != text.device:
+                raise ValueError(f"{who}: candidates {candidates.dtype} {tuple(candidates.shape)} on {candidates.device}, expected "
+                                 f"(B={B}, N in 1..{FORCED_MAX_N}, max_dec_len={S}) int64 on {text.device}")
+            return candidates, None
+        tokens, valid = candidate_tokens(candidates, text_len, S)
+        if tokens.shape[0] != B:
+            raise ValueError(f"{who}: candidates for {tokens.shape[0]} videos, the batch holds {B}")
+        return tokens.to(text.device), valid.to(text.device)
 
     def _encode(self, embedded_text, original_text_lengths, embedded_audio, original_audio_lengths, transformed_images,
                 original_image_lengths, decoder_start):

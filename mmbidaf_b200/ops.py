@@ -415,6 +415,72 @@ def decoder_forced_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, tokens, want_prob
     return probs, p_tok, terms
 
 
+def decoder_forced_train_fwd(seq: DecoderSeq, emb_text, h0, mask_u8, tokens):
+    """The forced roll-out of :func:`decoder_forced_fwd` for training (mmb_decoder_forced_train_fused): ONE launch whatever
+    ``decoder_cut`` says, the same p_tok and loss terms bit for bit, and every step's saved arrays for :func:`decoder_forced_bwd`.
+    Returns (p_tok (B,N,S), loss_terms (S,2,B N), saved) with ``saved`` = (probs (S,R,M), hw (S,R,4D), alpha (S,R,2,Lt), beta (S,R,2),
+    ctx12 (S,2,R,D), pb (S,2,R,D), xcat (S,R,D+E+H), gates (S,R,4H), att_cov (S,R,Lt), cell (S+1,R,H), cov (S+1,R,Lt), h_last (R,H)),
+    R = B N rows r = b N + n."""
+    lib = _lib.lib()
+    B, Lt, D, H, E, M = seq.B, seq.Lt, seq.D, seq.H, seq.E, seq.M
+    dev = h0.device
+    if emb_text.shape != (B, Lt, E) or h0.shape != (B, H) or mask_u8.shape != (B, M):
+        raise ValueError(f"decoder_forced_train_fwd: emb_text {tuple(emb_text.shape)}, h0 {tuple(h0.shape)}, mask "
+                         f"{tuple(mask_u8.shape)} for B={B} Lt={Lt} E={E} H={H} M={M}")
+    if tokens.dtype != torch.int64 or tokens.dim() != 3 or tokens.shape[0] != B or tokens.device != dev or \
+            not 1 <= tokens.shape[1] <= FORCED_MAX_N or tokens.shape[2] <= 0:
+        raise ValueError(f"decoder_forced_train_fwd: tokens {tokens.dtype} {tuple(tokens.shape)} on {tokens.device}, expected "
+                         f"(B={B}, N in 1..{FORCED_MAX_N}, S > 0) int64 on {dev}")
+    N, S = int(tokens.shape[1]), int(tokens.shape[2])
+    R = B * N
+    f32 = dict(device=dev, dtype=torch.float32)
+    p_tok = torch.empty(B, N, S, **f32)
+    terms = torch.empty(S, 2, R, **f32)
+    saved = (torch.empty(S, R, M, **f32), torch.empty(S, R, 4 * D, **f32), torch.empty(S, R, 2, Lt, **f32), torch.empty(S, R, 2, **f32),
+             torch.empty(S, 2, R, D, **f32), torch.empty(S, 2, R, D, **f32), torch.empty(S, R, D + E + H, **f32),
+             torch.empty(S, R, 4 * H, **f32), torch.empty(S, R, Lt, **f32), torch.empty(S + 1, R, H, **f32),
+             torch.empty(S + 1, R, Lt, **f32), torch.empty(R, H, **f32))
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_forced_train_fused(
+        p(seq.proj_a), p(seq.proj_i), p(seq.enc_a), p(seq.enc_i), p(seq.Wh4t), p(seq.bh4), p(seq.v1), p(seq.wc1), p(seq.v2),
+        p(seq.wc2), p(seq.v1b), p(seq.v2b), p(seq.Wb13t), p(seq.vb1), p(seq.vb2), p(seq.vb1b), p(seq.vb2b), p(seq.Wcatt),
+        p(seq.bcat), p(seq.out_wt), p(seq.out_b), p(emb_text), p(h0), p(mask_u8), p(tokens.contiguous()), p(saved[0]), p(p_tok),
+        p(terms), *(p(t) for t in saved[1:]), B, Lt, D, H, E, M, S, N, _lib.stream()), "mmb_decoder_forced_train_fused")
+    _count(1)
+    return p_tok, terms, saved
+
+
+def decoder_forced_bwd(seq: DecoderSeq, saved, tokens, g_terms, d_proj_a, d_proj_i, vec_acc, scal_acc):
+    """The backward of :func:`decoder_forced_train_fwd` (mmb_decoder_forced_bwd_fused): every step's whole-step backward, s = S-1 .. 0,
+    as ONE launch whatever ``decoder_cut`` says.  ``g_terms`` (S,2,R) fp32 = d objective / d loss_terms (entry [s, 0, r] the nll term's,
+    [s, 1, r] the coverage term's; a token outside 0..M-1 contributes nothing through its nll).  ``d_proj_*`` (B,Lt,D), ``vec_acc``
+    (R,6,D), ``scal_acc`` (R,4) are accumulated in place.  Returns (d_logits (S,R,M), d_gates (S,R,4H), d_hw4 (S,R,4D), d_ctx12
+    (S,2,R,D), d_pre_b (S,2,R,D), d_h0 (R,H))."""
+    lib = _lib.lib()
+    B, Lt, D, H, M = seq.B, seq.Lt, seq.D, seq.H, seq.M
+    probs, hw, alpha, beta, ctx12, pb, xcat, gates, att_cov, cell, cov, _ = saved
+    S, R = probs.shape[0], probs.shape[1]
+    N = R // B
+    dev = probs.device
+    if tokens.shape != (B, N, S) or g_terms.shape != (S, 2, R) or g_terms.dtype != torch.float32:
+        raise ValueError(f"decoder_forced_bwd: tokens {tuple(tokens.shape)}, g_terms {g_terms.dtype} {tuple(g_terms.shape)} for "
+                         f"B={B} N={N} S={S}")
+    f32 = dict(device=dev, dtype=torch.float32)
+    d_logits = torch.empty(S, R, seq.Mp, **f32)                                # zero-padded columns, as the step's
+    gbuf = torch.empty(S, R, 4 * H + 4 * D, **f32)                             # [d_gates | d_hw4] side by side
+    d_ctx12, d_pre_b = torch.empty(S, 2, R, D, **f32), torch.empty(S, 2, R, D, **f32)
+    d_h0 = torch.empty(R, H, **f32)
+    p = _lib.ptr
+    _lib.check(lib.mmb_decoder_forced_bwd_fused(
+        p(probs), p(tokens.contiguous()), p(g_terms.contiguous()), p(seq.out_w), p(gates), p(cell), p(seq.Wcat_ctx), p(alpha),
+        p(beta), p(ctx12), p(pb), p(hw), p(seq.vb1), p(seq.vb2), p(att_cov), p(cov), p(seq.Wb13), p(seq.proj_a), p(seq.proj_i),
+        p(seq.enc_a), p(seq.enc_i), p(seq.v1), p(seq.wc1), p(seq.v2), p(seq.wc2), p(seq.Wh_stack), p(d_logits), seq.Mp, p(gbuf),
+        4 * H + 4 * D, p(d_pre_b), p(d_ctx12), p(vec_acc), p(scal_acc), p(d_proj_a), p(d_proj_i), p(d_h0), B, Lt, D, H, M, S, N,
+        _lib.stream()), "mmb_decoder_forced_bwd_fused")
+    _count(1)
+    return d_logits[..., :M], gbuf[..., :4 * H], gbuf[..., 4 * H:], d_ctx12, d_pre_b, d_h0
+
+
 def _check_constraints(who: str, no_repeat, min_sentences) -> None:
     if not isinstance(no_repeat, int) or no_repeat not in (0, 1):
         raise ValueError(f"{who}: no_repeat {no_repeat!r}, expected a bool")
